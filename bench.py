@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- batched MPC step solves/s on B200 (BASELINE.json metric) and the CPU reference arm.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (nearest index -> reference sampling -> rollout -> linearise/condense ->
@@ -19,6 +19,9 @@ step kernel's own epilogue (NVLink peer stores into every rank's table) and made
 
 Timed region: CUDA events on the launching stream around each step, L2 flushed (256 MiB write) and the in-place
 warm-start buffers restored before every step outside the events; sum over K steps, max over ranks.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what its last timed step returned (last_step_outputs) as
+DIR/<name>.npy.  The inputs are seeded, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import json
@@ -152,6 +155,39 @@ def host_slices(args, rank, world):
     return out
 
 
+DUMP_BYTES = 60 << 20          # array data of --dump-outputs; the .npy headers fit in the rest of 64 MB
+
+
+def last_step_outputs(devs, has_obs):
+    """name -> float64 host array: what the timed step hands its caller (controls and target index updated in place,
+    predicted states, reference, cost, status, solver iterations, result records; with obstacles the flags and the
+    cut course lengths), instance-major.  Several horizon slices (config 5) are prefixed `T<T>_`.  When the whole
+    batch would exceed DUMP_BYTES, every array of a slice holds the same seeded sample of instances, sorted, whose
+    indices are `rows`."""
+    import torch
+    slices = []
+    for d in devs:
+        a = {"oa": d.oa, "od": d.od, "target_ind": d.tgt, "ox": d.out.ox, "oy": d.out.oy, "ov": d.out.ov,
+             "oyaw": d.out.oyaw, "xref": d.out.xref, "cost": d.out.cost, "status": d.out.status, "iters": d.out.iters,
+             "record": d.out.record}
+        if has_obs:
+            a["flag"], a["course_len"] = d.flag, d.clen
+        slices.append(a)
+    total = sum(8 * (sum(t.numel() for t in a.values()) + d.B) for d, a in zip(devs, slices))   # + d.B: `rows`
+    frac = min(1.0, DUMP_BYTES / total)
+    out = {}
+    for d, a in zip(devs, slices):
+        prefix = f"T{d.T}_" if len(devs) > 1 else ""
+        rows = None
+        if frac < 1.0:
+            rows = np.sort(np.random.default_rng(0).choice(d.B, int(d.B * frac), replace=False))
+            out[prefix + "rows"] = rows.astype(np.float64)
+            rows = torch.as_tensor(rows, device=d.oa.device)
+        for name, t in a.items():
+            out[prefix + name] = (t if rows is None else t.index_select(0, rows)).to(torch.float64).cpu().numpy()
+    return out
+
+
 def cpu_solver():
     """Which CPU implementation the CPU legs time: the reference's own solver stack when it imports here
     (cvxpy + ECOS through the reference's formulation, oracle/reference_solver.py), else the oracle port."""
@@ -261,7 +297,14 @@ def main():
                          "waiting for its own table (flags) or for the previous step's (deferred: ranks run uncoupled, "
                          "the last step pays the skew); or one NCCL all-gather per step")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs as DIR/<name>.npy (float64, at most 64 MB: a seeded "
+                         "sample of instances when the batch is larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -429,6 +472,8 @@ def main():
     clocks = sampler.finish()
     gc.enable()
     launches = mpc.launch_count - launches0
+    # taken now: the passes below overwrite the output buffers
+    dump = last_step_outputs(devs, has_obs) if args.dump_outputs and rank == 0 else None
     # per step: [flag kernel] + step launches + gather.  The metric counts MPC step solves: flag production is timed
     # separately (SURVEY.md 8d: "solves/s must not be diluted or inflated by it").
     coll_ms = np.array([e0.elapsed_time(ec) for e0, e1, ec, _ in evs]) if has_obs else np.zeros(args.steps)
@@ -652,6 +697,10 @@ def main():
                                 "sample": f"{per_slice} solved instances strided over each slice of the same batch "
                                           f"({len(jobs)} solves), one solve per call, {cores} processes, {dt:.1f} s wall",
                                 "reference_solver_probe": pr}
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

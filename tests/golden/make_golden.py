@@ -607,10 +607,27 @@ def record_planner(max_seconds=20):
     return out
 
 
+def savez_planner(path, arrays):
+    """np.savez_compressed with every trajectory that equals an earlier variant's stored once, which keeps
+    planner.npz under 1 MB: the rows (name, stored name) of `aliases` restore it (tests/helpers.py
+    load_planner_golden)."""
+    arrays, stored, aliases = dict(arrays), {}, []
+    for name in list(arrays):
+        if name.endswith("/trajectory"):
+            a = np.asarray(arrays[name])
+            key = (a.dtype.str, a.shape, a.tobytes())
+            if key in stored:
+                aliases.append((name, stored[key]))
+                del arrays[name]
+            else:
+                stored[key] = name
+    np.savez_compressed(path, aliases=np.array(aliases, dtype=str).reshape(-1, 2), **arrays)
+
+
 def main():
     install_shims()
     if "--planner" in sys.argv:
-        np.savez_compressed(os.path.join(HERE, "planner.npz"), **record_planner())
+        savez_planner(os.path.join(HERE, "planner.npz"), record_planner())
         return
     if "--obstacles" in sys.argv:
         np.savez_compressed(os.path.join(HERE, "scripted_obstacles.npz"), **record_scripted_obstacles())

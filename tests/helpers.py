@@ -30,6 +30,16 @@ def params_from_vector(v, T, max_iter=1):
         max_iter=max_iter)
 
 
+def load_planner_golden(golden_dir):
+    """tests/golden/planner.npz as a dict.  A trajectory equal to an earlier variant's is stored once; the rows
+    (name, stored name) of `aliases` give it back under every name it was recorded under."""
+    with np.load(os.path.join(golden_dir, "planner.npz")) as z:
+        d = {k: z[k] for k in z.files}
+    for name, stored in d.pop("aliases"):
+        d[str(name)] = d[str(stored)]
+    return d
+
+
 def default_vector(w, cfg=None):
     cfg = cfg or MPCConfig.default()
     return cfg.with_T(w["T"]).param_vector(dl=w["dl"])

@@ -4,11 +4,12 @@ reference's own MotionPrimitiveSearch / AStar (tests/golden/planner.npz).
 Exact: status, number of expansions, the primitive of every edge (i.e. the node path as a sequence of decisions).
 Node coordinates, expansion log and trajectory: 1e-9 (sin / cos come from CUDA's libm, numpy's from the host's);
 cost: 1e-12 relative."""
-import os
 import types
 
 import numpy as np
 import pytest
+
+from helpers import load_planner_golden
 
 pytestmark = pytest.mark.gpu
 
@@ -18,7 +19,7 @@ def fx(golden_dir):
     import __graft_entry__ as g
     g.build()
     from junction_mpc import planner as P
-    z = np.load(os.path.join(golden_dir, "planner.npz"))
+    z = load_planner_golden(golden_dir)
     return z, P
 
 

@@ -47,8 +47,9 @@ def test_gpu_matches_ecos_on_frozen_inputs(golden_dir):
         if e > 1.0:
             loose += 1
             assert out.cost[k] <= ref.cost + 1e-9 * abs(ref.cost), (k, e)
-    os.makedirs(os.path.join(os.path.dirname(golden_dir), "..", "profiles"), exist_ok=True)
-    with open(os.path.join(os.path.dirname(golden_dir), "..", "profiles", "r2_reference_solver_parity.json"), "w") as f:
-        json.dump({"probe": r, "instances": 96, "worst_scaled_error": worst, "outside_gate_but_better_objective": loose,
-                   "gate": {"abs": ABS_TOL, "rel": REL_TOL}}, f, indent=1)
+    report_dir = os.environ.get("JMPC_REPORT_DIR")          # summary only on request: the source tree is never written
+    if report_dir:
+        with open(os.path.join(report_dir, "r2_reference_solver_parity.json"), "w") as f:
+            json.dump({"probe": r, "instances": 96, "worst_scaled_error": worst, "outside_gate_but_better_objective": loose,
+                       "gate": {"abs": ABS_TOL, "rel": REL_TOL}}, f, indent=1)
     assert loose <= 96 // 10

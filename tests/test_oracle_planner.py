@@ -1,16 +1,15 @@
 """The planner restatement (oracle/planner_oracle.py) against searches recorded from the reference's own
 MotionPrimitiveSearch / AStar (tests/golden/planner.npz, made by tests/golden/make_golden.py --planner)."""
-import os
-
 import numpy as np
 import pytest
 
+from helpers import load_planner_golden
 from oracle import planner_oracle as PO
 
 
 @pytest.fixture(scope="module")
 def fx(golden_dir):
-    z = np.load(os.path.join(golden_dir, "planner.npz"))
+    z = load_planner_golden(golden_dir)
     planner = PO.Planner(z["mp_points"], z["mp_total_length"], float(z["car_radius"]), z["car_circle_centers"])
     return z, planner
 
