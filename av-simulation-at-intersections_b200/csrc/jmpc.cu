@@ -14,6 +14,7 @@
 #include "jmpc_step.cuh"
 #include "jmpc_episode.cuh"
 #include "jmpc_planner.cuh"
+#include "jmpc_courses.cuh"
 
 namespace {
 
@@ -254,12 +255,12 @@ int refresh_circle_tables(jmpc_handle h) {
 }
 
 // Arc-length tables of the uploaded courses (jmpc_collision.cuh: arc_table_kernel), N (N + 1) / 2 doubles per course;
-// courses are left without a table (the kernel then sums on the fly) once 256 MB are used.
-int refresh_arc_tables(jmpc_handle h) {
-  CK(cudaSetDevice(h->device));
+// courses are left without a table (the kernel then sums on the fly) once 256 MB are used.  Frees the old tables,
+// places the courses of h->course_n and allocates the new block; off[c] = -1 for a course without a table.
+int place_arc_tables(jmpc_handle h, std::vector<long long>& off) {
   if (h->d_arc) { cudaFree(h->d_arc); h->d_arc = nullptr; }
   if (!h->d_arc_off) CK(cudaMalloc(&h->d_arc_off, (size_t)h->max_courses * sizeof(long long)));
-  std::vector<long long> off(h->n_courses, -1);
+  off.assign(h->n_courses, -1);
   long long total = 0;
   h->arc_all = true;
   const long long cap = (256ll << 20) / (long long)sizeof(double);
@@ -269,6 +270,13 @@ int refresh_arc_tables(jmpc_handle h) {
     off[c] = total; total += need;
   }
   if (total > 0) CK(cudaMalloc(&h->d_arc, (size_t)total * sizeof(double)));
+  return 0;
+}
+
+int refresh_arc_tables(jmpc_handle h) {
+  CK(cudaSetDevice(h->device));
+  std::vector<long long> off;
+  if (place_arc_tables(h, off)) return -1;
   for (int c = 0; c < h->n_courses; ++c) {
     if (off[c] < 0) continue;
     const size_t coff = (size_t)c * h->course_stride;
@@ -1078,7 +1086,7 @@ int32_t jmpc_plan_host(int32_t device, int32_t B, int32_t n_mp, int32_t n_pts, i
   CK(cudaSetDevice(device));
   jmpc::PlanArgs a;
   memset(&a, 0, sizeof a);
-  a.B = B; a.n_mp = n_mp; a.n_pts = n_pts; a.n_cc = n_cc; a.max_obs = max_obs;
+  a.B = B; a.n_mp = n_mp; a.n_pts = n_pts; a.n_cc = n_cc; a.max_obs = max_obs; a.n_scenes = n_scenes;
   a.max_expansions = max_expansions; a.max_path = max_path; a.max_traj = (max_path - 1) * (n_pts - 1); a.max_log = max_log;
   a.pool_cap = max_expansions * n_mp + 1;
   int ts = 64;
@@ -1147,6 +1155,229 @@ int32_t jmpc_plan_host(int32_t device, int32_t B, int32_t n_mp, int32_t n_pts, i
   if (st) cudaStreamDestroy(st);
   cudaFree(d);
   return rc;
+}
+
+}  // extern "C"
+
+struct jmpc_planner_s {
+  int device = 0, max_B = 0, n_mp = 0, n_pts = 0, n_cc = 0;
+  int max_expansions = 0, max_path = 0, max_log = 0, pool_cap = 0, table_size = 0;
+  double *d_pts = nullptr, *d_len = nullptr, *d_cc = nullptr;                    // primitives
+  double* d_hp = nullptr; int* d_hp_n = nullptr; int* d_n_obs = nullptr;           // scenes
+  size_t hp_bytes = 0, hpn_bytes = 0, nobs_bytes = 0;
+  int n_scenes = 0, max_obs = 0;
+  jmpc::PlanNode* d_pool = nullptr; int* d_heap = nullptr; int* d_table = nullptr; // per-search workspace
+};
+
+namespace {
+// (re)allocate *p to hold `bytes` when it is smaller
+template <typename T>
+int grow(T** p, size_t* have, size_t bytes) {
+  if (bytes <= *have) return 0;
+  if (*p) cudaFree(*p);
+  *p = nullptr; *have = 0;
+  CK(cudaMalloc(p, bytes));
+  *have = bytes;
+  return 0;
+}
+}  // namespace
+
+extern "C" {
+
+int32_t jmpc_planner_create(int32_t device, int32_t max_B, int32_t n_mp, int32_t n_pts, int32_t n_cc, const double* mp_pts,
+                            const double* mp_len, const double* mp_cc, int32_t max_expansions, int32_t max_path,
+                            int32_t max_log, jmpc_planner* out) {
+  if (!out) return fail("jmpc_planner_create: out is NULL");
+  *out = nullptr;
+  if (!mp_pts || !mp_len || !mp_cc) return fail("jmpc_planner_create: NULL argument");
+  if (max_B < 1 || n_mp < 1 || n_mp > 32 || n_pts < 2 || n_cc < 1)
+    return fail("jmpc_planner_create: size out of range (max_B >= 1, 1 <= n_mp <= 32)");
+  if (max_expansions < 1 || max_path < 2 || max_log < 0) return fail("jmpc_planner_create: limits out of range");
+  int count = 0;
+  CK(cudaGetDeviceCount(&count));
+  if (device < 0 || device >= count) return fail("jmpc_planner_create: no such CUDA device");
+  CK(cudaSetDevice(device));
+  jmpc_planner p = new (std::nothrow) jmpc_planner_s();
+  if (!p) return fail("jmpc_planner_create: out of host memory");
+  p->device = device; p->max_B = max_B; p->n_mp = n_mp; p->n_pts = n_pts; p->n_cc = n_cc;
+  p->max_expansions = max_expansions; p->max_path = max_path; p->max_log = max_log;
+  p->pool_cap = max_expansions * n_mp + 1;                  // as jmpc_plan_host sizes them
+  int ts = 64;
+  while (ts < 2 * max_expansions + 2) ts <<= 1;
+  p->table_size = ts;
+  const size_t b = (size_t)max_B, pts = (size_t)n_mp * n_pts * 3, cc = (size_t)n_mp * n_cc * 2;
+  cudaError_t e;
+  if ((e = cudaMalloc(&p->d_pts, pts * 8)) != cudaSuccess || (e = cudaMalloc(&p->d_len, (size_t)n_mp * 8)) != cudaSuccess ||
+      (e = cudaMalloc(&p->d_cc, cc * 8)) != cudaSuccess ||
+      (e = cudaMalloc(&p->d_pool, b * p->pool_cap * sizeof(jmpc::PlanNode))) != cudaSuccess ||
+      (e = cudaMalloc(&p->d_heap, b * p->pool_cap * sizeof(int))) != cudaSuccess ||
+      (e = cudaMalloc(&p->d_table, b * ts * sizeof(int))) != cudaSuccess ||
+      (e = cudaMemcpy(p->d_pts, mp_pts, pts * 8, cudaMemcpyHostToDevice)) != cudaSuccess ||
+      (e = cudaMemcpy(p->d_len, mp_len, (size_t)n_mp * 8, cudaMemcpyHostToDevice)) != cudaSuccess ||
+      (e = cudaMemcpy(p->d_cc, mp_cc, cc * 8, cudaMemcpyHostToDevice)) != cudaSuccess) {
+    jmpc_planner_destroy(p);
+    return fail("jmpc_planner_create: workspace allocation failed (lower max_B or max_expansions)", e);
+  }
+  *out = p;
+  return 0;
+}
+
+int32_t jmpc_planner_destroy(jmpc_planner p) {
+  if (!p) return 0;
+  cudaSetDevice(p->device);
+  cudaFree(p->d_pts); cudaFree(p->d_len); cudaFree(p->d_cc); cudaFree(p->d_hp); cudaFree(p->d_hp_n); cudaFree(p->d_n_obs);
+  cudaFree(p->d_pool); cudaFree(p->d_heap); cudaFree(p->d_table);
+  delete p;
+  return 0;
+}
+
+int32_t jmpc_planner_set_scenes(jmpc_planner p, int32_t n_scenes, int32_t max_obs, const double* hp, const int32_t* hp_n,
+                                const int32_t* n_obs) {
+  if (!p || !hp || !hp_n || !n_obs) return fail("jmpc_planner_set_scenes: NULL argument");
+  if (n_scenes < 1 || max_obs < 0) return fail("jmpc_planner_set_scenes: size out of range");
+  for (int s = 0; s < n_scenes; ++s) {
+    if (n_obs[s] < 0 || n_obs[s] > max_obs) return fail("jmpc_planner_set_scenes: n_obs out of range");
+    for (int o = 0; o < n_obs[s]; ++o)
+      if (hp_n[(size_t)s * max_obs + o] < 1 || hp_n[(size_t)s * max_obs + o] > JMPC_PLAN_MAX_HP)
+        return fail("jmpc_planner_set_scenes: hp_n out of range");
+  }
+  CK(cudaSetDevice(p->device));
+  CK(cudaDeviceSynchronize());                             // searches in flight may still read the old scenes
+  const size_t hpd = (size_t)n_scenes * max_obs * JMPC_PLAN_MAX_HP * 3, hpn = (size_t)n_scenes * max_obs;
+  if (grow(&p->d_hp, &p->hp_bytes, std::max<size_t>(hpd, 1) * 8) || grow(&p->d_hp_n, &p->hpn_bytes, std::max<size_t>(hpn, 1) * 4) ||
+      grow(&p->d_n_obs, &p->nobs_bytes, (size_t)n_scenes * 4))
+    return -1;
+  if (hpd) CK(cudaMemcpy(p->d_hp, hp, hpd * 8, cudaMemcpyHostToDevice));
+  if (hpn) CK(cudaMemcpy(p->d_hp_n, hp_n, hpn * 4, cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(p->d_n_obs, n_obs, (size_t)n_scenes * 4, cudaMemcpyHostToDevice));
+  p->n_scenes = n_scenes; p->max_obs = max_obs;
+  return 0;
+}
+
+int32_t jmpc_plan(jmpc_planner p, int32_t B, const int32_t* scene_id, const double* start, const double* goal_point,
+                  const double* goal_area, const double* allowed, const double* weights, double* cost, int32_t* status,
+                  int32_t* n_path, double* path, int32_t* path_mp, int32_t* n_traj, double* traj, int32_t* expansions,
+                  double* log, void* stream) {
+  if (!p) return fail("jmpc_plan: NULL handle");
+  if (B < 0 || B > p->max_B) return fail("jmpc_plan: B out of range (B <= max_B of jmpc_planner_create)");
+  if (!start || !goal_point || !goal_area || !allowed || !weights || !cost || !status || !n_path || !path || !path_mp ||
+      !n_traj || !traj || !expansions)
+    return fail("jmpc_plan: NULL argument");
+  if (p->n_scenes < 1) return fail("jmpc_plan: no scenes (jmpc_planner_set_scenes)");
+  if (B == 0) return 0;
+  CK(cudaSetDevice(p->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  jmpc::PlanArgs a;
+  memset(&a, 0, sizeof a);
+  a.B = B; a.n_mp = p->n_mp; a.n_pts = p->n_pts; a.n_cc = p->n_cc; a.max_obs = p->max_obs; a.n_scenes = p->n_scenes;
+  a.max_expansions = p->max_expansions; a.max_path = p->max_path; a.max_traj = (p->max_path - 1) * (p->n_pts - 1);
+  a.max_log = log ? p->max_log : 0;
+  a.pool_cap = p->pool_cap; a.table_size = p->table_size;
+  a.mp_pts = p->d_pts; a.mp_len = p->d_len; a.mp_cc = p->d_cc;
+  a.hp = p->d_hp; a.hp_n = p->d_hp_n; a.n_obs = p->d_n_obs;
+  a.scene_id = scene_id; a.start = start; a.goal_point = goal_point; a.goal_area = goal_area; a.allowed = allowed;
+  a.weights = weights;
+  a.pool = p->d_pool; a.heap = p->d_heap; a.table = p->d_table;
+  a.cost = cost; a.status = status; a.n_path = n_path; a.path = path; a.path_mp = path_mp; a.n_traj = n_traj;
+  a.traj = traj; a.expansions = expansions; a.log = a.max_log ? log : nullptr;
+  // the kernel writes path / trajectory / log rows only as far as a search got: clear them, as jmpc_plan_host does
+  const size_t b = (size_t)B;
+  CK(cudaMemsetAsync(cost, 0, b * 8, st)); CK(cudaMemsetAsync(status, 0, b * 4, st)); CK(cudaMemsetAsync(n_path, 0, b * 4, st));
+  CK(cudaMemsetAsync(path, 0, b * p->max_path * 24, st)); CK(cudaMemsetAsync(path_mp, 0, b * p->max_path * 4, st));
+  CK(cudaMemsetAsync(n_traj, 0, b * 4, st)); CK(cudaMemsetAsync(traj, 0, b * a.max_traj * 24, st));
+  CK(cudaMemsetAsync(expansions, 0, b * 4, st));
+  if (a.log) CK(cudaMemsetAsync(log, 0, b * a.max_log * 40, st));
+  jmpc::plan_kernel<<<(B + 3) / 4, 128, 0, st>>>(a);
+  CK(cudaGetLastError());
+  return 0;
+}
+
+int32_t jmpc_set_courses_device(jmpc_handle h, int32_t n_courses, int32_t traj_stride, const int32_t* n_traj,
+                                const double* traj, const int32_t* plan_status, double* dl_out, int32_t* course_ok,
+                                void* stream) {
+  if (!h || !n_traj || !traj || !dl_out || !course_ok) return fail("jmpc_set_courses_device: NULL argument");
+  if (n_courses < 1 || n_courses > h->max_courses) return fail("jmpc_set_courses_device: n_courses out of range");
+  if (traj_stride < 1) return fail("jmpc_set_courses_device: traj_stride must be positive");
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  jmpc::IngestArgs a;
+  a.n_courses = n_courses; a.traj_stride = traj_stride; a.max_N = h->max_N; a.course_stride = h->course_stride;
+  a.n_traj = n_traj; a.traj = traj; a.plan_status = plan_status;
+  a.cx = h->d_cx; a.cy = h->d_cy; a.cyaw = h->d_cyaw; a.course_n = h->d_course_n; a.dl = dl_out; a.ok = course_ok;
+  jmpc::course_ingest_kernel<<<(n_courses + 3) / 4, 128, 0, st>>>(a);
+  CK(cudaGetLastError());
+  h->launches++;
+  // the lengths decide the arc-table budget (and are what course_len reports): the call's one readback
+  if (ensure_stage(h, (size_t)n_courses * sizeof(int))) return -1;
+  CK(cudaMemcpyAsync(h->h_stage, h->d_course_n, (size_t)n_courses * sizeof(int), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  const int* lens = (const int*)h->h_stage;
+  h->course_n.assign(lens, lens + n_courses);
+  h->n_courses = n_courses;
+  h->have_cv = false;
+  int max_n = 1;
+  for (int c = 0; c < n_courses; ++c) max_n = std::max(max_n, h->course_n[c]);
+  std::vector<long long> off;
+  if (place_arc_tables(h, off)) return -1;
+  CK(cudaMemcpyAsync(h->d_arc_off, off.data(), (size_t)n_courses * sizeof(long long), cudaMemcpyHostToDevice, st));
+  const unsigned gy = (unsigned)std::min(n_courses, 65535);
+  if (h->d_arc) {
+    jmpc::arc_tables_kernel<<<dim3((max_n + 63) / 64, gy), 64, 0, st>>>(n_courses, h->course_stride, h->d_course_n,
+                                                                      h->d_arc_off, h->d_cx, h->d_cy, h->d_arc);
+    CK(cudaGetLastError());
+    h->launches++;
+  }
+  jmpc::circle_tables_kernel<<<dim3((max_n + 127) / 128, gy), 128, 0, st>>>(
+      n_courses, h->course_stride, h->d_course_n, h->d_cx, h->d_cy, h->d_cyaw, h->off_front, h->off_rear, h->d_ccfx,
+      h->d_ccfy, h->d_ccrx, h->d_ccry);
+  CK(cudaGetLastError());
+  h->launches++;
+  // the *_host entry points run on the handle's own stream: order it after the tables without a host wait
+  cudaEvent_t ev;
+  CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+  cudaError_t e = cudaEventRecord(ev, st);
+  if (e == cudaSuccess) e = cudaStreamWaitEvent(h->own_stream, ev, 0);
+  cudaEventDestroy(ev);
+  if (e != cudaSuccess) return fail("jmpc_set_courses_device: stream ordering failed", e);
+  return 0;
+}
+
+int32_t jmpc_get_courses(jmpc_handle h, int32_t first, int32_t n, int32_t stride, int32_t* len, double* cx, double* cy,
+                         double* cyaw) {
+  if (!h || !len) return fail("jmpc_get_courses: NULL argument");
+  const bool pts = cx || cy || cyaw;
+  if (pts && !(cx && cy && cyaw)) return fail("jmpc_get_courses: give all of cx, cy, cyaw or none");
+  if (first < 0 || n < 0 || first + n > h->n_courses) return fail("jmpc_get_courses: course range out of range");
+  int width = 0;
+  for (int k = 0; k < n; ++k) { len[k] = h->course_n[first + k]; width = std::max(width, len[k]); }
+  if (!pts || n == 0) return 0;
+  if (stride < width) return fail("jmpc_get_courses: stride shorter than a course");
+  CK(cudaSetDevice(h->device));
+  CK(cudaDeviceSynchronize());
+  const size_t spitch = (size_t)h->course_stride * 8, dpitch = (size_t)stride * 8, off = (size_t)first * h->course_stride;
+  CK(cudaMemcpy2D(cx, dpitch, h->d_cx + off, spitch, (size_t)width * 8, n, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy2D(cy, dpitch, h->d_cy + off, spitch, (size_t)width * 8, n, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy2D(cyaw, dpitch, h->d_cyaw + off, spitch, (size_t)width * 8, n, cudaMemcpyDeviceToHost));
+  for (int k = 0; k < n; ++k) {
+    const size_t o = (size_t)k * stride + len[k], cnt = (size_t)stride - len[k];
+    memset(cx + o, 0, cnt * 8); memset(cy + o, 0, cnt * 8); memset(cyaw + o, 0, cnt * 8);
+  }
+  return 0;
+}
+
+int32_t jmpc_episode_init_from_courses(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* course_ok,
+                                       const double* dl, double* state, double* params, int32_t* done, void* stream) {
+  if (!h) return fail("jmpc_episode_init_from_courses: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_episode_init_from_courses: B out of range");
+  if (!state || !done) return fail("jmpc_episode_init_from_courses: NULL array");
+  if (h->n_courses < 1) return fail("jmpc_episode_init_from_courses: no courses uploaded");
+  if (B == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::episode_init_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
+      B, h->n_courses, h->course_stride, course_id, course_ok, dl, h->d_cx, h->d_cy, h->d_cyaw, state, params, done);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
 }
 
 int64_t jmpc_launch_count(jmpc_handle h) { return h ? h->launches : 0; }

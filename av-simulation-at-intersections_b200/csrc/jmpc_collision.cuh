@@ -60,16 +60,23 @@ __device__ __forceinline__ void circle_centre(double x, double y, double c, doub
   oy = __dadd_rn(__dmul_rn(s, off), y);
 }
 
+__device__ __forceinline__ void circle_table_point(int i, const double* __restrict__ cx, const double* __restrict__ cy,
+                                                   const double* __restrict__ cyaw, double off_front, double off_rear,
+                                                   double* __restrict__ fx, double* __restrict__ fy, double* __restrict__ rx,
+                                                   double* __restrict__ ry) {
+  double s, c;
+  sincos(cyaw[i], &s, &c);
+  circle_centre(cx[i], cy[i], c, s, off_front, fx[i], fy[i]);
+  circle_centre(cx[i], cy[i], c, s, off_rear, rx[i], ry[i]);
+}
+
 __global__ void circle_table_kernel(int n, const double* __restrict__ cx, const double* __restrict__ cy,
                                     const double* __restrict__ cyaw, double off_front, double off_rear,
                                     double* __restrict__ fx, double* __restrict__ fy, double* __restrict__ rx,
                                     double* __restrict__ ry) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  double s, c;
-  sincos(cyaw[i], &s, &c);
-  circle_centre(cx[i], cy[i], c, s, off_front, fx[i], fy[i]);
-  circle_centre(cx[i], cy[i], c, s, off_rear, rx[i], ry[i]);
+  circle_table_point(i, cx, cy, cyaw, off_front, off_rear, fx, fy, rx, ry);
 }
 
 // Running arc length of trajectory_full[a0:] for every start index a0 of a course: np.cumsum of the segment lengths,
@@ -77,9 +84,8 @@ __global__ void circle_table_kernel(int n, const double* __restrict__ cx, const 
 // is summed on its own; one thread per row).  Built once per course; the collision kernel then reads the row
 // instead of letting one lane re-do up to N sequential adds per instance.
 __host__ __device__ inline long long arc_row_offset(int a0, int N) { return (long long)a0 * N - ((long long)a0 * (a0 - 1)) / 2; }
-__global__ void arc_table_kernel(int N, const double* __restrict__ cx, const double* __restrict__ cy, double* __restrict__ tab) {
-  const int a0 = blockIdx.x * blockDim.x + threadIdx.x;
-  if (a0 >= N) return;
+__device__ __forceinline__ void arc_table_row(int a0, int N, const double* __restrict__ cx, const double* __restrict__ cy,
+                                              double* __restrict__ tab) {
   double* row = tab + arc_row_offset(a0, N);
   double acc = 0.0;
   for (int i = 0; i < N - a0; ++i) {
@@ -91,6 +97,11 @@ __global__ void arc_table_kernel(int N, const double* __restrict__ cx, const dou
     acc = __dadd_rn(acc, seg);
     row[i] = acc;
   }
+}
+__global__ void arc_table_kernel(int N, const double* __restrict__ cx, const double* __restrict__ cy, double* __restrict__ tab) {
+  const int a0 = blockIdx.x * blockDim.x + threadIdx.x;
+  if (a0 >= N) return;
+  arc_table_row(a0, N, cx, cy, tab);
 }
 
 // dist(a, b) <= reach with numpy's sqrt(dx*dx + dy*dy); the square root is only evaluated when the squared

@@ -32,7 +32,7 @@ struct PlanNode {           // one pushed tuple of the reference's heap
 };
 
 struct PlanArgs {
-  int B, n_mp, n_pts, n_cc, max_obs;
+  int B, n_mp, n_pts, n_cc, max_obs, n_scenes;
   // primitives (shared by all searches)
   const double* mp_pts;     // [n_mp][n_pts][3] points of each primitive, relative to its start pose
   const double* mp_len;     // [n_mp] total_length
@@ -140,7 +140,7 @@ __global__ void __launch_bounds__(128) plan_kernel(const PlanArgs A) {
   int* table = A.table + (size_t)b * A.table_size;
   const int mask = A.table_size - 1;
   for (int i = lane; i < A.table_size; i += 32) table[i] = -1;
-  const int scene = A.scene_id ? A.scene_id[b] : 0;
+  const int scene = A.scene_id ? min(max(A.scene_id[b], 0), A.n_scenes - 1) : 0;     // validated on the host by jmpc_plan_host
   const double* hp = A.hp + (size_t)scene * A.max_obs * JMPC_PLAN_MAX_HP * 3;
   const int* hp_n = A.hp_n + (size_t)scene * A.max_obs;
   const int n_obs = A.n_obs[scene];

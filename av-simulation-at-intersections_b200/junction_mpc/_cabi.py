@@ -65,6 +65,13 @@ SIGNATURES = {
                                                 C.c_void_p, C.c_int32, C.c_void_p]),
     "jmpc_plan_host": (C.c_int32, [C.c_int32] * 5 + [C.c_void_p] * 3 + [C.c_int32] * 2 + [C.c_void_p] * 9 + [C.c_int32] * 3
                        + [C.c_void_p] * 10),
+    "jmpc_planner_create": (C.c_int32, [C.c_int32] * 5 + [C.c_void_p] * 3 + [C.c_int32] * 3 + [C.POINTER(C.c_void_p)]),
+    "jmpc_planner_destroy": (C.c_int32, [C.c_void_p]),
+    "jmpc_planner_set_scenes": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "jmpc_plan": (C.c_int32, [C.c_void_p, C.c_int32] + [C.c_void_p] * 16),
+    "jmpc_set_courses_device": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32] + [C.c_void_p] * 6),
+    "jmpc_get_courses": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 4),
+    "jmpc_episode_init_from_courses": (C.c_int32, [C.c_void_p, C.c_int32] + [C.c_void_p] * 7),
     "jmpc_launch_count": (C.c_int64, [C.c_void_p]),
     "jmpc_measure_fma_peak": (C.c_int32, [C.c_void_p, c_f64p, c_f64p]),
     "jmpc_debug_linalg": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

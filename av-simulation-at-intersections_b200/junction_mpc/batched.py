@@ -62,6 +62,13 @@ class BatchedMPC:
                  max_T: Optional[int] = None, schedule: str = "history", du_th: float = 0.0):
         """courses: list of (N_c, >=3) arrays [x, y, yaw(smoothed)].  `du_th` > 0 switches on the early exit of the
         linearisation loop the reference left commented out (mpc.py:236-240)."""
+        self._open(max(len(c) for c in courses), len(courses), dl, T, config, dt, L, speed, max_batch, device,
+                   max_solver_iters, linearisation_iters, mu_tol, warps_per_sm, max_T, du_th)
+        self.set_courses(courses)
+        self.set_schedule(schedule)
+
+    def _open(self, max_N, max_courses, dl, T, config, dt, L, speed, max_batch, device, max_solver_iters,
+              linearisation_iters, mu_tol, warps_per_sm, max_T, du_th):
         self._lib = _cabi.load()
         cfg = config or MPCConfig.default()
         self.T = int(T if T is not None else cfg.T)
@@ -70,19 +77,72 @@ class BatchedMPC:
         self.default_params = self.config.param_vector(dl=self.dl, dt=self.dt, L=self.L, speed=self.speed)
         self.max_batch = int(max_batch)
         self.device = int(device)
-        lens = [len(c) for c in courses]
-        self.max_N = max(lens)
+        self.max_N = int(max_N)
+        self.car_radius = 2.0 / 2 ** 0.5                 # jmpc_set_car_geometry's default (car_dimensions.py:82-90)
+        self.course_ok = self.course_dl = None            # set by set_courses_from_plans
         opt = _cabi.Options(int(max_solver_iters), int(linearisation_iters or cfg.max_iter), float(mu_tol),
                             int(warps_per_sm), float(du_th))
         h = C.c_void_p()
         _cabi.check(self._lib.jmpc_create(self.device, self.max_batch, int(max_T or max(self.T, 25)), self.max_N,
-                                          len(courses), _ptr(self.default_params), C.byref(opt), C.byref(h)),
+                                          int(max_courses), _ptr(self.default_params), C.byref(opt), C.byref(h)),
                     "jmpc_create")
         self._h = h
         self._pinned = []
         self._host_out = {}
-        self.set_courses(courses)
-        self.set_schedule(schedule)
+
+    @classmethod
+    def from_plans(cls, plans, T: Optional[int] = None, config: Optional[MPCConfig] = None, dt: float = 0.2,
+                   L: float = 2.86, speed: float = 30.0 / 3.6, max_N: Optional[int] = None, max_batch: int = 1 << 20,
+                   device: int = 0, max_solver_iters: int = 40, linearisation_iters: Optional[int] = None,
+                   mu_tol: float = 1e-13, warps_per_sm: int = 0, max_T: Optional[int] = None, schedule: str = "history",
+                   du_th: float = 0.0) -> "BatchedMPC":
+        """An engine whose courses are the planned ones of a `planner.DevicePlanBatch`, ingested on the device
+        (`set_courses_from_plans`): course c = plan c.  `max_N` (default: the longest trajectory the plans can hold)
+        bounds the course length; a longer plan is reported unusable.  The engine's default dl is that of the first
+        usable course; `BatchedEpisodes.from_plans` gives every episode its own course's dl."""
+        obj = cls.__new__(cls)
+        obj._open(int(max_N or plans.traj.shape[1]), len(plans), float("nan"), T, config, dt, L, speed, max_batch, device,
+                  max_solver_iters, linearisation_iters, mu_tol, warps_per_sm, max_T, du_th)
+        obj.set_courses_from_plans(plans)
+        obj.set_schedule(schedule)
+        return obj
+
+    def set_courses_from_plans(self, plans):
+        """Replace the courses by the planned trajectories of `plans` (a `planner.DevicePlanBatch`) without a host round
+        trip (jmpc_set_courses_device): yaw unwrapped as MPC.__init__ does it (mpc.py:260), dl of the first segment
+        (mpc_intersection.py:73), collision tables built, on torch's current stream.  Sets `course_ok` (int32, 1 =
+        usable) and `course_dl` (float64, NaN when unusable) as CUDA tensors [n_plans], and `course_len`."""
+        import torch
+        n = len(plans)
+        dev = torch.device("cuda", self.device)
+        ok = torch.empty(n, dtype=torch.int32, device=dev)
+        dl = torch.empty(n, dtype=torch.float64, device=dev)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        _cabi.check(self._lib.jmpc_set_courses_device(
+            self._h, n, int(plans.traj.shape[1]), self._dp(plans.n_traj, torch.int32), self._dp(plans.traj, torch.float64),
+            self._dp(plans.status, torch.int32), self._dp(dl, torch.float64), self._dp(ok, torch.int32),
+            C.c_void_p(stream)), "jmpc_set_courses_device")
+        self.course_len = self.get_courses(0, n, lengths_only=True)
+        self.course_ok, self.course_dl = ok, dl
+        self._ok_host, self._dl_host = ok.cpu().numpy(), dl.cpu().numpy()
+        if self._ok_host.any():
+            self.dl = float(self._dl_host[np.argmax(self._ok_host)])
+            self.default_params = self.config.param_vector(dl=self.dl, dt=self.dt, L=self.L, speed=self.speed)
+            _cabi.check(self._lib.jmpc_set_default_params(self._h, _ptr(self.default_params)), "jmpc_set_default_params")
+
+    def get_courses(self, first: int = 0, n: Optional[int] = None, lengths_only: bool = False):
+        """The uploaded courses first .. first + n - 1 as (N_c, 3) arrays [x, y, smoothed yaw] (jmpc_get_courses);
+        with `lengths_only` just their lengths."""
+        n = len(self.course_len) - first if n is None else int(n)
+        lens = np.zeros(n, np.int32)
+        if lengths_only:
+            _cabi.check(self._lib.jmpc_get_courses(self._h, int(first), n, 0, _ptr(lens), None, None, None), "jmpc_get_courses")
+            return lens
+        stride = self.max_N
+        tab = np.zeros((3, n, stride))
+        _cabi.check(self._lib.jmpc_get_courses(self._h, int(first), n, stride, _ptr(lens), _ptr(tab[0]), _ptr(tab[1]),
+                                               _ptr(tab[2])), "jmpc_get_courses")
+        return [np.ascontiguousarray(tab[:, k, :lens[k]].T) for k in range(n)]
 
     # ---- configuration ----------------------------------------------------------------------------------
     def set_courses(self, courses: Sequence[np.ndarray]):
@@ -97,6 +157,7 @@ class BatchedMPC:
         _cabi.check(self._lib.jmpc_set_courses(self._h, len(courses), stride, _ptr(lens), _ptr(tab[0]), _ptr(tab[1]),
                                                _ptr(tab[2])), "jmpc_set_courses")
         self.course_len = lens.copy()
+        self.course_ok = self.course_dl = None
 
     def set_course_speed(self, speeds: Optional[Sequence[np.ndarray]]):
         """Reference speed profile per course point (`cv` of main/lib/mpc_with_speed.py:104): one array per uploaded
@@ -130,6 +191,7 @@ class BatchedMPC:
     def set_car_geometry(self, front_offset: float, rear_offset: float, radius: float):
         _cabi.check(self._lib.jmpc_set_car_geometry(self._h, float(front_offset), float(rear_offset), float(radius)),
                     "jmpc_set_car_geometry")
+        self.car_radius = float(radius)
 
     SCHEDULES = {"index": 0, "apriori": 1, "history": 2}
 

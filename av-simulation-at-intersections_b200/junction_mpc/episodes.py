@@ -10,12 +10,14 @@ per-step recording (`obstacle_script`).
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Optional
 
 import numpy as np
 
 from . import _cabi
 from .batched import BatchedMPC
+from .config import NPARAM
 
 
 OBS_KINDS = {"constant": 0, "t_intersection": 1, "roundabout": 2, "arterial": 3}
@@ -52,7 +54,57 @@ def scripted_obstacles(specs, L: float = 2.86):
     return script, model
 
 
+def plan_episode_setup(course_ok, course_dl, plan_id, n_plans: int, car_radius: float):
+    """Host-side checks of `BatchedEpisodes.from_plans`: returns (plan_id as int32 [B], margin).
+    plan_id None -> one episode per plan.  The margin is EXTRA_CUTOFF_MARGIN = 4 * ceil(radius / dl)
+    (mpc_intersection.py:87-88) over the usable courses the episodes drive; it is one scalar for the batch, so courses
+    that disagree on it are an error (0 when no episode has a usable course)."""
+    course_ok, course_dl = np.asarray(course_ok), np.asarray(course_dl, np.float64)
+    if course_ok.shape != (n_plans,) or course_dl.shape != (n_plans,):
+        raise ValueError(f"course_ok / course_dl must be [{n_plans}]")
+    pid = np.arange(n_plans, dtype=np.int64) if plan_id is None else np.asarray(plan_id)
+    if pid.ndim != 1 or len(pid) < 1 or not np.issubdtype(pid.dtype, np.integer):
+        raise ValueError("plan_id must be a non-empty 1-D integer array")
+    if pid.min() < 0 or pid.max() >= n_plans:
+        raise ValueError(f"plan_id out of range [0, {n_plans})")
+    used = np.unique(pid[course_ok[pid] != 0])
+    margins = {4 * int(math.ceil(car_radius / float(course_dl[c]))) for c in used}
+    if len(margins) > 1:
+        raise ValueError(f"the planned courses disagree on the cut-off margin 4 * ceil(radius / dl): {sorted(margins)}")
+    return np.ascontiguousarray(pid, dtype=np.int32), (margins.pop() if margins else 0)
+
+
 class BatchedEpisodes:
+    @classmethod
+    def from_plans(cls, engine: BatchedMPC, plans, plan_id=None, params=None, obstacle_program=None, obstacles=None,
+                   frame_window: int = 10, max_steps: int = 256, record_history: bool = True, horizon_s: float = 7.0,
+                   obstacle_script=None) -> "BatchedEpisodes":
+        """Episodes on the planned courses of `engine` (filled by `BatchedMPC.from_plans(plans)` /
+        `set_courses_from_plans(plans)`), the second half of main/scenarios/mpc_intersection.py:63-163 for a batch:
+        episode b drives plan `plan_id[b]` (default: one episode per plan; zeros = one course, many controllers).
+        Its start state (the course's first pose at v = 0), its params row `dl` and done = 3 for a plan without a usable
+        course are written on the device (jmpc_episode_init_from_courses); such episodes are never stepped.
+        `params` [B, NPARAM] (default: the engine's defaults) supplies every other parameter row.  `run()` adds
+        plan_status, plan_cost and expansions per episode."""
+        if engine.course_ok is None or len(engine.course_ok) != len(plans):
+            raise ValueError("the engine's courses do not come from these plans (BatchedMPC.from_plans)")
+        import torch
+        pid, margin = plan_episode_setup(engine._ok_host, engine._dl_host, plan_id, len(plans), engine.car_radius)
+        B = len(pid)
+        if params is None:
+            params = np.repeat(engine.default_params[None, :], B, axis=0)
+        elif np.shape(params) != (B, NPARAM):
+            raise ValueError(f"params must be [{B}, {NPARAM}]")
+        ep = cls(engine, np.zeros((B, 4)), course_id=pid, obstacles=obstacles, obstacle_script=obstacle_script,
+                 frame_window=frame_window, margin=margin, params=params, max_steps=max_steps,
+                 record_history=record_history, horizon_s=horizon_s, obstacle_program=obstacle_program)
+        stream = C.c_void_p(torch.cuda.current_stream(engine.device).cuda_stream)
+        _cabi.check(engine._lib.jmpc_episode_init_from_courses(
+            engine._h, B, ep._p(ep.course_id), ep._p(engine.course_ok), ep._p(engine.course_dl), ep._p(ep.state),
+            ep._p(ep.params), ep._p(ep.done), stream), "jmpc_episode_init_from_courses")
+        ep._plans = (plans, ep.course_id.long())
+        return ep
+
     def __init__(self, engine: BatchedMPC, state0, course_id=None, obstacles=None, obstacle_script=None,
                  frame_window: int = 10, margin: int = 72, params=None, max_steps: int = 256,
                  record_history: bool = True, horizon_s: float = 7.0, obstacle_program=None):
@@ -93,6 +145,7 @@ class BatchedEpisodes:
         self.flags = torch.zeros(self.max_steps, B, dtype=i32, device=self.dev) if record_history else None
         self.iteration = 0
         self.iter_dev = torch.zeros(1, dtype=i32, device=self.dev)     # the same counter on the device (graph replay)
+        self._plans = None                                           # (DevicePlanBatch, plan index per episode): from_plans
         if self.program is not None:                                 # get() before the first iteration
             self._scripted_step(advance=0)
 
@@ -201,4 +254,8 @@ class BatchedEpisodes:
             # (t = (i + 2) dt: HistorySimulation stores the initial state first, at t = dt; simulation.py:53-61)
             res["history"] = self.history[:n].cpu().numpy()
             res["flags"] = self.flags[:n].cpu().numpy()
+        if self._plans is not None:
+            plans, pid = self._plans
+            res.update(plan_status=plans.status[pid].cpu().numpy(), plan_cost=plans.cost[pid].cpu().numpy(),
+                       expansions=plans.expansions[pid].cpu().numpy())
         return res

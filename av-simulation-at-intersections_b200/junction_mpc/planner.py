@@ -66,6 +66,60 @@ def collision_check_points(mp_points: np.ndarray, radius: float, circle_centers:
     return np.concatenate(out, axis=0)
 
 
+def pack_plan_inputs(start, goal_point, goal_area, allowed_dtheta, scenes, scene_id=None, weights=None):
+    """The arguments of `BatchedPlanner.plan` in the C ABI's layout: (start, goal_point, goal_area, allowed, weights,
+    scene_id or None, (n_scenes, max_obs, hp, hp_n, n_obs))."""
+    f = lambda a, shape: np.ascontiguousarray(np.broadcast_to(np.asarray(a, np.float64), shape))   # noqa: E731
+    start = np.ascontiguousarray(np.asarray(start, np.float64).reshape(-1, 3))
+    B = len(start)
+    goal_point, goal_area = f(goal_point, (B, 3)), f(goal_area, (B, 4))
+    allowed = f(allowed_dtheta, (B,))
+    if weights is None or isinstance(weights, dict):
+        w = dict(DEFAULT_WEIGHTS, **(weights or {}))
+        weights = [w[k] for k in WEIGHT_KEYS]
+    weights = f(weights, (B, 9))
+    n_scenes = len(scenes)
+    max_obs = max(1, max(len(s) for s in scenes))
+    hp = np.zeros((n_scenes, max_obs, MAX_HP, 3))
+    hp_n = np.zeros((n_scenes, max_obs), np.int32)
+    n_obs = np.array([len(s) for s in scenes], np.int32)
+    for i, s in enumerate(scenes):
+        for k, rows in enumerate(s):
+            rows = np.asarray(rows, float).reshape(-1, 3)
+            if not 1 <= len(rows) <= MAX_HP:
+                raise ValueError(f"an obstacle needs 1..{MAX_HP} half-planes")
+            hp[i, k, :len(rows)] = rows
+            hp_n[i, k] = len(rows)
+    sid = None if scene_id is None else np.ascontiguousarray(scene_id, dtype=np.int32)
+    return start, goal_point, goal_area, allowed, weights, sid, (n_scenes, max_obs, hp, hp_n, n_obs)
+
+
+@dataclass
+class DevicePlanBatch:
+    """What `BatchedPlanner.plan_device` returns: the fields of `PlanBatch` as torch CUDA tensors (same shapes), still
+    being computed on the stream they were enqueued on.  Feed it to `BatchedMPC.from_plans` to drive the courses
+    without a host round trip."""
+    cost: object
+    status: object
+    n_path: object
+    path: object
+    path_mp: object
+    n_traj: object
+    traj: object                # [B, max_traj, 3] x, y, raw yaw
+    expansions: object
+    log: object = None
+
+    def __len__(self) -> int:
+        return int(self.cost.shape[0])
+
+    def to_host(self) -> PlanBatch:
+        """Synchronising copy into a `PlanBatch` (kernel_ms = NaN: the launch was not timed)."""
+        c = lambda t: None if t is None else t.cpu().numpy()            # noqa: E731
+        return PlanBatch(cost=c(self.cost), status=c(self.status), n_path=c(self.n_path), path=c(self.path),
+                         path_mp=c(self.path_mp), n_traj=c(self.n_traj), traj=c(self.traj),
+                         expansions=c(self.expansions), log=c(self.log), kernel_ms=float("nan"))
+
+
 @dataclass
 class PlanBatch:
     cost: np.ndarray            # [B]
@@ -91,9 +145,12 @@ class PlanBatch:
 
 class BatchedPlanner:
     def __init__(self, mp_points: Optional[np.ndarray] = None, mp_total_length: Optional[np.ndarray] = None,
-                 car_radius: float = 2.0 / 2 ** 0.5, circle_centers=((2.18, 0.0), (0.68, 0.0)), device: int = 0):
+                 car_radius: float = 2.0 / 2 ** 0.5, circle_centers=((2.18, 0.0), (0.68, 0.0)), device: int = 0,
+                 max_batch: int = 4096):
         """Defaults: the reference's bicycle-model primitives and BicycleModelDimensions (car_dimensions.py:62-90:
-        width 2, length 3.5, circle centres at L/2 +- (length - width)/2 ahead of the rear axle: 2.18 and 0.68)."""
+        width 2, length 3.5, circle centres at L/2 +- (length - width)/2 ahead of the rear axle: 2.18 and 0.68).
+        `max_batch`: searches per launch of `plan_device`, whose persistent workspace is allocated for that many
+        (about 2 MB per search at max_expansions = 4096); larger batches run in chunks."""
         self._lib = _cabi.load()
         if mp_points is None:
             _, mp_points, mp_total_length = load_motion_primitives()
@@ -106,34 +163,19 @@ class BatchedPlanner:
             raise ValueError("primitives with different numbers of collision-check points are not supported")
         self.mp_cc = np.ascontiguousarray(np.stack(cc), dtype=np.float64)
         self.device = int(device)
+        if int(max_batch) < 1:
+            raise ValueError("max_batch must be positive")
+        self.max_batch = int(max_batch)
+        self._handle, self._handle_key = None, None         # jmpc_planner of plan_device, created on first use
 
     def plan(self, start, goal_point, goal_area, allowed_dtheta, scenes: Sequence[Sequence[np.ndarray]], scene_id=None,
              weights=None, max_expansions: int = 4096, max_path: int = 48, log: bool = False) -> PlanBatch:
         """start, goal_point [B, 3]; goal_area [B, 4] = x1, y1, x2, y2; allowed_dtheta [B] or scalar;
         scenes: list of scenes, each a list of half-plane arrays [m, 3] (one per obstacle, m <= 8); scene_id [B];
         weights [B, 9] in WEIGHT_KEYS order, a dict, or None for the reference defaults."""
-        f = lambda a, shape: np.ascontiguousarray(np.broadcast_to(np.asarray(a, np.float64), shape))   # noqa: E731
-        start = np.ascontiguousarray(np.asarray(start, np.float64).reshape(-1, 3))
+        start, goal_point, goal_area, allowed, weights, sid, (n_scenes, max_obs, hp, hp_n, n_obs) = pack_plan_inputs(
+            start, goal_point, goal_area, allowed_dtheta, scenes, scene_id, weights)
         B = len(start)
-        goal_point, goal_area = f(goal_point, (B, 3)), f(goal_area, (B, 4))
-        allowed = f(allowed_dtheta, (B,))
-        if weights is None or isinstance(weights, dict):
-            w = dict(DEFAULT_WEIGHTS, **(weights or {}))
-            weights = [w[k] for k in WEIGHT_KEYS]
-        weights = f(weights, (B, 9))
-        n_scenes = len(scenes)
-        max_obs = max(1, max(len(s) for s in scenes))
-        hp = np.zeros((n_scenes, max_obs, MAX_HP, 3))
-        hp_n = np.zeros((n_scenes, max_obs), np.int32)
-        n_obs = np.array([len(s) for s in scenes], np.int32)
-        for i, s in enumerate(scenes):
-            for k, rows in enumerate(s):
-                rows = np.asarray(rows, float).reshape(-1, 3)
-                if not 1 <= len(rows) <= MAX_HP:
-                    raise ValueError(f"an obstacle needs 1..{MAX_HP} half-planes")
-                hp[i, k, :len(rows)] = rows
-                hp_n[i, k] = len(rows)
-        sid = None if scene_id is None else np.ascontiguousarray(scene_id, dtype=np.int32)
         n_mp, n_pts = self.mp_points.shape[:2]
         n_cc = self.mp_cc.shape[1]
         max_traj = (max_path - 1) * (n_pts - 1)
@@ -151,6 +193,78 @@ class BatchedPlanner:
             p(out.traj), p(out.expansions), p(out.log), C.cast(C.byref(ms), C.c_void_p)), "jmpc_plan_host")
         out.kernel_ms = float(ms.value)
         return out
+
+    def plan_device(self, start, goal_point, goal_area, allowed_dtheta, scenes: Sequence[Sequence[np.ndarray]],
+                    scene_id=None, weights=None, max_expansions: int = 4096, max_path: int = 48,
+                    log: bool = False) -> DevicePlanBatch:
+        """`plan` with the results left on the device: the same arguments, the same kernel and bit-identical
+        results, as torch CUDA tensors enqueued on torch's current stream (nothing is synchronised).  The workspace
+        is this planner's persistent `jmpc_planner`, created on first use for `max_batch` searches (re-created when
+        max_expansions / max_path / log change); batches larger than `max_batch` run in chunks on the same stream."""
+        import torch
+        start, goal_point, goal_area, allowed, weights, sid, (n_scenes, max_obs, hp, hp_n, n_obs) = pack_plan_inputs(
+            start, goal_point, goal_area, allowed_dtheta, scenes, scene_id, weights)
+        B = len(start)
+        if sid is not None and (sid.shape != (B,) or (B and (sid.min() < 0 or sid.max() >= n_scenes))):
+            raise ValueError("scene_id must be [B] with values in [0, len(scenes))")
+        max_expansions, max_path = int(max_expansions), int(max_path)
+        max_log = max_expansions if log else 0
+        p = self._planner_handle(max_expansions, max_path, max_log)
+        _cabi.check(self._lib.jmpc_planner_set_scenes(p, n_scenes, max_obs, hp.ctypes.data_as(C.c_void_p),
+                                                      hp_n.ctypes.data_as(C.c_void_p), n_obs.ctypes.data_as(C.c_void_p)),
+                    "jmpc_planner_set_scenes")
+        dev = torch.device("cuda", self.device)
+        f64, i32 = torch.float64, torch.int32
+        # np.array copies: the packed inputs can be read-only broadcast views, which torch does not wrap
+        up = lambda a, dt: None if a is None else torch.as_tensor(np.array(a), dtype=dt).to(dev)      # noqa: E731
+        d_start, d_goal, d_area, d_allowed, d_w, d_sid = (up(start, f64), up(goal_point, f64), up(goal_area, f64),
+                                                          up(allowed, f64), up(weights, f64), up(sid, i32))
+        max_traj = (max_path - 1) * (self.mp_points.shape[1] - 1)
+        out = DevicePlanBatch(cost=torch.empty(B, dtype=f64, device=dev), status=torch.empty(B, dtype=i32, device=dev),
+                              n_path=torch.empty(B, dtype=i32, device=dev),
+                              path=torch.empty(B, max_path, 3, dtype=f64, device=dev),
+                              path_mp=torch.empty(B, max_path, dtype=i32, device=dev),
+                              n_traj=torch.empty(B, dtype=i32, device=dev),
+                              traj=torch.empty(B, max_traj, 3, dtype=f64, device=dev),
+                              expansions=torch.empty(B, dtype=i32, device=dev),
+                              log=torch.empty(B, max_log, 5, dtype=f64, device=dev) if log else None)
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        q = lambda t, lo: None if t is None else C.c_void_p(t[lo:].data_ptr())           # noqa: E731
+        for lo in range(0, B, self.max_batch):
+            n = min(self.max_batch, B - lo)
+            _cabi.check(self._lib.jmpc_plan(
+                p, n, q(d_sid, lo), q(d_start, lo), q(d_goal, lo), q(d_area, lo), q(d_allowed, lo), q(d_w, lo),
+                q(out.cost, lo), q(out.status, lo), q(out.n_path, lo), q(out.path, lo), q(out.path_mp, lo),
+                q(out.n_traj, lo), q(out.traj, lo), q(out.expansions, lo), q(out.log, lo), stream), "jmpc_plan")
+        return out
+
+    def _planner_handle(self, max_expansions: int, max_path: int, max_log: int):
+        key = (max_expansions, max_path, max_log)
+        if self._handle is not None and self._handle_key == key:
+            return self._handle
+        self.close()
+        n_mp, n_pts = self.mp_points.shape[:2]
+        h = C.c_void_p()
+        p = lambda a: a.ctypes.data_as(C.c_void_p)                                       # noqa: E731
+        _cabi.check(self._lib.jmpc_planner_create(self.device, self.max_batch, n_mp, n_pts, self.mp_cc.shape[1],
+                                                  p(self.mp_points), p(self.mp_len), p(self.mp_cc), max_expansions,
+                                                  max_path, max_log, C.byref(h)), "jmpc_planner_create")
+        self._handle, self._handle_key = h, key
+        return h
+
+    def close(self):
+        """Free the persistent workspace of `plan_device` (waits for the device first)."""
+        if getattr(self, "_handle", None) is not None:
+            import torch
+            torch.cuda.synchronize(self.device)
+            self._lib.jmpc_planner_destroy(self._handle)
+            self._handle, self._handle_key = None, None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class MotionPrimitiveSearch:

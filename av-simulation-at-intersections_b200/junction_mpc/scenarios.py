@@ -1,0 +1,44 @@
+"""Planned scenarios from scene to goal on the device: main/scenarios/mpc_intersection.py:27-163 for a batch.
+
+The reference script plans a course with MotionPrimitiveSearch (:63-66), derives dl from its first segment (:73), builds
+an MPC on it (yaw smoothed in place, mpc.py:260), starts the ego at trajectory_full[0] with v = 0 (:76-79) and runs the
+closed loop against its scripted obstacles (:99-163).  `run_planned_scenarios` does the same for many (scene, start,
+goal, weights) at once: the searches, the course ingestion and the loop all run in libjmpc.so kernels and the planned
+courses never leave the GPU.
+"""
+from __future__ import annotations
+
+from typing import Optional, Sequence
+
+from .batched import BatchedMPC
+from .config import MPCConfig
+from .episodes import BatchedEpisodes, scripted_obstacles
+from .planner import BatchedPlanner
+
+
+def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_area, allowed_dtheta, scene_id=None,
+                          weights=None, obstacles: Optional[Sequence[Sequence[dict]]] = None, frame_window: int = 10,
+                          T: Optional[int] = None, config: Optional[MPCConfig] = None, dt: float = 0.2,
+                          max_steps: int = 256, max_expansions: int = 4096, max_path: int = 48,
+                          max_N: Optional[int] = None, planner: Optional[BatchedPlanner] = None, device: int = 0) -> dict:
+    """One episode per search.  scenes / start / goal_point / goal_area / allowed_dtheta / scene_id / weights as in
+    `BatchedPlanner.plan`; obstacles: per episode a list of the reference's scripted-obstacle dicts (see
+    `episodes.scripted_obstacles`), or None for an empty road; frame_window: FRAME_WINDOW of the script (10 for the
+    intersection, 20 for the roundabout).  Returns `BatchedEpisodes.run`'s dict (steps, done -- 3 where the search
+    found no course --, state, history, flags, plan_status, plan_cost, expansions) plus the episodes' `dl` and
+    `margin`."""
+    import torch
+    planner = planner or BatchedPlanner(device=device)
+    plans = planner.plan_device(start, goal_point, goal_area, allowed_dtheta, scenes, scene_id=scene_id, weights=weights,
+                                max_expansions=max_expansions, max_path=max_path)
+    engine = BatchedMPC.from_plans(plans, T=T, config=config, dt=dt, max_N=max_N, max_batch=len(plans), device=device)
+    try:
+        program = None if obstacles is None else scripted_obstacles(obstacles)
+        ep = BatchedEpisodes.from_plans(engine, plans, obstacle_program=program, frame_window=frame_window,
+                                        max_steps=max_steps)
+        res = ep.run(max_steps=max_steps)
+        res.update(dl=engine.course_dl.cpu().numpy(), margin=ep.margin)
+        torch.cuda.synchronize(engine.device)
+        return res
+    finally:
+        engine.close()

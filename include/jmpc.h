@@ -232,7 +232,8 @@ int32_t jmpc_plant_step(jmpc_handle h, int32_t B, double* state, const double* a
                         const double* params, void* stream);
 
 /* Closed-loop episodes on the device (the scenario loop around the step, main/scenarios/mpc_intersection.py:99-163).
- * DEVICE pointers; all arrays [B] unless noted; episodes with done != 0 are left untouched by all three.
+ * DEVICE pointers; all arrays [B] unless noted; episodes with done != 0 are left untouched by all three.  done codes:
+ * 1 goal reached, 2 the index rule raised, 3 no planned course (jmpc_episode_init_from_courses: the plan failed).
  *   jmpc_episode_pre : done |= is_goal(state) (mpc.py:314-330; done = 2 when the index rule raises), then
  *                      agent_idx = nearest forward index on the full course unless the truncated course has
  *                      collapsed onto the ego's point (mpc_intersection.py:107-109).  course_len = length of the
@@ -319,6 +320,70 @@ int32_t jmpc_plan_host(int32_t device, int32_t B, int32_t n_mp, int32_t n_pts, i
                        int32_t max_expansions, int32_t max_path, int32_t max_log, double* cost, int32_t* status,
                        int32_t* n_path, double* path, int32_t* path_mp, int32_t* n_traj, double* traj,
                        int32_t* expansions, double* log, double* kernel_ms);
+
+/* Persistent planner: the same plan_kernel as jmpc_plan_host with the primitives, scenes and per-search workspace
+ * allocated once, so that planned courses can stay on the device (jmpc_set_courses_device) instead of taking the
+ * allocate / upload / run / download / free round trip of jmpc_plan_host on every call.  Replaces the per-scenario
+ * MotionPrimitiveSearch(...).run() of main/scenarios/mpc_intersection.py:63-66 for a batch of scenarios.
+ * One handle per (host thread, device); calls on one handle must be serialised by the caller (one stream).
+ *
+ * jmpc_planner_create: uploads the primitive set (layouts as jmpc_plan_host) and allocates, for max_B searches, the
+ *   workspace of each search -- node pool (pool_cap = max_expansions * n_mp + 1 entries of 48 bytes), heap
+ *   (pool_cap int32) and closed-set hash table (table_size = smallest power of two >= 2 * max_expansions + 2, at
+ *   least 64, int32 slots) -- i.e. pool_cap * 52 + table_size * 4 bytes per search (about 2 MB at max_expansions =
+ *   4096 with the reference's nine primitives).  max_log = 0 disables the expansion log. */
+typedef struct jmpc_planner_s* jmpc_planner;
+int32_t jmpc_planner_create(int32_t device, int32_t max_B, int32_t n_mp, int32_t n_pts, int32_t n_cc, const double* mp_pts,
+                            const double* mp_len, const double* mp_cc, int32_t max_expansions, int32_t max_path,
+                            int32_t max_log, jmpc_planner* out);
+int32_t jmpc_planner_destroy(jmpc_planner p);
+/* Scenes (HOST pointers, layouts as jmpc_plan_host), uploaded once and kept until the next call.  Waits for the
+ * device to finish earlier work of the handle before replacing them. */
+int32_t jmpc_planner_set_scenes(jmpc_planner p, int32_t n_scenes, int32_t max_obs, const double* hp, const int32_t* hp_n,
+                                const int32_t* n_obs);
+/* B <= max_B searches with DEVICE pointers; only enqueues on `stream` (no allocation, no synchronisation).  Inputs
+ * and results have the layouts of jmpc_plan_host with the handle's max_path and max_log (log may be NULL; a handle
+ * created with max_log = 0 writes none).  scene_id [B] or NULL (all scene 0); values outside [0, n_scenes) are
+ * clamped, as device entry points cannot validate.  The results are bit-identical to jmpc_plan_host's for the same
+ * inputs and limits, and do not depend on what an earlier call left in the workspace: the outputs are cleared first
+ * and every search resets its own hash table. */
+int32_t jmpc_plan(jmpc_planner p, int32_t B, const int32_t* scene_id, const double* start, const double* goal_point,
+                  const double* goal_area, const double* allowed, const double* weights, double* cost, int32_t* status,
+                  int32_t* n_path, double* path, int32_t* path_mp, int32_t* n_traj, double* traj, int32_t* expansions,
+                  double* log, void* stream);
+
+/* Course tables straight from the planner's output (DEVICE pointers): course c is traj[c][0 : n_traj[c]] of a
+ * [n_courses][traj_stride][3] array (jmpc_plan's traj, x, y, raw yaw).  Replaces, for a batch, what the scenario
+ * script does between planning and driving (mpc_intersection.py:63-79): MPC(trajectory_full) smoothing the yaw in
+ * place (mpc.py:260 -> the sequential unwrap of mpc.py:46-58, one thread per course, the same compares with pi/2 and
+ * the same adds of 2 pi, so bit-identical to it) and dl = norm(trajectory_full[0, :2] - trajectory_full[1, :2])
+ * (mpc_intersection.py:73, as sqrt(dx*dx + dy*dy) without fused multiply-adds).  Then the circle and arc-length
+ * tables of jmpc_set_courses are built, in O(1) launches for all courses.  No trajectory byte leaves the device; the
+ * call reads the n_courses lengths back (one synchronisation of `stream`) so that the handle's course lengths and the
+ * arc-table budget behave as after jmpc_set_courses.
+ *   plan_status [n_courses] jmpc_plan_status or NULL (all found)
+ *   dl_out [n_courses]: dl of the course, NaN when unusable;  course_ok [n_courses]: 1 usable, 0 unusable
+ * A course whose plan failed (status != JMPC_PLAN_FOUND), with fewer than 2 or more than max_N points, or with a
+ * non-finite value is unusable: it gets a one-point placeholder -- its first trajectory point (the start pose) when
+ * the plan produced one, the origin otherwise -- and never fails the call.  The tables are built on `stream`; the
+ * handle's own stream (the *_host entry points) is ordered after them, other streams must be ordered by the caller. */
+int32_t jmpc_set_courses_device(jmpc_handle h, int32_t n_courses, int32_t traj_stride, const int32_t* n_traj,
+                                const double* traj, const int32_t* plan_status, double* dl_out, int32_t* course_ok,
+                                void* stream);
+
+/* Read courses first .. first + n - 1 back (HOST pointers): len [n], and cx / cy / cyaw [n][stride] with the points
+ * beyond a course's length zeroed (all three NULL: lengths only).  Waits for the device.  For tests and for callers
+ * that want to keep what was planned and smoothed. */
+int32_t jmpc_get_courses(jmpc_handle h, int32_t first, int32_t n, int32_t stride, int32_t* len, double* cx, double* cy,
+                         double* cyaw);
+
+/* Episode start on the ingested courses (DEVICE pointers), the reference's State(x=trajectory_full[0, 0],
+ * y=trajectory_full[0, 1], yaw=trajectory_full[0, 2], v=0) of mpc_intersection.py:76-79 after the smoothing:
+ *   state [B][4] = (cx[0], cy[0], 0, cyaw[0]) of course course_id[b] (NULL: course 0; clamped to the courses)
+ *   params [B][JMPC_NPARAM] or NULL: row JMPC_P_DL = dl[course] (dl NULL: untouched); other rows are left as they are
+ *   done [B] = 3 ("no planned course") where course_ok[course] == 0 (course_ok NULL: all usable); untouched otherwise */
+int32_t jmpc_episode_init_from_courses(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* course_ok,
+                                       const double* dl, double* state, double* params, int32_t* done, void* stream);
 
 /* Number of kernel launches issued through this handle since creation (for bench.py's gpu_launches). */
 int64_t jmpc_launch_count(jmpc_handle h);

@@ -1,0 +1,197 @@
+"""Plan-and-drive study through the device pipeline and through the host pipeline it replaces.
+
+Workload: the recorded planner variants that find a course (tests/golden/planner.npz), replicated to 1 024 / 4 096 /
+16 384 scenarios, each driven from its start to its goal against the reference's scripted obstacles (roundabout
+variants: the roundabout script, all others: the intersection script; FRAME_WINDOW = 10 for the whole batch).
+
+  device: BatchedPlanner.plan_device -> BatchedMPC.from_plans (max_N = 1024, the longest recorded course is 1020
+          points) -> BatchedEpisodes.from_plans -> run
+  host:   BatchedPlanner.plan -> PlanBatch.courses() -> synth.smooth_yaw_inplace per course -> BatchedMPC(courses)
+          -> BatchedEpisodes -> run
+
+Per stage: planning (kernel by CUDA events, wall), course ingestion, episodes (steps/s, episodes/s), total wall; the
+share of courses that got an arc-length table (the collision kernel sums the others on the fly).  Both pipelines must
+give bit-identical episodes; the script checks that and reports it.  Each size runs twice after a warm-up batch and
+the second pass is reported; the device planner's kernel time comes from a separate torch.profiler pass
+(plan_device_span_ms is the event span around plan_device, host-side input packing and uploads included).
+Writes plan_and_drive.json into --out (default: the current directory).
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+for p in (ROOT, os.path.join(ROOT, "av-simulation-at-intersections_b200"), os.path.join(ROOT, "tests")):
+    sys.path.insert(0, p)
+import numpy as np  # noqa: E402
+
+from helpers import load_planner_golden  # noqa: E402
+
+SCRIPTS = {
+    "intersection": [dict(kind="t_intersection", direction=1, offset=2., turning=False, speed=25 / 3.6, dt=0.2),
+                     dict(kind="t_intersection", direction=-1, offset=4., turning=True, speed=25 / 3.6, dt=0.2)],
+    "roundabout": [dict(kind="roundabout", direction=1, offset=1., turning=True, speed=25 / 3.6, dt=0.2),
+                   dict(kind="roundabout", direction=-1, offset=4., turning=True, speed=25 / 3.6, dt=0.2)],
+}
+ARC_CAP_DOUBLES = (256 << 20) // 8      # the handle's arc-table budget (jmpc.cu: place_arc_tables)
+
+
+def workload(z, B):
+    names = [str(n) for n in z["variants"] if not np.isnan(z[f"{n}/cost"])]
+    g = lambda n, k: z[f"{n}/{k}"]             # noqa: E731
+    scenes = [[g(n, "hp")[k, :g(n, "hp_n")[k]] for k in range(len(g(n, "hp_n")))] for n in names]
+    idx = np.arange(B) % len(names)
+    inp = dict(start=np.stack([g(names[i], "start") for i in idx]), goal_point=np.stack([g(names[i], "goal_point") for i in idx]),
+               goal_area=np.stack([g(names[i], "goal_area") for i in idx]),
+               allowed_dtheta=np.array([float(g(names[i], "allowed_dtheta")) for i in idx]), scenes=scenes, scene_id=idx,
+               weights=np.stack([g(names[i], "weights") for i in idx]))
+    obstacles = [SCRIPTS["roundabout" if names[i].startswith("roundabout") else "intersection"] for i in idx]
+    return inp, obstacles
+
+
+def arc_table_share(lens):
+    total, have = 0, 0
+    for n in lens:
+        need = int(n) * (int(n) + 1) // 2
+        if total + need <= ARC_CAP_DOUBLES:
+            total += need
+            have += 1
+    return have / max(len(lens), 1)
+
+
+def device_pipeline(planner, inp, obstacles, steps, T):
+    import torch
+    from junction_mpc.batched import BatchedMPC
+    from junction_mpc.episodes import BatchedEpisodes, scripted_obstacles
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    ev[0].record()
+    plans = planner.plan_device(**inp)
+    ev[1].record()
+    torch.cuda.synchronize()
+    t1 = time.perf_counter()
+    engine = BatchedMPC.from_plans(plans, T=T, max_N=1024, max_batch=len(plans))
+    torch.cuda.synchronize()
+    t2 = time.perf_counter()
+    ev[2].record()                              # ingestion alone, on the engine that exists now
+    engine.set_courses_from_plans(plans)
+    ev[3].record()
+    torch.cuda.synchronize()
+    t3 = time.perf_counter()
+    ep = BatchedEpisodes.from_plans(engine, plans, obstacle_program=scripted_obstacles(obstacles), frame_window=10,
+                                    max_steps=steps)
+    res = ep.run(max_steps=steps)
+    t4 = time.perf_counter()
+    stages = dict(plan_device_span_ms=ev[0].elapsed_time(ev[1]), plan_wall_ms=(t1 - t0) * 1e3,
+                  engine_create_and_ingest_wall_ms=(t2 - t1) * 1e3, ingest_wall_ms=(t3 - t2) * 1e3,
+                  ingest_device_span_ms=ev[2].elapsed_time(ev[3]), episodes_wall_ms=(t4 - t3) * 1e3,
+                  total_wall_ms=(t2 - t0 + t4 - t3) * 1e3, launches_engine=engine.launch_count)
+    lens = engine.course_len.copy()
+    stages["usable_courses"] = int(engine.course_ok.sum().item())
+    engine.close()
+    return stages, res, lens
+
+
+def host_pipeline(planner, inp, obstacles, steps, T, dl_margin):
+    import torch
+    from junction_mpc import synth
+    from junction_mpc.batched import BatchedMPC
+    from junction_mpc.config import PARAM_INDEX
+    from junction_mpc.episodes import BatchedEpisodes, scripted_obstacles
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    r = planner.plan(**inp)
+    t1 = time.perf_counter()
+    courses = r.courses()
+    for c in courses:
+        synth.smooth_yaw_inplace(c[:, 2])
+    dl = np.array([np.sqrt((c[0, 0] - c[1, 0]) ** 2 + (c[0, 1] - c[1, 1]) ** 2) for c in courses])
+    t2 = time.perf_counter()
+    engine = BatchedMPC(courses, dl=float(dl[0]), T=T, max_batch=len(courses))
+    t3 = time.perf_counter()
+    B = len(courses)
+    state0 = np.array([[c[0, 0], c[0, 1], 0.0, c[0, 2]] for c in courses])
+    params = np.repeat(engine.default_params[None, :], B, axis=0)
+    params[:, PARAM_INDEX["dl"]] = dl
+    ep = BatchedEpisodes(engine, state0, course_id=np.arange(B), obstacle_program=scripted_obstacles(obstacles),
+                         frame_window=10, margin=dl_margin, params=params, max_steps=steps)
+    res = ep.run(max_steps=steps)
+    t4 = time.perf_counter()
+    stages = dict(plan_kernel_ms=r.kernel_ms, plan_wall_ms=(t1 - t0) * 1e3, courses_and_smoothing_wall_ms=(t2 - t1) * 1e3,
+                  engine_create_and_upload_wall_ms=(t3 - t2) * 1e3, episodes_wall_ms=(t4 - t3) * 1e3,
+                  total_wall_ms=(t4 - t0) * 1e3, launches_engine=engine.launch_count)
+    engine.close()
+    return stages, res
+
+
+def plan_kernel_ms_profiled(planner, inp):
+    """Device time of the plan_kernel launches of one plan_device call, by torch.profiler in a call of its own."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        planner.plan_device(**inp)
+        torch.cuda.synchronize()
+    us = 0.0
+    for e in prof.key_averages():
+        if "plan_kernel" in e.key:
+            us += getattr(e, "device_time_total", None) or getattr(e, "cuda_time_total", 0.0)
+    return us / 1e3
+
+
+def episode_rates(res):
+    steps = int(res["steps"].sum())
+    return dict(episode_steps=steps, iterations=int(res["iterations"]), goal_reached=int((res["done"] == 1).sum()))
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--sizes", default="1024,4096,16384")
+    ap.add_argument("--steps", type=int, default=256)
+    ap.add_argument("--out", default=None)
+    a = ap.parse_args()
+    import torch
+    from junction_mpc import planner as P
+    z = load_planner_golden(os.path.join(ROOT, "tests", "golden"))
+    sizes = [int(s) for s in a.sizes.split(",")]
+    planner = P.BatchedPlanner(z["mp_points"], z["mp_total_length"], float(z["car_radius"]), z["car_circle_centers"],
+                               max_batch=max(sizes))
+    T, margin = 13, 72
+    gpu = dict(name=torch.cuda.get_device_name(0))
+    try:
+        gpu["power_limit"] = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
+                                            capture_output=True, text=True, timeout=30).stdout.strip()
+    except Exception as e:                       # noqa: BLE001
+        gpu["power_limit"] = f"unavailable ({e})"
+    out = dict(gpu=gpu, workload="recorded planner variants that find a course, replicated; scripted obstacles; T = 13; "
+               "plan() defaults max_expansions = 4096, max_path = 48", sizes={})
+    inp, obs = workload(z, 64)                   # warm-up: module loads, kernel attributes, both pipelines
+    device_pipeline(planner, inp, obs, 16, T)
+    host_pipeline(planner, inp, obs, 16, T, margin)
+    for B in sizes:
+        inp, obs = workload(z, B)
+        for _ in range(2):                      # the second pass is reported: buffers of this size already allocated
+            dev, dres, lens = device_pipeline(planner, inp, obs, a.steps, T)
+            host, hres = host_pipeline(planner, inp, obs, a.steps, T, margin)
+        dev["plan_kernel_ms"] = plan_kernel_ms_profiled(planner, inp)
+        same = all(np.array_equal(dres[k], hres[k], equal_nan=True) for k in ("steps", "done", "state", "history", "flags"))
+        for stages, res in ((dev, dres), (host, hres)):
+            stages.update(episode_rates(res))
+            stages["episode_steps_per_s"] = stages["episode_steps"] / (stages["episodes_wall_ms"] * 1e-3)
+            stages["episodes_per_s_end_to_end"] = B / (stages["total_wall_ms"] * 1e-3)
+        out["sizes"][str(B)] = dict(scenarios=B, device=dev, host=host, identical_episodes=bool(same),
+                                    arc_table_share=arc_table_share(lens),
+                                    speedup_total_wall=host["total_wall_ms"] / dev["total_wall_ms"])
+        print(B, json.dumps(out["sizes"][str(B)]), flush=True)
+    planner.close()
+    dest = a.out or os.getcwd()
+    os.makedirs(dest, exist_ok=True)
+    with open(os.path.join(dest, "plan_and_drive.json"), "w") as f:
+        json.dump(out, f, indent=1)
+
+
+if __name__ == "__main__":
+    main()
