@@ -48,6 +48,7 @@ struct jmpc_handle_s {
   double *d_ccfx = nullptr, *d_ccfy = nullptr, *d_ccrx = nullptr, *d_ccry = nullptr;   // collision-circle tables
   double* d_arc = nullptr; long long* d_arc_off = nullptr;                                // arc-length tables (collision kernel)
   bool arc_all = false;                                                                   // every uploaded course has a table
+  std::vector<int> arc_has;                                                               // per course: 1 = has a table (jmpc_get_arc_tables)
   double off_front = 2.86 / 2 + (3.5 / 2 - 1.0), off_rear = 2.86 / 2 - (3.5 / 2 - 1.0), radius = 2.0 / 1.4142135623730951;
   int* d_course_n = nullptr;
   int n_courses = 0, course_stride = 0;
@@ -261,13 +262,14 @@ int place_arc_tables(jmpc_handle h, std::vector<long long>& off) {
   if (h->d_arc) { cudaFree(h->d_arc); h->d_arc = nullptr; }
   if (!h->d_arc_off) CK(cudaMalloc(&h->d_arc_off, (size_t)h->max_courses * sizeof(long long)));
   off.assign(h->n_courses, -1);
+  h->arc_has.assign(h->n_courses, 0);
   long long total = 0;
   h->arc_all = true;
   const long long cap = (256ll << 20) / (long long)sizeof(double);
   for (int c = 0; c < h->n_courses; ++c) {
     const long long n = h->course_n[c], need = n * (n + 1) / 2;
     if (total + need > cap) { h->arc_all = false; continue; }
-    off[c] = total; total += need;
+    off[c] = total; total += need; h->arc_has[c] = 1;
   }
   if (total > 0) CK(cudaMalloc(&h->d_arc, (size_t)total * sizeof(double)));
   return 0;
@@ -845,17 +847,21 @@ int32_t jmpc_collision(jmpc_handle h, int32_t B, const int32_t* course_id, const
   a.horizon_s = horizon_s; a.params = params;
   memcpy(a.defaults.v, h->defaults, sizeof h->defaults);
   a.flag = flag; a.course_len_out = course_len_out; a.skip = h->skip;
-  const int wpb = 4;
-  const int blocks = (B + wpb - 1) / wpb;
   // with a table for every course the kernel needs no shared memory for the arc scan: 5 KB per warp instead of 12.6 KB
   // at max_N = 960 and two obstacles, i.e. more than twice the resident warps of this latency-bound kernel
   a.arc_smem = (a.arc_tab && h->arc_all) ? 0 : h->max_N;
-  const size_t smem = wpb * jmpc::collision_warp_smem_bytes(a.arc_smem, n_obs);
+  // 4 warps per block unless a long course's arc scan does not leave room for them: then 2, or 1 (jmpc.h states the
+  // resulting max_N limit).  The warps of a block share nothing, so the results do not depend on the count.
+  const size_t smem_cap = 200 * 1024, warp_smem = jmpc::collision_warp_smem_bytes(a.arc_smem, n_obs);
+  if (warp_smem > smem_cap) return fail("jmpc_collision: course too long for the shared-memory arc scan");
+  int wpb = 4;
+  while (wpb > 1 && wpb * warp_smem > smem_cap) wpb >>= 1;
+  const int blocks = (B + wpb - 1) / wpb;
+  const size_t smem = wpb * warp_smem;
   if (!h->collision_attr_set) {             // per handle: function attributes are per device
-    CK(cudaFuncSetAttribute(jmpc::collision_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    CK(cudaFuncSetAttribute(jmpc::collision_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_cap));
     h->collision_attr_set = true;
   }
-  if (smem > 200 * 1024) return fail("jmpc_collision: course too long for the shared-memory arc scan");
   jmpc::collision_kernel<<<blocks, wpb * 32, smem, (cudaStream_t)stream>>>(a);
   CK(cudaGetLastError());
   h->launches++;
@@ -1362,6 +1368,13 @@ int32_t jmpc_get_courses(jmpc_handle h, int32_t first, int32_t n, int32_t stride
     const size_t o = (size_t)k * stride + len[k], cnt = (size_t)stride - len[k];
     memset(cx + o, 0, cnt * 8); memset(cy + o, 0, cnt * 8); memset(cyaw + o, 0, cnt * 8);
   }
+  return 0;
+}
+
+int32_t jmpc_get_arc_tables(jmpc_handle h, int32_t first, int32_t n, int32_t* has_table) {
+  if (!h || !has_table) return fail("jmpc_get_arc_tables: NULL argument");
+  if (first < 0 || n < 0 || first + n > h->n_courses) return fail("jmpc_get_arc_tables: course range out of range");
+  for (int k = 0; k < n; ++k) has_table[k] = h->arc_has[first + k];
   return 0;
 }
 

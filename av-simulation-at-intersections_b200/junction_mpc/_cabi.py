@@ -71,6 +71,7 @@ SIGNATURES = {
     "jmpc_plan": (C.c_int32, [C.c_void_p, C.c_int32] + [C.c_void_p] * 16),
     "jmpc_set_courses_device": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32] + [C.c_void_p] * 6),
     "jmpc_get_courses": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 4),
+    "jmpc_get_arc_tables": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
     "jmpc_episode_init_from_courses": (C.c_int32, [C.c_void_p, C.c_int32] + [C.c_void_p] * 7),
     "jmpc_launch_count": (C.c_int64, [C.c_void_p]),
     "jmpc_measure_fma_peak": (C.c_int32, [C.c_void_p, c_f64p, c_f64p]),

@@ -144,6 +144,14 @@ class BatchedMPC:
                                                _ptr(tab[2])), "jmpc_get_courses")
         return [np.ascontiguousarray(tab[:, k, :lens[k]].T) for k in range(n)]
 
+    def arc_table_flags(self, first: int = 0, n: Optional[int] = None) -> np.ndarray:
+        """bool [n]: which of the uploaded courses first .. first + n - 1 got an arc-length table (jmpc_get_arc_tables);
+        the collision kernel sums the arc lengths of the others on the fly."""
+        n = len(self.course_len) - first if n is None else int(n)
+        has = np.zeros(n, np.int32)
+        _cabi.check(self._lib.jmpc_get_arc_tables(self._h, int(first), n, _ptr(has)), "jmpc_get_arc_tables")
+        return has != 0
+
     # ---- configuration ----------------------------------------------------------------------------------
     def set_courses(self, courses: Sequence[np.ndarray]):
         lens = _i32([len(c) for c in courses])

@@ -216,7 +216,12 @@ int32_t jmpc_host_free(jmpc_handle h, void* p);
  *   obstacles [B][n_obs][6];  frame_window: FRAME_WINDOW;  margin: EXTRA_CUTOFF_MARGIN (in course points)
  *   flag [B]: 1 when a collision is predicted;  course_len_out [B]: effective course length to feed
  *   jmpc_step (full length when flag == 0).  flag = -1 (full length) reports an instance outside the kernel's table
- *   sizes: more than 160 kept ego points or more than 71 obstacle prediction steps (the reference's scenes: 49 / 35). */
+ *   sizes: more than 160 kept ego points or more than 71 obstacle prediction steps (the reference's scenes: 49 / 35).
+ * params [B][JMPC_NPARAM] or NULL: dt, L, max_accel and sim_max_speed are read per instance.
+ * Arc lengths: a course with an arc-length table (jmpc_get_arc_tables) reads them from it; the others are summed on the
+ * fly in shared memory, max_N doubles per warp.  Then the kernel runs 4, 2 or 1 warps per block, the most whose
+ * (max_N + 288 n_obs + 32) * 8 + 320 bytes each fit in 200 KB, and the call fails when one warp does not fit:
+ * max_N <= 25528 - 288 n_obs (23224 at 8 obstacles) whenever some uploaded course lacks a table. */
 int32_t jmpc_collision(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* agent_idx,
                        const double* v, const double* obstacles, int32_t n_obs, int32_t frame_window,
                        int32_t margin, double horizon_s, const double* params, int32_t* flag,
@@ -248,7 +253,9 @@ int32_t jmpc_plant_step(jmpc_handle h, int32_t B, double* state, const double* a
  *                      flags_base[i] ([rows][B]), t = (i + 1) * dt_loop.  With jmpc_counter_add (*counter += delta,
  *                      one thread) closing the iteration, the whole loop body has no per-iteration host argument and
  *                      can be captured once as a CUDA graph and replayed.
- *   jmpc_obstacle_step: constant-input motion of obstacles [B][n_obs][6] (moving_obstacles_prediction.py:21-29). */
+ *   jmpc_obstacle_step: constant-input motion of obstacles [B][n_obs][6] (moving_obstacles_prediction.py:21-29), with
+ *                      one `dt` for the whole batch: a params row's dt reaches the collision prediction and the plant,
+ *                      not this step. */
 int32_t jmpc_episode_pre(jmpc_handle h, int32_t B, const double* state, const int32_t* course_id,
                          const int32_t* course_len, const int32_t* target_ind, const int32_t* steps,
                          int32_t* agent_idx, int32_t* done, double goal_dis, double stop_speed, void* stream);
@@ -376,6 +383,12 @@ int32_t jmpc_set_courses_device(jmpc_handle h, int32_t n_courses, int32_t traj_s
  * that want to keep what was planned and smoothed. */
 int32_t jmpc_get_courses(jmpc_handle h, int32_t first, int32_t n, int32_t stride, int32_t* len, double* cx, double* cy,
                          double* cyaw);
+
+/* Which courses first .. first + n - 1 got an arc-length table (HOST pointer): has_table [n], 1 = table, 0 = the
+ * collision kernel sums the arc lengths on the fly.  A course of N points needs N (N + 1) / 2 doubles; the uploads
+ * (jmpc_set_courses, jmpc_set_courses_device) place them in course order while they fit in 256 MB, skipping a course
+ * that does not fit.  Both paths give bit-identical results; the table saves the collision kernel a sequential sum. */
+int32_t jmpc_get_arc_tables(jmpc_handle h, int32_t first, int32_t n, int32_t* has_table);
 
 /* Episode start on the ingested courses (DEVICE pointers), the reference's State(x=trajectory_full[0, 0],
  * y=trajectory_full[0, 1], yaw=trajectory_full[0, 2], v=0) of mpc_intersection.py:76-79 after the smoothing:

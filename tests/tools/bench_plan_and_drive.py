@@ -36,7 +36,6 @@ SCRIPTS = {
     "roundabout": [dict(kind="roundabout", direction=1, offset=1., turning=True, speed=25 / 3.6, dt=0.2),
                    dict(kind="roundabout", direction=-1, offset=4., turning=True, speed=25 / 3.6, dt=0.2)],
 }
-ARC_CAP_DOUBLES = (256 << 20) // 8      # the handle's arc-table budget (jmpc.cu: place_arc_tables)
 
 
 def workload(z, B):
@@ -50,16 +49,6 @@ def workload(z, B):
                weights=np.stack([g(names[i], "weights") for i in idx]))
     obstacles = [SCRIPTS["roundabout" if names[i].startswith("roundabout") else "intersection"] for i in idx]
     return inp, obstacles
-
-
-def arc_table_share(lens):
-    total, have = 0, 0
-    for n in lens:
-        need = int(n) * (int(n) + 1) // 2
-        if total + need <= ARC_CAP_DOUBLES:
-            total += need
-            have += 1
-    return have / max(len(lens), 1)
 
 
 def device_pipeline(planner, inp, obstacles, steps, T):
@@ -90,10 +79,10 @@ def device_pipeline(planner, inp, obstacles, steps, T):
                   engine_create_and_ingest_wall_ms=(t2 - t1) * 1e3, ingest_wall_ms=(t3 - t2) * 1e3,
                   ingest_device_span_ms=ev[2].elapsed_time(ev[3]), episodes_wall_ms=(t4 - t3) * 1e3,
                   total_wall_ms=(t2 - t0 + t4 - t3) * 1e3, launches_engine=engine.launch_count)
-    lens = engine.course_len.copy()
+    has_table = engine.arc_table_flags()
     stages["usable_courses"] = int(engine.course_ok.sum().item())
     engine.close()
-    return stages, res, lens
+    return stages, res, has_table
 
 
 def host_pipeline(planner, inp, obstacles, steps, T, dl_margin):
@@ -174,7 +163,7 @@ def main():
     for B in sizes:
         inp, obs = workload(z, B)
         for _ in range(2):                      # the second pass is reported: buffers of this size already allocated
-            dev, dres, lens = device_pipeline(planner, inp, obs, a.steps, T)
+            dev, dres, has_table = device_pipeline(planner, inp, obs, a.steps, T)
             host, hres = host_pipeline(planner, inp, obs, a.steps, T, margin)
         dev["plan_kernel_ms"] = plan_kernel_ms_profiled(planner, inp)
         same = all(np.array_equal(dres[k], hres[k], equal_nan=True) for k in ("steps", "done", "state", "history", "flags"))
@@ -183,7 +172,7 @@ def main():
             stages["episode_steps_per_s"] = stages["episode_steps"] / (stages["episodes_wall_ms"] * 1e-3)
             stages["episodes_per_s_end_to_end"] = B / (stages["total_wall_ms"] * 1e-3)
         out["sizes"][str(B)] = dict(scenarios=B, device=dev, host=host, identical_episodes=bool(same),
-                                    arc_table_share=arc_table_share(lens),
+                                    arc_table_share=float(has_table.mean()),
                                     speedup_total_wall=host["total_wall_ms"] / dev["total_wall_ms"])
         print(B, json.dumps(out["sizes"][str(B)]), flush=True)
     planner.close()
