@@ -1033,6 +1033,38 @@ int32_t jmpc_counter_add(jmpc_handle h, int32_t* counter, int32_t delta, void* s
   return 0;
 }
 
+int32_t jmpc_episode_outcomes(jmpc_handle h, int32_t B, const double* state, const int32_t* course_id,
+                              const double* obstacles, int32_t n_obs, const double* record, const double* di,
+                              const int32_t* flag, const double* params, const int32_t* done, const int32_t* iter_dev,
+                              int32_t initial, double* outcomes, double* obstacle_history, int32_t history_rows,
+                              void* stream) {
+  if (!h) return fail("jmpc_episode_outcomes: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_episode_outcomes: B out of range");
+  if (n_obs < 0 || n_obs > jmpc::kMaxObstacles) return fail("jmpc_episode_outcomes: n_obs out of range");
+  if (history_rows < 0) return fail("jmpc_episode_outcomes: negative history_rows");
+  if (!state || !done || !outcomes) return fail("jmpc_episode_outcomes: NULL array");
+  if (n_obs > 0 && !obstacles) return fail("jmpc_episode_outcomes: obstacles is NULL");
+  if (!initial) {
+    if (!record || !di || !iter_dev) return fail("jmpc_episode_outcomes: NULL step array");
+    if (h->n_courses < 1) return fail("jmpc_episode_outcomes: no courses uploaded (jmpc_set_courses)");
+  }
+  if (B == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::OutcomeArgs a;
+  memset(&a, 0, sizeof a);
+  a.B = B; a.n_obs = n_obs; a.initial = initial ? 1 : 0; a.history_rows = history_rows;
+  a.cx = h->d_cx; a.cy = h->d_cy; a.cyaw = h->d_cyaw; a.course_stride = h->course_stride; a.course_id = course_id;
+  a.params = params;
+  memcpy(a.defaults.v, h->defaults, sizeof h->defaults);
+  a.off_front = h->off_front; a.off_rear = h->off_rear; a.radius = h->radius;
+  a.state = state; a.obstacles = obstacles; a.record = record; a.di = di; a.flag = flag; a.done = done;
+  a.iter_dev = iter_dev; a.outcomes = outcomes; a.obstacle_history = obstacle_history;
+  jmpc::episode_outcome_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(a);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
 int32_t jmpc_obstacle_step(jmpc_handle h, int32_t B, int32_t n_obs, double* obstacles, const int32_t* done,
                            double dt, void* stream) {
   if (!h) return fail("jmpc_obstacle_step: NULL handle");

@@ -85,6 +85,30 @@ __global__ void __launch_bounds__(128) episode_pre_kernel(const EpisodeArgs A) {
   if (lane == 0) A.agent_idx[b] = a0;
 }
 
+// ---- per-step arithmetic shared by episode_post_kernel and episode_outcome_kernel ---------------------------------
+// Applied controls of a step: any status but OPTIMAL is a failed solve, the previous steer `di` is kept and the ego
+// brakes with MAX_DECEL (mpc.py:298-301); that includes JMPC_MAX_ITER, whose record carries no controls.
+__device__ __forceinline__ bool applied_controls(const double* rec, const double* prm, double di, double& delta,
+                                                 double& acc) {
+  const bool ok = (int)rec[3] == JMPC_OPTIMAL;
+  delta = ok ? rec[0] : di;
+  acc = ok ? rec[1] : prm[JMPC_P_MAX_DECEL];
+  return ok;
+}
+// get_current_xref_deviation (mpc.py:305-312) at the course point `at`; (x, y) = ox[0], oy[0], the current position
+__device__ __forceinline__ double xref_deviation(const double* cx, const double* cy, const double* cyaw, size_t at,
+                                                 double x, double y) {
+  const double ang = cyaw[at] + M_PI / 2;
+  const double ex = cx[at] - x, ey = cy[at] - y;
+  const double px = cos(ang) * ex, py = sin(ang) * ey;
+  return sqrt(__dadd_rn(__dmul_rn(px, px), __dmul_rn(py, py)));
+}
+// the steer the plant applies and its yaw rate (simulation.py:38-43)
+__device__ __forceinline__ double clamped_steer(double delta, double max_steer) {
+  return fmax(fmin(delta, max_steer), -max_steer);
+}
+__device__ __forceinline__ double yaw_rate(double v, double L, double steer) { return __dmul_rn(v / L, tan(steer)); }
+
 // One thread per episode: controls from the step's record, xref deviation, plant step, history, counters.
 __global__ void episode_post_kernel(const EpisodeArgs A) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -108,24 +132,15 @@ __global__ void episode_post_kernel(const EpisodeArgs A) {
   double x = A.state[4 * b], y = A.state[4 * b + 1], v = A.state[4 * b + 2], yaw = A.state[4 * b + 3];
   const int target = (int)rec[4];
   A.target_ind[b] = target;
-  double delta = A.di[b], acc = prm[JMPC_P_MAX_DECEL];
-  double dev = nan("");
-  // any status but OPTIMAL is a failed solve: the previous steer is kept and the ego brakes with MAX_DECEL
-  // (mpc.py:298-301); that includes JMPC_MAX_ITER, whose record carries no controls
-  if (status == JMPC_OPTIMAL) {
-    delta = rec[0]; acc = rec[1];
-    // get_current_xref_deviation (mpc.py:305-312); ox[0], oy[0] are the current position
-    const double ang = A.cyaw[coff + target] + M_PI / 2;
-    const double ex = A.cx[coff + target] - x, ey = A.cy[coff + target] - y;
-    const double px = cos(ang) * ex, py = sin(ang) * ey;
-    dev = sqrt(__dadd_rn(__dmul_rn(px, px), __dmul_rn(py, py)));
-  }
+  double delta, acc;
+  const bool ok = applied_controls(rec, prm, A.di[b], delta, acc);
+  const double dev = ok ? xref_deviation(A.cx, A.cy, A.cyaw, coff + target, x, y) : nan("");
   A.di[b] = delta;
-  if (A.warm) A.warm[b] = (status == JMPC_OPTIMAL) ? 1 : 0;
+  if (A.warm) A.warm[b] = ok ? 1 : 0;
   // Simulation.step (simulation.py:35-47)
-  const double dt = prm[JMPC_P_DT], L = prm[JMPC_P_L], ms = prm[JMPC_P_MAX_STEER];
-  const double dcl = fmax(fmin(delta, ms), -ms);
-  const double xd = __dmul_rn(v, cos(yaw)), yd = __dmul_rn(v, sin(yaw)), td = __dmul_rn(v / L, tan(dcl));
+  const double dt = prm[JMPC_P_DT], L = prm[JMPC_P_L];
+  const double dcl = clamped_steer(delta, prm[JMPC_P_MAX_STEER]);
+  const double xd = __dmul_rn(v, cos(yaw)), yd = __dmul_rn(v, sin(yaw)), td = yaw_rate(v, L, dcl);
   x = __dadd_rn(x, __dmul_rn(xd, dt));
   y = __dadd_rn(y, __dmul_rn(yd, dt));
   yaw = __dadd_rn(yaw, __dmul_rn(td, dt));
@@ -141,6 +156,118 @@ __global__ void episode_post_kernel(const EpisodeArgs A) {
 }
 
 __global__ void counter_add_kernel(int* counter, int delta) { *counter += delta; }
+
+// ---- per-episode outcome record (enum jmpc_outcome) ----------------------------------------------------------------
+// private running state after the public columns
+enum { kOutPrevX = JMPC_NOUTCOME, kOutPrevY, kOutPrevV, kOutPrevA, kOutPrevSteer, kOutSteps, kOutEnd };
+static_assert(kOutEnd == JMPC_OUTCOME_LEN, "JMPC_OUTCOME_LEN must cover the private columns");
+
+struct OutcomeArgs {
+  int B, n_obs, initial, history_rows;
+  const double* cx; const double* cy; const double* cyaw; int course_stride;
+  const int* course_id;
+  const double* params; ParamBlock defaults;
+  double off_front, off_rear, radius;       // jmpc_set_car_geometry, as the collision kernel uses it
+  const double* state;                      // [B][4] after this iteration's plant step
+  const double* obstacles;                  // [B][n_obs][6] poses of the same instant
+  const double* record; const double* di; const int* flag; const int* done; const int* iter_dev;
+  double* outcomes;                         // [B][JMPC_OUTCOME_LEN]
+  double* obstacle_history;                 // [history_rows + 1][B][n_obs][6] or nullptr
+};
+
+// One thread per episode, once before the first loop iteration (initial: evaluation 0) and once per iteration after
+// the obstacles have advanced (evaluation i + 1).  At most kMaxObstacles x 4 circle pairs per evaluation.
+__global__ void episode_outcome_kernel(const OutcomeArgs A) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= A.B) return;
+  double* out = A.outcomes + (size_t)b * JMPC_OUTCOME_LEN;
+  const double x = A.state[4 * b], y = A.state[4 * b + 1], v = A.state[4 * b + 2], yaw = A.state[4 * b + 3];
+  int e = 0;
+  if (A.initial) {
+    out[JMPC_O_MIN_CLEARANCE] = INFINITY;
+    for (int c = JMPC_O_MIN_CLEARANCE_EVAL; c <= JMPC_O_FIRST_CONTACT_OBS; ++c) out[c] = -1.0;
+    for (int c = JMPC_O_CONTACT_EVALS; c < JMPC_NOUTCOME; ++c) out[c] = 0.0;
+    out[kOutPrevA] = 0.0; out[kOutPrevSteer] = 0.0; out[kOutSteps] = 0.0;
+    if (A.done[b]) return;
+  } else {
+    if (A.done[b]) return;                  // no step executed in this iteration (goal, index rule) or earlier
+    e = *A.iter_dev + 1;
+    // the step just executed, recomputed as episode_post_kernel computed it
+    const double* prm = A.params ? A.params + (size_t)b * JMPC_NPARAM : A.defaults.v;
+    const double* rec = A.record + (size_t)b * JMPC_RECORD_LEN;
+    const double px = out[kOutPrevX], py = out[kOutPrevY], pv = out[kOutPrevV];
+    double delta, acc;
+    const bool ok = applied_controls(rec, prm, A.di[b], delta, acc);
+    const double dt = prm[JMPC_P_DT];
+    const double steer = clamped_steer(delta, prm[JMPC_P_MAX_STEER]);
+    const double lat = __dmul_rn(pv, yaw_rate(pv, prm[JMPC_P_L], steer));
+    const int f = A.flag ? A.flag[b] : 0;
+    if (f == 1) out[JMPC_O_CUT_STEPS] += 1.0;
+    if (f == -1) out[JMPC_O_LIMIT_STEPS] += 1.0;
+    if (!ok) out[JMPC_O_FAILED_SOLVES] += 1.0;
+    if (ok) {
+      const int cid = A.course_id ? A.course_id[b] : 0;
+      const double dev = xref_deviation(A.cx, A.cy, A.cyaw, (size_t)cid * A.course_stride + (int)rec[4], px, py);
+      if (isfinite(dev)) {
+        out[JMPC_O_MAX_XREF_DEV] = fmax(out[JMPC_O_MAX_XREF_DEV], dev);
+        out[JMPC_O_SUM_XREF_DEV] = __dadd_rn(out[JMPC_O_SUM_XREF_DEV], dev);
+      }
+    }
+    out[JMPC_O_MAX_ABS_ACCEL] = fmax(out[JMPC_O_MAX_ABS_ACCEL], fabs(acc));
+    out[JMPC_O_MAX_ABS_LAT_ACCEL] = fmax(out[JMPC_O_MAX_ABS_LAT_ACCEL], fabs(lat));
+    if (out[kOutSteps] > 0.0) {
+      out[JMPC_O_MAX_ABS_JERK] = fmax(out[JMPC_O_MAX_ABS_JERK], fabs((acc - out[kOutPrevA]) / dt));
+      out[JMPC_O_MAX_ABS_STEER_RATE] = fmax(out[JMPC_O_MAX_ABS_STEER_RATE], fabs((steer - out[kOutPrevSteer]) / dt));
+    }
+    out[JMPC_O_DISTANCE] = __dadd_rn(out[JMPC_O_DISTANCE], hypot(x - px, y - py));
+    out[kOutPrevA] = acc; out[kOutPrevSteer] = steer; out[kOutSteps] += 1.0;
+  }
+  out[kOutPrevX] = x; out[kOutPrevY] = y; out[kOutPrevV] = v;
+
+  // evaluation e: the ego's circles against every obstacle's, same centres as the collision kernel
+  double s, c;
+  sincos(yaw, &s, &c);
+  double ex[2], ey[2];
+  circle_centre(x, y, c, s, A.off_front, ex[0], ey[0]);
+  circle_centre(x, y, c, s, A.off_rear, ex[1], ey[1]);
+  const double reach = 2.0 * A.radius;
+  double best = out[JMPC_O_MIN_CLEARANCE];
+  int best_obs = -1, contact_obs = -1;
+  double* track = (A.obstacle_history && e <= A.history_rows)
+                      ? A.obstacle_history + ((size_t)e * A.B + b) * A.n_obs * 6 : nullptr;
+  for (int k = 0; k < A.n_obs; ++k) {
+    const double* o = A.obstacles + ((size_t)b * A.n_obs + k) * 6;
+    if (track)
+      for (int j = 0; j < 6; ++j) track[6 * k + j] = o[j];
+    sincos(o[3], &s, &c);
+    double ox[2], oy[2];
+    circle_centre(o[0], o[1], c, s, A.off_front, ox[0], oy[0]);
+    circle_centre(o[0], o[1], c, s, A.off_rear, ox[1], oy[1]);
+    double clear = INFINITY;
+    bool touch = false;
+#pragma unroll
+    for (int p = 0; p < 4; ++p) {
+      const double dx = ex[p >> 1] - ox[p & 1], dy = ey[p >> 1] - oy[p & 1];
+      const double d = sqrt(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
+      clear = fmin(clear, d - reach);
+      touch |= d <= reach;
+    }
+    if (clear < best) { best = clear; best_obs = k; }
+    if (touch && contact_obs < 0) contact_obs = k;
+  }
+  if (best_obs >= 0) {
+    out[JMPC_O_MIN_CLEARANCE] = best;
+    out[JMPC_O_MIN_CLEARANCE_EVAL] = (double)e;
+    out[JMPC_O_MIN_CLEARANCE_OBS] = (double)best_obs;
+  }
+  if (contact_obs >= 0) {
+    out[JMPC_O_CONTACT_EVALS] += 1.0;
+    if (out[JMPC_O_FIRST_CONTACT_EVAL] < 0.0) {
+      out[JMPC_O_FIRST_CONTACT_EVAL] = (double)e;
+      out[JMPC_O_FIRST_CONTACT_OBS] = (double)contact_obs;
+    }
+  }
+}
 
 // Constant-input obstacle motion, one thread per obstacle: obstacles [B][n_obs][6] = x, y, v, yaw, a, steer.
 __global__ void obstacle_step_kernel(int count, double* __restrict__ obs, const int* __restrict__ done, int n_obs,

@@ -60,6 +60,8 @@ SIGNATURES = {
     "jmpc_episode_post_dev": (C.c_int32, [C.c_void_p, C.c_int32] + [C.c_void_p] * 10 + [C.c_int32, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_double, C.c_void_p]),
     "jmpc_counter_add": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "jmpc_episode_outcomes": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]
+                              + [C.c_void_p] * 6 + [C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "jmpc_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]),
     "jmpc_scripted_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                                 C.c_void_p, C.c_int32, C.c_void_p]),

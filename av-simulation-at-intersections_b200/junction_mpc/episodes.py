@@ -5,7 +5,8 @@ goal test -> ego index on the full course -> collision flag / cut -> MPC step ->
 Everything runs in libjmpc.so kernels on torch-owned device tensors; the host only sequences launches and looks
 at the `done` flags every few iterations.  Obstacles are the reference's scripted vehicles stepped on the device
 (`obstacle_program`, see `scripted_obstacles`), constant-input vehicles advanced on the device (`obstacles`), or a
-per-step recording (`obstacle_script`).
+per-step recording (`obstacle_script`).  With `outcomes=True` every episode also keeps a compact outcome record on
+the device (contact, clearance, comfort; enum jmpc_outcome in include/jmpc.h), so that a study needs no History.
 """
 from __future__ import annotations
 
@@ -21,6 +22,34 @@ from .config import NPARAM
 
 
 OBS_KINDS = {"constant": 0, "t_intersection": 1, "roundabout": 2, "arterial": 3}
+
+# public columns of the outcome record, in the order of enum jmpc_outcome (include/jmpc.h)
+OUTCOME_NAMES = ("min_clearance", "min_clearance_eval", "min_clearance_obs", "first_contact_eval", "first_contact_obs",
+                 "contact_evals", "cut_steps", "limit_steps", "failed_solves", "max_abs_accel", "max_abs_jerk",
+                 "max_abs_steer_rate", "max_abs_lat_accel", "max_xref_dev", "sum_xref_dev", "distance")
+OUTCOME_INT = frozenset(OUTCOME_NAMES[1:9])          # evaluation / obstacle indices and counts
+OUTCOME_LEN = 22                                     # JMPC_OUTCOME_LEN: the public columns, then private running state
+MAX_OBSTACLES = 8                                    # kMaxObstacles of the collision and outcome kernels
+
+
+def outcome_setup(outcomes: bool, record_obstacles: bool, n_obs: int) -> bool:
+    """Host-side checks of the outcome options of `BatchedEpisodes`: returns whether the outcome kernel runs.
+    The obstacle tracks are written by the outcome kernel, so `record_obstacles` needs `outcomes`."""
+    if record_obstacles and not outcomes:
+        raise ValueError("record_obstacles=True needs outcomes=True")
+    if outcomes and not 0 <= n_obs <= MAX_OBSTACLES:
+        raise ValueError(f"outcomes support at most {MAX_OBSTACLES} obstacles per episode, got {n_obs}")
+    return bool(outcomes)
+
+
+def outcome_columns(record) -> dict:
+    """[B, >= len(OUTCOME_NAMES)] float64 outcome records -> dict of [B] arrays keyed by OUTCOME_NAMES (the index and
+    count columns as int64)."""
+    record = np.asarray(record, dtype=np.float64)
+    if record.ndim != 2 or record.shape[1] < len(OUTCOME_NAMES):
+        raise ValueError(f"outcome records must be [B, >= {len(OUTCOME_NAMES)}]")
+    return {n: (record[:, k].astype(np.int64) if n in OUTCOME_INT else record[:, k].copy())
+            for k, n in enumerate(OUTCOME_NAMES)}
 
 
 def scripted_obstacles(specs, L: float = 2.86):
@@ -78,14 +107,15 @@ class BatchedEpisodes:
     @classmethod
     def from_plans(cls, engine: BatchedMPC, plans, plan_id=None, params=None, obstacle_program=None, obstacles=None,
                    frame_window: int = 10, max_steps: int = 256, record_history: bool = True, horizon_s: float = 7.0,
-                   obstacle_script=None) -> "BatchedEpisodes":
+                   obstacle_script=None, outcomes: bool = False, record_obstacles: bool = False) -> "BatchedEpisodes":
         """Episodes on the planned courses of `engine` (filled by `BatchedMPC.from_plans(plans)` /
         `set_courses_from_plans(plans)`), the second half of main/scenarios/mpc_intersection.py:63-163 for a batch:
         episode b drives plan `plan_id[b]` (default: one episode per plan; zeros = one course, many controllers).
         Its start state (the course's first pose at v = 0), its params row `dl` and done = 3 for a plan without a usable
         course are written on the device (jmpc_episode_init_from_courses); such episodes are never stepped.
         `params` [B, NPARAM] (default: the engine's defaults) supplies every other parameter row.  `run()` adds
-        plan_status, plan_cost and expansions per episode."""
+        plan_status, plan_cost and expansions per episode.  `outcomes` / `record_obstacles` as in `__init__`; evaluation
+        0 of the outcome record sees the planned start states."""
         if engine.course_ok is None or len(engine.course_ok) != len(plans):
             raise ValueError("the engine's courses do not come from these plans (BatchedMPC.from_plans)")
         import torch
@@ -97,7 +127,8 @@ class BatchedEpisodes:
             raise ValueError(f"params must be [{B}, {NPARAM}]")
         ep = cls(engine, np.zeros((B, 4)), course_id=pid, obstacles=obstacles, obstacle_script=obstacle_script,
                  frame_window=frame_window, margin=margin, params=params, max_steps=max_steps,
-                 record_history=record_history, horizon_s=horizon_s, obstacle_program=obstacle_program)
+                 record_history=record_history, horizon_s=horizon_s, obstacle_program=obstacle_program,
+                 outcomes=outcomes, record_obstacles=record_obstacles)
         stream = C.c_void_p(torch.cuda.current_stream(engine.device).cuda_stream)
         _cabi.check(engine._lib.jmpc_episode_init_from_courses(
             engine._h, B, ep._p(ep.course_id), ep._p(engine.course_ok), ep._p(engine.course_dl), ep._p(ep.state),
@@ -107,7 +138,13 @@ class BatchedEpisodes:
 
     def __init__(self, engine: BatchedMPC, state0, course_id=None, obstacles=None, obstacle_script=None,
                  frame_window: int = 10, margin: int = 72, params=None, max_steps: int = 256,
-                 record_history: bool = True, horizon_s: float = 7.0, obstacle_program=None):
+                 record_history: bool = True, horizon_s: float = 7.0, obstacle_program=None, outcomes: bool = False,
+                 record_obstacles: bool = False):
+        """outcomes: keep one outcome record per episode on the device (jmpc_episode_outcomes): contact and clearance
+        against the obstacles, cut / limit steps, failed solves, comfort and tracking columns; `run()` returns it as
+        `outcomes`.  It observes only: the episodes are exactly those of outcomes=False.  record_obstacles (needs
+        outcomes): also keep the obstacle poses of every evaluation, `run()`'s `obstacle_history`
+        [iterations + 1, B, n_obs, 6], whose row i + 1 is simultaneous with History row i."""
         import torch
         self.torch = torch
         self.e = engine
@@ -146,6 +183,19 @@ class BatchedEpisodes:
         self.iteration = 0
         self.iter_dev = torch.zeros(1, dtype=i32, device=self.dev)     # the same counter on the device (graph replay)
         self._plans = None                                           # (DevicePlanBatch, plan index per episode): from_plans
+        n_obs = 0
+        if self.obstacles is not None:
+            n_obs = int(self.obstacles.shape[1])
+        elif self.script is not None:
+            n_obs = int(self.script.shape[2])
+        self.n_obs = n_obs
+        self.outcomes = self.obstacle_history = None
+        if outcome_setup(outcomes, record_obstacles, n_obs):
+            self.outcomes = torch.empty(B, OUTCOME_LEN, dtype=f64, device=self.dev)     # evaluation 0 fills it
+            if record_obstacles:
+                self.obstacle_history = torch.full((self.max_steps + 1, B, n_obs, 6), float("nan"), dtype=f64,
+                                                   device=self.dev)
+        self._outcomes_started = False
         if self.program is not None:                                 # get() before the first iteration
             self._scripted_step(advance=0)
 
@@ -156,6 +206,26 @@ class BatchedEpisodes:
             e._h, self.B, int(self.program[0].shape[1]), self._p(self.program[0]), self._p(self.program[1]),
             self._p(self.obstacles), self._p(self.done), int(advance), stream), "jmpc_scripted_obstacle_step")
 
+    def _outcome_eval(self, obs, initial: int):
+        """Evaluation 0 (initial) or i + 1 of the outcome record; obs: the obstacle poses of that instant."""
+        e, torch = self.e, self.torch
+        stream = C.c_void_p(torch.cuda.current_stream(e.device).cuda_stream)
+        has_obs = obs is not None and self.n_obs > 0
+        _cabi.check(e._lib.jmpc_episode_outcomes(
+            e._h, self.B, self._p(self.state), self._p(self.course_id), self._p(obs) if has_obs else None,
+            self.n_obs if has_obs else 0, self._p(self.out.record), self._p(self.di),
+            self._p(self.flag) if has_obs else None, self._p(self.params), self._p(self.done), self._p(self.iter_dev),
+            int(initial), self._p(self.outcomes), self._p(self.obstacle_history), self.max_steps, stream),
+            "jmpc_episode_outcomes")
+
+    def _start_outcomes(self):
+        """Evaluation 0, launched once before the first iteration: after __init__ / from_plans wrote the start states."""
+        if self.outcomes is None or self._outcomes_started:
+            return
+        obs = self.obstacles if self.script is None else self.script[0]
+        self._outcome_eval(obs, initial=1)
+        self._outcomes_started = True
+
     def _p(self, ten):
         return None if ten is None else C.c_void_p(ten.data_ptr())
 
@@ -163,6 +233,7 @@ class BatchedEpisodes:
         """One loop iteration for every episode that is not done.  The engine-wide skip mask (finished episodes cost
         nothing in the step / collision kernels) is installed for the duration of the launches only: the engine never
         keeps a pointer into this object's tensors between calls."""
+        self._start_outcomes()
         self.e.set_skip_mask(self.done)
         try:
             self._iterate()
@@ -200,11 +271,16 @@ class BatchedEpisodes:
         elif self.obstacles is not None and self.obstacles.shape[1] > 0:
             _cabi.check(lib.jmpc_obstacle_step(e._h, self.B, int(self.obstacles.shape[1]), self._p(self.obstacles),
                                                self._p(self.done), float(e.dt), stream), "jmpc_obstacle_step")
+        if self.outcomes is not None:          # the obstacle poses that iteration i + 1's collision check reads
+            self._outcome_eval(self.obstacles if self.script is None else self.script[min(i + 1, self.script.shape[0] - 1)],
+                               initial=0)
         _cabi.check(lib.jmpc_counter_add(e._h, self._p(self.iter_dev), 1, stream), "jmpc_counter_add")
         self.iteration += 1
 
     def run(self, max_steps: Optional[int] = None, check_every: int = 8, use_graph: bool = False):
-        """Iterate until every episode reached its goal (or max_steps).  Returns a dict of numpy results.
+        """Iterate until every episode reached its goal (or max_steps).  Returns a dict of numpy results; with
+        outcomes=True also `outcomes` (dict of [B] arrays keyed by OUTCOME_NAMES, enum jmpc_outcome in include/jmpc.h)
+        and with record_obstacles=True `obstacle_history` [min(iterations, max_steps) + 1, B, n_obs, 6].
 
         With constant-input obstacles the loop body takes no per-iteration host argument, so with `use_graph`
         `check_every` iterations are captured once as a CUDA graph and replayed (one launch per 8 iterations instead
@@ -213,6 +289,7 @@ class BatchedEpisodes:
         it pays for long runs of small batches."""
         torch = self.torch
         max_steps = int(max_steps or self.max_steps)
+        self._start_outcomes()
         graph = None
         if use_graph and self.script is None and max_steps - self.iteration > 2 * check_every:
             self.iterate()                                    # eager once: scratch allocations, kernel attributes
@@ -254,6 +331,10 @@ class BatchedEpisodes:
             # (t = (i + 2) dt: HistorySimulation stores the initial state first, at t = dt; simulation.py:53-61)
             res["history"] = self.history[:n].cpu().numpy()
             res["flags"] = self.flags[:n].cpu().numpy()
+        if self.outcomes is not None:
+            res["outcomes"] = outcome_columns(self.outcomes.cpu().numpy())
+            if self.obstacle_history is not None:
+                res["obstacle_history"] = self.obstacle_history[:min(self.iteration, self.max_steps) + 1].cpu().numpy()
         if self._plans is not None:
             plans, pid = self._plans
             res.update(plan_status=plans.status[pid].cpu().numpy(), plan_cost=plans.cost[pid].cpu().numpy(),

@@ -20,13 +20,15 @@ def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_ar
                           weights=None, obstacles: Optional[Sequence[Sequence[dict]]] = None, frame_window: int = 10,
                           T: Optional[int] = None, config: Optional[MPCConfig] = None, dt: float = 0.2,
                           max_steps: int = 256, max_expansions: int = 4096, max_path: int = 48,
-                          max_N: Optional[int] = None, planner: Optional[BatchedPlanner] = None, device: int = 0) -> dict:
+                          max_N: Optional[int] = None, planner: Optional[BatchedPlanner] = None, device: int = 0,
+                          outcomes: bool = False, record_history: bool = True) -> dict:
     """One episode per search.  scenes / start / goal_point / goal_area / allowed_dtheta / scene_id / weights as in
     `BatchedPlanner.plan`; obstacles: per episode a list of the reference's scripted-obstacle dicts (see
     `episodes.scripted_obstacles`), or None for an empty road; frame_window: FRAME_WINDOW of the script (10 for the
     intersection, 20 for the roundabout).  Returns `BatchedEpisodes.run`'s dict (steps, done -- 3 where the search
     found no course --, state, history, flags, plan_status, plan_cost, expansions) plus the episodes' `dl` and
-    `margin`."""
+    `margin`.  outcomes=True adds the per-episode outcome record (`BatchedEpisodes(outcomes=True)`); with
+    record_history=False no History is kept on the device at all, which is what a large study wants."""
     import torch
     planner = planner or BatchedPlanner(device=device)
     plans = planner.plan_device(start, goal_point, goal_area, allowed_dtheta, scenes, scene_id=scene_id, weights=weights,
@@ -35,7 +37,7 @@ def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_ar
     try:
         program = None if obstacles is None else scripted_obstacles(obstacles)
         ep = BatchedEpisodes.from_plans(engine, plans, obstacle_program=program, frame_window=frame_window,
-                                        max_steps=max_steps)
+                                        max_steps=max_steps, record_history=record_history, outcomes=outcomes)
         res = ep.run(max_steps=max_steps)
         res.update(dl=engine.course_dl.cpu().numpy(), margin=ep.margin)
         torch.cuda.synchronize(engine.device)

@@ -268,6 +268,53 @@ int32_t jmpc_episode_post_dev(jmpc_handle h, int32_t B, double* state, const int
                               const int32_t* flag, const int32_t* iter_dev, double dt_loop, void* stream);
 int32_t jmpc_counter_add(jmpc_handle h, int32_t* counter, int32_t delta, void* stream);
 
+/* Per-episode outcome record (DEVICE pointers): contact, clearance and comfort of each closed-loop episode, accumulated
+ * on the device while it runs, so that a study needs neither the History nor the obstacle poses on the host.
+ * outcomes [B][JMPC_OUTCOME_LEN]: the public columns of enum jmpc_outcome, then private running state (previous pose,
+ * speed, applied a and clamped steer, executed steps).  One thread per episode; episodes with done != 0 are left
+ * untouched (also a done = 2 that jmpc_episode_post set in the same iteration).
+ *   Evaluation e pairs an ego pose with obstacle poses of the same instant.  e = 0: the start state with the obstacles'
+ *   initial poses (initial = 1: writes the empty record for every episode, then evaluates; reads no step data, record /
+ *   di / flag / iter_dev may be NULL).  e = i + 1 (initial = 0, i read from iter_dev): the state after loop iteration i
+ *   (History row i) with the poses iteration i + 1's collision check reads -- so enqueue it after the obstacles have
+ *   advanced (jmpc_scripted_obstacle_step(advance = 1) / jmpc_obstacle_step; a recording's frame min(i + 1, S - 1))
+ *   and before jmpc_counter_add.  With no step data besides the record the call also works in a captured graph.
+ *   Geometry is the collision kernel's (jmpc_set_car_geometry): two circles of radius r per car, for the ego at
+ *   state (x, y, yaw) and for obstacle k at obstacles[b][k] (x, y, yaw = columns 0, 1, 3).  Clearance of (ego,
+ *   obstacle) = min over the 4 circle pairs of dist - 2r; contact <=> dist <= 2r for some pair (the test jmpc_collision
+ *   applies to predictions).  The record only observes:
+ *   nothing here changes an episode.
+ *   The step columns count executed steps: flag [B] is the iteration's jmpc_collision flag (NULL: no obstacles,
+ *   counts 0), the applied controls and the xref deviation are recomputed from record, di, params and the previous
+ *   pose exactly as jmpc_episode_post computes them; course_id [B] or NULL (course 0) locates the target point.
+ *   obstacle_history [rows + 1][B][n_obs][6] or NULL: the poses of evaluation e go to row e (skipped once e > rows),
+ *   so row i + 1 is simultaneous with History row i.  Episodes that are done get no row. */
+#define JMPC_OUTCOME_LEN 22       /* doubles per episode in the outcome record (JMPC_NOUTCOME public, then private) */
+enum jmpc_outcome {
+  JMPC_O_MIN_CLEARANCE = 0,  /* min over evaluations and obstacles of the clearance [m]            empty: +inf */
+  JMPC_O_MIN_CLEARANCE_EVAL, /* evaluation where that minimum was first reached (strict <)         empty: -1   */
+  JMPC_O_MIN_CLEARANCE_OBS,  /*   and its obstacle (the lowest index within the evaluation)        empty: -1   */
+  JMPC_O_FIRST_CONTACT_EVAL, /* first evaluation with contact                                      empty: -1   */
+  JMPC_O_FIRST_CONTACT_OBS,  /*   and the lowest obstacle index in contact then                    empty: -1   */
+  JMPC_O_CONTACT_EVALS,      /* evaluations with contact                                           empty: 0    */
+  JMPC_O_CUT_STEPS,          /* executed steps whose collision flag was 1 (course cut)             empty: 0    */
+  JMPC_O_LIMIT_STEPS,        /* executed steps whose flag was -1 (no valid collision check)        empty: 0    */
+  JMPC_O_FAILED_SOLVES,      /* executed steps whose status was not JMPC_OPTIMAL (braked, MAX_DECEL) empty: 0  */
+  JMPC_O_MAX_ABS_ACCEL,      /* max |a| applied                                                    empty: 0    */
+  JMPC_O_MAX_ABS_JERK,       /* max |a_i - a_{i-1}| / dt over consecutive executed steps           empty: 0    */
+  JMPC_O_MAX_ABS_STEER_RATE, /* the same for the applied steer clamp(delta, +-MAX_STEER)           empty: 0    */
+  JMPC_O_MAX_ABS_LAT_ACCEL,  /* max |v * (v / L) * tan(steer)|, v the speed before the step        empty: 0    */
+  JMPC_O_MAX_XREF_DEV,       /* max of the xref deviation over optimal solves (History column 7)   empty: 0    */
+  JMPC_O_SUM_XREF_DEV,       /*   and its sum                                                      empty: 0    */
+  JMPC_O_DISTANCE,           /* path length driven: sum of hypot(dx, dy) over executed steps [m]   empty: 0    */
+  JMPC_NOUTCOME
+};
+int32_t jmpc_episode_outcomes(jmpc_handle h, int32_t B, const double* state, const int32_t* course_id,
+                              const double* obstacles, int32_t n_obs, const double* record, const double* di,
+                              const int32_t* flag, const double* params, const int32_t* done, const int32_t* iter_dev,
+                              int32_t initial, double* outcomes, double* obstacle_history, int32_t history_rows,
+                              void* stream);
+
 /* The reference's scripted obstacles on the device (main/lib/moving_obstacles.py: MovingObstacleTIntersection :166-232,
  * MovingObstacleRoundabout :28-123 including its dt = 0.2 quirk at :45 and the theta overwrite inside its steering
  * property, MovingObstacleArterial :125-164).  DEVICE pointers.
