@@ -143,10 +143,11 @@ int step_geometry(jmpc_handle h, int B, int T, StepGeom* g, StepKernel* kernel) 
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, wpb * 32, smem));
     if (per_sm < 1) return fail("step kernel does not fit on an SM for this horizon");
     if (cap > 0) per_sm = std::max(1, std::min(per_sm, cap / wpb));
-    // Shared memory and L1 share 256 KB per SM, and the spilled registers of the solver loop (ish / isl, 64 bytes per
-    // thread, read back three times per iteration) live in L1.  Ask for no more shared memory than the resident
-    // blocks use: T = 20 / T = 8 fit into the 196 KB configuration, which leaves 60 KB of L1 instead of 28 KB
-    // (measured: T = 20 0.833 -> 0.808 ms on config 2, T = 8 +1.5 %); T = 13 / T = 25 need the full 228 KB either way.
+    // Shared memory and L1 share 256 KB per SM.  Ask for no more shared memory than the resident blocks use: T = 20 /
+    // T = 8 fit into the 196 KB configuration, which leaves 60 KB of L1 instead of 28 KB for the course tables and
+    // the T = 8 kernel's spilled registers (measured when the T = 20 solver loop still spilled: 0.833 -> 0.808 ms on
+    // config 2, T = 8 +1.5 %; with that loop spill-free the two configurations time the same on config 2,
+    // profiles/r5_ab.txt); T = 13 / T = 25 need the full 228 KB either way.
     if (carve == cudaSharedmemCarveoutMaxShared) {
       int smem_sm = 0;
       CK(cudaDeviceGetAttribute(&smem_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, h->device));

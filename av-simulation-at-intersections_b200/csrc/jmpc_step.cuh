@@ -88,8 +88,9 @@ struct StepArgs {
 };
 
 constexpr int kSlotHi3 = JMPC_NPARAM, kSlotLo3 = JMPC_NPARAM + 1, kSlotLim = JMPC_NPARAM + 2;   // derived bounds
+constexpr int kSlotGscale = JMPC_NPARAM + 3;     // the solver's dual-residual scale
 constexpr int kParamSlots = 32;
-static_assert(JMPC_NPARAM + 3 <= kParamSlots, "parameter block too small");
+static_assert(JMPC_NPARAM + 4 <= kParamSlots, "parameter block too small");
 
 // suffix-moment slots of the Hessian assembly (step_prep): weight x centred prefix products
 enum MomentSlot {
@@ -653,6 +654,22 @@ __device__ __noinline__ int step_prep(const StepArgs& A, int b, bool active, dou
   return JMPC_OPTIMAL;
 }
 
+// 1 / s of a lane's slacks, recomputed after the factorisation and after the triangular solves instead of being held
+// across them: 16 registers fewer live through the solver loop's register peaks.  rcp_pos with a volatile seed, so that
+// the recomputations are not merged back into one value; the same instructions on the same slacks, the same bits.
+__device__ __forceinline__ double rcp_pos_again(double a) {
+  double y;
+  asm volatile("rcp.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(a));
+  double e = fma(-a, y, 1.0);
+  y = fma(y, e, y);
+  e = fma(-a, y, 1.0);
+  return fma(y, e, y);
+}
+__device__ __forceinline__ void slack_rcp(const double sh[4], const double sl[4], double ish[4], double isl[4]) {
+#pragma unroll
+  for (int r = 0; r < 4; ++r) { ish[r] = rcp_pos_again(sh[r]); isl[r] = rcp_pos_again(sl[r]); }
+}
+
 // ---- phase B: Mehrotra predictor-corrector on the condensed QP -----------------------------------------------
 // Returns the group's iteration count; `converged_out` says whether its KKT tolerances were met.  The groups of a
 // warp iterate in lock step until all of them are done; a group that is done (or never active) keeps executing on
@@ -693,9 +710,12 @@ __device__ __noinline__ int step_solve(const StepArgs& A, bool active, double* s
     else { lh[r] = is_live(r) ? 1.0 : 0.0; ll[r] = lh[r]; }
   }
   const double inv_rows = 1.0 / (double)(2 * (4 * T - 1));
-  double gscale = 0.0;
-  if (gl < T) gscale = fmax(fabs(M.q[gl]), fabs(M.q[T + gl]));
-  gscale = 1.0 + grp_max<G>(gscale, gm);
+  {
+    double gscale = 0.0;
+    if (gl < T) gscale = fmax(fabs(M.q[gl]), fabs(M.q[T + gl]));
+    gscale = 1.0 + grp_max<G>(gscale, gm);
+    if (gl == 0) M.prm[kSlotGscale] = gscale;    // read back by the exit tests (not held in a register across the loop)
+  }
   const int ntd = tiles_doubles(n);
   bool converged = false;
   bool acceptable = false;          // last evaluated iterate meets the reduced tolerances (see below)
@@ -722,12 +742,12 @@ __device__ __noinline__ int step_solve(const StepArgs& A, bool active, double* s
     // and the triangular solves: with them in registers the compiler spilled 0.5 KB per thread to local memory,
     // which misses the small L1 left beside 222 KB of shared memory and waits on L2.
     double* stash = M.grad;                         // [8][T]: rph[0..3], rpl[0..3] of stage = lane
-    double z[4], ish[4], isl[4], t4[4];
+    double z[4], t4[4];
     rows_apply<G>(M.u, T, gl, gm, z);
     double mu = 0.0, rpmax = 0.0;                   // rpmax: this lane's largest primal row residual
     double w2, w3;
     {
-      double w[4];
+      double w[4], ish[4], isl[4];
 #pragma unroll
       for (int r = 0; r < 4; ++r) {
         const bool lv = is_live(r);
@@ -781,6 +801,7 @@ __device__ __noinline__ int step_solve(const StepArgs& A, bool active, double* s
     // 64-bit shuffle steps with their compares and selects).
     const double rdmax_l = dmax(fabs(g0), fabs(g1));
     const bool rp_strict = grp_all<G>(rpmax <= A.tol_res), rp_red = grp_all<G>(rpmax <= 1e-7), rp_brk = grp_all<G>(rpmax <= 1e-9);
+    const double gscale = M.prm[kSlotGscale];
     const bool rd_strict = grp_all<G>(rdmax_l <= A.tol_res * gscale), rd_red = grp_all<G>(rdmax_l <= 1e-7 * gscale);
     const bool rd_brk = grp_all<G>(rdmax_l <= 1e-9 * gscale);
 #ifdef JMPC_DEBUG_RESID
@@ -822,29 +843,26 @@ __device__ __noinline__ int step_solve(const StepArgs& A, bool active, double* s
     }
     if (!kLock && done) break;
 
+    // dlh / dll enter each phase's direction recovery holding the complementarity targets rc: l s for the predictor, l s
+    // + ds_aff dl_aff - sigma mu for the corrector (formed at the end of the predictor, so that only rc and not the four
+    // affine directions live into the corrector)
     double dsh[4], dsl[4], dlh[4], dll[4];
-    double sigma_mu = 0.0, aff_step = 0.0;
+    double aff_step = 0.0;
 #pragma unroll 1
     for (int phase = 0; phase < 2; ++phase) {
-      // complementarity targets: predictor rc = l s ; corrector rc = l s + ds_aff dl_aff - sigma mu
-      double rph[4], rpl[4];
       double sw_lo = 0.0, sw_hi = 0.0;
       (void)sw_lo; (void)sw_hi;
-#pragma unroll
-      for (int r = 0; r < 4; ++r) {
-        rph[r] = (gl < T) ? stash[r * T + gl] : 0.0; rpl[r] = (gl < T) ? stash[(4 + r) * T + gl] : 0.0;
-      }
+      // the primal row residual k (rph[0..3], rpl[0..3]), read from the stash where it is used
+      auto rp = [&](int k) -> double { return (gl < T) ? stash[k * T + gl] : 0.0; };
       if (phase == 1) {
-        double th[4];
-        const double sm013 = live013 ? sigma_mu : 0.0, sm2 = live2 ? sigma_mu : 0.0;
+        double th[4], ish[4], isl[4];
+        slack_rcp(sh, sl, ish, isl);
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
-          const double sm = (r == 2) ? sm2 : sm013;
-          const double rch = fma(lh[r], sh[r], dsh[r] * dlh[r] - sm), rcl = fma(ll[r], sl[r], dsl[r] * dll[r] - sm);
-          const double a_h = fma(lh[r], rph[r], -rch) * ish[r];
-          const double a_l = fma(ll[r], rpl[r], -rcl) * isl[r];
-          th[r] = a_h - a_l;
-          dlh[r] = rch; dll[r] = rcl;               // stash rc for the direction recovery below
+          // th = a_h - a_l with a_l rounded and a_h's product fused into the difference, written out: left to the
+          // compiler, which of the two products it fuses changes with the surrounding code, and so would the iterates
+          const double a_l = __dmul_rn(fma(ll[r], rp(4 + r), -dll[r]), isl[r]);
+          th[r] = fma(fma(lh[r], rp(r), -dlh[r]), ish[r], -a_l);
         }
         rows_apply_T<G>(th, gl, gm, ra, rd);
         if (gl < T) { M.rhs[gl] = -g0 - ra; M.rhs[T + gl] = -g1 - rd; }
@@ -881,13 +899,14 @@ __device__ __noinline__ int step_solve(const StepArgs& A, bool active, double* s
       // (ish, isl), so their ratios are one multiplication each; the multipliers' ratios are tracked as a
       // (numerator, denominator) pair compared by cross-multiplication and turned into a ratio once per lane (no
       // fp64 division anywhere: ~20 instructions each).  Dead rows carry zero directions and never bind.
-      double rho = 0.0, wn = 0.0, wd = 1.0;
+      double rho = 0.0, wn = 0.0, wd = 1.0, ish[4], isl[4];
+      slack_rcp(sh, sl, ish, isl);
       auto cand = [&](double num, double den) { if (num * wd > wn * den) { wn = num; wd = den; } };
 #pragma unroll
       for (int r = 0; r < 4; ++r) {
         const double rch = dlh[r], rcl = dll[r];
-        dsh[r] = -rph[r] - dz[r];
-        dsl[r] = -rpl[r] + dz[r];
+        dsh[r] = -rp(r) - dz[r];
+        dsl[r] = -rp(4 + r) + dz[r];
         dlh[r] = -(fma(lh[r], dsh[r], rch)) * ish[r];
         dll[r] = -(fma(ll[r], dsl[r], rcl)) * isl[r];
         rho = dmax(rho, dmax(-dsh[r] * ish[r], -dsl[r] * isl[r]));
@@ -906,7 +925,13 @@ __device__ __noinline__ int step_solve(const StepArgs& A, bool active, double* s
           mu_aff += fma(aa, dlh[r], lh[r]) * fma(aa, dsh[r], sh[r]) + fma(aa, dll[r], ll[r]) * fma(aa, dsl[r], sl[r]);
         mu_aff = grp_sum<G>(mu_aff, gm) * inv_rows;
         const double ratio = mu_aff * rcp_pos(mu);
-        sigma_mu = ratio * ratio * ratio * mu;
+        const double sigma_mu = ratio * ratio * ratio * mu;
+        const double sm013 = live013 ? sigma_mu : 0.0, sm2 = live2 ? sigma_mu : 0.0;
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {                // the corrector's rc
+          const double sm = (r == 2) ? sm2 : sm013;
+          dlh[r] = fma(lh[r], sh[r], dsh[r] * dlh[r] - sm); dll[r] = fma(ll[r], sl[r], dsl[r] * dll[r] - sm);
+        }
       } else if (!kLock || !done) {
         // Fraction to the boundary tied to the length aa of the affine (predictor) step: a long predictor step
         // means the iterate is well centred and the corrector may go almost to the boundary (0.9999); a short
