@@ -1066,6 +1066,43 @@ int32_t jmpc_episode_outcomes(jmpc_handle h, int32_t B, const double* state, con
   return 0;
 }
 
+int32_t jmpc_scene_exchange(jmpc_handle h, int32_t B, int32_t k, int32_t n_extra, const double* state,
+                            const double* record, const double* di, const double* params, const int32_t* done,
+                            const int32_t* steps, const double* extras, double* obstacles_out, void* stream) {
+  if (!h) return fail("jmpc_scene_exchange: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_scene_exchange: B out of range");
+  if (k < 1 || B % k != 0) return fail("jmpc_scene_exchange: B must be a multiple of k >= 1");
+  if (n_extra < 0 || (k - 1) + n_extra > jmpc::kMaxObstacles)
+    return fail("jmpc_scene_exchange: (k - 1) + n_extra must be in [0, 8]");
+  if (!state || !record || !di || !done || !steps || !obstacles_out) return fail("jmpc_scene_exchange: NULL array");
+  if (n_extra > 0 && !extras) return fail("jmpc_scene_exchange: extras is NULL");
+  const int n_obs = (k - 1) + n_extra;
+  if (B == 0 || n_obs == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::ParamBlock defaults;
+  memcpy(defaults.v, h->defaults, sizeof h->defaults);
+  const int count = B * n_obs;
+  jmpc::scene_exchange_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
+      count, k, n_obs, state, record, di, params, defaults, done, steps, extras, obstacles_out);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
+int32_t jmpc_scene_init(jmpc_handle h, int32_t B, int32_t k, int32_t* done, void* stream) {
+  if (!h) return fail("jmpc_scene_init: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_scene_init: B out of range");
+  if (k < 1 || B % k != 0) return fail("jmpc_scene_init: B must be a multiple of k >= 1");
+  if (!done) return fail("jmpc_scene_init: NULL array");
+  if (B == 0 || k == 1) return 0;
+  CK(cudaSetDevice(h->device));
+  const int n_scenes = B / k;
+  jmpc::scene_init_kernel<<<(n_scenes + 127) / 128, 128, 0, (cudaStream_t)stream>>>(n_scenes, k, done);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
 int32_t jmpc_obstacle_step(jmpc_handle h, int32_t B, int32_t n_obs, double* obstacles, const int32_t* done,
                            double dt, void* stream) {
   if (!h) return fail("jmpc_obstacle_step: NULL handle");

@@ -269,6 +269,54 @@ __global__ void episode_outcome_kernel(const OutcomeArgs A) {
   }
 }
 
+// ---- scenes of k vehicles that see each other as obstacles (jmpc_scene_exchange, jmpc_scene_init) -----------------
+// One thread per (episode, slot) of obstacles_out [B][n_obs][6], n_obs = (k - 1) + n_extra.  Slots 0 .. k - 2 are the
+// scene mates of episode b = s * k + j in episode order without b itself, slots k - 1 .. are b's own extras.  A mate's
+// row is the tuple the flag kernel consumes: its pose and speed, and the (a, clamped steer) it applied in its last
+// step; (0, 0) before its first step; a finished mate (done != 0) is parked: v = a = steer = 0.  Copies, a select and
+// the shared clamp only, so the rows are bit-exact with the state and the applied controls.
+__global__ void scene_exchange_kernel(int count, int k, int n_obs, const double* __restrict__ state,
+                                      const double* __restrict__ record, const double* __restrict__ di,
+                                      const double* __restrict__ params, const ParamBlock defaults,
+                                      const int* __restrict__ done, const int* __restrict__ steps,
+                                      const double* __restrict__ extras, double* __restrict__ obstacles_out) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= count) return;
+  const int b = t / n_obs, slot = t - b * n_obs;
+  double* o = obstacles_out + (size_t)t * 6;
+  if (slot >= k - 1) {
+    const double* e = extras + ((size_t)b * (n_obs - (k - 1)) + (slot - (k - 1))) * 6;
+    for (int c = 0; c < 6; ++c) o[c] = e[c];
+    return;
+  }
+  const int j = b % k;
+  const int m = b - j + (slot < j ? slot : slot + 1);
+  const double* s = state + 4 * (size_t)m;
+  double v = s[2], acc = 0.0, steer = 0.0;
+  if (done[m]) {
+    v = 0.0;
+  } else if (steps[m] > 0) {
+    const double* prm = params ? params + (size_t)m * JMPC_NPARAM : defaults.v;
+    double delta;
+    applied_controls(record + (size_t)m * JMPC_RECORD_LEN, prm, di[m], delta, acc);
+    steer = clamped_steer(delta, prm[JMPC_P_MAX_STEER]);
+  }
+  o[0] = s[0]; o[1] = s[1]; o[2] = v; o[3] = s[3]; o[4] = acc; o[5] = steer;
+}
+
+// One thread per scene: a scene with an episode that has no course (done = 3) is not driven; its other episodes get
+// done = 4.
+__global__ void scene_init_kernel(int n_scenes, int k, int* __restrict__ done) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n_scenes) return;
+  int* d = done + (size_t)s * k;
+  bool unplannable = false;
+  for (int j = 0; j < k; ++j) unplannable |= d[j] == JMPC_DONE_NO_COURSE;
+  if (!unplannable) return;
+  for (int j = 0; j < k; ++j)
+    if (d[j] == JMPC_DONE_RUNNING) d[j] = JMPC_DONE_MATE_NO_COURSE;
+}
+
 // Constant-input obstacle motion, one thread per obstacle: obstacles [B][n_obs][6] = x, y, v, yaw, a, steer.
 __global__ void obstacle_step_kernel(int count, double* __restrict__ obs, const int* __restrict__ done, int n_obs,
                                      double dt, double L) {

@@ -11,6 +11,8 @@ ABI_VERSION = 2
 JMPC_MAX_T = 31
 RECORD_LEN = 8
 STATUS_OPTIMAL, STATUS_MAX_ITER, STATUS_INFEASIBLE, STATUS_INDEX_RULE = 0, 1, 2, 3
+# enum jmpc_done: why an episode stopped
+DONE_RUNNING, DONE_GOAL, DONE_INDEX_RULE, DONE_NO_COURSE, DONE_MATE_NO_COURSE = 0, 1, 2, 3, 4
 
 c_i32p = C.POINTER(C.c_int32)
 c_f64p = C.POINTER(C.c_double)
@@ -62,6 +64,8 @@ SIGNATURES = {
     "jmpc_counter_add": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "jmpc_episode_outcomes": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]
                               + [C.c_void_p] * 6 + [C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "jmpc_scene_exchange": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 9),
+    "jmpc_scene_init": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     "jmpc_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]),
     "jmpc_scripted_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                                 C.c_void_p, C.c_int32, C.c_void_p]),

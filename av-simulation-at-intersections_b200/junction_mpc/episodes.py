@@ -7,6 +7,8 @@ at the `done` flags every few iterations.  Obstacles are the reference's scripte
 (`obstacle_program`, see `scripted_obstacles`), constant-input vehicles advanced on the device (`obstacles`), or a
 per-step recording (`obstacle_script`).  With `outcomes=True` every episode also keeps a compact outcome record on
 the device (contact, clearance, comfort; enum jmpc_outcome in include/jmpc.h), so that a study needs no History.
+With `agents_per_scene=k` every k consecutive episodes form a scene whose MPC-driven vehicles see each other as moving
+obstacles (jmpc_scene_exchange).
 """
 from __future__ import annotations
 
@@ -40,6 +42,25 @@ def outcome_setup(outcomes: bool, record_obstacles: bool, n_obs: int) -> bool:
     if outcomes and not 0 <= n_obs <= MAX_OBSTACLES:
         raise ValueError(f"outcomes support at most {MAX_OBSTACLES} obstacles per episode, got {n_obs}")
     return bool(outcomes)
+
+
+def scene_setup(B: int, agents_per_scene: int, n_extra: int, has_script: bool) -> int:
+    """Host-side checks of the scene option of `BatchedEpisodes`: returns the obstacle slots per episode,
+    (agents_per_scene - 1) scene mates + n_extra own obstacles (enum jmpc_done / jmpc_scene_exchange in include/jmpc.h)."""
+    k = agents_per_scene
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or k < 1:
+        raise ValueError(f"agents_per_scene must be an integer >= 1, got {k!r}")
+    k = int(k)
+    if B % k:
+        raise ValueError(f"the batch of {B} episodes is not a whole number of scenes of {k} vehicles")
+    if k > 1 and has_script:
+        raise ValueError("obstacle_script cannot be combined with agents_per_scene > 1: a recording cannot react to the "
+                         "scene's vehicles; give obstacles or obstacle_program for the scripted traffic")
+    n_obs = (k - 1) + int(n_extra)
+    if n_obs > MAX_OBSTACLES:
+        raise ValueError(f"{k - 1} scene mates + {n_extra} obstacles exceed the {MAX_OBSTACLES} obstacle slots of an "
+                         "episode")
+    return n_obs
 
 
 def outcome_columns(record) -> dict:
@@ -107,15 +128,17 @@ class BatchedEpisodes:
     @classmethod
     def from_plans(cls, engine: BatchedMPC, plans, plan_id=None, params=None, obstacle_program=None, obstacles=None,
                    frame_window: int = 10, max_steps: int = 256, record_history: bool = True, horizon_s: float = 7.0,
-                   obstacle_script=None, outcomes: bool = False, record_obstacles: bool = False) -> "BatchedEpisodes":
+                   obstacle_script=None, outcomes: bool = False, record_obstacles: bool = False,
+                   agents_per_scene: int = 1) -> "BatchedEpisodes":
         """Episodes on the planned courses of `engine` (filled by `BatchedMPC.from_plans(plans)` /
         `set_courses_from_plans(plans)`), the second half of main/scenarios/mpc_intersection.py:63-163 for a batch:
         episode b drives plan `plan_id[b]` (default: one episode per plan; zeros = one course, many controllers).
         Its start state (the course's first pose at v = 0), its params row `dl` and done = 3 for a plan without a usable
         course are written on the device (jmpc_episode_init_from_courses); such episodes are never stepped.
         `params` [B, NPARAM] (default: the engine's defaults) supplies every other parameter row.  `run()` adds
-        plan_status, plan_cost and expansions per episode.  `outcomes` / `record_obstacles` as in `__init__`; evaluation
-        0 of the outcome record sees the planned start states."""
+        plan_status, plan_cost and expansions per episode.  `outcomes` / `record_obstacles` / `agents_per_scene` as in
+        `__init__`; evaluation 0 of the outcome record sees the planned start states.  With agents_per_scene > 1 a scene
+        with a done = 3 vehicle is not driven: its other vehicles get done = 4 (jmpc_scene_init)."""
         if engine.course_ok is None or len(engine.course_ok) != len(plans):
             raise ValueError("the engine's courses do not come from these plans (BatchedMPC.from_plans)")
         import torch
@@ -128,23 +151,33 @@ class BatchedEpisodes:
         ep = cls(engine, np.zeros((B, 4)), course_id=pid, obstacles=obstacles, obstacle_script=obstacle_script,
                  frame_window=frame_window, margin=margin, params=params, max_steps=max_steps,
                  record_history=record_history, horizon_s=horizon_s, obstacle_program=obstacle_program,
-                 outcomes=outcomes, record_obstacles=record_obstacles)
+                 outcomes=outcomes, record_obstacles=record_obstacles, agents_per_scene=agents_per_scene)
         stream = C.c_void_p(torch.cuda.current_stream(engine.device).cuda_stream)
         _cabi.check(engine._lib.jmpc_episode_init_from_courses(
             engine._h, B, ep._p(ep.course_id), ep._p(engine.course_ok), ep._p(engine.course_dl), ep._p(ep.state),
             ep._p(ep.params), ep._p(ep.done), stream), "jmpc_episode_init_from_courses")
+        if ep.k > 1:
+            _cabi.check(engine._lib.jmpc_scene_init(engine._h, B, ep.k, ep._p(ep.done), stream), "jmpc_scene_init")
         ep._plans = (plans, ep.course_id.long())
         return ep
 
     def __init__(self, engine: BatchedMPC, state0, course_id=None, obstacles=None, obstacle_script=None,
                  frame_window: int = 10, margin: int = 72, params=None, max_steps: int = 256,
                  record_history: bool = True, horizon_s: float = 7.0, obstacle_program=None, outcomes: bool = False,
-                 record_obstacles: bool = False):
+                 record_obstacles: bool = False, agents_per_scene: int = 1):
         """outcomes: keep one outcome record per episode on the device (jmpc_episode_outcomes): contact and clearance
         against the obstacles, cut / limit steps, failed solves, comfort and tracking columns; `run()` returns it as
         `outcomes`.  It observes only: the episodes are exactly those of outcomes=False.  record_obstacles (needs
         outcomes): also keep the obstacle poses of every evaluation, `run()`'s `obstacle_history`
-        [iterations + 1, B, n_obs, 6], whose row i + 1 is simultaneous with History row i."""
+        [iterations + 1, B, n_obs, 6], whose row i + 1 is simultaneous with History row i.
+
+        agents_per_scene = k > 1: k consecutive episodes form a scene of MPC-driven vehicles that see each other as
+        moving obstacles (jmpc_scene_exchange in include/jmpc.h).  Each episode's obstacle slots are its k - 1 scene mates
+        in episode order (itself skipped), then its own `obstacles` / `obstacle_program` (n_extra of them), at most 8
+        in all; the outcome record's *_obs columns index these slots.  A mate's row is its state and the (a, clamped
+        steer) it last applied; a finished mate stays parked at its last pose with v = a = steer = 0.  All vehicles move
+        simultaneously: the rows iteration i + 1 reads are those after iteration i.  k = 1 is the single-vehicle loop,
+        with nothing launched or allocated for scenes."""
         import torch
         self.torch = torch
         self.e = engine
@@ -188,6 +221,10 @@ class BatchedEpisodes:
             n_obs = int(self.obstacles.shape[1])
         elif self.script is not None:
             n_obs = int(self.script.shape[2])
+        n_obs = scene_setup(B, agents_per_scene, n_obs, self.script is not None)
+        self.k = int(agents_per_scene)
+        # k > 1: the obstacle rows every kernel reads, written by jmpc_scene_exchange from the vehicles and the extras
+        self.scene_obs = torch.empty(B, n_obs, 6, dtype=f64, device=self.dev) if self.k > 1 else None
         self.n_obs = n_obs
         self.outcomes = self.obstacle_history = None
         if outcome_setup(outcomes, record_obstacles, n_obs):
@@ -195,7 +232,7 @@ class BatchedEpisodes:
             if record_obstacles:
                 self.obstacle_history = torch.full((self.max_steps + 1, B, n_obs, 6), float("nan"), dtype=f64,
                                                    device=self.dev)
-        self._outcomes_started = False
+        self._started = False
         if self.program is not None:                                 # get() before the first iteration
             self._scripted_step(advance=0)
 
@@ -218,13 +255,32 @@ class BatchedEpisodes:
             int(initial), self._p(self.outcomes), self._p(self.obstacle_history), self.max_steps, stream),
             "jmpc_episode_outcomes")
 
-    def _start_outcomes(self):
-        """Evaluation 0, launched once before the first iteration: after __init__ / from_plans wrote the start states."""
-        if self.outcomes is None or self._outcomes_started:
+    def _scene_exchange(self):
+        """The obstacle rows of every episode from its scene mates' states and its own extras (jmpc_scene_exchange)."""
+        e = self.e
+        stream = C.c_void_p(self.torch.cuda.current_stream(e.device).cuda_stream)
+        n_extra = 0 if self.obstacles is None else int(self.obstacles.shape[1])
+        _cabi.check(e._lib.jmpc_scene_exchange(
+            e._h, self.B, self.k, n_extra, self._p(self.state), self._p(self.out.record), self._p(self.di),
+            self._p(self.params), self._p(self.done), self._p(self.steps), self._p(self.obstacles) if n_extra else None,
+            self._p(self.scene_obs), stream), "jmpc_scene_exchange")
+
+    def _current_obstacles(self, frame: int):
+        """The obstacle rows that loop iteration `frame`'s collision check reads (evaluation `frame`)."""
+        if self.scene_obs is not None:
+            return self.scene_obs
+        return self.obstacles if self.script is None else self.script[min(frame, self.script.shape[0] - 1)]
+
+    def _start(self):
+        """Launched once before the first iteration, after __init__ / from_plans wrote the start states: the scene's
+        first exchange, then evaluation 0 of the outcome record."""
+        if self._started:
             return
-        obs = self.obstacles if self.script is None else self.script[0]
-        self._outcome_eval(obs, initial=1)
-        self._outcomes_started = True
+        if self.scene_obs is not None:
+            self._scene_exchange()
+        if self.outcomes is not None:
+            self._outcome_eval(self._current_obstacles(0), initial=1)
+        self._started = True
 
     def _p(self, ten):
         return None if ten is None else C.c_void_p(ten.data_ptr())
@@ -233,7 +289,7 @@ class BatchedEpisodes:
         """One loop iteration for every episode that is not done.  The engine-wide skip mask (finished episodes cost
         nothing in the step / collision kernels) is installed for the duration of the launches only: the engine never
         keeps a pointer into this object's tensors between calls."""
-        self._start_outcomes()
+        self._start()
         self.e.set_skip_mask(self.done)
         try:
             self._iterate()
@@ -249,7 +305,7 @@ class BatchedEpisodes:
                                          self._p(self.target_ind), self._p(self.steps), self._p(self.agent_idx),
                                          self._p(self.done), float(cfg.goal_dis), float(cfg.stop_speed), stream),
                     "jmpc_episode_pre")
-        obs = self.obstacles if self.script is None else self.script[min(i, self.script.shape[0] - 1)]
+        obs = self._current_obstacles(i)
         if obs is not None and obs.shape[1] > 0:
             self.v.copy_(self.state[:, 2])
             e.collision(self.agent_idx, self.v, obs, self.frame_window, self.margin, self.flag, self.course_len,
@@ -271,9 +327,10 @@ class BatchedEpisodes:
         elif self.obstacles is not None and self.obstacles.shape[1] > 0:
             _cabi.check(lib.jmpc_obstacle_step(e._h, self.B, int(self.obstacles.shape[1]), self._p(self.obstacles),
                                                self._p(self.done), float(e.dt), stream), "jmpc_obstacle_step")
+        if self.scene_obs is not None:         # all vehicles have moved: the scene's rows of evaluation i + 1
+            self._scene_exchange()
         if self.outcomes is not None:          # the obstacle poses that iteration i + 1's collision check reads
-            self._outcome_eval(self.obstacles if self.script is None else self.script[min(i + 1, self.script.shape[0] - 1)],
-                               initial=0)
+            self._outcome_eval(self._current_obstacles(i + 1), initial=0)
         _cabi.check(lib.jmpc_counter_add(e._h, self._p(self.iter_dev), 1, stream), "jmpc_counter_add")
         self.iteration += 1
 
@@ -289,7 +346,7 @@ class BatchedEpisodes:
         it pays for long runs of small batches."""
         torch = self.torch
         max_steps = int(max_steps or self.max_steps)
-        self._start_outcomes()
+        self._start()
         graph = None
         if use_graph and self.script is None and max_steps - self.iteration > 2 * check_every:
             self.iterate()                                    # eager once: scratch allocations, kernel attributes

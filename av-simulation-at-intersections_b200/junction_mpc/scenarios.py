@@ -21,15 +21,25 @@ def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_ar
                           T: Optional[int] = None, config: Optional[MPCConfig] = None, dt: float = 0.2,
                           max_steps: int = 256, max_expansions: int = 4096, max_path: int = 48,
                           max_N: Optional[int] = None, planner: Optional[BatchedPlanner] = None, device: int = 0,
-                          outcomes: bool = False, record_history: bool = True) -> dict:
+                          outcomes: bool = False, record_history: bool = True, agents_per_scene: int = 1) -> dict:
     """One episode per search.  scenes / start / goal_point / goal_area / allowed_dtheta / scene_id / weights as in
     `BatchedPlanner.plan`; obstacles: per episode a list of the reference's scripted-obstacle dicts (see
     `episodes.scripted_obstacles`), or None for an empty road; frame_window: FRAME_WINDOW of the script (10 for the
     intersection, 20 for the roundabout).  Returns `BatchedEpisodes.run`'s dict (steps, done -- 3 where the search
     found no course --, state, history, flags, plan_status, plan_cost, expansions) plus the episodes' `dl` and
     `margin`.  outcomes=True adds the per-episode outcome record (`BatchedEpisodes(outcomes=True)`); with
-    record_history=False no History is kept on the device at all, which is what a large study wants."""
+    record_history=False no History is kept on the device at all, which is what a large study wants.
+
+    agents_per_scene = k > 1: searches [s k, (s + 1) k) are the k MPC-driven vehicles of scene s, which see each other
+    as moving obstacles (`BatchedEpisodes(agents_per_scene=k)`); `obstacles` is then given per scene (len = B / k) and
+    replicated to its vehicles.  A scene with a failed search is not driven: that vehicle gets done = 3, its mates
+    done = 4."""
     import torch
+    k = int(agents_per_scene)
+    if obstacles is not None and k > 1:
+        if len(start) % k or len(obstacles) != len(start) // k:
+            raise ValueError(f"with agents_per_scene = {k}, obstacles must hold one list per scene ({len(start)} // {k})")
+        obstacles = [specs for specs in obstacles for _ in range(k)]
     planner = planner or BatchedPlanner(device=device)
     plans = planner.plan_device(start, goal_point, goal_area, allowed_dtheta, scenes, scene_id=scene_id, weights=weights,
                                 max_expansions=max_expansions, max_path=max_path)
@@ -37,7 +47,8 @@ def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_ar
     try:
         program = None if obstacles is None else scripted_obstacles(obstacles)
         ep = BatchedEpisodes.from_plans(engine, plans, obstacle_program=program, frame_window=frame_window,
-                                        max_steps=max_steps, record_history=record_history, outcomes=outcomes)
+                                        max_steps=max_steps, record_history=record_history, outcomes=outcomes,
+                                        agents_per_scene=k)
         res = ep.run(max_steps=max_steps)
         res.update(dl=engine.course_dl.cpu().numpy(), margin=ep.margin)
         torch.cuda.synchronize(engine.device)

@@ -237,8 +237,9 @@ int32_t jmpc_plant_step(jmpc_handle h, int32_t B, double* state, const double* a
                         const double* params, void* stream);
 
 /* Closed-loop episodes on the device (the scenario loop around the step, main/scenarios/mpc_intersection.py:99-163).
- * DEVICE pointers; all arrays [B] unless noted; episodes with done != 0 are left untouched by all three.  done codes:
- * 1 goal reached, 2 the index rule raised, 3 no planned course (jmpc_episode_init_from_courses: the plan failed).
+ * DEVICE pointers; all arrays [B] unless noted; episodes with done != 0 are left untouched by all three.  done codes
+ * (enum jmpc_done): 1 goal reached, 2 the index rule raised, 3 no planned course (jmpc_episode_init_from_courses: the
+ * plan failed), 4 a scene mate has no planned course (jmpc_scene_init).
  *   jmpc_episode_pre : done |= is_goal(state) (mpc.py:314-330; done = 2 when the index rule raises), then
  *                      agent_idx = nearest forward index on the full course unless the truncated course has
  *                      collapsed onto the ego's point (mpc_intersection.py:107-109).  course_len = length of the
@@ -256,6 +257,13 @@ int32_t jmpc_plant_step(jmpc_handle h, int32_t B, double* state, const double* a
  *   jmpc_obstacle_step: constant-input motion of obstacles [B][n_obs][6] (moving_obstacles_prediction.py:21-29), with
  *                      one `dt` for the whole batch: a params row's dt reaches the collision prediction and the plant,
  *                      not this step. */
+enum jmpc_done {
+  JMPC_DONE_RUNNING = 0,         /* still driving                                                                  */
+  JMPC_DONE_GOAL = 1,            /* is_goal fired                                                    mpc.py:314-330 */
+  JMPC_DONE_INDEX_RULE = 2,      /* the nearest-index rule raised                             trajectories.py:120 */
+  JMPC_DONE_NO_COURSE = 3,       /* no usable planned course: never stepped      jmpc_episode_init_from_courses */
+  JMPC_DONE_MATE_NO_COURSE = 4   /* a scene mate has no usable planned course: never stepped    jmpc_scene_init */
+};
 int32_t jmpc_episode_pre(jmpc_handle h, int32_t B, const double* state, const int32_t* course_id,
                          const int32_t* course_len, const int32_t* target_ind, const int32_t* steps,
                          int32_t* agent_idx, int32_t* done, double goal_dis, double stop_speed, void* stream);
@@ -314,6 +322,33 @@ int32_t jmpc_episode_outcomes(jmpc_handle h, int32_t B, const double* state, con
                               const int32_t* flag, const double* params, const int32_t* done, const int32_t* iter_dev,
                               int32_t initial, double* outcomes, double* obstacle_history, int32_t history_rows,
                               void* stream);
+
+/* Scenes of several MPC-driven vehicles that see each other as moving obstacles (DEVICE pointers).  k consecutive
+ * episodes form a scene: episode b = s * k + j is vehicle j of scene s (B % k == 0, k >= 1).  Every vehicle runs the
+ * single-vehicle loop above unchanged; only its obstacle rows come from its scene mates.
+ *   jmpc_scene_exchange writes obstacles_out [B][n_obs][6], n_obs = (k - 1) + n_extra <= 8 (the collision and outcome
+ *   kernels' limit), the obstacle rows of every episode:
+ *     slots 0 .. k - 2: the scene mates in episode order, skipping the episode itself (the outcome record's *_obs
+ *       columns index these slots).  A mate's row is (x, y, v, yaw, a, steer): its state at that instant, the
+ *       acceleration it applied in its last executed step (MAX_DECEL after a failed solve, mpc.py:298-301) and the
+ *       steer it applied, clamped to +-MAX_STEER as the plant clamps it (simulation.py:38-43) -- both from the step's
+ *       record, di and params as jmpc_episode_post applies them; a = steer = 0 before the mate's first step (steps = 0).
+ *       Parked rule: a mate with done != 0 no longer moves and stays in the scene at its last pose with
+ *       v = a = steer = 0.
+ *     slots k - 1 .. n_obs - 1: the episode's own extras [B][n_extra][6] (constant-input or scripted obstacles,
+ *       advanced by jmpc_obstacle_step / jmpc_scripted_obstacle_step as for a single vehicle), copied.
+ *   Timing: all vehicles move simultaneously.  Enqueue one exchange before evaluation 0 / loop iteration 0 (on the start
+ *   states) and one per loop iteration after jmpc_episode_post_dev and the extras' advance, before jmpc_episode_outcomes:
+ *   the rows written in iteration i are the poses of evaluation i + 1 and what iteration i + 1's jmpc_collision reads,
+ *   the contract of a recording's frame.  No per-iteration host argument: the call can be captured in a CUDA graph.
+ *   record [B][JMPC_RECORD_LEN], di, params ([B][JMPC_NPARAM] or NULL: handle defaults), done, steps: as
+ *   jmpc_episode_post leaves them; extras NULL when n_extra = 0.  Rows of every episode are written, done or not.
+ *   jmpc_scene_init: the scene pass after jmpc_episode_init_from_courses.  A scene in which some episode has done = 3 is
+ *   not driven: its episodes with done = 0 get done = 4 (JMPC_DONE_MATE_NO_COURSE), so no mate row is ever absent. */
+int32_t jmpc_scene_exchange(jmpc_handle h, int32_t B, int32_t k, int32_t n_extra, const double* state,
+                            const double* record, const double* di, const double* params, const int32_t* done,
+                            const int32_t* steps, const double* extras, double* obstacles_out, void* stream);
+int32_t jmpc_scene_init(jmpc_handle h, int32_t B, int32_t k, int32_t* done, void* stream);
 
 /* The reference's scripted obstacles on the device (main/lib/moving_obstacles.py: MovingObstacleTIntersection :166-232,
  * MovingObstacleRoundabout :28-123 including its dt = 0.2 quirk at :45 and the theta overwrite inside its steering
