@@ -70,7 +70,7 @@ struct jmpc_handle_s {
   int n_flag_peers = 0;
   unsigned long long gather_step = 0;
   int* d_gather_timeout = nullptr;
-  bool collision_attr_set = false;
+  bool collision_attr_set = false, collision_planned_attr_set = false;
   const int* skip = nullptr;           // jmpc_set_skip_mask
   // longest-first scheduling (jmpc_set_schedule)
   int host_transfer = 1;               // jmpc_set_host_transfer
@@ -822,17 +822,24 @@ int32_t jmpc_step_host_io(jmpc_handle h, int32_t B, int32_t T, const double* sta
   return 0;
 }
 
-int32_t jmpc_collision(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* agent_idx,
-                       const double* v, const double* obstacles, int32_t n_obs, int32_t frame_window,
-                       int32_t margin, double horizon_s, const double* params, int32_t* flag,
-                       int32_t* course_len_out, void* stream) {
-  if (!h) return fail("jmpc_collision: NULL handle");
-  if (B < 0 || B > h->max_B) return fail("jmpc_collision: B out of range");
-  if (!agent_idx || !v || !flag || !course_len_out) return fail("jmpc_collision: NULL array");
-  if (n_obs < 0 || n_obs > jmpc::kMaxObstacles) return fail("jmpc_collision: n_obs out of range");
-  if (n_obs > 0 && !obstacles) return fail("jmpc_collision: obstacles is NULL");
-  if (frame_window < 0 || frame_window > jmpc::kMaxFrameWindow) return fail("jmpc_collision: frame_window out of range");
-  if (h->n_courses < 1) return fail("jmpc_collision: no courses uploaded (jmpc_set_courses)");
+// jmpc_collision and jmpc_collision_planned: the same checks and launch sizing for both instantiations of the kernel
+// (section B of the planned one uses no extra shared memory).
+extern "C++" {
+template <bool Planned>
+static int32_t launch_collision(const char* name, jmpc_handle h, int32_t B, const int32_t* course_id,
+                                const int32_t* agent_idx, const double* v, const double* obstacles, int32_t n_obs,
+                                const double* plans, int32_t n_planned, int32_t plan_len, int32_t frame_window,
+                                int32_t margin, double horizon_s, const double* params, int32_t* flag,
+                                int32_t* course_len_out, void* stream) {
+  char msg[160];
+  auto err = [&](const char* what) { snprintf(msg, sizeof msg, "%s: %s", name, what); return fail(msg); };
+  if (!h) return err("NULL handle");
+  if (B < 0 || B > h->max_B) return err("B out of range");
+  if (!agent_idx || !v || !flag || !course_len_out) return err("NULL array");
+  if (n_obs < 0 || n_obs > jmpc::kMaxObstacles) return err("n_obs out of range");
+  if (n_obs > 0 && !obstacles) return err("obstacles is NULL");
+  if (frame_window < 0 || frame_window > jmpc::kMaxFrameWindow) return err("frame_window out of range");
+  if (h->n_courses < 1) return err("no courses uploaded (jmpc_set_courses)");
   if (B == 0) return 0;
   CK(cudaSetDevice(h->device));
   jmpc::CollisionArgs a;
@@ -848,25 +855,49 @@ int32_t jmpc_collision(jmpc_handle h, int32_t B, const int32_t* course_id, const
   a.horizon_s = horizon_s; a.params = params;
   memcpy(a.defaults.v, h->defaults, sizeof h->defaults);
   a.flag = flag; a.course_len_out = course_len_out; a.skip = h->skip;
+  a.plans = plans; a.n_planned = n_planned; a.plan_len = plan_len;
   // with a table for every course the kernel needs no shared memory for the arc scan: 5 KB per warp instead of 12.6 KB
   // at max_N = 960 and two obstacles, i.e. more than twice the resident warps of this latency-bound kernel
   a.arc_smem = (a.arc_tab && h->arc_all) ? 0 : h->max_N;
   // 4 warps per block unless a long course's arc scan does not leave room for them: then 2, or 1 (jmpc.h states the
   // resulting max_N limit).  The warps of a block share nothing, so the results do not depend on the count.
   const size_t smem_cap = 200 * 1024, warp_smem = jmpc::collision_warp_smem_bytes(a.arc_smem, n_obs);
-  if (warp_smem > smem_cap) return fail("jmpc_collision: course too long for the shared-memory arc scan");
+  if (warp_smem > smem_cap) return err("course too long for the shared-memory arc scan");
   int wpb = 4;
   while (wpb > 1 && wpb * warp_smem > smem_cap) wpb >>= 1;
   const int blocks = (B + wpb - 1) / wpb;
   const size_t smem = wpb * warp_smem;
-  if (!h->collision_attr_set) {             // per handle: function attributes are per device
-    CK(cudaFuncSetAttribute(jmpc::collision_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_cap));
-    h->collision_attr_set = true;
+  bool& attr_set = Planned ? h->collision_planned_attr_set : h->collision_attr_set;
+  if (!attr_set) {                          // per handle: function attributes are per device
+    CK(cudaFuncSetAttribute(jmpc::collision_kernel<Planned>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_cap));
+    attr_set = true;
   }
-  jmpc::collision_kernel<<<blocks, wpb * 32, smem, (cudaStream_t)stream>>>(a);
+  jmpc::collision_kernel<Planned><<<blocks, wpb * 32, smem, (cudaStream_t)stream>>>(a);
   CK(cudaGetLastError());
   h->launches++;
   return 0;
+}
+}  // extern "C++"
+
+int32_t jmpc_collision(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* agent_idx,
+                       const double* v, const double* obstacles, int32_t n_obs, int32_t frame_window,
+                       int32_t margin, double horizon_s, const double* params, int32_t* flag,
+                       int32_t* course_len_out, void* stream) {
+  return launch_collision<false>("jmpc_collision", h, B, course_id, agent_idx, v, obstacles, n_obs, nullptr, 0, 1,
+                                 frame_window, margin, horizon_s, params, flag, course_len_out, stream);
+}
+
+int32_t jmpc_collision_planned(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* agent_idx,
+                               const double* v, const double* obstacles, int32_t n_obs, const double* plans,
+                               int32_t n_planned, int32_t plan_len, int32_t frame_window, int32_t margin,
+                               double horizon_s, const double* params, int32_t* flag, int32_t* course_len_out,
+                               void* stream) {
+  if (n_planned < 0 || n_planned > n_obs) return fail("jmpc_collision_planned: n_planned must be in [0, n_obs]");
+  if (plan_len < 1) return fail("jmpc_collision_planned: plan_len must be >= 1");
+  if (n_planned > 0 && !plans) return fail("jmpc_collision_planned: plans is NULL");
+  return launch_collision<true>("jmpc_collision_planned", h, B, course_id, agent_idx, v, obstacles, n_obs, plans,
+                                n_planned, plan_len, frame_window, margin, horizon_s, params, flag, course_len_out,
+                                stream);
 }
 
 int32_t jmpc_collision_host(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* agent_idx,
@@ -1084,6 +1115,28 @@ int32_t jmpc_scene_exchange(jmpc_handle h, int32_t B, int32_t k, int32_t n_extra
   const int count = B * n_obs;
   jmpc::scene_exchange_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
       count, k, n_obs, state, record, di, params, defaults, done, steps, extras, obstacles_out);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
+int32_t jmpc_scene_plans(jmpc_handle h, int32_t B, int32_t k, int32_t T, const double* oa, const double* od,
+                         const int32_t* warm, const int32_t* done, const double* params, const double* obstacles,
+                         int32_t n_obs, double* plans_out, void* stream) {
+  if (!h) return fail("jmpc_scene_plans: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_scene_plans: B out of range");
+  if (k < 1 || B % k != 0) return fail("jmpc_scene_plans: B must be a multiple of k >= 1");
+  if (T < 2) return fail("jmpc_scene_plans: T must be >= 2");
+  if (n_obs < k - 1 || n_obs > jmpc::kMaxObstacles) return fail("jmpc_scene_plans: n_obs must be in [k - 1, 8]");
+  if (B == 0 || k == 1) return 0;
+  if (!oa || !od || !warm || !done || !obstacles || !plans_out) return fail("jmpc_scene_plans: NULL array");
+  CK(cudaSetDevice(h->device));
+  jmpc::ParamBlock defaults;
+  memcpy(defaults.v, h->defaults, sizeof h->defaults);
+  const long long count = (long long)B * (k - 1) * (T - 1);
+  if (count > INT32_MAX) return fail("jmpc_scene_plans: B * (k - 1) * (T - 1) too large");
+  jmpc::scene_plans_kernel<<<(unsigned)((count + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+      (int)count, k, T, n_obs, oa, od, warm, done, params, defaults, obstacles, plans_out);
   CK(cudaGetLastError());
   h->launches++;
   return 0;

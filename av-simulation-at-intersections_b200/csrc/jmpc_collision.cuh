@@ -44,6 +44,9 @@ struct CollisionArgs {
   // starts at arc_tab + arc_off[c] + a0 * N - a0 (a0 - 1) / 2 and has N - a0 entries; arc_off[c] < 0 = no table
   const double* arc_tab; const long long* arc_off;
   const int* skip;                                   // [B] or nullptr: skip[b] != 0 -> instance left untouched
+  // collision_kernel<true> only: per-step inputs [B][n_planned][plan_len][2] (a, steer) of obstacle slots 0 ..
+  // n_planned - 1; predictor step t uses input min(t, plan_len - 1)
+  const double* plans; int n_planned, plan_len;
 };
 
 // dynamic shared memory of one warp: arc[arc_cap] | ocx[n_obs][kMaxObsFrames][2] | ocy[...] | bbox[kMaxObstacles][4] |
@@ -131,6 +134,10 @@ struct CollisionSmem {
   __device__ __forceinline__ int oi(int ob, int frame, int circle) const { return (ob * kMaxObsFrames + frame) * 2 + circle; }
 };
 
+// Planned = false: every obstacle is predicted with the constant input (a, steer) of its row (columns 4, 5).
+// Planned = true: slots < A.n_planned are predicted with their per-step inputs from A.plans instead; only section B
+// differs, and a plan whose entries all equal the row's (a, steer) gives the constant-input prediction bit for bit.
+template <bool Planned>
 __global__ void __launch_bounds__(128) collision_kernel(const CollisionArgs A) {
   extern __shared__ unsigned char smem_raw[];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -222,15 +229,39 @@ __global__ void __launch_bounds__(128) collision_kernel(const CollisionArgs A) {
   // Each value is produced by the same operations in the same order as in the reference's loop, which evaluates
   // sin / cos of every heading twice (2 x 35 sequential sincos per obstacle on 2-4 active lanes before).
   const int n_of = min((int)ceil(A.horizon_s / dt), kMaxObsFrames - 1);
+  // Planned slots: the recurrence is the same, with input min(k, plan_len - 1) at step k.  tan(steer_k) of every
+  // (slot, step) is evaluated across the lanes first, into ocy[ob][k][1] (free until the centres are written); the
+  // yaw / speed walk then replaces it with the speed before step k, which the position pass reads back.
+  const double* plan = nullptr;
+  if constexpr (Planned) {
+    const double* pb = A.plans + (size_t)b * A.n_planned * A.plan_len * 2;
+    for (int j = lane; j < A.n_planned * n_of; j += 32) {
+      const int ob = j / n_of, k = j - ob * n_of;
+      S.ocy[S.oi(ob, k, 1)] = tan(pb[((size_t)ob * A.plan_len + min(k, A.plan_len - 1)) * 2 + 1]);
+    }
+    if (lane < A.n_planned) plan = pb + (size_t)lane * A.plan_len * 2;
+    __syncwarp();
+  }
   if (lane < A.n_obs) {
     const double* o = A.obstacles + ((size_t)b * A.n_obs + lane) * 6;
     double vo = o[2], yaw = o[3];
-    const double acc = o[4], tn = tan(o[5]);
-    S.ocy[S.oi(lane, 0, 0)] = yaw;                   // scratch: heading k in ocy[ob][k][0]
-    for (int k = 0; k < n_of; ++k) {
-      vo = __dadd_rn(vo, __dmul_rn(acc, dt));
-      yaw = __dadd_rn(yaw, __dmul_rn(__dmul_rn(vo / L, tn), dt));
-      S.ocy[S.oi(lane, k + 1, 0)] = yaw;
+    if (Planned && plan) {
+      S.ocy[S.oi(lane, 0, 0)] = yaw;                 // scratch: heading k in ocy[ob][k][0]
+      for (int k = 0; k < n_of; ++k) {
+        const double tn = S.ocy[S.oi(lane, k, 1)];
+        S.ocy[S.oi(lane, k, 1)] = vo;
+        vo = __dadd_rn(vo, __dmul_rn(plan[2 * min(k, A.plan_len - 1)], dt));
+        yaw = __dadd_rn(yaw, __dmul_rn(__dmul_rn(vo / L, tn), dt));
+        S.ocy[S.oi(lane, k + 1, 0)] = yaw;
+      }
+    } else {
+      const double acc = o[4], tn = tan(o[5]);
+      S.ocy[S.oi(lane, 0, 0)] = yaw;
+      for (int k = 0; k < n_of; ++k) {
+        vo = __dadd_rn(vo, __dmul_rn(acc, dt));
+        yaw = __dadd_rn(yaw, __dmul_rn(__dmul_rn(vo / L, tn), dt));
+        S.ocy[S.oi(lane, k + 1, 0)] = yaw;
+      }
     }
   }
   __syncwarp();
@@ -247,9 +278,10 @@ __global__ void __launch_bounds__(128) collision_kernel(const CollisionArgs A) {
     const double acc = o[4];
     double c = S.ocx[S.oi(lane, 0, 0)], s = S.ocx[S.oi(lane, 0, 1)];
     for (int k = 0; k < n_of; ++k) {
+      if (Planned && plan) vo = S.ocy[S.oi(lane, k, 1)];
       x = __dadd_rn(x, __dmul_rn(__dmul_rn(vo, c), dt));
       y = __dadd_rn(y, __dmul_rn(__dmul_rn(vo, s), dt));
-      vo = __dadd_rn(vo, __dmul_rn(acc, dt));
+      if (!(Planned && plan)) vo = __dadd_rn(vo, __dmul_rn(acc, dt));
       c = S.ocx[S.oi(lane, k + 1, 0)]; s = S.ocx[S.oi(lane, k + 1, 1)];       // heading after the step
       // slot k is overwritten with the circle centres only now that its cos / sin have been consumed
       circle_centre(x, y, c, s, A.off_front, S.ocx[S.oi(lane, k, 0)], S.ocy[S.oi(lane, k, 0)]);

@@ -275,6 +275,11 @@ __global__ void episode_outcome_kernel(const OutcomeArgs A) {
 // row is the tuple the flag kernel consumes: its pose and speed, and the (a, clamped steer) it applied in its last
 // step; (0, 0) before its first step; a finished mate (done != 0) is parked: v = a = steer = 0.  Copies, a select and
 // the shared clamp only, so the rows are bit-exact with the state and the applied controls.
+// Mate slot `slot` (0 .. k - 2) of episode b = s * k + j: the scene's episodes in order, b itself skipped.
+__device__ __forceinline__ int scene_mate(int b, int k, int slot) {
+  const int j = b % k;
+  return b - j + (slot < j ? slot : slot + 1);
+}
 __global__ void scene_exchange_kernel(int count, int k, int n_obs, const double* __restrict__ state,
                                       const double* __restrict__ record, const double* __restrict__ di,
                                       const double* __restrict__ params, const ParamBlock defaults,
@@ -289,8 +294,7 @@ __global__ void scene_exchange_kernel(int count, int k, int n_obs, const double*
     for (int c = 0; c < 6; ++c) o[c] = e[c];
     return;
   }
-  const int j = b % k;
-  const int m = b - j + (slot < j ? slot : slot + 1);
+  const int m = scene_mate(b, k, slot);
   const double* s = state + 4 * (size_t)m;
   double v = s[2], acc = 0.0, steer = 0.0;
   if (done[m]) {
@@ -302,6 +306,34 @@ __global__ void scene_exchange_kernel(int count, int k, int n_obs, const double*
     steer = clamped_steer(delta, prm[JMPC_P_MAX_STEER]);
   }
   o[0] = s[0]; o[1] = s[1]; o[2] = v; o[3] = s[3]; o[4] = acc; o[5] = steer;
+}
+
+// One thread per (episode, mate slot, plan step) of plans_out [B][k - 1][T - 1][2] (jmpc_scene_plans): the input of
+// predictor step t for mate m is what m's last solve planned for its step t + 1, (oa[m][t + 1], clamp(od[m][t + 1])).
+// A mate without a valid plan -- finished (done != 0) or without a usable warm start (warm = 0: before its first step,
+// after a failed solve) -- repeats its row's (a, steer), so that its slot predicts exactly as the constant-input row.
+__global__ void scene_plans_kernel(int count, int k, int T, int n_obs, const double* __restrict__ oa,
+                                   const double* __restrict__ od, const int* __restrict__ warm,
+                                   const int* __restrict__ done, const double* __restrict__ params,
+                                   const ParamBlock defaults, const double* __restrict__ obstacles,
+                                   double* __restrict__ plans_out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  const int row = i / (T - 1), t = i - row * (T - 1);       // row = b * (k - 1) + slot
+  const int b = row / (k - 1), slot = row - b * (k - 1);
+  const int m = scene_mate(b, k, slot);
+  double acc, steer;
+  if (done[m] == 0 && warm[m] != 0) {
+    const double* prm = params ? params + (size_t)m * JMPC_NPARAM : defaults.v;
+    acc = oa[(size_t)m * T + t + 1];
+    steer = clamped_steer(od[(size_t)m * T + t + 1], prm[JMPC_P_MAX_STEER]);
+  } else {
+    const double* o = obstacles + ((size_t)b * n_obs + slot) * 6;
+    acc = o[4];
+    steer = o[5];
+  }
+  plans_out[2 * (size_t)i] = acc;
+  plans_out[2 * (size_t)i + 1] = steer;
 }
 
 // One thread per scene: a scene with an episode that has no course (done = 3) is not driven; its other episodes get

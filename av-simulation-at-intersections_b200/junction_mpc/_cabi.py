@@ -52,6 +52,8 @@ SIGNATURES = {
     "jmpc_host_free": (C.c_int32, [C.c_void_p, C.c_void_p]),
     "jmpc_collision": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                    C.c_int32, C.c_int32, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "jmpc_collision_planned": (C.c_int32, [C.c_void_p, C.c_int32] + [C.c_void_p] * 4 + [C.c_int32, C.c_void_p]
+                               + [C.c_int32] * 4 + [C.c_double] + [C.c_void_p] * 4),
     "jmpc_collision_host": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_void_p, C.c_void_p,
                                         C.c_void_p]),
@@ -65,6 +67,8 @@ SIGNATURES = {
     "jmpc_episode_outcomes": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]
                               + [C.c_void_p] * 6 + [C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "jmpc_scene_exchange": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 9),
+    "jmpc_scene_plans": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 6
+                         + [C.c_int32, C.c_void_p, C.c_void_p]),
     "jmpc_scene_init": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     "jmpc_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]),
     "jmpc_scripted_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,

@@ -8,7 +8,8 @@ at the `done` flags every few iterations.  Obstacles are the reference's scripte
 per-step recording (`obstacle_script`).  With `outcomes=True` every episode also keeps a compact outcome record on
 the device (contact, clearance, comfort; enum jmpc_outcome in include/jmpc.h), so that a study needs no History.
 With `agents_per_scene=k` every k consecutive episodes form a scene whose MPC-driven vehicles see each other as moving
-obstacles (jmpc_scene_exchange).
+obstacles (jmpc_scene_exchange); with `share_plans=True` they predict each other along their MPC plans
+(jmpc_scene_plans, jmpc_collision_planned).
 """
 from __future__ import annotations
 
@@ -20,7 +21,7 @@ import numpy as np
 
 from . import _cabi
 from .batched import BatchedMPC
-from .config import NPARAM
+from .config import NPARAM, PARAM_INDEX
 
 
 OBS_KINDS = {"constant": 0, "t_intersection": 1, "roundabout": 2, "arterial": 3}
@@ -61,6 +62,22 @@ def scene_setup(B: int, agents_per_scene: int, n_extra: int, has_script: bool) -
         raise ValueError(f"{k - 1} scene mates + {n_extra} obstacles exceed the {MAX_OBSTACLES} obstacle slots of an "
                          "episode")
     return n_obs
+
+
+def plan_share_setup(share_plans: bool, k: int, params) -> bool:
+    """Host-side checks of the shared-plans option of `BatchedEpisodes`: returns whether the plans are exchanged.
+    A mate's plan is in its own steps and the predictor runs at the evaluating vehicle's dt, so every vehicle of a scene
+    needs the same dt (params [B, NPARAM] rows; None = the engine's defaults for all)."""
+    if not share_plans:
+        return False
+    if k < 2:
+        raise ValueError("share_plans=True needs agents_per_scene > 1: there are no scene mates to share plans with")
+    if params is not None:
+        dt = np.asarray(params, np.float64)[:, PARAM_INDEX["dt"]].reshape(-1, k)
+        bad = np.flatnonzero((dt != dt[:, :1]).any(axis=1))
+        if len(bad):
+            raise ValueError(f"share_plans=True needs one dt per scene: scene {int(bad[0])} has dt {dt[bad[0]].tolist()}")
+    return True
 
 
 def outcome_columns(record) -> dict:
@@ -129,15 +146,15 @@ class BatchedEpisodes:
     def from_plans(cls, engine: BatchedMPC, plans, plan_id=None, params=None, obstacle_program=None, obstacles=None,
                    frame_window: int = 10, max_steps: int = 256, record_history: bool = True, horizon_s: float = 7.0,
                    obstacle_script=None, outcomes: bool = False, record_obstacles: bool = False,
-                   agents_per_scene: int = 1) -> "BatchedEpisodes":
+                   agents_per_scene: int = 1, share_plans: bool = False) -> "BatchedEpisodes":
         """Episodes on the planned courses of `engine` (filled by `BatchedMPC.from_plans(plans)` /
         `set_courses_from_plans(plans)`), the second half of main/scenarios/mpc_intersection.py:63-163 for a batch:
         episode b drives plan `plan_id[b]` (default: one episode per plan; zeros = one course, many controllers).
         Its start state (the course's first pose at v = 0), its params row `dl` and done = 3 for a plan without a usable
         course are written on the device (jmpc_episode_init_from_courses); such episodes are never stepped.
         `params` [B, NPARAM] (default: the engine's defaults) supplies every other parameter row.  `run()` adds
-        plan_status, plan_cost and expansions per episode.  `outcomes` / `record_obstacles` / `agents_per_scene` as in
-        `__init__`; evaluation 0 of the outcome record sees the planned start states.  With agents_per_scene > 1 a scene
+        plan_status, plan_cost and expansions per episode.  `outcomes` / `record_obstacles` / `agents_per_scene` /
+        `share_plans` as in `__init__`; evaluation 0 of the outcome record sees the planned start states.  With agents_per_scene > 1 a scene
         with a done = 3 vehicle is not driven: its other vehicles get done = 4 (jmpc_scene_init)."""
         if engine.course_ok is None or len(engine.course_ok) != len(plans):
             raise ValueError("the engine's courses do not come from these plans (BatchedMPC.from_plans)")
@@ -151,7 +168,8 @@ class BatchedEpisodes:
         ep = cls(engine, np.zeros((B, 4)), course_id=pid, obstacles=obstacles, obstacle_script=obstacle_script,
                  frame_window=frame_window, margin=margin, params=params, max_steps=max_steps,
                  record_history=record_history, horizon_s=horizon_s, obstacle_program=obstacle_program,
-                 outcomes=outcomes, record_obstacles=record_obstacles, agents_per_scene=agents_per_scene)
+                 outcomes=outcomes, record_obstacles=record_obstacles, agents_per_scene=agents_per_scene,
+                 share_plans=share_plans)
         stream = C.c_void_p(torch.cuda.current_stream(engine.device).cuda_stream)
         _cabi.check(engine._lib.jmpc_episode_init_from_courses(
             engine._h, B, ep._p(ep.course_id), ep._p(engine.course_ok), ep._p(engine.course_dl), ep._p(ep.state),
@@ -164,7 +182,7 @@ class BatchedEpisodes:
     def __init__(self, engine: BatchedMPC, state0, course_id=None, obstacles=None, obstacle_script=None,
                  frame_window: int = 10, margin: int = 72, params=None, max_steps: int = 256,
                  record_history: bool = True, horizon_s: float = 7.0, obstacle_program=None, outcomes: bool = False,
-                 record_obstacles: bool = False, agents_per_scene: int = 1):
+                 record_obstacles: bool = False, agents_per_scene: int = 1, share_plans: bool = False):
         """outcomes: keep one outcome record per episode on the device (jmpc_episode_outcomes): contact and clearance
         against the obstacles, cut / limit steps, failed solves, comfort and tracking columns; `run()` returns it as
         `outcomes`.  It observes only: the episodes are exactly those of outcomes=False.  record_obstacles (needs
@@ -177,7 +195,14 @@ class BatchedEpisodes:
         in all; the outcome record's *_obs columns index these slots.  A mate's row is its state and the (a, clamped
         steer) it last applied; a finished mate stays parked at its last pose with v = a = steer = 0.  All vehicles move
         simultaneously: the rows iteration i + 1 reads are those after iteration i.  k = 1 is the single-vehicle loop,
-        with nothing launched or allocated for scenes."""
+        with nothing launched or allocated for scenes.
+
+        share_plans (needs k > 1 and one dt per scene): each vehicle predicts its mates along their MPC plans instead of
+        holding their last applied (a, steer) for the whole horizon (jmpc_scene_plans / jmpc_collision_planned in
+        include/jmpc.h).  The mate rows, the outcome record and obstacle_history are unchanged; only the prediction of
+        the mate slots changes.  A mate's plan is the rest of its last solve, oa / od[1:], its last input held past the
+        end; a mate that is done, or has no usable warm start (before its first step, after a failed solve), is
+        predicted from its row as without the option.  Extras keep their constant-input prediction."""
         import torch
         self.torch = torch
         self.e = engine
@@ -225,6 +250,9 @@ class BatchedEpisodes:
         self.k = int(agents_per_scene)
         # k > 1: the obstacle rows every kernel reads, written by jmpc_scene_exchange from the vehicles and the extras
         self.scene_obs = torch.empty(B, n_obs, 6, dtype=f64, device=self.dev) if self.k > 1 else None
+        # share_plans: the mates' remaining plans [B, k - 1, T - 1, 2], written by jmpc_scene_plans after every exchange
+        self.scene_plans = (torch.empty(B, self.k - 1, self.T - 1, 2, dtype=f64, device=self.dev)
+                            if plan_share_setup(share_plans, self.k, params) else None)
         self.n_obs = n_obs
         self.outcomes = self.obstacle_history = None
         if outcome_setup(outcomes, record_obstacles, n_obs):
@@ -256,7 +284,8 @@ class BatchedEpisodes:
             "jmpc_episode_outcomes")
 
     def _scene_exchange(self):
-        """The obstacle rows of every episode from its scene mates' states and its own extras (jmpc_scene_exchange)."""
+        """The obstacle rows of every episode from its scene mates' states and its own extras (jmpc_scene_exchange), and
+        with share_plans the mates' plans (jmpc_scene_plans)."""
         e = self.e
         stream = C.c_void_p(self.torch.cuda.current_stream(e.device).cuda_stream)
         n_extra = 0 if self.obstacles is None else int(self.obstacles.shape[1])
@@ -264,6 +293,11 @@ class BatchedEpisodes:
             e._h, self.B, self.k, n_extra, self._p(self.state), self._p(self.out.record), self._p(self.di),
             self._p(self.params), self._p(self.done), self._p(self.steps), self._p(self.obstacles) if n_extra else None,
             self._p(self.scene_obs), stream), "jmpc_scene_exchange")
+        if self.scene_plans is not None:
+            _cabi.check(e._lib.jmpc_scene_plans(
+                e._h, self.B, self.k, self.T, self._p(self.oa), self._p(self.od), self._p(self.warm), self._p(self.done),
+                self._p(self.params), self._p(self.scene_obs), self.n_obs, self._p(self.scene_plans), stream),
+                "jmpc_scene_plans")
 
     def _current_obstacles(self, frame: int):
         """The obstacle rows that loop iteration `frame`'s collision check reads (evaluation `frame`)."""
@@ -309,7 +343,8 @@ class BatchedEpisodes:
         if obs is not None and obs.shape[1] > 0:
             self.v.copy_(self.state[:, 2])
             e.collision(self.agent_idx, self.v, obs, self.frame_window, self.margin, self.flag, self.course_len,
-                        course_id=self.course_id, params=self.params, horizon_s=self.horizon_s)
+                        course_id=self.course_id, params=self.params, horizon_s=self.horizon_s, plans=self.scene_plans,
+                        n_planned=self.k - 1)
             has_flags = True
         else:
             has_flags = False

@@ -21,7 +21,8 @@ def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_ar
                           T: Optional[int] = None, config: Optional[MPCConfig] = None, dt: float = 0.2,
                           max_steps: int = 256, max_expansions: int = 4096, max_path: int = 48,
                           max_N: Optional[int] = None, planner: Optional[BatchedPlanner] = None, device: int = 0,
-                          outcomes: bool = False, record_history: bool = True, agents_per_scene: int = 1) -> dict:
+                          outcomes: bool = False, record_history: bool = True, agents_per_scene: int = 1,
+                          share_plans: bool = False) -> dict:
     """One episode per search.  scenes / start / goal_point / goal_area / allowed_dtheta / scene_id / weights as in
     `BatchedPlanner.plan`; obstacles: per episode a list of the reference's scripted-obstacle dicts (see
     `episodes.scripted_obstacles`), or None for an empty road; frame_window: FRAME_WINDOW of the script (10 for the
@@ -33,7 +34,8 @@ def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_ar
     agents_per_scene = k > 1: searches [s k, (s + 1) k) are the k MPC-driven vehicles of scene s, which see each other
     as moving obstacles (`BatchedEpisodes(agents_per_scene=k)`); `obstacles` is then given per scene (len = B / k) and
     replicated to its vehicles.  A scene with a failed search is not driven: that vehicle gets done = 3, its mates
-    done = 4."""
+    done = 4.  share_plans=True: the vehicles of a scene predict each other along their MPC plans
+    (`BatchedEpisodes(share_plans=True)`)."""
     import torch
     k = int(agents_per_scene)
     if obstacles is not None and k > 1:
@@ -48,7 +50,7 @@ def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_ar
         program = None if obstacles is None else scripted_obstacles(obstacles)
         ep = BatchedEpisodes.from_plans(engine, plans, obstacle_program=program, frame_window=frame_window,
                                         max_steps=max_steps, record_history=record_history, outcomes=outcomes,
-                                        agents_per_scene=k)
+                                        agents_per_scene=k, share_plans=share_plans)
         res = ep.run(max_steps=max_steps)
         res.update(dl=engine.course_dl.cpu().numpy(), margin=ep.margin)
         torch.cuda.synchronize(engine.device)

@@ -231,6 +231,21 @@ int32_t jmpc_collision_host(jmpc_handle h, int32_t B, const int32_t* course_id, 
                             int32_t margin, double horizon_s, const double* params, int32_t* flag,
                             int32_t* course_len_out);
 
+/* jmpc_collision with per-step inputs for the first n_planned obstacle slots (DEVICE pointers; every other argument,
+ * check, limit, the skip mask and the launch sizing as jmpc_collision; no extra shared memory).
+ *   plans [B][n_planned][plan_len][2]: (a, steer) per predictor step; 0 <= n_planned <= n_obs, plan_len >= 1, plans
+ *   may be NULL only when n_planned = 0.  A planned slot is predicted with the reference's constant-input recurrence
+ *   (moving_obstacles_prediction.py:21-47) fed a sequence: predictor step t uses input min(t, plan_len - 1), so past
+ *   the plan the last input is held (speed unclamped, as for a constant input).  Per step the position advances with
+ *   the old v and yaw, then v += a_t dt, then yaw += (v / L) tan(steer_t) dt.  The rows' columns 4 and 5 are not read
+ *   for planned slots; slots n_planned .. n_obs - 1 use them as jmpc_collision does.  A plan whose entries all equal
+ *   the row's (a, steer) gives jmpc_collision's flags and cut lengths bit for bit. */
+int32_t jmpc_collision_planned(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* agent_idx,
+                               const double* v, const double* obstacles, int32_t n_obs, const double* plans,
+                               int32_t n_planned, int32_t plan_len, int32_t frame_window, int32_t margin,
+                               double horizon_s, const double* params, int32_t* flag, int32_t* course_len_out,
+                               void* stream);
+
 /* Plant step for B instances (Simulation.step, simulation.py:35-47 -> Bicycle.step, bicycle/main.py:28-41).
  * DEVICE pointers; state [B][4] is advanced in place with (a, delta). */
 int32_t jmpc_plant_step(jmpc_handle h, int32_t B, double* state, const double* a, const double* delta,
@@ -349,6 +364,21 @@ int32_t jmpc_scene_exchange(jmpc_handle h, int32_t B, int32_t k, int32_t n_extra
                             const double* record, const double* di, const double* params, const int32_t* done,
                             const int32_t* steps, const double* extras, double* obstacles_out, void* stream);
 int32_t jmpc_scene_init(jmpc_handle h, int32_t B, int32_t k, int32_t* done, void* stream);
+
+/* Shared plans (opt-in): scene mates predicted along their own MPC plans instead of their last applied controls.
+ *   jmpc_scene_plans writes plans_out [B][k - 1][T - 1][2], the inputs jmpc_collision_planned reads for the mate slots
+ *   0 .. k - 2 (n_planned = k - 1, plan_len = T - 1).  The mate rows of jmpc_scene_exchange are unchanged; only their
+ *   prediction changes.  For mate m of a slot and predictor step t = 0 .. T - 2 the input is
+ *   (oa[m][t + 1], clamp(od[m][t + 1], +-MAX_STEER of m)): the rest of the plan of m's last solve, whose step 0 m has
+ *   just applied.  A mate without a valid plan -- done[m] != 0 (parked), or warm[m] = 0 (before its first step, after a
+ *   failed solve) -- gets its row's (a, steer) repeated, so that its slot predicts exactly as the constant-input row.
+ *   oa, od [B][T] and warm, done [B] as jmpc_step / jmpc_episode_post_dev leave them; params [B][JMPC_NPARAM] or NULL;
+ *   obstacles [B][n_obs][6] the rows jmpc_scene_exchange wrote, n_obs in [k - 1, 8].  T >= 2.  k = 1 writes nothing.
+ *   Timing: enqueue it after every jmpc_scene_exchange (before iteration 0 and once per iteration); no per-iteration
+ *   host argument.  The predictor runs at the evaluating vehicle's dt, so the vehicles of a scene must share dt. */
+int32_t jmpc_scene_plans(jmpc_handle h, int32_t B, int32_t k, int32_t T, const double* oa, const double* od,
+                         const int32_t* warm, const int32_t* done, const double* params, const double* obstacles,
+                         int32_t n_obs, double* plans_out, void* stream);
 
 /* The reference's scripted obstacles on the device (main/lib/moving_obstacles.py: MovingObstacleTIntersection :166-232,
  * MovingObstacleRoundabout :28-123 including its dt = 0.2 quirk at :45 and the theta overwrite inside its steering
