@@ -71,6 +71,7 @@ struct jmpc_handle_s {
   unsigned long long gather_step = 0;
   int* d_gather_timeout = nullptr;
   bool collision_attr_set = false, collision_planned_attr_set = false;
+  bool collision_masked_attr_set[2] = {false, false};   // masked_collision_kernel<false / true>
   const int* skip = nullptr;           // jmpc_set_skip_mask
   // longest-first scheduling (jmpc_set_schedule)
   int host_transfer = 1;               // jmpc_set_host_transfer
@@ -822,15 +823,15 @@ int32_t jmpc_step_host_io(jmpc_handle h, int32_t B, int32_t T, const double* sta
   return 0;
 }
 
-// jmpc_collision and jmpc_collision_planned: the same checks and launch sizing for both instantiations of the kernel
-// (section B of the planned one uses no extra shared memory).
+// jmpc_collision, jmpc_collision_planned and jmpc_collision_masked: the same checks and launch sizing for every
+// instantiation of the kernel (section B of the planned one and the mask use no extra shared memory).
 extern "C++" {
-template <bool Planned>
+template <bool Planned, bool Masked = false>
 static int32_t launch_collision(const char* name, jmpc_handle h, int32_t B, const int32_t* course_id,
                                 const int32_t* agent_idx, const double* v, const double* obstacles, int32_t n_obs,
                                 const double* plans, int32_t n_planned, int32_t plan_len, int32_t frame_window,
                                 int32_t margin, double horizon_s, const double* params, int32_t* flag,
-                                int32_t* course_len_out, void* stream) {
+                                int32_t* course_len_out, void* stream, const int32_t* consider = nullptr) {
   char msg[160];
   auto err = [&](const char* what) { snprintf(msg, sizeof msg, "%s: %s", name, what); return fail(msg); };
   if (!h) return err("NULL handle");
@@ -867,12 +868,23 @@ static int32_t launch_collision(const char* name, jmpc_handle h, int32_t B, cons
   while (wpb > 1 && wpb * warp_smem > smem_cap) wpb >>= 1;
   const int blocks = (B + wpb - 1) / wpb;
   const size_t smem = wpb * warp_smem;
-  bool& attr_set = Planned ? h->collision_planned_attr_set : h->collision_attr_set;
-  if (!attr_set) {                          // per handle: function attributes are per device
-    CK(cudaFuncSetAttribute(jmpc::collision_kernel<Planned>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_cap));
-    attr_set = true;
+  bool& attr_set = Masked ? h->collision_masked_attr_set[Planned]
+                          : (Planned ? h->collision_planned_attr_set : h->collision_attr_set);
+  if constexpr (Masked) {
+    if (!attr_set) {                        // per handle: function attributes are per device
+      CK(cudaFuncSetAttribute(jmpc::masked_collision_kernel<Planned>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              (int)smem_cap));
+      attr_set = true;
+    }
+    jmpc::masked_collision_kernel<Planned><<<blocks, wpb * 32, smem, (cudaStream_t)stream>>>(a, consider);
+  } else {
+    if (!attr_set) {
+      CK(cudaFuncSetAttribute(jmpc::collision_kernel<Planned>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              (int)smem_cap));
+      attr_set = true;
+    }
+    jmpc::collision_kernel<Planned><<<blocks, wpb * 32, smem, (cudaStream_t)stream>>>(a);
   }
-  jmpc::collision_kernel<Planned><<<blocks, wpb * 32, smem, (cudaStream_t)stream>>>(a);
   CK(cudaGetLastError());
   h->launches++;
   return 0;
@@ -898,6 +910,24 @@ int32_t jmpc_collision_planned(jmpc_handle h, int32_t B, const int32_t* course_i
   return launch_collision<true>("jmpc_collision_planned", h, B, course_id, agent_idx, v, obstacles, n_obs, plans,
                                 n_planned, plan_len, frame_window, margin, horizon_s, params, flag, course_len_out,
                                 stream);
+}
+
+int32_t jmpc_collision_masked(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* agent_idx,
+                              const double* v, const double* obstacles, int32_t n_obs, const double* plans,
+                              int32_t n_planned, int32_t plan_len, const int32_t* consider, int32_t frame_window,
+                              int32_t margin, double horizon_s, const double* params, int32_t* flag,
+                              int32_t* course_len_out, void* stream) {
+  if (n_planned < 0 || n_planned > n_obs) return fail("jmpc_collision_masked: n_planned must be in [0, n_obs]");
+  if (plan_len < 1) return fail("jmpc_collision_masked: plan_len must be >= 1");
+  if (n_planned > 0 && !plans) return fail("jmpc_collision_masked: plans is NULL");
+  if (!consider) return fail("jmpc_collision_masked: consider is NULL");
+  if (n_planned > 0)
+    return launch_collision<true, true>("jmpc_collision_masked", h, B, course_id, agent_idx, v, obstacles, n_obs, plans,
+                                        n_planned, plan_len, frame_window, margin, horizon_s, params, flag,
+                                        course_len_out, stream, consider);
+  return launch_collision<false, true>("jmpc_collision_masked", h, B, course_id, agent_idx, v, obstacles, n_obs,
+                                       nullptr, 0, 1, frame_window, margin, horizon_s, params, flag, course_len_out,
+                                       stream, consider);
 }
 
 int32_t jmpc_collision_host(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* agent_idx,
@@ -1137,6 +1167,46 @@ int32_t jmpc_scene_plans(jmpc_handle h, int32_t B, int32_t k, int32_t T, const d
   if (count > INT32_MAX) return fail("jmpc_scene_plans: B * (k - 1) * (T - 1) too large");
   jmpc::scene_plans_kernel<<<(unsigned)((count + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
       (int)count, k, T, n_obs, oa, od, warm, done, params, defaults, obstacles, plans_out);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
+int32_t jmpc_right_of_way_init(jmpc_handle h, int32_t B, int32_t k, const int32_t* course_id, const double* junction,
+                               int32_t n_junction, int32_t* zone_out, void* stream) {
+  if (!h) return fail("jmpc_right_of_way_init: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_right_of_way_init: B out of range");
+  if (k < 1 || B % k != 0) return fail("jmpc_right_of_way_init: B must be a multiple of k >= 1");
+  if (n_junction != 1 && n_junction != B / k) return fail("jmpc_right_of_way_init: n_junction must be 1 or B / k");
+  if (!junction || !zone_out) return fail("jmpc_right_of_way_init: NULL array");
+  if (h->n_courses < 1) return fail("jmpc_right_of_way_init: no courses uploaded (jmpc_set_courses)");
+  if (B == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::right_of_way_init_kernel<<<(B + 3) / 4, 128, 0, (cudaStream_t)stream>>>(
+      B, k, h->d_cx, h->d_cy, h->d_course_n, h->course_stride, h->n_courses, course_id, junction,
+      n_junction > 1 ? 1 : 0, zone_out);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
+int32_t jmpc_right_of_way(jmpc_handle h, int32_t B, int32_t k, int32_t rule, const int32_t* agent_idx,
+                          const int32_t* done, const double* params, const int32_t* zone, const double* priority,
+                          int32_t* consider_out, void* stream) {
+  if (!h) return fail("jmpc_right_of_way: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_right_of_way: B out of range");
+  if (k < 2 || k > jmpc::kMaxObstacles + 1 || B % k != 0)
+    return fail("jmpc_right_of_way: B must be a multiple of k in [2, 9]");
+  if (rule != JMPC_ROW_FIXED && rule != JMPC_ROW_FIRST_COME) return fail("jmpc_right_of_way: unknown rule");
+  if (!agent_idx || !done || !consider_out) return fail("jmpc_right_of_way: NULL array");
+  if (rule == JMPC_ROW_FIXED && !priority) return fail("jmpc_right_of_way: the fixed rule needs priority");
+  if (rule == JMPC_ROW_FIRST_COME && !zone) return fail("jmpc_right_of_way: the first-come rule needs zone");
+  if (B == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::ParamBlock defaults;
+  memcpy(defaults.v, h->defaults, sizeof h->defaults);
+  jmpc::right_of_way_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(B, k, rule, agent_idx, done, params,
+                                                                               defaults, zone, priority, consider_out);
   CK(cudaGetLastError());
   h->launches++;
   return 0;

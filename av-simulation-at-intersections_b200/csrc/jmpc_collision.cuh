@@ -118,6 +118,14 @@ __device__ __forceinline__ bool within(double ax, double ay, double bx, double b
   return sqrt(d2) <= reach;
 }
 
+// consider[b] of the masked kernel, loaded where it is used (volatile: not merged with an earlier load of the same word
+// and kept in a register across sections A and B).  The generic pointer is converted to the global window explicitly.
+__device__ __forceinline__ unsigned ld_mask(const int* p) {
+  unsigned m;
+  asm volatile("{\n\t.reg .u64 g;\n\tcvta.to.global.u64 g, %1;\n\tld.global.nc.u32 %0, [g];\n\t}" : "=r"(m) : "l"(p));
+  return m;
+}
+
 struct CollisionSmem {
   double* arc;          // segment lengths, then running arc length
   double* ocx;          // obstacle circle centres [obstacle][frame][circle]
@@ -134,11 +142,18 @@ struct CollisionSmem {
   __device__ __forceinline__ int oi(int ob, int frame, int circle) const { return (ob * kMaxObsFrames + frame) * 2 + circle; }
 };
 
+// The body of collision_kernel and masked_collision_kernel, one warp per instance.
 // Planned = false: every obstacle is predicted with the constant input (a, steer) of its row (columns 4, 5).
 // Planned = true: slots < A.n_planned are predicted with their per-step inputs from A.plans instead; only section B
 // differs, and a plan whose entries all equal the row's (a, steer) gives the constant-input prediction bit for bit.
-template <bool Planned>
-__global__ void __launch_bounds__(128) collision_kernel(const CollisionArgs A) {
+// Masked = true: only the slots whose bit is set in consider[b] take part in section C.  Dropping slots keeps the
+// reference's row order of the others (obstacle major within an ego circle), so the result is that of the same call on
+// the considered rows alone; a mask without a bit among the n_obs slots is the n_obs = 0 case (flag 0, the full length:
+// section C finds no pair, and the table-limit exit reports 0 instead of -1).  An ignored slot gets an empty bounding
+// box (+inf .. -inf), which section C's box test skips like any box out of reach; the mask is read where it is used,
+// so that no register holds it across sections A and B.
+template <bool Planned, bool Masked>
+__device__ __forceinline__ void collision_body(const CollisionArgs& A, const int* __restrict__ consider) {
   extern __shared__ unsigned char smem_raw[];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const int b = blockIdx.x * (blockDim.x >> 5) + wib;
@@ -219,7 +234,12 @@ __global__ void __launch_bounds__(128) collision_kernel(const CollisionArgs A) {
   // or whose obstacle prediction needs more than kMaxObsFrames - 1 steps cannot be decided here; it is reported
   // (flag = -1, full course length) instead of being silently truncated.  The reference's scenes need 49 / 35.
   if (n_ego > kMaxEgoFrames || (int)ceil(A.horizon_s / dt) > kMaxObsFrames - 1) {
-    if (lane == 0) { A.flag[b] = -1; A.course_len_out[b] = N; }
+    // a mask without a considered slot is the n_obs = 0 case: flag 0 (tested here, on this rare path, and not before
+    // section A: a test up there costs the masked kernels spills of the loop state)
+    if (lane == 0) {
+      A.flag[b] = (Masked && (ld_mask(consider + b) & ((1u << A.n_obs) - 1u)) == 0u) ? 0 : -1;
+      A.course_len_out[b] = N;
+    }
     return;
   }
 
@@ -304,6 +324,7 @@ __global__ void __launch_bounds__(128) collision_kernel(const CollisionArgs A) {
       x0 = fmin(x0, __shfl_xor_sync(full, x0, o)); x1 = fmax(x1, __shfl_xor_sync(full, x1, o));
       y0 = fmin(y0, __shfl_xor_sync(full, y0, o)); y1 = fmax(y1, __shfl_xor_sync(full, y1, o));
     }
+    if (Masked && !((ld_mask(consider + b) >> ob) & 1u)) { x0 = y0 = INFINITY; x1 = y1 = -INFINITY; }
     if (lane == 0) { S.bbox[4 * ob] = x0; S.bbox[4 * ob + 1] = x1; S.bbox[4 * ob + 2] = y0; S.bbox[4 * ob + 3] = y1; }
   }
   __syncwarp();
@@ -390,6 +411,18 @@ __global__ void __launch_bounds__(128) collision_kernel(const CollisionArgs A) {
     A.flag[b] = 1;
     A.course_len_out[b] = max(a0 + 1, first - A.margin);
   }
+}
+
+// jmpc_collision / jmpc_collision_planned
+template <bool Planned>
+__global__ void __launch_bounds__(128) collision_kernel(const CollisionArgs A) {
+  collision_body<Planned, false>(A, nullptr);
+}
+
+// jmpc_collision_masked: consider [B] int32, bit s set = obstacle slot s takes part in the cut
+template <bool Planned>
+__global__ void __launch_bounds__(128) masked_collision_kernel(const CollisionArgs A, const int32_t* consider) {
+  collision_body<Planned, true>(A, consider);
 }
 
 }  // namespace jmpc

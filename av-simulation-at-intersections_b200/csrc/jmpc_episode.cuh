@@ -336,6 +336,80 @@ __global__ void scene_plans_kernel(int count, int k, int T, int n_obs, const dou
   plans_out[2 * (size_t)i + 1] = steer;
 }
 
+// ---- right-of-way rules (jmpc_right_of_way_init, jmpc_right_of_way) ----------------------------------------------
+// One warp per episode: the first and last point of its course inside the junction zone of its scene b / k,
+// dx * dx + dy * dy <= r * r without fused multiply-add; -1 / -1 when the course never enters it.  zone_out [B][2].
+__global__ void __launch_bounds__(128) right_of_way_init_kernel(int B, int k, const double* __restrict__ cx,
+                                                                const double* __restrict__ cy,
+                                                                const int* __restrict__ course_n, int course_stride,
+                                                                int n_courses, const int* __restrict__ course_id,
+                                                                const double* __restrict__ junction, int per_scene,
+                                                                int* __restrict__ zone_out) {
+  const int lane = threadIdx.x & 31;
+  const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (b >= B) return;
+  const int cid = course_id ? min(max(course_id[b], 0), n_courses - 1) : 0;
+  const double* px = cx + (size_t)cid * course_stride;
+  const double* py = cy + (size_t)cid * course_stride;
+  const int N = course_n[cid];
+  const double* J = junction + (per_scene ? 3 * (size_t)(b / k) : 0);
+  const double jx = J[0], jy = J[1], r2 = __dmul_rn(J[2], J[2]);
+  int entry = 0x7fffffff, exit = -1;
+  for (int i = lane; i < N; i += 32) {
+    const double dx = px[i] - jx, dy = py[i] - jy;
+    if (__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)) <= r2) { entry = min(entry, i); exit = max(exit, i); }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    entry = min(entry, __shfl_xor_sync(0xffffffffu, entry, o));
+    exit = max(exit, __shfl_xor_sync(0xffffffffu, exit, o));
+  }
+  if (lane == 0) {
+    zone_out[2 * (size_t)b] = exit < 0 ? -1 : entry;
+    zone_out[2 * (size_t)b + 1] = exit;
+  }
+}
+
+// The right-of-way key (cls, key) of episode m, compared lexicographically and then by episode index.
+//   JMPC_ROW_FIXED: (0, priority[m]).
+//   JMPC_ROW_FIRST_COME, a = agent_idx[m], zone [entry, exit]: committed (a >= entry) (0, (exit - a) dl), approaching
+//   (1, (entry - a) dl), a course that never enters the zone (2, 0).
+struct RowKey { int cls; double key; int idx; };
+__device__ __forceinline__ bool row_before(const RowKey& p, const RowKey& q) {
+  if (p.cls != q.cls) return p.cls < q.cls;
+  if (p.key != q.key) return p.key < q.key;
+  return p.idx < q.idx;
+}
+__device__ __forceinline__ RowKey row_key(int m, int rule, const int* __restrict__ agent_idx,
+                                          const double* __restrict__ params, const ParamBlock& defaults,
+                                          const int* __restrict__ zone, const double* __restrict__ priority) {
+  if (rule == JMPC_ROW_FIXED) return RowKey{0, priority[m], m};
+  const int entry = zone[2 * (size_t)m], exit = zone[2 * (size_t)m + 1], a = agent_idx[m];
+  if (entry < 0) return RowKey{2, 0.0, m};
+  const double dl = (params ? params + (size_t)m * JMPC_NPARAM : defaults.v)[JMPC_P_DL];
+  if (a >= entry) return RowKey{0, __dmul_rn((double)(exit - a), dl), m};
+  return RowKey{1, __dmul_rn((double)(entry - a), dl), m};
+}
+// One thread per episode b: consider[b] has every bit set except the mate slots s (0 .. k - 2) whose mate is moving
+// (done = 0) and does not come before b.  Parked mates and the extras are always considered; a finished b gets -1.
+__global__ void right_of_way_kernel(int B, int k, int rule, const int* __restrict__ agent_idx,
+                                    const int* __restrict__ done, const double* __restrict__ params,
+                                    const ParamBlock defaults, const int* __restrict__ zone,
+                                    const double* __restrict__ priority, int* __restrict__ consider) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  unsigned mask = 0xffffffffu;
+  if (done[b] == 0) {
+    const RowKey own = row_key(b, rule, agent_idx, params, defaults, zone, priority);
+    for (int slot = 0; slot < k - 1; ++slot) {
+      const int m = scene_mate(b, k, slot);
+      if (done[m] == 0 && !row_before(row_key(m, rule, agent_idx, params, defaults, zone, priority), own))
+        mask &= ~(1u << slot);
+    }
+  }
+  consider[b] = (int)mask;
+}
+
 // One thread per scene: a scene with an episode that has no course (done = 3) is not driven; its other episodes get
 // done = 4.
 __global__ void scene_init_kernel(int n_scenes, int k, int* __restrict__ done) {

@@ -433,10 +433,11 @@ class BatchedMPC:
 
     def collision(self, agent_idx, v, obstacles, frame_window: int, margin: int, flag, course_len_out,
                   course_id=None, params=None, horizon_s: float = 7.0, stream: Optional[int] = None, plans=None,
-                  n_planned: int = 0):
+                  n_planned: int = 0, consider=None):
         """Collision flags and cut lengths on the device.  plans [B, n_planned, plan_len, 2] float64 (optional): per-step
         (a, steer) inputs that predict obstacle slots 0 .. n_planned - 1 instead of their rows' constant inputs
-        (jmpc_collision_planned in include/jmpc.h)."""
+        (jmpc_collision_planned in include/jmpc.h).  consider [B] int32 (optional): bit s set = obstacle slot s takes
+        part in the cut; the others are ignored (jmpc_collision_masked)."""
         import torch
         B = agent_idx.shape[0]
         n_obs = int(obstacles.shape[1]) if obstacles is not None else 0
@@ -446,6 +447,19 @@ class BatchedMPC:
             n_planned = int(n_planned)
             if plans.dim() != 4 or plans.shape[0] != B or plans.shape[1] != n_planned or plans.shape[3] != 2:
                 raise ValueError(f"plans must be [{B}, {n_planned}, plan_len, 2]")
+        if consider is not None:
+            if tuple(consider.shape) != (B,):
+                raise ValueError(f"consider must be [{B}]")
+            planned = plans is not None and n_planned > 0
+            _cabi.check(self._lib.jmpc_collision_masked(
+                self._h, B, self._dp(course_id, torch.int32), self._dp(agent_idx, torch.int32),
+                self._dp(v, torch.float64), self._dp(obstacles, torch.float64), n_obs,
+                self._dp(plans, torch.float64) if planned else None, n_planned if planned else 0,
+                int(plans.shape[2]) if planned else 1, self._dp(consider, torch.int32), int(frame_window), int(margin),
+                float(horizon_s), self._dp(params, torch.float64), self._dp(flag, torch.int32),
+                self._dp(course_len_out, torch.int32), C.c_void_p(stream)), "jmpc_collision_masked")
+            return flag, course_len_out
+        if plans is not None:
             _cabi.check(self._lib.jmpc_collision_planned(
                 self._h, B, self._dp(course_id, torch.int32), self._dp(agent_idx, torch.int32),
                 self._dp(v, torch.float64), self._dp(obstacles, torch.float64), n_obs, self._dp(plans, torch.float64),

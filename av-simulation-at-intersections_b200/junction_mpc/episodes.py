@@ -9,7 +9,8 @@ per-step recording (`obstacle_script`).  With `outcomes=True` every episode also
 the device (contact, clearance, comfort; enum jmpc_outcome in include/jmpc.h), so that a study needs no History.
 With `agents_per_scene=k` every k consecutive episodes form a scene whose MPC-driven vehicles see each other as moving
 obstacles (jmpc_scene_exchange); with `share_plans=True` they predict each other along their MPC plans
-(jmpc_scene_plans, jmpc_collision_planned).
+(jmpc_scene_plans, jmpc_collision_planned); with `right_of_way` a rule decides which mates each vehicle yields to
+(jmpc_right_of_way, jmpc_collision_masked).
 """
 from __future__ import annotations
 
@@ -80,6 +81,47 @@ def plan_share_setup(share_plans: bool, k: int, params) -> bool:
     return True
 
 
+RIGHT_OF_WAY_RULES = {"fixed": _cabi.ROW_FIXED, "first_come": _cabi.ROW_FIRST_COME}
+
+
+def right_of_way_setup(right_of_way, k: int, B: int, priority=None, junction=None):
+    """Host-side checks of the right-of-way option of `BatchedEpisodes`.  Returns None without a rule, else
+    (rule code of enum jmpc_right_of_way_rule, priority float64 [B] or None, junction float64 [1 or B / k, 3] or None).
+    "fixed" takes priority [B] (finite; default: each episode's position j in its scene) and no junction; "first_come"
+    takes junction = (x, y, r), once for all scenes or [B / k, 3], finite with r > 0, and no priority."""
+    if right_of_way is None:
+        if priority is not None or junction is not None:
+            raise ValueError("priority / junction are arguments of a right-of-way rule: give right_of_way too")
+        return None
+    if right_of_way not in RIGHT_OF_WAY_RULES:
+        raise ValueError(f"right_of_way must be None, 'fixed' or 'first_come', got {right_of_way!r}")
+    if k < 2:
+        raise ValueError("a right-of-way rule needs agents_per_scene > 1: there are no scene mates to yield to")
+    if right_of_way == "fixed":
+        if junction is not None:
+            raise ValueError("the fixed rule takes no junction")
+        if priority is None:
+            return _cabi.ROW_FIXED, (np.arange(B) % k).astype(np.float64), None
+        prio = np.asarray(priority, np.float64)
+        if prio.shape != (B,):
+            raise ValueError(f"priority must be [{B}] (one key per episode), got shape {prio.shape}")
+        if not np.isfinite(prio).all():
+            raise ValueError("priority must be finite")
+        return _cabi.ROW_FIXED, np.ascontiguousarray(prio), None
+    if priority is not None:
+        raise ValueError("the first_come rule takes no priority: its keys come from the junction zone")
+    if junction is None:
+        raise ValueError("the first_come rule needs junction = (x, y, r)")
+    junc = np.asarray(junction, np.float64)
+    if junc.shape == (3,):
+        junc = junc[None, :]
+    if junc.shape not in ((1, 3), (B // k, 3)):
+        raise ValueError(f"junction must be (x, y, r) or [{B // k}, 3] (one per scene), got shape {np.shape(junction)}")
+    if not np.isfinite(junc).all() or not (junc[:, 2] > 0).all():
+        raise ValueError("junction must be finite with r > 0")
+    return _cabi.ROW_FIRST_COME, None, np.ascontiguousarray(junc)
+
+
 def outcome_columns(record) -> dict:
     """[B, >= len(OUTCOME_NAMES)] float64 outcome records -> dict of [B] arrays keyed by OUTCOME_NAMES (the index and
     count columns as int64)."""
@@ -146,7 +188,8 @@ class BatchedEpisodes:
     def from_plans(cls, engine: BatchedMPC, plans, plan_id=None, params=None, obstacle_program=None, obstacles=None,
                    frame_window: int = 10, max_steps: int = 256, record_history: bool = True, horizon_s: float = 7.0,
                    obstacle_script=None, outcomes: bool = False, record_obstacles: bool = False,
-                   agents_per_scene: int = 1, share_plans: bool = False) -> "BatchedEpisodes":
+                   agents_per_scene: int = 1, share_plans: bool = False, right_of_way=None, priority=None,
+                   junction=None) -> "BatchedEpisodes":
         """Episodes on the planned courses of `engine` (filled by `BatchedMPC.from_plans(plans)` /
         `set_courses_from_plans(plans)`), the second half of main/scenarios/mpc_intersection.py:63-163 for a batch:
         episode b drives plan `plan_id[b]` (default: one episode per plan; zeros = one course, many controllers).
@@ -154,8 +197,10 @@ class BatchedEpisodes:
         course are written on the device (jmpc_episode_init_from_courses); such episodes are never stepped.
         `params` [B, NPARAM] (default: the engine's defaults) supplies every other parameter row.  `run()` adds
         plan_status, plan_cost and expansions per episode.  `outcomes` / `record_obstacles` / `agents_per_scene` /
-        `share_plans` as in `__init__`; evaluation 0 of the outcome record sees the planned start states.  With agents_per_scene > 1 a scene
-        with a done = 3 vehicle is not driven: its other vehicles get done = 4 (jmpc_scene_init)."""
+        `share_plans` / `right_of_way` / `priority` / `junction` as in `__init__`; evaluation 0 of the outcome record sees
+        the planned start states; the junction zones are found on the planned courses, and first_come distances use
+        each course's dl.  With agents_per_scene > 1 a scene with a done = 3 vehicle is not driven: its other vehicles get
+        done = 4 (jmpc_scene_init)."""
         if engine.course_ok is None or len(engine.course_ok) != len(plans):
             raise ValueError("the engine's courses do not come from these plans (BatchedMPC.from_plans)")
         import torch
@@ -169,7 +214,7 @@ class BatchedEpisodes:
                  frame_window=frame_window, margin=margin, params=params, max_steps=max_steps,
                  record_history=record_history, horizon_s=horizon_s, obstacle_program=obstacle_program,
                  outcomes=outcomes, record_obstacles=record_obstacles, agents_per_scene=agents_per_scene,
-                 share_plans=share_plans)
+                 share_plans=share_plans, right_of_way=right_of_way, priority=priority, junction=junction)
         stream = C.c_void_p(torch.cuda.current_stream(engine.device).cuda_stream)
         _cabi.check(engine._lib.jmpc_episode_init_from_courses(
             engine._h, B, ep._p(ep.course_id), ep._p(engine.course_ok), ep._p(engine.course_dl), ep._p(ep.state),
@@ -182,7 +227,8 @@ class BatchedEpisodes:
     def __init__(self, engine: BatchedMPC, state0, course_id=None, obstacles=None, obstacle_script=None,
                  frame_window: int = 10, margin: int = 72, params=None, max_steps: int = 256,
                  record_history: bool = True, horizon_s: float = 7.0, obstacle_program=None, outcomes: bool = False,
-                 record_obstacles: bool = False, agents_per_scene: int = 1, share_plans: bool = False):
+                 record_obstacles: bool = False, agents_per_scene: int = 1, share_plans: bool = False,
+                 right_of_way=None, priority=None, junction=None):
         """outcomes: keep one outcome record per episode on the device (jmpc_episode_outcomes): contact and clearance
         against the obstacles, cut / limit steps, failed solves, comfort and tracking columns; `run()` returns it as
         `outcomes`.  It observes only: the episodes are exactly those of outcomes=False.  record_obstacles (needs
@@ -202,7 +248,20 @@ class BatchedEpisodes:
         include/jmpc.h).  The mate rows, the outcome record and obstacle_history are unchanged; only the prediction of
         the mate slots changes.  A mate's plan is the rest of its last solve, oa / od[1:], its last input held past the
         end; a mate that is done, or has no usable warm start (before its first step, after a failed solve), is
-        predicted from its row as without the option.  Extras keep their constant-input prediction."""
+        predicted from its row as without the option.  Extras keep their constant-input prediction.
+
+        right_of_way = "fixed" | "first_come" (needs k > 1; None: every mate is considered, as before): a rule that
+        decides which moving mates a vehicle yields to (jmpc_right_of_way / jmpc_collision_masked in include/jmpc.h).
+        Every iteration, after the goal test, each vehicle gets a consider mask (`consider` [B] int32, bit s = obstacle
+        slot s takes part in its collision cut).  Extras and parked mates (done != 0) are always considered; a moving
+        mate only if its key (class, key, episode index) is smaller than the vehicle's own, so no cycle of waiting can
+        form.  The rule changes nothing else: the mate rows, obstacle_history and the outcome record are unchanged, and
+        contacts with ignored mates are still measured.
+          "fixed": class 0, key priority[b] (float64 [B], finite; default: the position j of b in its scene).
+          "first_come": junction = (x, y, r), for all scenes or [B / k, 3].  entry / exit are the first and last points
+          of b's course within r of the centre (jmpc_right_of_way_init, `zone` [B, 2]; -1 when it never enters), a its
+          course index, dl its params' dl: committed (a >= entry) class 0, key (exit - a) dl; approaching class 1,
+          key (entry - a) dl; a course that never enters the zone class 2 (it yields to every moving mate)."""
         import torch
         self.torch = torch
         self.e = engine
@@ -254,6 +313,21 @@ class BatchedEpisodes:
         self.scene_plans = (torch.empty(B, self.k - 1, self.T - 1, 2, dtype=f64, device=self.dev)
                             if plan_share_setup(share_plans, self.k, params) else None)
         self.n_obs = n_obs
+        # right_of_way: the per-episode consider mask (jmpc_right_of_way, every iteration) and the rule's constant inputs
+        self.consider = self.zone = self.priority = self.junction = None
+        row = right_of_way_setup(right_of_way, self.k, B, priority, junction)
+        if row is not None:
+            self.row_rule, prio, junc = row
+            self.consider = torch.full((B,), -1, dtype=i32, device=self.dev)
+            self.priority = t(prio, f64)
+            if junc is not None:
+                # the course ids are final here (from_plans passes its plan ids): the zones are found once
+                self.junction = t(junc, f64)
+                self.zone = torch.empty(B, 2, dtype=i32, device=self.dev)
+                stream = C.c_void_p(torch.cuda.current_stream(engine.device).cuda_stream)
+                _cabi.check(engine._lib.jmpc_right_of_way_init(
+                    engine._h, B, self.k, self._p(self.course_id), self._p(self.junction), int(junc.shape[0]),
+                    self._p(self.zone), stream), "jmpc_right_of_way_init")
         self.outcomes = self.obstacle_history = None
         if outcome_setup(outcomes, record_obstacles, n_obs):
             self.outcomes = torch.empty(B, OUTCOME_LEN, dtype=f64, device=self.dev)     # evaluation 0 fills it
@@ -339,12 +413,16 @@ class BatchedEpisodes:
                                          self._p(self.target_ind), self._p(self.steps), self._p(self.agent_idx),
                                          self._p(self.done), float(cfg.goal_dis), float(cfg.stop_speed), stream),
                     "jmpc_episode_pre")
+        if self.consider is not None:          # this iteration's agent_idx and done: who yields to whom
+            _cabi.check(lib.jmpc_right_of_way(
+                e._h, self.B, self.k, self.row_rule, self._p(self.agent_idx), self._p(self.done), self._p(self.params),
+                self._p(self.zone), self._p(self.priority), self._p(self.consider), stream), "jmpc_right_of_way")
         obs = self._current_obstacles(i)
         if obs is not None and obs.shape[1] > 0:
             self.v.copy_(self.state[:, 2])
             e.collision(self.agent_idx, self.v, obs, self.frame_window, self.margin, self.flag, self.course_len,
                         course_id=self.course_id, params=self.params, horizon_s=self.horizon_s, plans=self.scene_plans,
-                        n_planned=self.k - 1)
+                        n_planned=self.k - 1, consider=self.consider)
             has_flags = True
         else:
             has_flags = False

@@ -22,7 +22,7 @@ def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_ar
                           max_steps: int = 256, max_expansions: int = 4096, max_path: int = 48,
                           max_N: Optional[int] = None, planner: Optional[BatchedPlanner] = None, device: int = 0,
                           outcomes: bool = False, record_history: bool = True, agents_per_scene: int = 1,
-                          share_plans: bool = False) -> dict:
+                          share_plans: bool = False, right_of_way=None, priority=None, junction=None) -> dict:
     """One episode per search.  scenes / start / goal_point / goal_area / allowed_dtheta / scene_id / weights as in
     `BatchedPlanner.plan`; obstacles: per episode a list of the reference's scripted-obstacle dicts (see
     `episodes.scripted_obstacles`), or None for an empty road; frame_window: FRAME_WINDOW of the script (10 for the
@@ -35,7 +35,8 @@ def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_ar
     as moving obstacles (`BatchedEpisodes(agents_per_scene=k)`); `obstacles` is then given per scene (len = B / k) and
     replicated to its vehicles.  A scene with a failed search is not driven: that vehicle gets done = 3, its mates
     done = 4.  share_plans=True: the vehicles of a scene predict each other along their MPC plans
-    (`BatchedEpisodes(share_plans=True)`)."""
+    (`BatchedEpisodes(share_plans=True)`).  right_of_way / priority / junction: a rule that decides which mates each
+    vehicle yields to (`BatchedEpisodes(right_of_way=...)`); priority per search, junction once or per scene."""
     import torch
     k = int(agents_per_scene)
     if obstacles is not None and k > 1:
@@ -50,7 +51,8 @@ def run_planned_scenarios(scenes: Sequence[Sequence], start, goal_point, goal_ar
         program = None if obstacles is None else scripted_obstacles(obstacles)
         ep = BatchedEpisodes.from_plans(engine, plans, obstacle_program=program, frame_window=frame_window,
                                         max_steps=max_steps, record_history=record_history, outcomes=outcomes,
-                                        agents_per_scene=k, share_plans=share_plans)
+                                        agents_per_scene=k, share_plans=share_plans, right_of_way=right_of_way,
+                                        priority=priority, junction=junction)
         res = ep.run(max_steps=max_steps)
         res.update(dl=engine.course_dl.cpu().numpy(), margin=ep.margin)
         torch.cuda.synchronize(engine.device)

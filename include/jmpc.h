@@ -380,6 +380,49 @@ int32_t jmpc_scene_plans(jmpc_handle h, int32_t B, int32_t k, int32_t T, const d
                          const int32_t* warm, const int32_t* done, const double* params, const double* obstacles,
                          int32_t n_obs, double* plans_out, void* stream);
 
+/* Right-of-way rules (opt-in): which scene mates a vehicle yields to.  Without a rule every vehicle cuts its course in
+ * front of every mate whose prediction crosses it, so two vehicles that cross both stop and wait for each other.
+ * A rule sets a per-episode consider mask, consider [B] int32: bit s set = obstacle slot s takes part in the episode's
+ * collision cut (jmpc_collision_masked).  It changes nothing else: the mate rows, the outcome record (contacts with
+ * ignored mates are still measured) and obstacle_history stay as they are.
+ *   Always considered: the extras (slots k - 1 ..; they do not react) and parked mates (done != 0 at the collision
+ *   instant).  A moving mate m is considered by b only if m comes before b in the scene's total order of keys
+ *   (cls, key, episode index), compared lexicographically; so the first vehicle of a scene yields only to parked cars
+ *   and extras, and no cycle of waiting forms between moving vehicles.  The mask has every bit set except the mate
+ *   slots b ignores; a finished episode (done != 0) gets -1.  Mate slot s is mate s of jmpc_scene_exchange.
+ *   JMPC_ROW_FIXED: cls 0, key = priority[b] (finite).
+ *   JMPC_ROW_FIRST_COME: zone [B][2] = (entry, exit) from jmpc_right_of_way_init, a = agent_idx[b], dl = params
+ *     JMPC_P_DL of b: committed (a >= entry; inside the zone or past it) cls 0, key (exit - a) * dl, so the vehicle
+ *     closest to leaving or furthest past the zone goes first; approaching (a < entry) cls 1, key (entry - a) * dl;
+ *     a course that never enters the zone (entry = -1) cls 2: it yields to every moving mate.  Distances are course
+ *     indices x dl, the arc length on the uniformly resampled courses.
+ * jmpc_right_of_way_init writes zone_out [B][2]: the first and last index i of episode b's course (course_id [B] or
+ *   NULL = course 0) with dx * dx + dy * dy <= r * r, dx = cx[i] - x, dy = cy[i] - y, evaluated without fused
+ *   multiply-add; -1 / -1 when no point is inside.  junction [n_junction][3] = (x, y, r): n_junction = 1 (one zone for
+ *   every scene) or B / k (scene b / k).  Enqueue it once the course ids are final.
+ * jmpc_right_of_way writes consider_out [B] from agent_idx, done (as jmpc_episode_pre leaves them), params
+ *   ([B][JMPC_NPARAM] or NULL: handle defaults; first_come reads JMPC_P_DL), zone (first_come) and priority [B]
+ *   (fixed).  k in [2, 9].  Timing: every iteration after jmpc_episode_pre and before jmpc_collision_masked; no
+ *   per-iteration host argument, so the call can be captured in a CUDA graph.
+ * jmpc_collision_masked: jmpc_collision (plans = NULL, n_planned = 0) or jmpc_collision_planned with every check, the
+ *   skip mask and the launch sizing of those, where only the slots whose bit is set in consider [B] (DEVICE, not NULL)
+ *   take part in the cut.  The result equals the same call on the considered rows (and plans) alone, in slot order; a
+ *   mask with no bit set among the n_obs slots gives flag = 0 and the full course length, as n_obs = 0 does. */
+enum jmpc_right_of_way_rule {
+  JMPC_ROW_FIXED = 1,            /* key = priority[b]                                                              */
+  JMPC_ROW_FIRST_COME = 2        /* committed before approaching, then by distance to the zone's exit / entry     */
+};
+int32_t jmpc_right_of_way_init(jmpc_handle h, int32_t B, int32_t k, const int32_t* course_id, const double* junction,
+                               int32_t n_junction, int32_t* zone_out, void* stream);
+int32_t jmpc_right_of_way(jmpc_handle h, int32_t B, int32_t k, int32_t rule, const int32_t* agent_idx,
+                          const int32_t* done, const double* params, const int32_t* zone, const double* priority,
+                          int32_t* consider_out, void* stream);
+int32_t jmpc_collision_masked(jmpc_handle h, int32_t B, const int32_t* course_id, const int32_t* agent_idx,
+                              const double* v, const double* obstacles, int32_t n_obs, const double* plans,
+                              int32_t n_planned, int32_t plan_len, const int32_t* consider, int32_t frame_window,
+                              int32_t margin, double horizon_s, const double* params, int32_t* flag,
+                              int32_t* course_len_out, void* stream);
+
 /* The reference's scripted obstacles on the device (main/lib/moving_obstacles.py: MovingObstacleTIntersection :166-232,
  * MovingObstacleRoundabout :28-123 including its dt = 0.2 quirk at :45 and the theta overwrite inside its steering
  * property, MovingObstacleArterial :125-164).  DEVICE pointers.
