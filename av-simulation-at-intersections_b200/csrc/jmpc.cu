@@ -242,24 +242,26 @@ __global__ void plant_step_kernel(int B, double* __restrict__ state, const doubl
   state[4 * b] = x; state[4 * b + 1] = y; state[4 * b + 2] = v; state[4 * b + 3] = yaw;
 }
 
-int refresh_circle_tables(jmpc_handle h) {
-  CK(cudaSetDevice(h->device));
-  for (int c = 0; c < h->n_courses; ++c) {
-    const size_t off = (size_t)c * h->course_stride;
-    const int n = h->course_n[c];
-    jmpc::circle_table_kernel<<<(n + 127) / 128, 128, 0, h->own_stream>>>(
-        n, h->d_cx + off, h->d_cy + off, h->d_cyaw + off, h->off_front, h->off_rear, h->d_ccfx + off,
-        h->d_ccfy + off, h->d_ccrx + off, h->d_ccry + off);
-    CK(cudaGetLastError());
-    h->launches++;
-  }
-  CK(cudaStreamSynchronize(h->own_stream));
+// Grid of the table kernels (jmpc_courses.cuh) over the uploaded courses: x = point, y = course.
+dim3 course_grid(jmpc_handle h, int threads) {
+  int max_n = 1;
+  for (int n : h->course_n) max_n = std::max(max_n, n);
+  return dim3((max_n + threads - 1) / threads, (unsigned)std::min(h->n_courses, 65535));
+}
+
+// Circle-centre tables of the uploaded courses for the handle's car geometry, on `st`.
+int build_circle_tables(jmpc_handle h, cudaStream_t st) {
+  jmpc::circle_tables_kernel<<<course_grid(h, 128), 128, 0, st>>>(
+      h->n_courses, h->course_stride, h->d_course_n, h->d_cx, h->d_cy, h->d_cyaw, h->off_front, h->off_rear, h->d_ccfx,
+      h->d_ccfy, h->d_ccrx, h->d_ccry);
+  CK(cudaGetLastError());
+  h->launches++;
   return 0;
 }
 
-// Arc-length tables of the uploaded courses (jmpc_collision.cuh: arc_table_kernel), N (N + 1) / 2 doubles per course;
-// courses are left without a table (the kernel then sums on the fly) once 256 MB are used.  Frees the old tables,
-// places the courses of h->course_n and allocates the new block; off[c] = -1 for a course without a table.
+// Arc-length tables of the uploaded courses, N (N + 1) / 2 doubles per course; courses are left without a table (the
+// kernel then sums on the fly) once 256 MB are used.  Frees the old tables, places the courses of h->course_n and
+// allocates the new block; off[c] = -1 for a course without a table.
 int place_arc_tables(jmpc_handle h, std::vector<long long>& off) {
   if (h->d_arc) { cudaFree(h->d_arc); h->d_arc = nullptr; }
   if (!h->d_arc_off) CK(cudaMalloc(&h->d_arc_off, (size_t)h->max_courses * sizeof(long long)));
@@ -277,21 +279,19 @@ int place_arc_tables(jmpc_handle h, std::vector<long long>& off) {
   return 0;
 }
 
-int refresh_arc_tables(jmpc_handle h) {
-  CK(cudaSetDevice(h->device));
+// The collision kernel's tables of the uploaded courses (h->n_courses, h->course_n, the course points on the device),
+// enqueued on `st`: arc-length tables, then circle-centre tables.
+int build_course_tables(jmpc_handle h, cudaStream_t st) {
   std::vector<long long> off;
   if (place_arc_tables(h, off)) return -1;
-  for (int c = 0; c < h->n_courses; ++c) {
-    if (off[c] < 0) continue;
-    const size_t coff = (size_t)c * h->course_stride;
-    const int n = h->course_n[c];
-    jmpc::arc_table_kernel<<<(n + 63) / 64, 64, 0, h->own_stream>>>(n, h->d_cx + coff, h->d_cy + coff, h->d_arc + off[c]);
+  CK(cudaMemcpyAsync(h->d_arc_off, off.data(), (size_t)h->n_courses * sizeof(long long), cudaMemcpyHostToDevice, st));
+  if (h->d_arc) {
+    jmpc::arc_tables_kernel<<<course_grid(h, 64), 64, 0, st>>>(h->n_courses, h->course_stride, h->d_course_n,
+                                                               h->d_arc_off, h->d_cx, h->d_cy, h->d_arc);
     CK(cudaGetLastError());
     h->launches++;
   }
-  CK(cudaMemcpyAsync(h->d_arc_off, off.data(), (size_t)h->n_courses * sizeof(long long), cudaMemcpyHostToDevice, h->own_stream));
-  CK(cudaStreamSynchronize(h->own_stream));
-  return 0;
+  return build_circle_tables(h, st);
 }
 
 template <typename F>
@@ -432,8 +432,9 @@ int32_t jmpc_set_courses(jmpc_handle h, int32_t n_courses, int32_t stride, const
   h->course_n.assign(len, len + n_courses);
   h->n_courses = n_courses;
   h->have_cv = false;                               // a speed profile belongs to the courses it was uploaded for
-  if (refresh_arc_tables(h)) return -1;
-  return refresh_circle_tables(h);
+  if (build_course_tables(h, st)) return -1;
+  CK(cudaStreamSynchronize(st));
+  return 0;
 }
 
 int32_t jmpc_set_course_speed(jmpc_handle h, int32_t n_courses, int32_t stride, const double* cv) {
@@ -459,7 +460,11 @@ int32_t jmpc_set_car_geometry(jmpc_handle h, double front_offset, double rear_of
   if (!h) return fail("jmpc_set_car_geometry: NULL handle");
   if (!(radius > 0)) return fail("jmpc_set_car_geometry: radius must be positive");
   h->off_front = front_offset; h->off_rear = rear_offset; h->radius = radius;
-  return h->n_courses ? refresh_circle_tables(h) : 0;
+  if (!h->n_courses) return 0;
+  CK(cudaSetDevice(h->device));
+  if (build_circle_tables(h, h->own_stream)) return -1;
+  CK(cudaStreamSynchronize(h->own_stream));
+  return 0;
 }
 
 namespace {
@@ -1256,6 +1261,74 @@ int32_t jmpc_scripted_obstacle_step(jmpc_handle h, int32_t B, int32_t n_obs, con
   return 0;
 }
 
+}  // extern "C"
+
+struct jmpc_planner_s {
+  int device = 0, max_B = 0, n_mp = 0, n_pts = 0, n_cc = 0;
+  int max_expansions = 0, max_path = 0, max_log = 0, pool_cap = 0, table_size = 0, max_traj = 0;
+  double *d_pts = nullptr, *d_len = nullptr, *d_cc = nullptr;                    // primitives
+  double* d_hp = nullptr; int* d_hp_n = nullptr; int* d_n_obs = nullptr;           // scenes
+  size_t hp_bytes = 0, hpn_bytes = 0, nobs_bytes = 0;
+  int n_scenes = 0, max_obs = 0;
+  jmpc::PlanNode* d_pool = nullptr; int* d_heap = nullptr; int* d_table = nullptr; // per-search workspace
+
+  // Per search: a node pool and a heap of pool_cap entries, a closed-set hash table of table_size slots (a power of
+  // two, at least 64 and 2 * max_expansions + 2) and max_traj trajectory points.
+  jmpc_planner_s(int device, int max_B, int n_mp, int n_pts, int n_cc, int max_expansions, int max_path, int max_log)
+      : device(device), max_B(max_B), n_mp(n_mp), n_pts(n_pts), n_cc(n_cc), max_expansions(max_expansions),
+        max_path(max_path), max_log(max_log), pool_cap(max_expansions * n_mp + 1), max_traj((max_path - 1) * (n_pts - 1)) {
+    table_size = 64;
+    while (table_size < 2 * max_expansions + 2) table_size <<= 1;
+  }
+};
+
+namespace {
+// (re)allocate *p to hold `bytes` when it is smaller
+template <typename T>
+int grow(T** p, size_t* have, size_t bytes) {
+  if (bytes <= *have) return 0;
+  if (*p) cudaFree(*p);
+  *p = nullptr; *have = 0;
+  CK(cudaMalloc(p, bytes));
+  *have = bytes;
+  return 0;
+}
+
+// B searches on planner p's primitives, scenes and workspace, enqueued on `st`.  The outputs are cleared first: the
+// kernel writes path / trajectory / log rows only as far as a search got.  e0 / e1, when given, bracket plan_kernel.
+int launch_plan(const jmpc_planner_s* p, int B, const int* scene_id, const double* start, const double* goal_point,
+                const double* goal_area, const double* allowed, const double* weights, double* cost, int* status,
+                int* n_path, double* path, int* path_mp, int* n_traj, double* traj, int* expansions, double* log,
+                cudaStream_t st, cudaEvent_t e0 = nullptr, cudaEvent_t e1 = nullptr) {
+  jmpc::PlanArgs a;
+  memset(&a, 0, sizeof a);
+  a.B = B; a.n_mp = p->n_mp; a.n_pts = p->n_pts; a.n_cc = p->n_cc; a.max_obs = p->max_obs; a.n_scenes = p->n_scenes;
+  a.max_expansions = p->max_expansions; a.max_path = p->max_path; a.max_traj = p->max_traj;
+  a.max_log = log ? p->max_log : 0;
+  a.pool_cap = p->pool_cap; a.table_size = p->table_size;
+  a.mp_pts = p->d_pts; a.mp_len = p->d_len; a.mp_cc = p->d_cc;
+  a.hp = p->d_hp; a.hp_n = p->d_hp_n; a.n_obs = p->d_n_obs;
+  a.scene_id = scene_id; a.start = start; a.goal_point = goal_point; a.goal_area = goal_area; a.allowed = allowed;
+  a.weights = weights;
+  a.pool = p->d_pool; a.heap = p->d_heap; a.table = p->d_table;
+  a.cost = cost; a.status = status; a.n_path = n_path; a.path = path; a.path_mp = path_mp; a.n_traj = n_traj;
+  a.traj = traj; a.expansions = expansions; a.log = a.max_log ? log : nullptr;
+  const size_t b = (size_t)B;
+  CK(cudaMemsetAsync(cost, 0, b * 8, st)); CK(cudaMemsetAsync(status, 0, b * 4, st)); CK(cudaMemsetAsync(n_path, 0, b * 4, st));
+  CK(cudaMemsetAsync(path, 0, b * p->max_path * 24, st)); CK(cudaMemsetAsync(path_mp, 0, b * p->max_path * 4, st));
+  CK(cudaMemsetAsync(n_traj, 0, b * 4, st)); CK(cudaMemsetAsync(traj, 0, b * a.max_traj * 24, st));
+  CK(cudaMemsetAsync(expansions, 0, b * 4, st));
+  if (a.log) CK(cudaMemsetAsync(log, 0, b * a.max_log * 40, st));
+  if (e0) CK(cudaEventRecord(e0, st));
+  jmpc::plan_kernel<<<(B + 3) / 4, 128, 0, st>>>(a);
+  CK(cudaGetLastError());
+  if (e1) CK(cudaEventRecord(e1, st));
+  return 0;
+}
+}  // namespace
+
+extern "C" {
+
 int32_t jmpc_plan_host(int32_t device, int32_t B, int32_t n_mp, int32_t n_pts, int32_t n_cc, const double* mp_pts,
                        const double* mp_len, const double* mp_cc, int32_t n_scenes, int32_t max_obs, const double* hp,
                        const int32_t* hp_n, const int32_t* n_obs, const int32_t* scene_id, const double* start,
@@ -1283,14 +1356,8 @@ int32_t jmpc_plan_host(int32_t device, int32_t B, int32_t n_mp, int32_t n_pts, i
   CK(cudaGetDeviceCount(&count));
   if (device < 0 || device >= count) return fail("jmpc_plan_host: no such CUDA device");
   CK(cudaSetDevice(device));
-  jmpc::PlanArgs a;
-  memset(&a, 0, sizeof a);
-  a.B = B; a.n_mp = n_mp; a.n_pts = n_pts; a.n_cc = n_cc; a.max_obs = max_obs; a.n_scenes = n_scenes;
-  a.max_expansions = max_expansions; a.max_path = max_path; a.max_traj = (max_path - 1) * (n_pts - 1); a.max_log = max_log;
-  a.pool_cap = max_expansions * n_mp + 1;
-  int ts = 64;
-  while (ts < 2 * max_expansions + 2) ts <<= 1;
-  a.table_size = ts;
+  jmpc_planner_s p(device, B, n_mp, n_pts, n_cc, max_expansions, max_path, max_log);
+  p.n_scenes = n_scenes; p.max_obs = max_obs;
   const size_t b = (size_t)B;
   // one device block [inputs | workspace | results]
   size_t off = 0;
@@ -1300,10 +1367,10 @@ int32_t jmpc_plan_host(int32_t device, int32_t B, int32_t n_mp, int32_t n_pts, i
   const size_t o_hp = seg(hp_doubles * 8), o_hpn = seg((size_t)n_scenes * max_obs * 4 + 4), o_nobs = seg((size_t)n_scenes * 4);
   const size_t o_sid = seg(b * 4), o_start = seg(b * 24), o_goal = seg(b * 24), o_area = seg(b * 32), o_allow = seg(b * 8);
   const size_t o_w = seg(b * 72);
-  const size_t o_pool = seg(b * a.pool_cap * sizeof(jmpc::PlanNode)), o_heap = seg(b * a.pool_cap * 4), o_tab = seg(b * ts * 4);
-  const size_t o_res = off;
+  const size_t o_pool = seg(b * p.pool_cap * sizeof(jmpc::PlanNode)), o_heap = seg(b * p.pool_cap * 4);
+  const size_t o_tab = seg(b * p.table_size * 4);
   const size_t o_cost = seg(b * 8), o_status = seg(b * 4), o_npath = seg(b * 4), o_path = seg(b * max_path * 24);
-  const size_t o_pmp = seg(b * max_path * 4), o_ntraj = seg(b * 4), o_traj = seg(b * a.max_traj * 24), o_exp = seg(b * 4);
+  const size_t o_pmp = seg(b * max_path * 4), o_ntraj = seg(b * 4), o_traj = seg(b * p.max_traj * 24), o_exp = seg(b * 4);
   const size_t o_log = seg(log ? b * max_log * 40 : 0);
   char* d = nullptr;
   cudaError_t err = cudaMalloc(&d, off);
@@ -1325,26 +1392,17 @@ int32_t jmpc_plan_host(int32_t device, int32_t B, int32_t n_mp, int32_t n_pts, i
   if (scene_id) up(o_sid, scene_id, b * 4);
   up(o_start, start, b * 24); up(o_goal, goal_point, b * 24); up(o_area, goal_area, b * 32); up(o_allow, allowed, b * 8);
   up(o_w, weights, b * 72);
-  if (!rc) {
-    a.mp_pts = (const double*)(d + o_pts); a.mp_len = (const double*)(d + o_len); a.mp_cc = (const double*)(d + o_cc);
-    a.hp = (const double*)(d + o_hp); a.hp_n = (const int*)(d + o_hpn); a.n_obs = (const int*)(d + o_nobs);
-    a.scene_id = scene_id ? (const int*)(d + o_sid) : nullptr;
-    a.start = (const double*)(d + o_start); a.goal_point = (const double*)(d + o_goal); a.goal_area = (const double*)(d + o_area);
-    a.allowed = (const double*)(d + o_allow); a.weights = (const double*)(d + o_w);
-    a.pool = (jmpc::PlanNode*)(d + o_pool); a.heap = (int*)(d + o_heap); a.table = (int*)(d + o_tab);
-    a.cost = (double*)(d + o_cost); a.status = (int*)(d + o_status); a.n_path = (int*)(d + o_npath); a.path = (double*)(d + o_path);
-    a.path_mp = (int*)(d + o_pmp); a.n_traj = (int*)(d + o_ntraj); a.traj = (double*)(d + o_traj); a.expansions = (int*)(d + o_exp);
-    a.log = log ? (double*)(d + o_log) : nullptr;
-    if (cudaMemsetAsync(d + o_res, 0, off - o_res, st) != cudaSuccess) rc = fail("jmpc_plan_host: memset failed");
-  }
-  if (!rc) {
-    cudaEventRecord(e0, st);
-    jmpc::plan_kernel<<<(B + 3) / 4, 128, 0, st>>>(a);
-    cudaEventRecord(e1, st);
-    if ((err = cudaGetLastError()) != cudaSuccess) rc = fail("jmpc_plan_host: launch failed", err);
-  }
+  p.d_pts = (double*)(d + o_pts); p.d_len = (double*)(d + o_len); p.d_cc = (double*)(d + o_cc);
+  p.d_hp = (double*)(d + o_hp); p.d_hp_n = (int*)(d + o_hpn); p.d_n_obs = (int*)(d + o_nobs);
+  p.d_pool = (jmpc::PlanNode*)(d + o_pool); p.d_heap = (int*)(d + o_heap); p.d_table = (int*)(d + o_tab);
+  if (!rc && launch_plan(&p, B, scene_id ? (const int*)(d + o_sid) : nullptr, (const double*)(d + o_start),
+                         (const double*)(d + o_goal), (const double*)(d + o_area), (const double*)(d + o_allow),
+                         (const double*)(d + o_w), (double*)(d + o_cost), (int*)(d + o_status), (int*)(d + o_npath),
+                         (double*)(d + o_path), (int*)(d + o_pmp), (int*)(d + o_ntraj), (double*)(d + o_traj),
+                         (int*)(d + o_exp), log ? (double*)(d + o_log) : nullptr, st, e0, e1))
+    rc = -1;
   down(cost, o_cost, b * 8); down(status, o_status, b * 4); down(n_path, o_npath, b * 4); down(path, o_path, b * max_path * 24);
-  down(path_mp, o_pmp, b * max_path * 4); down(n_traj, o_ntraj, b * 4); down(traj, o_traj, b * a.max_traj * 24);
+  down(path_mp, o_pmp, b * max_path * 4); down(n_traj, o_ntraj, b * 4); down(traj, o_traj, b * p.max_traj * 24);
   down(expansions, o_exp, b * 4);
   if (log) down(log, o_log, b * max_log * 40);
   if (!rc && (err = cudaStreamSynchronize(st)) != cudaSuccess) rc = fail("jmpc_plan_host: kernel failed", err);
@@ -1355,33 +1413,6 @@ int32_t jmpc_plan_host(int32_t device, int32_t B, int32_t n_mp, int32_t n_pts, i
   cudaFree(d);
   return rc;
 }
-
-}  // extern "C"
-
-struct jmpc_planner_s {
-  int device = 0, max_B = 0, n_mp = 0, n_pts = 0, n_cc = 0;
-  int max_expansions = 0, max_path = 0, max_log = 0, pool_cap = 0, table_size = 0;
-  double *d_pts = nullptr, *d_len = nullptr, *d_cc = nullptr;                    // primitives
-  double* d_hp = nullptr; int* d_hp_n = nullptr; int* d_n_obs = nullptr;           // scenes
-  size_t hp_bytes = 0, hpn_bytes = 0, nobs_bytes = 0;
-  int n_scenes = 0, max_obs = 0;
-  jmpc::PlanNode* d_pool = nullptr; int* d_heap = nullptr; int* d_table = nullptr; // per-search workspace
-};
-
-namespace {
-// (re)allocate *p to hold `bytes` when it is smaller
-template <typename T>
-int grow(T** p, size_t* have, size_t bytes) {
-  if (bytes <= *have) return 0;
-  if (*p) cudaFree(*p);
-  *p = nullptr; *have = 0;
-  CK(cudaMalloc(p, bytes));
-  *have = bytes;
-  return 0;
-}
-}  // namespace
-
-extern "C" {
 
 int32_t jmpc_planner_create(int32_t device, int32_t max_B, int32_t n_mp, int32_t n_pts, int32_t n_cc, const double* mp_pts,
                             const double* mp_len, const double* mp_cc, int32_t max_expansions, int32_t max_path,
@@ -1396,21 +1427,15 @@ int32_t jmpc_planner_create(int32_t device, int32_t max_B, int32_t n_mp, int32_t
   CK(cudaGetDeviceCount(&count));
   if (device < 0 || device >= count) return fail("jmpc_planner_create: no such CUDA device");
   CK(cudaSetDevice(device));
-  jmpc_planner p = new (std::nothrow) jmpc_planner_s();
+  jmpc_planner p = new (std::nothrow) jmpc_planner_s(device, max_B, n_mp, n_pts, n_cc, max_expansions, max_path, max_log);
   if (!p) return fail("jmpc_planner_create: out of host memory");
-  p->device = device; p->max_B = max_B; p->n_mp = n_mp; p->n_pts = n_pts; p->n_cc = n_cc;
-  p->max_expansions = max_expansions; p->max_path = max_path; p->max_log = max_log;
-  p->pool_cap = max_expansions * n_mp + 1;                  // as jmpc_plan_host sizes them
-  int ts = 64;
-  while (ts < 2 * max_expansions + 2) ts <<= 1;
-  p->table_size = ts;
   const size_t b = (size_t)max_B, pts = (size_t)n_mp * n_pts * 3, cc = (size_t)n_mp * n_cc * 2;
   cudaError_t e;
   if ((e = cudaMalloc(&p->d_pts, pts * 8)) != cudaSuccess || (e = cudaMalloc(&p->d_len, (size_t)n_mp * 8)) != cudaSuccess ||
       (e = cudaMalloc(&p->d_cc, cc * 8)) != cudaSuccess ||
       (e = cudaMalloc(&p->d_pool, b * p->pool_cap * sizeof(jmpc::PlanNode))) != cudaSuccess ||
       (e = cudaMalloc(&p->d_heap, b * p->pool_cap * sizeof(int))) != cudaSuccess ||
-      (e = cudaMalloc(&p->d_table, b * ts * sizeof(int))) != cudaSuccess ||
+      (e = cudaMalloc(&p->d_table, b * p->table_size * sizeof(int))) != cudaSuccess ||
       (e = cudaMemcpy(p->d_pts, mp_pts, pts * 8, cudaMemcpyHostToDevice)) != cudaSuccess ||
       (e = cudaMemcpy(p->d_len, mp_len, (size_t)n_mp * 8, cudaMemcpyHostToDevice)) != cudaSuccess ||
       (e = cudaMemcpy(p->d_cc, mp_cc, cc * 8, cudaMemcpyHostToDevice)) != cudaSuccess) {
@@ -1465,30 +1490,8 @@ int32_t jmpc_plan(jmpc_planner p, int32_t B, const int32_t* scene_id, const doub
   if (p->n_scenes < 1) return fail("jmpc_plan: no scenes (jmpc_planner_set_scenes)");
   if (B == 0) return 0;
   CK(cudaSetDevice(p->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  jmpc::PlanArgs a;
-  memset(&a, 0, sizeof a);
-  a.B = B; a.n_mp = p->n_mp; a.n_pts = p->n_pts; a.n_cc = p->n_cc; a.max_obs = p->max_obs; a.n_scenes = p->n_scenes;
-  a.max_expansions = p->max_expansions; a.max_path = p->max_path; a.max_traj = (p->max_path - 1) * (p->n_pts - 1);
-  a.max_log = log ? p->max_log : 0;
-  a.pool_cap = p->pool_cap; a.table_size = p->table_size;
-  a.mp_pts = p->d_pts; a.mp_len = p->d_len; a.mp_cc = p->d_cc;
-  a.hp = p->d_hp; a.hp_n = p->d_hp_n; a.n_obs = p->d_n_obs;
-  a.scene_id = scene_id; a.start = start; a.goal_point = goal_point; a.goal_area = goal_area; a.allowed = allowed;
-  a.weights = weights;
-  a.pool = p->d_pool; a.heap = p->d_heap; a.table = p->d_table;
-  a.cost = cost; a.status = status; a.n_path = n_path; a.path = path; a.path_mp = path_mp; a.n_traj = n_traj;
-  a.traj = traj; a.expansions = expansions; a.log = a.max_log ? log : nullptr;
-  // the kernel writes path / trajectory / log rows only as far as a search got: clear them, as jmpc_plan_host does
-  const size_t b = (size_t)B;
-  CK(cudaMemsetAsync(cost, 0, b * 8, st)); CK(cudaMemsetAsync(status, 0, b * 4, st)); CK(cudaMemsetAsync(n_path, 0, b * 4, st));
-  CK(cudaMemsetAsync(path, 0, b * p->max_path * 24, st)); CK(cudaMemsetAsync(path_mp, 0, b * p->max_path * 4, st));
-  CK(cudaMemsetAsync(n_traj, 0, b * 4, st)); CK(cudaMemsetAsync(traj, 0, b * a.max_traj * 24, st));
-  CK(cudaMemsetAsync(expansions, 0, b * 4, st));
-  if (a.log) CK(cudaMemsetAsync(log, 0, b * a.max_log * 40, st));
-  jmpc::plan_kernel<<<(B + 3) / 4, 128, 0, st>>>(a);
-  CK(cudaGetLastError());
-  return 0;
+  return launch_plan(p, B, scene_id, start, goal_point, goal_area, allowed, weights, cost, status, n_path, path, path_mp,
+                     n_traj, traj, expansions, log, (cudaStream_t)stream);
 }
 
 int32_t jmpc_set_courses_device(jmpc_handle h, int32_t n_courses, int32_t traj_stride, const int32_t* n_traj,
@@ -1514,23 +1517,7 @@ int32_t jmpc_set_courses_device(jmpc_handle h, int32_t n_courses, int32_t traj_s
   h->course_n.assign(lens, lens + n_courses);
   h->n_courses = n_courses;
   h->have_cv = false;
-  int max_n = 1;
-  for (int c = 0; c < n_courses; ++c) max_n = std::max(max_n, h->course_n[c]);
-  std::vector<long long> off;
-  if (place_arc_tables(h, off)) return -1;
-  CK(cudaMemcpyAsync(h->d_arc_off, off.data(), (size_t)n_courses * sizeof(long long), cudaMemcpyHostToDevice, st));
-  const unsigned gy = (unsigned)std::min(n_courses, 65535);
-  if (h->d_arc) {
-    jmpc::arc_tables_kernel<<<dim3((max_n + 63) / 64, gy), 64, 0, st>>>(n_courses, h->course_stride, h->d_course_n,
-                                                                      h->d_arc_off, h->d_cx, h->d_cy, h->d_arc);
-    CK(cudaGetLastError());
-    h->launches++;
-  }
-  jmpc::circle_tables_kernel<<<dim3((max_n + 127) / 128, gy), 128, 0, st>>>(
-      n_courses, h->course_stride, h->d_course_n, h->d_cx, h->d_cy, h->d_cyaw, h->off_front, h->off_rear, h->d_ccfx,
-      h->d_ccfy, h->d_ccrx, h->d_ccry);
-  CK(cudaGetLastError());
-  h->launches++;
+  if (build_course_tables(h, st)) return -1;
   // the *_host entry points run on the handle's own stream: order it after the tables without a host wait
   cudaEvent_t ev;
   CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));

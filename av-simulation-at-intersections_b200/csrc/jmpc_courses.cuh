@@ -1,5 +1,6 @@
-// jmpc_courses.cuh -- planned courses into the controller's course tables on the device (jmpc_set_courses_device), and
-// the episode start on them (jmpc_episode_init_from_courses).
+// jmpc_courses.cuh -- course tables on the device: planned courses into the controller's course tables
+// (jmpc_set_courses_device), the collision kernel's circle-centre and arc-length tables of all uploaded courses (both
+// jmpc_set_courses and jmpc_set_courses_device), and the episode start on them (jmpc_episode_init_from_courses).
 //
 // Reference (relative to SaeedRahmani/AV-Simulation-at-Intersections):
 //   main/scenarios/mpc_intersection.py:63-79   plan, dl of the first segment, MPC(trajectory_full), State at its start
@@ -7,8 +8,8 @@
 //
 // What the host pipeline did per course (slice the planner's output, unwrap the yaw in a Python loop, upload through a
 // pinned row, one table kernel per course) is three launches for all courses here: course_ingest_kernel (one warp per
-// course: AoS -> SoA copy by the lanes, the sequential unwrap by lane 0), then circle_tables_kernel and
-// arc_tables_kernel with the course index in the grid's y dimension.
+// course: AoS -> SoA copy by the lanes, the sequential unwrap by lane 0), then arc_tables_kernel and
+// circle_tables_kernel with the course index in the grid's y dimension.
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
@@ -81,12 +82,18 @@ __global__ void circle_tables_kernel(int n_courses, int stride, const int* __res
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   for (int c = blockIdx.y; c < n_courses; c += gridDim.y) {
     if (i >= course_n[c]) continue;
-    const size_t o = (size_t)c * stride;
-    circle_table_point(i, cx + o, cy + o, cyaw + o, off_front, off_rear, fx + o, fy + o, rx + o, ry + o);
+    const size_t k = (size_t)c * stride + i;
+    double s, co;
+    sincos(cyaw[k], &s, &co);
+    circle_centre(cx[k], cy[k], co, s, off_front, fx[k], fy[k]);
+    circle_centre(cx[k], cy[k], co, s, off_rear, rx[k], ry[k]);
   }
 }
 
-// Arc-length tables of every course that has a slot (arc_off[c] >= 0): x = start index, y = course.
+// Arc-length tables of every course that has a slot (arc_off[c] >= 0): x = start index, y = course.  Row a0 is the
+// running arc length of trajectory_full[a0:], np.cumsum of the segment lengths, i.e. strictly sequential float64 adds
+// starting at a0 (the partial sums depend on a0 through rounding, so every row is summed on its own).  The collision
+// kernel then reads the row instead of letting one lane re-do up to N sequential adds per instance.
 __global__ void arc_tables_kernel(int n_courses, int stride, const int* __restrict__ course_n,
                                   const long long* __restrict__ arc_off, const double* __restrict__ cx,
                                   const double* __restrict__ cy, double* __restrict__ tab) {
@@ -94,8 +101,19 @@ __global__ void arc_tables_kernel(int n_courses, int stride, const int* __restri
   for (int c = blockIdx.y; c < n_courses; c += gridDim.y) {
     const int N = course_n[c];
     if (a0 >= N || arc_off[c] < 0) continue;
-    const size_t o = (size_t)c * stride;
-    arc_table_row(a0, N, cx + o, cy + o, tab + arc_off[c]);
+    const double* x = cx + (size_t)c * stride;
+    const double* y = cy + (size_t)c * stride;
+    double* row = tab + arc_off[c] + arc_row_offset(a0, N);
+    double acc = 0.0;
+    for (int i = 0; i < N - a0; ++i) {
+      double seg = 0.0;
+      if (i > 0) {
+        const double dx = x[a0 + i] - x[a0 + i - 1], dy = y[a0 + i] - y[a0 + i - 1];
+        seg = sqrt(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
+      }
+      acc = __dadd_rn(acc, seg);
+      row[i] = acc;
+    }
   }
 }
 

@@ -140,7 +140,8 @@ __global__ void __launch_bounds__(128) plan_kernel(const PlanArgs A) {
   int* table = A.table + (size_t)b * A.table_size;
   const int mask = A.table_size - 1;
   for (int i = lane; i < A.table_size; i += 32) table[i] = -1;
-  const int scene = A.scene_id ? min(max(A.scene_id[b], 0), A.n_scenes - 1) : 0;     // validated on the host by jmpc_plan_host
+  // jmpc_plan_host rejects an out-of-range scene id on the host; jmpc_plan's ids live on the device and are clamped here
+  const int scene = A.scene_id ? min(max(A.scene_id[b], 0), A.n_scenes - 1) : 0;
   const double* hp = A.hp + (size_t)scene * A.max_obs * JMPC_PLAN_MAX_HP * 3;
   const int* hp_n = A.hp_n + (size_t)scene * A.max_obs;
   const int n_obs = A.n_obs[scene];

@@ -35,7 +35,7 @@ torch.cuda.synchronize()
 # config 3: flag kernel, step kernel T = 13, plant; closed loop kernels on the same batch
 w = synth.make_workload(3)
 B = w["B"]
-mpc3 = BatchedMPC(w["courses"], dl=w["dl"], T=13, max_batch=B)          # arc_table_kernel + circle_table_kernel
+mpc3 = BatchedMPC(w["courses"], dl=w["dl"], T=13, max_batch=B)          # arc_tables_kernel + circle_tables_kernel
 state, tgt = t(w["state"], torch.float64), t(w["target_ind"], torch.int32)
 oa, od = t(w["oa"], torch.float64), t(w["od"], torch.float64)
 agent, v, obs = t(w["agent_idx"], torch.int32), t(w["state"][:, 2], torch.float64), t(w["obstacles"], torch.float64)
