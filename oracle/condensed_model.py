@@ -283,8 +283,29 @@ def _assemble_K_cum(T, P, w):
 
 def ipm_solve(c: CondensedQP, max_iter: int = 40, mu_tol: float = 1e-13, s_min: float = 1e-2, lam0: float = 1.0,
               cumulative: bool = False):
-    """Returns (u, iterations, converged).  `cumulative`: iterate in the kernel's unknowns [s; delta] (c.P, c.q must
-    then be the Hessian / linear term in those unknowns); the result is still returned as controls [a; delta]."""
+    """Returns (u, iterations, converged) of `ipm_solve_exit` with the kernel's default tolerances."""
+    return ipm_solve_exit(c, max_iter=max_iter, mu_tol=mu_tol, s_min=s_min, lam0=lam0, cumulative=cumulative)[:3]
+
+
+def ipm_solve_exit(c: CondensedQP, max_iter: int = 40, mu_tol: float = 1e-13, s_min: float = 1e-2, lam0: float = 1.0,
+                   cumulative: bool = False, tol_res: float = 1e-9, init_mu: float = 0.0):
+    """Returns (u, iterations, converged, exit).  `cumulative`: iterate in the kernel's unknowns [s; delta] (c.P, c.q must
+    then be the Hessian / linear term in those unknowns); the result is still returned as controls [a; delta].
+
+    The exits are those of step_solve in csrc/jmpc_step.cuh, tested in the same order on the same quantities:
+
+      "strict"           mu <= mu_tol, every primal row <= tol_res, dual residual <= tol_res * gscale;
+      "complementarity"  mu <= 1e-3 mu_tol with the primal rows strict;
+      "reduced"          the iteration cap, with the last iterate tested inside mu <= 1e-9, rows <= 1e-7 and
+                         dual <= 1e-7 gscale (accepted: the kernel reports the solve as converged);
+      "breakdown"        the factorisation fails (a non-positive pivot in the kernel, numpy's cholesky raising here) on
+                         an iterate with mu <= 1e-11, rows and dual <= 1e-9 (times gscale);
+      "cap"              the iteration cap without the reduced tolerances (a failed solve);
+      "diverged"         the factorisation fails anywhere else: the kernel patches the pivot and carries on, which this
+                         model cannot follow (a failed solve here, whatever the kernel makes of it).
+
+    gscale = 1 + max |q|.  `iterations` counts the completed Newton steps, as the kernel's `iters` output does.
+    `init_mu > 0` starts the multipliers centred at init_mu / s, as the kernel does; otherwise at `lam0`."""
     T = len(c.q) // 2
     n = 2 * T
     _rows_apply, _rows_apply_T, _assemble_K = ((_rows_apply_cum, _rows_apply_T_cum, _assemble_K_cum) if cumulative else
@@ -298,27 +319,39 @@ def ipm_solve(c: CondensedQP, max_iter: int = 40, mu_tol: float = 1e-13, s_min: 
     z = _rows_apply(T, u)
     sh = np.maximum(hi - z, s_min)
     sl = np.maximum(z - lo, s_min)
-    lh = np.where(live, lam0, 0.0)
-    ll = np.where(live, lam0, 0.0)
+    if init_mu > 0.0:
+        lh = np.where(live, init_mu / sh, 0.0)
+        ll = np.where(live, init_mu / sl, 0.0)
+    else:
+        lh = np.where(live, lam0, 0.0)
+        ll = np.where(live, lam0, 0.0)
     gscale = 1.0 + np.abs(c.q).max()
-    ok = False
-    it = 0
-    for it in range(1, max_iter + 1):
+
+    def result(it, ok, kind):
+        return (cumulative_transform(T) @ u if cumulative else u), it, ok, kind
+
+    acceptable = False
+    for it in range(max_iter):
         z = _rows_apply(T, u)
         rd = c.P @ u + c.q + _rows_apply_T(T, np.where(live, lh - ll, 0.0))
         rph = np.where(live, z + sh - hi, 0.0)
         rpl = np.where(live, -z + sl + lo, 0.0)
         mu = float((lh * sh + ll * sl)[live].sum()) / nrow
-        if mu <= mu_tol and max(np.abs(rph).max(), np.abs(rpl).max()) <= 1e-9 and np.abs(rd).max() <= 1e-9 * gscale:
-            ok = True
-            it -= 1
-            break
+        rp = max(np.abs(rph).max(), np.abs(rpl).max())
+        rdm = np.abs(rd).max()
+        if mu <= mu_tol and rp <= tol_res and rdm <= tol_res * gscale:
+            return result(it, True, "strict")
+        if mu <= 1e-3 * mu_tol and rp <= tol_res:
+            return result(it, True, "complementarity")
+        acceptable = mu <= 1e-9 and rp <= 1e-7 and rdm <= 1e-7 * gscale
         w = np.where(live, lh / sh + ll / sl, 0.0)
         K = _assemble_K(T, c.P, w)
         try:
             Lc = np.linalg.cholesky(K)
         except np.linalg.LinAlgError:
-            break
+            if mu <= 1e-11 and rp <= 1e-9 and rdm <= 1e-9 * gscale:
+                return result(it, True, "breakdown")
+            return result(it, False, "diverged")
 
         def newton(rch, rcl):
             th = np.where(live, (-rch + lh * rph) / sh, 0.0)
@@ -350,6 +383,6 @@ def ipm_solve(c: CondensedQP, max_iter: int = 40, mu_tol: float = 1e-13, s_min: 
         u = u + alpha * du
         sh, sl = sh + alpha * dsh, sl + alpha * dsl
         lh, ll = lh + alpha * dlh, ll + alpha * dll
-    if cumulative:
-        u = cumulative_transform(T) @ u
-    return u, it, ok
+    # the cap: the kernel reports the last iterate it tested against the reduced tolerances as converged (the step
+    # taken after that test is not undone, nor is the iterate it leads to tested)
+    return result(max_iter, acceptable, "reduced" if acceptable else "cap")

@@ -1,9 +1,11 @@
 """CPU check of the algorithm the CUDA kernel runs: exact condensing of the reference QP and the predictor-corrector
 iteration (oracle/condensed_model.py is the numpy model of both) against the sparse-form oracle."""
+import dataclasses
+
 import numpy as np
 import pytest
 
-from helpers import default_vector, params_from_vector, scaled_err
+from helpers import default_vector, make_pool, params_from_vector, scaled_err
 from oracle import condensed_model as CM
 from oracle import mpc_oracle as O
 from oracle.qp import solve_qp
@@ -105,3 +107,59 @@ def test_interior_point_iterates_do_not_depend_on_the_unknowns(cases):
         np.testing.assert_allclose(u_s, u_a, rtol=0, atol=1e-7)
         T = p.T
         assert scaled_err(u_s[:T], r.oa) <= 1.0 and scaled_err(u_s[T:], r.od) <= 1.0
+
+
+def _model_against_oracle(args):
+    pv, T, state, oa, od, course, n, target = args
+    p = params_from_vector(pv, T)
+    r = O.mpc_step(p, state, oa, od, course[:n, 0], course[:n, 1], course[:n, 2], int(target))
+    assert r.status == O.STATUS_OPTIMAL
+    cq = CM.condense(p, r.xref, r.xbar, state, r.reaches_end)
+    P, q = CM.condense_cumulative(p, r.xref, r.xbar, state, r.reaches_end)
+    u, it, ok, kind = CM.ipm_solve_exit(dataclasses.replace(cq, P=P, q=q), cumulative=True)
+    u_or = np.concatenate([r.oa, r.od])
+    f_star = CM.objective(cq, u_or)
+    # multipliers of the rows active at the oracle's optimum (least squares on P u + q + A_act' y = 0)
+    z = cq.A @ u_or
+    act = np.flatnonzero(np.minimum(cq.hi - z, z - cq.lo) <= 1e-7)
+    y = np.linalg.lstsq(cq.A[act].T, -(cq.P @ u_or + cq.q), rcond=None)[0] if len(act) else np.zeros(0)
+    return dict(gap=(CM.objective(cq, u) - f_star) / max(1.0, abs(f_star)), du=float(np.abs(u - u_or).max()),
+                exit=kind, ok=ok, iters=it, weakest=float(np.abs(y).min()) if len(y) else np.inf)
+
+
+def test_interior_point_model_is_as_accurate_as_the_certified_oracle():
+    """What the kernel's algorithm delivers, measured against the certified oracle (mpc_oracle + qp.solve_qp) on about
+    100 instances each of config 2, sweep points at T = 8 and 25 and the degenerate set (T = 13).  The model iterates
+    in the kernel's unknowns with the kernel's tolerances and all four of its exits.
+
+      * cost: (f(u_model) - f*) / max(1, |f*|) within 1e-10 (measured: -1.3e-12 .. 1.8e-12);
+      * exits: every solve ends at the strict or the complementarity exit, never at reduced tolerances;
+      * controls: within 1e-7 of the oracle's where every row active at the optimum carries a multiplier of at least
+        1e-3 (measured: at most 9.9e-9; 392 of the 400 instances).  Where an active row's multiplier vanishes (strict
+        complementarity fails: on config 2 the speed row of the last stage, which bounds the sum of all accelerations)
+        an interior point approaches the optimum along that row only at the rate of sqrt(mu), so at mu <= 1e-13 the
+        last acceleration can be off by ~1e-5 (measured: 1.5e-5 on config 2, 5.7e-7 at T = 8) while the cost is
+        within 1e-12.  Those instances are held to 1e-4.
+
+    Iterations: 5 to 20 (measured), every exit strict.
+
+    The GPU test of the kernel against this model (tests/test_gpu_solver_accuracy.py) relies on these figures: its tight
+    band belongs to the algorithm, not to luck."""
+    from junction_mpc import synth
+    sets = {"config2": synth.make_workload(2, B=100), "sweep_T8": synth.make_sweep(8, states_per_point=1, max_points=100),
+            "sweep_T25": synth.make_sweep(25, states_per_point=1, max_points=100),
+            "degenerate_T13": synth.make_degenerate(13, B=100)}
+    with make_pool() as pool:
+        for name, w in sets.items():
+            base = default_vector(w)
+            jobs = [(base if w["params"] is None else w["params"][k], w["T"], w["state"][k], w["oa"][k], w["od"][k],
+                     w["courses"][0], int(w["course_len"][k]), int(w["target_ind"][k])) for k in range(w["B"])]
+            res = pool.map(_model_against_oracle, jobs)
+            gap = np.array([r["gap"] for r in res])
+            du = np.array([r["du"] for r in res])
+            strict_compl = np.array([r["weakest"] >= 1e-3 for r in res])
+            assert all(r["ok"] and r["exit"] in ("strict", "complementarity") for r in res), name
+            assert np.abs(gap).max() <= 1e-10, (name, gap.min(), gap.max())
+            assert du[strict_compl].max() <= 1e-7, (name, np.sort(du[strict_compl])[-3:])
+            assert du.max() <= 1e-4, (name, du.max())
+            assert strict_compl.mean() >= 0.9, name
