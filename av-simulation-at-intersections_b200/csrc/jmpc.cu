@@ -593,6 +593,109 @@ bool is_pinned(jmpc_handle h, const void* p, void** mapped) {
   *mapped = at.devicePointer;
   return true;
 }
+
+// The host arrays of one *_host call, staged on the handle's stream.  Layout [inputs | outputs], 16-byte aligned, at
+// the same offsets on the device (d_stage) and in the handle's page-locked host block (h_stage).  Transfer modes
+// (jmpc_set_host_transfer):
+//   1  (default) inputs by cudaMemcpyAsync: page-locked ones straight from the caller's memory, the others through
+//      h_stage (one copy for the whole input region when no input is page-locked).  The kernels store their results
+//      directly into page-locked host memory through the device mapping (unified addressing): the caller's own array
+//      where that is page-locked (jmpc_host_alloc, cudaHostAlloc, torch pin_memory), the h_stage slot otherwise (one
+//      host memcpy).  A step warp writes ~1.7 KB when it is done with an instance; the stores ride under the other
+//      warps' solves, and at ~6 GB/s of results the PCIe link is far from saturated, so the device -> host transfer
+//      leaves the critical path (measured: 1.61 -> 1.43 ms per 4096-instance step).
+//   2  the kernels also read their inputs through the mapping: no copy ahead of the kernel, every warp waits a PCIe
+//      round trip when it picks an instance up instead.  Faster than 1 on large batches (65 536 instances at T = 13:
+//      4.26 instead of 4.44 ms per call), the same at 4096 and at 1 (profiles/r10_host_transfer.txt).
+//   0  staged DMA both ways (results to d_stage, cudaMemcpyAsync back).
+// Mode 1 runs as 0 when an output has no device mapping, mode 2 as 1 when an input has none.
+struct HostCall {
+  struct Seg { size_t off, bytes; void* host; bool pinned; void* mapped; };
+  jmpc_handle h;
+  Seg segs[20];                         // jmpc_step_host_io's 20 arrays
+  int ns = 0, first_out = 0;
+  size_t off = 0, in_end = 0;
+  bool zc_in = false, zc_out = false;
+
+  explicit HostCall(jmpc_handle h) : h(h) {}
+
+  // A NULL host array is an empty segment: nullptr on the device side.  Inputs are registered before outputs.
+  const Seg* add(size_t bytes, const void* host) {
+    Seg& s = segs[ns++];
+    s.off = off; s.bytes = host ? bytes : 0; s.host = const_cast<void*>(host); s.mapped = nullptr;
+    s.pinned = s.bytes && is_pinned(h, host, &s.mapped);
+    off += (s.bytes + 15) & ~size_t(15);
+    return &s;
+  }
+  const Seg* in(size_t bytes, const void* host) { const Seg* s = add(bytes, host); first_out = ns; in_end = off; return s; }
+  const Seg* out(size_t bytes, void* host) { return add(bytes, host); }
+
+  // Device addresses of segments k0 .. k1 - 1: the caller's mapping where page-locked, the h_stage slot otherwise.
+  // False when one has none.
+  bool map(int k0, int k1, char* hs_dev) {
+    for (int k = k0; k < k1; ++k) {
+      Seg& s = segs[k];
+      if (s.bytes && !s.pinned) s.mapped = hs_dev + s.off;
+      if (s.bytes && !s.mapped) return false;
+    }
+    return true;
+  }
+
+  // Sizes the staging blocks, picks the transfer paths and enqueues the input copies.
+  int upload() {
+    if (ensure_stage(h, off)) return -1;
+    char *hs = h->h_stage, *ds = h->d_stage, *hs_dev = nullptr;
+    zc_out = h->host_transfer >= 1;
+    if (zc_out && cudaHostGetDevicePointer((void**)&hs_dev, hs, 0) != cudaSuccess) { cudaGetLastError(); zc_out = false; }
+    zc_out = zc_out && map(first_out, ns, hs_dev);
+    zc_in = zc_out && h->host_transfer == 2 && map(0, first_out, hs_dev);
+    bool one_copy = !zc_in;
+    for (int k = 0; k < first_out; ++k) one_copy = one_copy && !segs[k].pinned;
+    for (int k = 0; k < first_out; ++k) {
+      const Seg& s = segs[k];
+      if (!s.bytes) continue;
+      if (!s.pinned) memcpy(hs + s.off, s.host, s.bytes);
+      if (!zc_in && !one_copy)
+        CK(cudaMemcpyAsync(ds + s.off, s.pinned ? s.host : hs + s.off, s.bytes, cudaMemcpyHostToDevice, h->own_stream));
+    }
+    if (one_copy) CK(cudaMemcpyAsync(ds, hs, in_end, cudaMemcpyHostToDevice, h->own_stream));
+    return 0;
+  }
+
+  // Kernel arguments: where an input is read and where an output is written.
+  const char* rd(const Seg* s) const { return s->bytes ? (zc_in ? (char*)s->mapped : h->d_stage + s->off) : nullptr; }
+  char* wr(const Seg* s) const { return s->bytes ? (zc_out ? (char*)s->mapped : h->d_stage + s->off) : nullptr; }
+
+  // After the launch: the staged download, if any, and the wait for the stream.
+  int wait() {
+    for (int k = first_out; k < ns && !zc_out; ++k) {
+      const Seg& s = segs[k];
+      if (!s.bytes) continue;
+      CK(cudaMemcpyAsync(s.pinned ? s.host : (void*)(h->h_stage + s.off), h->d_stage + s.off, s.bytes,
+                         cudaMemcpyDeviceToHost, h->own_stream));
+    }
+    CK(cudaStreamSynchronize(h->own_stream));
+    return 0;
+  }
+
+  // Results of the pageable outputs from h_stage.
+  void copy_out() const {
+    for (int k = first_out; k < ns; ++k)
+      if (segs[k].bytes && !segs[k].pinned) memcpy(segs[k].host, h->h_stage + segs[k].off, segs[k].bytes);
+  }
+};
+
+// Checks the host entry points share.  Host arrays can be validated (the device entry points clamp instead,
+// jmpc_step.cuh); the skip mask is a device array for the device entry points.
+int check_host_call(jmpc_handle h, const char* name, int B, const int32_t* course_id) {
+  const char* what = h->skip ? "a skip mask is set (jmpc_set_skip_mask is for the device entry points)" : nullptr;
+  for (int k = 0; course_id && !what && k < B; ++k)
+    if (course_id[k] < 0 || course_id[k] >= h->n_courses) what = "course_id out of range";
+  if (!what) return 0;
+  char msg[160];
+  snprintf(msg, sizeof msg, "%s: %s", name, what);
+  return fail(msg);
+}
 }  // namespace
 
 int32_t jmpc_debug_cycles(jmpc_handle h, uint64_t* out32, int32_t reset) {
@@ -693,30 +796,10 @@ int32_t jmpc_step_host_io(jmpc_handle h, int32_t B, int32_t T, const double* sta
       !xref || !cost || !status)
     return fail("jmpc_step_host: NULL array");
   if (h->n_courses < 1) return fail("jmpc_step_host: no courses uploaded (jmpc_set_courses)");
-  if (h->skip) return fail("jmpc_step_host: a skip mask is set (jmpc_set_skip_mask is for the device entry points)");
-  if (course_id)             // host arrays can be validated (the device entry points clamp instead, jmpc_step.cuh)
-    for (int k = 0; k < B; ++k)
-      if (course_id[k] < 0 || course_id[k] >= h->n_courses) return fail("jmpc_step_host: course_id out of range");
+  if (int rc = check_host_call(h, "jmpc_step_host", B, course_id)) return rc;
   if (B == 0) return 0;
   CK(cudaSetDevice(h->device));
   const size_t T1 = T + 1, b = (size_t)B;
-  // Staging block layout [inputs | outputs], the same offsets on the device (d_stage) and in the handle's
-  // page-locked host block (h_stage).  Transfer modes (jmpc_set_host_transfer):
-  //   1  (default) inputs by cudaMemcpyAsync into d_stage; the kernel stores its results directly into page-locked
-  //      host memory through the device mapping (unified addressing): the caller's own array where that is
-  //      page-locked (jmpc_host_alloc, cudaHostAlloc, torch pin_memory), the h_stage slot otherwise (one host
-  //      memcpy).  A warp writes ~1.7 KB when it is done with an instance; the stores ride under the other warps'
-  //      solves, and at ~6 GB/s of results the PCIe link is far from saturated, so the device -> host transfer
-  //      leaves the critical path (measured: 1.61 -> 1.43 ms per 4096-instance step).
-  //   2  the kernel also reads its inputs from page-locked host memory (no copy engine at all).  Measured slower
-  //      than 1: every warp waits a PCIe round trip when it picks an instance up (kernel 1.24 -> 1.30 ms).
-  //   0  staged DMA both ways (results to d_stage, cudaMemcpyAsync back).
-  // Instances that fail the index rule or are infeasible get their input values in oa_out / od_out / target_out
-  // (the kernel carries them over), so "in-out arrays keep their values" holds whether or not the arrays alias.
-  struct Seg { size_t off, bytes; void* host; bool pinned; void* mapped; };
-  size_t off = 0;
-  Seg segs[20];
-  int ns = 0;
 #ifdef JMPC_EXPERIMENT
   const bool timing = getenv("JMPC_TIMING") != nullptr;                 // host-side breakdown on stderr
 #else
@@ -725,99 +808,46 @@ int32_t jmpc_step_host_io(jmpc_handle h, int32_t B, int32_t T, const double* sta
   auto now = [] { return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   const double t_begin = timing ? now() : 0.0;
   const int mode = h->host_transfer;
-  auto seg = [&](size_t bytes, const void* host) -> Seg& {
-    Seg& s = segs[ns++];
-    s.off = off; s.bytes = host ? bytes : 0; s.host = const_cast<void*>(host);
-    s.mapped = nullptr;
-    s.pinned = host ? is_pinned(h, host, &s.mapped) : false;
-    off += (s.bytes + 15) & ~size_t(15);
-    return s;
-  };
-  const Seg& s_state = seg(b * 4 * 8, state);
-  const Seg& s_params = seg(b * JMPC_NPARAM * 8, params);
-  const Seg& s_cid = seg(b * 4, course_id);
-  const Seg& s_clen = seg(b * 4, course_len);
-  const Seg& s_warm = seg(b * 4, warm);
-  const Seg& s_oa_in = seg(b * T * 8, oa_in);
-  const Seg& s_od_in = seg(b * T * 8, od_in);
-  const Seg& s_tgt_in = seg(b * 4, target_in);
-  const int first_out = ns;
-  const size_t in_end = off;
-  const Seg& s_oa = seg(b * T * 8, oa_out);
-  const Seg& s_od = seg(b * T * 8, od_out);
-  const Seg& s_tgt = seg(b * 4, target_out);
-  const Seg& s_ox = seg(b * T1 * 8, ox);
-  const Seg& s_oy = seg(b * T1 * 8, oy);
-  const Seg& s_ov = seg(b * T1 * 8, ov);
-  const Seg& s_oyaw = seg(b * T1 * 8, oyaw);
-  const Seg& s_xref = seg(b * 4 * T1 * 8, xref);
-  const Seg& s_cost = seg(b * 8, cost);
-  const Seg& s_status = seg(b * 4, status);
-  const Seg& s_iters = seg(b * 4, iters);
-  const Seg& s_rec = seg(b * JMPC_RECORD_LEN * 8, record);
-  const size_t total = off;
-  if (ensure_stage(h, total)) return -1;
-  char* hs = h->h_stage; char* ds = h->d_stage;
+  // Instances that fail the index rule or are infeasible get their input values in oa_out / od_out / target_out
+  // (the kernel carries them over), so "in-out arrays keep their values" holds whether or not the arrays alias.
+  HostCall io(h);
+  auto s_state = io.in(b * 4 * 8, state);
+  auto s_params = io.in(b * JMPC_NPARAM * 8, params);
+  auto s_cid = io.in(b * 4, course_id);
+  auto s_clen = io.in(b * 4, course_len);
+  auto s_warm = io.in(b * 4, warm);
+  auto s_oa_in = io.in(b * T * 8, oa_in);
+  auto s_od_in = io.in(b * T * 8, od_in);
+  auto s_tgt_in = io.in(b * 4, target_in);
+  auto s_oa = io.out(b * T * 8, oa_out);
+  auto s_od = io.out(b * T * 8, od_out);
+  auto s_tgt = io.out(b * 4, target_out);
+  auto s_ox = io.out(b * T1 * 8, ox);
+  auto s_oy = io.out(b * T1 * 8, oy);
+  auto s_ov = io.out(b * T1 * 8, ov);
+  auto s_oyaw = io.out(b * T1 * 8, oyaw);
+  auto s_xref = io.out(b * 4 * T1 * 8, xref);
+  auto s_cost = io.out(b * 8, cost);
+  auto s_status = io.out(b * 4, status);
+  auto s_iters = io.out(b * 4, iters);
+  auto s_rec = io.out(b * JMPC_RECORD_LEN * 8, record);
+  if (int rc = io.upload()) return rc;
   cudaStream_t st = h->own_stream;
-  // device mappings of the page-locked arrays
-  char* hs_dev = nullptr;
-  bool map_ok = mode >= 1;
-  if (map_ok && cudaHostGetDevicePointer((void**)&hs_dev, hs, 0) != cudaSuccess) { cudaGetLastError(); map_ok = false; }
-  for (int k = 0; k < ns && map_ok; ++k) {
-    Seg& s = segs[k];
-    if (!s.bytes) continue;
-    if (s.pinned) { if (!s.mapped) map_ok = false; }
-    else s.mapped = hs_dev + s.off;
-  }
-  const bool zc_out = map_ok, zc_in = map_ok && mode >= 2;
-  // ---- inputs
-  if (zc_in) {
-    for (int k = 0; k < first_out; ++k)
-      if (segs[k].bytes && !segs[k].pinned) memcpy(hs + segs[k].off, segs[k].host, segs[k].bytes);
-  } else {
-    bool any_pinned_in = false;
-    for (int k = 0; k < first_out; ++k) any_pinned_in = any_pinned_in || (segs[k].bytes && segs[k].pinned);
-    if (!any_pinned_in) {
-      for (int k = 0; k < first_out; ++k)
-        if (segs[k].bytes) memcpy(hs + segs[k].off, segs[k].host, segs[k].bytes);
-      CK(cudaMemcpyAsync(ds, hs, in_end, cudaMemcpyHostToDevice, st));
-    } else {
-      for (int k = 0; k < first_out; ++k) {
-        const Seg& s = segs[k];
-        if (!s.bytes) continue;
-        const void* src = s.host;
-        if (!s.pinned) { memcpy(hs + s.off, s.host, s.bytes); src = hs + s.off; }
-        CK(cudaMemcpyAsync(ds + s.off, src, s.bytes, cudaMemcpyHostToDevice, st));
-      }
-    }
-  }
-  auto rp = [&](const Seg& s) -> char* { return s.bytes ? (zc_in ? (char*)s.mapped : ds + s.off) : nullptr; };    // read side
-  auto wp = [&](const Seg& s) -> char* { return s.bytes ? (zc_out ? (char*)s.mapped : ds + s.off) : nullptr; };   // write side
   const double t_prep = timing ? now() : 0.0;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   if (timing) { cudaEventCreate(&ev0); cudaEventCreate(&ev1); cudaEventRecord(ev0, st); }
-  int rc = launch_step(h, B, T, (const double*)rp(s_state), (const int*)rp(s_cid), (const int*)rp(s_clen),
-                       (const int*)rp(s_tgt_in), (int*)wp(s_tgt), (const int*)rp(s_warm), (const double*)rp(s_oa_in),
-                       (const double*)rp(s_od_in), (double*)wp(s_oa), (double*)wp(s_od), (const double*)rp(s_params),
-                       (double*)wp(s_ox), (double*)wp(s_oy), (double*)wp(s_ov), (double*)wp(s_oyaw), (double*)wp(s_xref),
-                       (double*)wp(s_cost), (int*)wp(s_status), (int*)wp(s_iters), (double*)wp(s_rec), st);
+  int rc = launch_step(h, B, T, (const double*)io.rd(s_state), (const int*)io.rd(s_cid), (const int*)io.rd(s_clen),
+                       (const int*)io.rd(s_tgt_in), (int*)io.wr(s_tgt), (const int*)io.rd(s_warm),
+                       (const double*)io.rd(s_oa_in), (const double*)io.rd(s_od_in), (double*)io.wr(s_oa),
+                       (double*)io.wr(s_od), (const double*)io.rd(s_params), (double*)io.wr(s_ox), (double*)io.wr(s_oy),
+                       (double*)io.wr(s_ov), (double*)io.wr(s_oyaw), (double*)io.wr(s_xref), (double*)io.wr(s_cost),
+                       (int*)io.wr(s_status), (int*)io.wr(s_iters), (double*)io.wr(s_rec), st);
   if (rc) return rc;
   if (timing) cudaEventRecord(ev1, st);
   const double t_launch = timing ? now() : 0.0;
-  // ---- results
-  if (!zc_out) {
-    for (int k = first_out; k < ns; ++k) {
-      const Seg& s = segs[k];
-      if (!s.bytes) continue;
-      CK(cudaMemcpyAsync(s.pinned ? s.host : (void*)(hs + s.off), ds + s.off, s.bytes, cudaMemcpyDeviceToHost, st));
-    }
-  }
-  CK(cudaStreamSynchronize(st));
+  if ((rc = io.wait())) return rc;
   const double t_sync = timing ? now() : 0.0;
-  for (int k = first_out; k < ns; ++k) {
-    const Seg& s = segs[k];
-    if (s.bytes && !s.pinned) memcpy(s.host, hs + s.off, s.bytes);
-  }
+  io.copy_out();
   if (timing) {
     float kms = 0.f;
     cudaEventElapsedTime(&kms, ev0, ev1);
@@ -944,67 +974,24 @@ int32_t jmpc_collision_host(jmpc_handle h, int32_t B, const int32_t* course_id, 
   if (!agent_idx || !v || !flag || !course_len_out) return fail("jmpc_collision_host: NULL array");
   if (n_obs < 0 || n_obs > jmpc::kMaxObstacles) return fail("jmpc_collision_host: n_obs out of range");
   if (n_obs > 0 && !obstacles) return fail("jmpc_collision_host: obstacles is NULL");
-  if (h->skip) return fail("jmpc_collision_host: a skip mask is set (jmpc_set_skip_mask is for the device entry points)");
-  if (course_id)
-    for (int k = 0; k < B; ++k)
-      if (course_id[k] < 0 || course_id[k] >= h->n_courses) return fail("jmpc_collision_host: course_id out of range");
+  if (int rc = check_host_call(h, "jmpc_collision_host", B, course_id)) return rc;
   if (B == 0) return 0;
   CK(cudaSetDevice(h->device));
   const size_t b = (size_t)B;
-  // Inputs: page-locked caller arrays (jmpc_host_alloc) are copied to the device straight from where they are, others
-  // through the handle's pinned block.  Results: the kernel stores flag / course_len_out into page-locked host memory
-  // through its device mapping (the caller's arrays when they are page-locked, the pinned block + one memcpy otherwise),
-  // as the step's host entry point does: no device->host copy pass.
-  struct Seg { size_t off, bytes; const void* host; bool pinned; void* mapped; };
-  Seg segs[7];
-  int ns = 0;
-  size_t off = 0;
-  auto seg = [&](size_t bytes, const void* host) -> Seg& {
-    Seg& s = segs[ns++];
-    s.off = off; s.bytes = host ? bytes : 0; s.host = host; s.mapped = nullptr;
-    s.pinned = (host && s.bytes) ? is_pinned(h, host, &s.mapped) : false;
-    off += (s.bytes + 15) & ~size_t(15);
-    return s;
-  };
-  const Seg& s_v = seg(b * 8, v);
-  const Seg& s_obs = seg(b * n_obs * 6 * 8, n_obs ? obstacles : nullptr);
-  const Seg& s_prm = seg(b * JMPC_NPARAM * 8, params);
-  const Seg& s_cid = seg(b * 4, course_id);
-  const Seg& s_idx = seg(b * 4, agent_idx);
-  const int first_out = ns;
-  Seg& s_flag = seg(b * 4, flag);
-  Seg& s_len = seg(b * 4, course_len_out);
-  if (ensure_stage(h, off)) return -1;
-  char* hs = h->h_stage; char* ds = h->d_stage;
-  cudaStream_t st = h->own_stream;
-  for (int k = 0; k < first_out; ++k) {
-    const Seg& s = segs[k];
-    if (!s.bytes) continue;
-    const void* src = s.host;
-    if (!s.pinned) { memcpy(hs + s.off, s.host, s.bytes); src = hs + s.off; }
-    CK(cudaMemcpyAsync(ds + s.off, src, s.bytes, cudaMemcpyHostToDevice, st));
-  }
-  char* hs_dev = nullptr;
-  bool zc_out = h->host_transfer >= 1;
-  if (zc_out && cudaHostGetDevicePointer((void**)&hs_dev, hs, 0) != cudaSuccess) { cudaGetLastError(); zc_out = false; }
-  for (int k = first_out; k < ns && zc_out; ++k) {
-    Seg& s = segs[k];
-    if (s.pinned) { if (!s.mapped) zc_out = false; }
-    else s.mapped = hs_dev + s.off;
-  }
-  auto rp = [&](const Seg& s) -> const char* { return s.bytes ? ds + s.off : nullptr; };
-  auto wp = [&](const Seg& s) -> char* { return zc_out ? (char*)s.mapped : ds + s.off; };
-  int rc = jmpc_collision(h, B, (const int*)rp(s_cid), (const int*)rp(s_idx), (const double*)rp(s_v),
-                          (const double*)rp(s_obs), n_obs, frame_window, margin, horizon_s, (const double*)rp(s_prm),
-                          (int*)wp(s_flag), (int*)wp(s_len), (void*)st);
-  if (rc) return rc;
-  if (!zc_out)
-    for (int k = first_out; k < ns; ++k)
-      CK(cudaMemcpyAsync(segs[k].pinned ? const_cast<void*>(segs[k].host) : (void*)(hs + segs[k].off), ds + segs[k].off,
-                         segs[k].bytes, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
-  for (int k = first_out; k < ns; ++k)
-    if (!segs[k].pinned) memcpy(const_cast<void*>(segs[k].host), hs + segs[k].off, segs[k].bytes);
+  HostCall io(h);
+  auto s_v = io.in(b * 8, v);
+  auto s_obs = io.in(b * n_obs * 6 * 8, n_obs ? obstacles : nullptr);
+  auto s_prm = io.in(b * JMPC_NPARAM * 8, params);
+  auto s_cid = io.in(b * 4, course_id);
+  auto s_idx = io.in(b * 4, agent_idx);
+  auto s_flag = io.out(b * 4, flag);
+  auto s_len = io.out(b * 4, course_len_out);
+  if (int rc = io.upload()) return rc;
+  int rc = jmpc_collision(h, B, (const int*)io.rd(s_cid), (const int*)io.rd(s_idx), (const double*)io.rd(s_v),
+                          (const double*)io.rd(s_obs), n_obs, frame_window, margin, horizon_s,
+                          (const double*)io.rd(s_prm), (int*)io.wr(s_flag), (int*)io.wr(s_len), (void*)h->own_stream);
+  if (rc || (rc = io.wait())) return rc;
+  io.copy_out();
   return 0;
 }
 

@@ -34,7 +34,10 @@ def _i32(a, shape=None):
 
 
 def _ptr(a):
-    return None if a is None else a.ctypes.data_as(C.c_void_p)
+    """Address of `a`'s data for a ctypes argument (None for None).  A plain integer costs half what `data_as` does,
+    which matters on the single-instance host step (20 arrays); it does not keep `a` alive, so every array handed to
+    a call is bound to a name until the call returns."""
+    return None if a is None else a.ctypes.data
 
 
 @dataclass
@@ -314,42 +317,21 @@ class BatchedMPC:
     # ---- host path --------------------------------------------------------------------------------------
     def step_host(self, state, target_ind, oa=None, od=None, course_id=None, course_len=None, warm=None,
                   params=None, T: Optional[int] = None, out: Optional[StepOutput] = None) -> StepOutput:
+        """One step per row of `state` [B, 4]; the inputs are only read.  Results go to fresh arrays, or into `out`
+        (e.g. page-locked ones from `host_outputs`) when it is given.  `oa` / `od` / `target_ind` may be `out`'s own
+        arrays (a closed loop feeding its previous solution back), in which case nothing is copied."""
         T = int(T or self.T)
-        if out is not None:
-            return self._step_host_into(out, T, state, target_ind, oa, od, course_id, course_len, warm, params)
         state = _f64(state)
         B = state.shape[0]
         if state.shape != (B, 4):
             raise ValueError("state must be [B, 4] (x, y, v, yaw)")
-        T1 = T + 1
-        if oa is None or od is None:
-            oa_b, od_b = np.zeros((B, T)), np.zeros((B, T))
-            warm = np.zeros(B, np.int32)
-        else:
-            oa_b, od_b = _f64(oa, (B, T)).copy(), _f64(od, (B, T)).copy()
-        tgt = _i32(target_ind, (B,)).copy()
-        cid = None if course_id is None else _i32(course_id, (B,))
-        clen = None if course_len is None else _i32(course_len, (B,))
-        wrm = None if warm is None else _i32(warm, (B,))
-        prm = None if params is None else _f64(params, (B, NPARAM))
-        ox, oy, ov, oyaw = (np.zeros((B, T1)) for _ in range(4))
-        xref = np.zeros((B, 4, T1))
-        cost = np.full(B, np.nan)
-        status = np.zeros(B, np.int32)
-        iters = np.zeros(B, np.int32)
-        record = np.zeros((B, _cabi.RECORD_LEN))
-        _cabi.check(self._lib.jmpc_step_host(self._h, B, T, _ptr(state), _ptr(cid), _ptr(clen), _ptr(tgt), _ptr(wrm),
-                                             _ptr(oa_b), _ptr(od_b), _ptr(prm), _ptr(ox), _ptr(oy), _ptr(ov),
-                                             _ptr(oyaw), _ptr(xref), _ptr(cost), _ptr(status), _ptr(iters),
-                                             _ptr(record)), "jmpc_step_host")
-        return StepOutput(oa_b, od_b, ox, oy, ov, oyaw, xref, cost, status, iters, tgt, record)
-
-    def _step_host_into(self, out, T, state, target_ind, oa, od, course_id, course_len, warm, params) -> StepOutput:
-        """Results into the caller's (page-locked) `out`; the inputs are only read.  `oa` / `od` / `target_ind` may be
-        `out`'s own arrays (a closed loop feeding its previous solution back), in which case nothing is copied."""
-        state = _f64(state)
-        B = state.shape[0]
-        if out.oa.shape != (B, T):
+        if out is None:
+            f = np.zeros
+            out = StepOutput(oa=f((B, T)), od=f((B, T)), ox=f((B, T + 1)), oy=f((B, T + 1)), ov=f((B, T + 1)),
+                             oyaw=f((B, T + 1)), xref=f((B, 4, T + 1)), cost=np.full(B, np.nan),
+                             status=f(B, np.int32), iters=f(B, np.int32), target_ind=f(B, np.int32),
+                             record=f((B, _cabi.RECORD_LEN)))
+        elif out.oa.shape != (B, T):
             raise ValueError("`out` was made for another batch size / horizon")
         if oa is None or od is None:
             out.oa[...] = 0.0
@@ -386,10 +368,12 @@ class BatchedMPC:
         else:
             flag = np.zeros(B, np.int32)
             clen = np.zeros(B, np.int32)
+        cid = None if course_id is None else _i32(course_id, (B,))
+        v = _f64(v, (B,))
+        prm = None if params is None else _f64(params, (B, NPARAM))
         _cabi.check(self._lib.jmpc_collision_host(
-            self._h, B, _ptr(None if course_id is None else _i32(course_id, (B,))), _ptr(agent_idx), _ptr(_f64(v, (B,))),
-            _ptr(obstacles) if n_obs else None, n_obs, int(frame_window), int(margin), float(horizon_s),
-            _ptr(None if params is None else _f64(params, (B, NPARAM))), _ptr(flag), _ptr(clen)), "jmpc_collision_host")
+            self._h, B, _ptr(cid), _ptr(agent_idx), _ptr(v), _ptr(obstacles) if n_obs else None, n_obs,
+            int(frame_window), int(margin), float(horizon_s), _ptr(prm), _ptr(flag), _ptr(clen)), "jmpc_collision_host")
         return flag, clen
 
     # ---- device path (torch tensors) -----------------------------------------------------------------------

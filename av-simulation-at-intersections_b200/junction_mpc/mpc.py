@@ -9,7 +9,7 @@ Everything a scenario runner touches keeps its name, signature and types (SURVEY
     mpc.get_current_xref_deviation(); mpc.is_goal(state)                  mpc.py:305-330
     mpc.ox, mpc.oy, mpc.xref, mpc.di                                      mpc_intersection.py:301-306
 
-A single ego is a batch of one: `step` runs the same CUDA kernel as `BatchedMPC` through `jmpc_step_host`.
+A single ego is a batch of one: `step` runs the same CUDA kernel as `BatchedMPC` through `jmpc_step_host_io`.
 `install()` registers this module as `lib.mpc` (and the sensitivity / speed-profile flavours as
 `lib.mpc_sensitivity` / `lib.mpc_with_speed`) so the
 reference's scenario scripts run unmodified; see INTEGRATION.md.

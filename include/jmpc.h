@@ -11,8 +11,8 @@
  *   - `jmpc_step` / `jmpc_collision` take DEVICE pointers (e.g. torch tensors' data_ptr()) and only enqueue
  *     work on `stream`; they never synchronise.
  *   - `jmpc_step_host[_io]` / `jmpc_collision_host` take HOST pointers, run the same kernels and return after the
- *     results are on the host (step: the kernel accesses page-locked host memory directly; collision: staged
- *     through pinned buffers owned by the handle).
+ *     results are on the host (inputs staged through pinned buffers owned by the handle, results stored by the
+ *     kernels into page-locked host memory directly; jmpc_set_host_transfer).
  *   - Arrays are instance-major ("batch first"), float64 / int32, densely packed:
  *       state      [B][4]         x, y, v, yaw            (main/lib/mpc.py:291)
  *       oa, od     [B][T]         accelerations / steering angles; in: previous solution (the linearisation
@@ -184,9 +184,10 @@ int32_t jmpc_gather_timed_out(jmpc_handle h, int32_t* out);
 /* Same with HOST pointers: runs the step and returns when the results are in the host arrays.  The inputs are
  * copied to the device with cudaMemcpyAsync; the results take no copy pass: the kernel's epilogue stores them into
  * page-locked host memory through its device mapping -- the caller's arrays where they are page-locked
- * (jmpc_host_alloc), the handle's staging block otherwise (one host memcpy per such array).  jmpc_set_host_transfer
- * selects the other two modes: 0 stages both directions through device memory, 2 also reads the inputs through the
- * mapping (measured slower: every warp waits a PCIe round trip when it picks an instance up). */
+ * (jmpc_host_alloc), the handle's staging block otherwise (one host memcpy per such array).  jmpc_collision_host
+ * moves its arrays the same way.  jmpc_set_host_transfer selects the other two modes: 0 stages both directions
+ * through device memory, 2 also reads the inputs through the mapping (no input copy ahead of the kernel; faster on
+ * large batches: 4.26 instead of 4.44 ms for 65 536 instances at T = 13 on a B200 at 1000 W, the same at 4096 and 1). */
 int32_t jmpc_step_host(jmpc_handle h, int32_t B, int32_t T, const double* state, const int32_t* course_id,
                        const int32_t* course_len, int32_t* target_ind, const int32_t* warm, double* oa,
                        double* od, const double* params, double* ox, double* oy, double* ov, double* oyaw,
