@@ -1087,20 +1087,26 @@ int32_t jmpc_counter_add(jmpc_handle h, int32_t* counter, int32_t delta, void* s
   return 0;
 }
 
-int32_t jmpc_episode_outcomes(jmpc_handle h, int32_t B, const double* state, const int32_t* course_id,
-                              const double* obstacles, int32_t n_obs, const double* record, const double* di,
-                              const int32_t* flag, const double* params, const int32_t* done, const int32_t* iter_dev,
-                              int32_t initial, double* outcomes, double* obstacle_history, int32_t history_rows,
-                              void* stream) {
-  if (!h) return fail("jmpc_episode_outcomes: NULL handle");
-  if (B < 0 || B > h->max_B) return fail("jmpc_episode_outcomes: B out of range");
-  if (n_obs < 0 || n_obs > jmpc::kMaxObstacles) return fail("jmpc_episode_outcomes: n_obs out of range");
-  if (history_rows < 0) return fail("jmpc_episode_outcomes: negative history_rows");
-  if (!state || !done || !outcomes) return fail("jmpc_episode_outcomes: NULL array");
-  if (n_obs > 0 && !obstacles) return fail("jmpc_episode_outcomes: obstacles is NULL");
+// jmpc_episode_outcomes and jmpc_episode_outcomes_scene: the same checks and launch
+extern "C++" {
+template <bool Scene>
+static int32_t launch_outcomes(const char* name, jmpc_handle h, int32_t B, const double* state,
+                               const int32_t* course_id, const double* obstacles, int32_t n_obs, const double* record,
+                               const double* di, const int32_t* flag, const double* params, const int32_t* done,
+                               const int32_t* present, const int32_t* depart, const int32_t* iter_dev, int32_t initial,
+                               double* outcomes, double* obstacle_history, int32_t history_rows, void* stream) {
+  char msg[160];
+  auto err = [&](const char* what) { snprintf(msg, sizeof msg, "%s: %s", name, what); return fail(msg); };
+  if (!h) return err("NULL handle");
+  if (B < 0 || B > h->max_B) return err("B out of range");
+  if (n_obs < 0 || n_obs > jmpc::kMaxObstacles) return err("n_obs out of range");
+  if (history_rows < 0) return err("negative history_rows");
+  if (!state || !done || !outcomes) return err("NULL array");
+  if (n_obs > 0 && !obstacles) return err("obstacles is NULL");
+  if (Scene && !depart) return err("depart is NULL");
   if (!initial) {
-    if (!record || !di || !iter_dev) return fail("jmpc_episode_outcomes: NULL step array");
-    if (h->n_courses < 1) return fail("jmpc_episode_outcomes: no courses uploaded (jmpc_set_courses)");
+    if (!record || !di || !iter_dev) return err("NULL step array");
+    if (h->n_courses < 1) return err("no courses uploaded (jmpc_set_courses)");
   }
   if (B == 0) return 0;
   CK(cudaSetDevice(h->device));
@@ -1113,7 +1119,74 @@ int32_t jmpc_episode_outcomes(jmpc_handle h, int32_t B, const double* state, con
   a.off_front = h->off_front; a.off_rear = h->off_rear; a.radius = h->radius;
   a.state = state; a.obstacles = obstacles; a.record = record; a.di = di; a.flag = flag; a.done = done;
   a.iter_dev = iter_dev; a.outcomes = outcomes; a.obstacle_history = obstacle_history;
-  jmpc::episode_outcome_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(a);
+  a.present = present; a.depart = depart;
+  if (Scene)
+    jmpc::scene_outcome_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(a);
+  else
+    jmpc::episode_outcome_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(a);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+}  // extern "C++"
+
+int32_t jmpc_episode_outcomes(jmpc_handle h, int32_t B, const double* state, const int32_t* course_id,
+                              const double* obstacles, int32_t n_obs, const double* record, const double* di,
+                              const int32_t* flag, const double* params, const int32_t* done, const int32_t* iter_dev,
+                              int32_t initial, double* outcomes, double* obstacle_history, int32_t history_rows,
+                              void* stream) {
+  return launch_outcomes<false>("jmpc_episode_outcomes", h, B, state, course_id, obstacles, n_obs, record, di, flag,
+                                params, done, nullptr, nullptr, iter_dev, initial, outcomes, obstacle_history,
+                                history_rows, stream);
+}
+
+int32_t jmpc_episode_outcomes_scene(jmpc_handle h, int32_t B, const double* state, const int32_t* course_id,
+                                    const double* obstacles, int32_t n_obs, const double* record, const double* di,
+                                    const int32_t* flag, const double* params, const int32_t* done,
+                                    const int32_t* present, const int32_t* depart, const int32_t* iter_dev,
+                                    int32_t initial, double* outcomes, double* obstacle_history, int32_t history_rows,
+                                    void* stream) {
+  return launch_outcomes<true>("jmpc_episode_outcomes_scene", h, B, state, course_id, obstacles, n_obs, record, di,
+                               flag, params, done, present, depart, iter_dev, initial, outcomes, obstacle_history,
+                               history_rows, stream);
+}
+
+int32_t jmpc_scene_depart_init(jmpc_handle h, int32_t B, const int32_t* depart, int32_t* done, void* stream) {
+  if (!h) return fail("jmpc_scene_depart_init: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_scene_depart_init: B out of range");
+  if (!depart || !done) return fail("jmpc_scene_depart_init: NULL array");
+  if (B == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::scene_depart_init_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(B, depart, done);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
+int32_t jmpc_scene_enter(jmpc_handle h, int32_t B, const int32_t* depart, const int32_t* iter_dev, int32_t* done,
+                         void* stream) {
+  if (!h) return fail("jmpc_scene_enter: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_scene_enter: B out of range");
+  if (!depart || !iter_dev || !done) return fail("jmpc_scene_enter: NULL array");
+  if (B == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::scene_enter_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(B, depart, iter_dev, done);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
+int32_t jmpc_scene_presence(jmpc_handle h, int32_t B, int32_t k, int32_t leave, const int32_t* done, int32_t* mask,
+                            int32_t combine, void* stream) {
+  if (!h) return fail("jmpc_scene_presence: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_scene_presence: B out of range");
+  if (k < 1 || k > jmpc::kMaxObstacles + 1 || B % k != 0)
+    return fail("jmpc_scene_presence: B must be a multiple of k in [1, 9]");
+  if (!done || !mask) return fail("jmpc_scene_presence: NULL array");
+  if (B == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::scene_presence_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(B, k, leave ? 1 : 0, done, mask,
+                                                                                 combine ? 1 : 0);
   CK(cudaGetLastError());
   h->launches++;
   return 0;

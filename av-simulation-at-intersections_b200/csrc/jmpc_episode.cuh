@@ -173,17 +173,28 @@ struct OutcomeArgs {
   const double* record; const double* di; const int* flag; const int* done; const int* iter_dev;
   double* outcomes;                         // [B][JMPC_OUTCOME_LEN]
   double* obstacle_history;                 // [history_rows + 1][B][n_obs][6] or nullptr
+  // scene_outcome_kernel only (jmpc_episode_outcomes_scene)
+  const int* present;                       // [B] bit s = obstacle slot s is present, or nullptr: every slot
+  const int* depart;                        // [B] entry iteration: evaluation depart[b] > 0 starts b's record
 };
 
 // One thread per episode, once before the first loop iteration (initial: evaluation 0) and once per iteration after
 // the obstacles have advanced (evaluation i + 1).  At most kMaxObstacles x 4 circle pairs per evaluation.
-__global__ void episode_outcome_kernel(const OutcomeArgs A) {
+// Scene: absent slots (bit clear in present[b]) are skipped and get a NaN track row, and evaluation depart[b] takes
+// the path of evaluation 0 for b.
+template <bool Scene>
+__device__ __forceinline__ void episode_outcome_body(const OutcomeArgs& A) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= A.B) return;
   double* out = A.outcomes + (size_t)b * JMPC_OUTCOME_LEN;
   const double x = A.state[4 * b], y = A.state[4 * b + 1], v = A.state[4 * b + 2], yaw = A.state[4 * b + 3];
   int e = 0;
-  if (A.initial) {
+  bool first = A.initial != 0;
+  if (Scene && !first && !A.done[b]) {      // b entered after iteration e - 1 and has taken no step yet
+    e = *A.iter_dev + 1;
+    first = e == A.depart[b];
+  }
+  if (first) {
     out[JMPC_O_MIN_CLEARANCE] = INFINITY;
     for (int c = JMPC_O_MIN_CLEARANCE_EVAL; c <= JMPC_O_FIRST_CONTACT_OBS; ++c) out[c] = -1.0;
     for (int c = JMPC_O_CONTACT_EVALS; c < JMPC_NOUTCOME; ++c) out[c] = 0.0;
@@ -235,8 +246,14 @@ __global__ void episode_outcome_kernel(const OutcomeArgs A) {
   int best_obs = -1, contact_obs = -1;
   double* track = (A.obstacle_history && e <= A.history_rows)
                       ? A.obstacle_history + ((size_t)e * A.B + b) * A.n_obs * 6 : nullptr;
+  const unsigned present = (Scene && A.present) ? (unsigned)A.present[b] : 0xffffffffu;
   for (int k = 0; k < A.n_obs; ++k) {
     const double* o = A.obstacles + ((size_t)b * A.n_obs + k) * 6;
+    if (Scene && !((present >> k) & 1u)) {
+      if (track)
+        for (int j = 0; j < 6; ++j) track[6 * k + j] = nan("");
+      continue;
+    }
     if (track)
       for (int j = 0; j < 6; ++j) track[6 * k + j] = o[j];
     sincos(o[3], &s, &c);
@@ -268,6 +285,8 @@ __global__ void episode_outcome_kernel(const OutcomeArgs A) {
     }
   }
 }
+__global__ void episode_outcome_kernel(const OutcomeArgs A) { episode_outcome_body<false>(A); }
+__global__ void scene_outcome_kernel(const OutcomeArgs A) { episode_outcome_body<true>(A); }
 
 // ---- scenes of k vehicles that see each other as obstacles (jmpc_scene_exchange, jmpc_scene_init) -----------------
 // One thread per (episode, slot) of obstacles_out [B][n_obs][6], n_obs = (k - 1) + n_extra.  Slots 0 .. k - 2 are the
@@ -423,12 +442,43 @@ __global__ void scene_init_kernel(int n_scenes, int k, int* __restrict__ done) {
     if (d[j] == JMPC_DONE_RUNNING) d[j] = JMPC_DONE_MATE_NO_COURSE;
 }
 
+// ---- lifetimes of scene vehicles (jmpc_scene_depart_init, jmpc_scene_enter, jmpc_scene_presence) ---------------
+// One thread per episode: a vehicle that enters later waits (done 0 -> JMPC_WAITING where depart > 0).
+__global__ void scene_depart_init_kernel(int B, const int* __restrict__ depart, int* __restrict__ done) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  if (done[b] == JMPC_DONE_RUNNING && depart[b] > 0) done[b] = JMPC_WAITING;
+}
+// One thread per episode, at the end of loop iteration i: the vehicles that take their first step in iteration i + 1
+// enter (JMPC_WAITING -> 0), so that evaluation i + 1 sees them.
+__global__ void scene_enter_kernel(int B, const int* __restrict__ depart, const int* __restrict__ iter_dev,
+                                   int* __restrict__ done) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  if (done[b] == JMPC_WAITING && depart[b] <= *iter_dev + 1) done[b] = JMPC_DONE_RUNNING;
+}
+// One thread per episode b: clears bit s of mask[b] for every absent mate in slot s (waiting, or gone after its goal
+// with leave != 0).  combine = 0 starts from -1, combine = 1 from mask[b] (a right-of-way rule's consider mask).
+__global__ void scene_presence_kernel(int B, int k, int leave, const int* __restrict__ done, int* __restrict__ mask,
+                                      int combine) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  unsigned m = combine ? (unsigned)mask[b] : 0xffffffffu;
+  for (int slot = 0; slot < k - 1; ++slot) {
+    const int d = done[scene_mate(b, k, slot)];
+    if (d == JMPC_WAITING || (leave && d == JMPC_DONE_GOAL)) m &= ~(1u << slot);
+  }
+  mask[b] = (int)m;
+}
+// The extras of a waiting vehicle keep to the loop's clock: they advance as those of a running one.
+__device__ __forceinline__ bool extras_advance(int done) { return done == JMPC_DONE_RUNNING || done == JMPC_WAITING; }
+
 // Constant-input obstacle motion, one thread per obstacle: obstacles [B][n_obs][6] = x, y, v, yaw, a, steer.
 __global__ void obstacle_step_kernel(int count, double* __restrict__ obs, const int* __restrict__ done, int n_obs,
                                      double dt, double L) {
   const int k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= count) return;
-  if (done && done[k / n_obs]) return;
+  if (done && !extras_advance(done[k / n_obs])) return;
   double* o = obs + (size_t)k * 6;
   double x = o[0], y = o[1], v = o[2], yaw = o[3];
   double s, c;
@@ -487,7 +537,7 @@ __global__ void scripted_obstacle_kernel(int count, const double* __restrict__ s
                                          double L) {
   const int k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= count) return;
-  if (done && done[k / n_obs]) return;
+  if (done && !extras_advance(done[k / n_obs])) return;
   const double* sc = script + (size_t)k * JMPC_OBS_SCRIPT_LEN;
   double* m = model + (size_t)k * 4;
   double xc = m[0], yc = m[1], theta = m[2], counter = m[3];

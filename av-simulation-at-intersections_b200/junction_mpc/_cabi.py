@@ -15,6 +15,8 @@ STATUS_OPTIMAL, STATUS_MAX_ITER, STATUS_INFEASIBLE, STATUS_INDEX_RULE = 0, 1, 2,
 DONE_RUNNING, DONE_GOAL, DONE_INDEX_RULE, DONE_NO_COURSE, DONE_MATE_NO_COURSE = 0, 1, 2, 3, 4
 # enum jmpc_right_of_way_rule
 ROW_FIXED, ROW_FIRST_COME = 1, 2
+# enum jmpc_scene_lifetime: the done code of a vehicle that has not entered its scene yet
+WAITING = 5
 
 c_i32p = C.POINTER(C.c_int32)
 c_f64p = C.POINTER(C.c_double)
@@ -77,6 +79,12 @@ SIGNATURES = {
     "jmpc_right_of_way": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 7),
     "jmpc_collision_masked": (C.c_int32, [C.c_void_p, C.c_int32] + [C.c_void_p] * 4 + [C.c_int32, C.c_void_p]
                               + [C.c_int32] * 2 + [C.c_void_p] + [C.c_int32] * 2 + [C.c_double] + [C.c_void_p] * 4),
+    "jmpc_scene_depart_init": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "jmpc_scene_enter": (C.c_int32, [C.c_void_p, C.c_int32] + [C.c_void_p] * 4),
+    "jmpc_scene_presence": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
+                                        C.c_void_p]),
+    "jmpc_episode_outcomes_scene": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]
+                                    + [C.c_void_p] * 8 + [C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "jmpc_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]),
     "jmpc_scripted_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                                 C.c_void_p, C.c_int32, C.c_void_p]),

@@ -10,7 +10,8 @@ the device (contact, clearance, comfort; enum jmpc_outcome in include/jmpc.h), s
 With `agents_per_scene=k` every k consecutive episodes form a scene whose MPC-driven vehicles see each other as moving
 obstacles (jmpc_scene_exchange); with `share_plans=True` they predict each other along their MPC plans
 (jmpc_scene_plans, jmpc_collision_planned); with `right_of_way` a rule decides which mates each vehicle yields to
-(jmpc_right_of_way, jmpc_collision_masked).
+(jmpc_right_of_way, jmpc_collision_masked); with `depart` / `on_goal="leave"` every vehicle has a lifetime in its scene:
+it enters at its departure iteration and may leave at its goal (jmpc_scene_enter, jmpc_scene_presence).
 """
 from __future__ import annotations
 
@@ -122,6 +123,36 @@ def right_of_way_setup(right_of_way, k: int, B: int, priority=None, junction=Non
     return _cabi.ROW_FIRST_COME, None, np.ascontiguousarray(junc)
 
 
+ON_GOAL = ("park", "leave")
+
+
+def lifetime_setup(depart, on_goal: str, k: int, B: int):
+    """Host-side checks of the lifetime options of `BatchedEpisodes`.  Returns None when every vehicle is present from
+    evaluation 0 and parks at its goal (depart None or all zero, on_goal "park": the run without lifetimes), else
+    (depart int32 [B], leave).  depart: integer array [B] >= 0, the loop iteration of each vehicle's first step;
+    on_goal "park" | "leave" (leave needs agents_per_scene > 1)."""
+    if on_goal not in ON_GOAL:
+        raise ValueError(f"on_goal must be 'park' or 'leave', got {on_goal!r}")
+    leave = on_goal == "leave"
+    if leave and k < 2:
+        raise ValueError("on_goal='leave' needs agents_per_scene > 1: there are no scene mates to leave")
+    if depart is None:
+        dep = np.zeros(B, np.int32)
+    else:
+        dep = np.asarray(depart)
+        if not np.issubdtype(dep.dtype, np.integer):
+            raise ValueError(f"depart must be an integer array, got dtype {dep.dtype}")
+        if dep.shape != (B,):
+            raise ValueError(f"depart must be [{B}] (one entry iteration per episode), got shape {dep.shape}")
+        if (dep < 0).any():
+            raise ValueError("depart must be >= 0")
+        if (dep > np.iinfo(np.int32).max).any():
+            raise ValueError("depart must fit in int32")
+    if not leave and not dep.any():
+        return None
+    return np.ascontiguousarray(dep, dtype=np.int32), leave
+
+
 def outcome_columns(record) -> dict:
     """[B, >= len(OUTCOME_NAMES)] float64 outcome records -> dict of [B] arrays keyed by OUTCOME_NAMES (the index and
     count columns as int64)."""
@@ -189,7 +220,7 @@ class BatchedEpisodes:
                    frame_window: int = 10, max_steps: int = 256, record_history: bool = True, horizon_s: float = 7.0,
                    obstacle_script=None, outcomes: bool = False, record_obstacles: bool = False,
                    agents_per_scene: int = 1, share_plans: bool = False, right_of_way=None, priority=None,
-                   junction=None) -> "BatchedEpisodes":
+                   junction=None, depart=None, on_goal: str = "park") -> "BatchedEpisodes":
         """Episodes on the planned courses of `engine` (filled by `BatchedMPC.from_plans(plans)` /
         `set_courses_from_plans(plans)`), the second half of main/scenarios/mpc_intersection.py:63-163 for a batch:
         episode b drives plan `plan_id[b]` (default: one episode per plan; zeros = one course, many controllers).
@@ -197,10 +228,10 @@ class BatchedEpisodes:
         course are written on the device (jmpc_episode_init_from_courses); such episodes are never stepped.
         `params` [B, NPARAM] (default: the engine's defaults) supplies every other parameter row.  `run()` adds
         plan_status, plan_cost and expansions per episode.  `outcomes` / `record_obstacles` / `agents_per_scene` /
-        `share_plans` / `right_of_way` / `priority` / `junction` as in `__init__`; evaluation 0 of the outcome record sees
+        `share_plans` / `right_of_way` / `priority` / `junction` / `depart` / `on_goal` as in `__init__`; evaluation 0 of the outcome record sees
         the planned start states; the junction zones are found on the planned courses, and first_come distances use
         each course's dl.  With agents_per_scene > 1 a scene with a done = 3 vehicle is not driven: its other vehicles get
-        done = 4 (jmpc_scene_init)."""
+        done = 4 (jmpc_scene_init); such vehicles never wait either: the waiting code is set after this pass."""
         if engine.course_ok is None or len(engine.course_ok) != len(plans):
             raise ValueError("the engine's courses do not come from these plans (BatchedMPC.from_plans)")
         import torch
@@ -214,7 +245,8 @@ class BatchedEpisodes:
                  frame_window=frame_window, margin=margin, params=params, max_steps=max_steps,
                  record_history=record_history, horizon_s=horizon_s, obstacle_program=obstacle_program,
                  outcomes=outcomes, record_obstacles=record_obstacles, agents_per_scene=agents_per_scene,
-                 share_plans=share_plans, right_of_way=right_of_way, priority=priority, junction=junction)
+                 share_plans=share_plans, right_of_way=right_of_way, priority=priority, junction=junction,
+                 depart=depart, on_goal=on_goal)
         stream = C.c_void_p(torch.cuda.current_stream(engine.device).cuda_stream)
         _cabi.check(engine._lib.jmpc_episode_init_from_courses(
             engine._h, B, ep._p(ep.course_id), ep._p(engine.course_ok), ep._p(engine.course_dl), ep._p(ep.state),
@@ -228,7 +260,7 @@ class BatchedEpisodes:
                  frame_window: int = 10, margin: int = 72, params=None, max_steps: int = 256,
                  record_history: bool = True, horizon_s: float = 7.0, obstacle_program=None, outcomes: bool = False,
                  record_obstacles: bool = False, agents_per_scene: int = 1, share_plans: bool = False,
-                 right_of_way=None, priority=None, junction=None):
+                 right_of_way=None, priority=None, junction=None, depart=None, on_goal: str = "park"):
         """outcomes: keep one outcome record per episode on the device (jmpc_episode_outcomes): contact and clearance
         against the obstacles, cut / limit steps, failed solves, comfort and tracking columns; `run()` returns it as
         `outcomes`.  It observes only: the episodes are exactly those of outcomes=False.  record_obstacles (needs
@@ -261,7 +293,21 @@ class BatchedEpisodes:
           "first_come": junction = (x, y, r), for all scenes or [B / k, 3].  entry / exit are the first and last points
           of b's course within r of the centre (jmpc_right_of_way_init, `zone` [B, 2]; -1 when it never enters), a its
           course index, dl its params' dl: committed (a >= entry) class 0, key (exit - a) dl; approaching class 1,
-          key (entry - a) dl; a course that never enters the zone class 2 (it yields to every moving mate)."""
+          key (entry - a) dl; a course that never enters the zone class 2 (it yields to every moving mate).
+
+        depart (integer [B] >= 0; None = all zeros) and on_goal = "park" | "leave": each vehicle's lifetime in its scene
+        (jmpc_scene_depart_init / jmpc_scene_enter / jmpc_scene_presence / jmpc_episode_outcomes_scene in
+        include/jmpc.h).  Vehicle b takes its first step in loop iteration depart[b]; until then it waits at its start
+        state with done = WAITING (5): not stepped, not goal-tested, no History row, absent for its mates.  It enters
+        between iteration depart[b] - 1 and evaluation depart[b] with its start state, speed kept.  Its extras follow the
+        loop's clock while it waits, so at entry it sees what a depart = 0 vehicle sees then.  With "leave" (needs k > 1)
+        a vehicle whose goal test fires at the top of iteration g is present in evaluation g and absent from iteration
+        g's collision check on; done = 2 (index rule) stays parked under both.  Absent mates take no part in the
+        collision cut (with a rule: the rule's mask AND presence, written into `consider`), and add no clearance or
+        contact to the outcome record, whose obstacle_history rows for them are NaN.  A vehicle's outcome record starts
+        at evaluation depart[b]; the *_eval columns stay global evaluation indices, and `steps` counts its own steps.
+        A vehicle that has not entered when the run ends keeps done = WAITING.  depart all zero with "park" is the run
+        without lifetimes, with nothing launched or allocated for them."""
         import torch
         self.torch = torch
         self.e = engine
@@ -328,6 +374,20 @@ class BatchedEpisodes:
                 _cabi.check(engine._lib.jmpc_right_of_way_init(
                     engine._h, B, self.k, self._p(self.course_id), self._p(self.junction), int(junc.shape[0]),
                     self._p(self.zone), stream), "jmpc_right_of_way_init")
+        # lifetimes: depart [B] int32; the collision mask (a rule's `consider` ANDed with presence, or presence alone)
+        # and the evaluation mask `presence` [B], both written by jmpc_scene_presence every iteration (k > 1)
+        self.depart = self.presence = None
+        self._collision_mask = self.consider
+        self._leave = self._entering = False
+        life = lifetime_setup(depart, on_goal, self.k, B)
+        if life is not None:
+            dep, self._leave = life
+            self.depart = t(dep, i32)
+            self._entering = bool(dep.any())
+            if self.k > 1:
+                self.presence = torch.full((B,), -1, dtype=i32, device=self.dev)
+                if self._collision_mask is None:
+                    self._collision_mask = torch.full((B,), -1, dtype=i32, device=self.dev)
         self.outcomes = self.obstacle_history = None
         if outcome_setup(outcomes, record_obstacles, n_obs):
             self.outcomes = torch.empty(B, OUTCOME_LEN, dtype=f64, device=self.dev)     # evaluation 0 fills it
@@ -350,6 +410,15 @@ class BatchedEpisodes:
         e, torch = self.e, self.torch
         stream = C.c_void_p(torch.cuda.current_stream(e.device).cuda_stream)
         has_obs = obs is not None and self.n_obs > 0
+        if self.depart is not None:
+            _cabi.check(e._lib.jmpc_episode_outcomes_scene(
+                e._h, self.B, self._p(self.state), self._p(self.course_id), self._p(obs) if has_obs else None,
+                self.n_obs if has_obs else 0, self._p(self.out.record), self._p(self.di),
+                self._p(self.flag) if has_obs else None, self._p(self.params), self._p(self.done),
+                self._p(self.presence), self._p(self.depart), self._p(self.iter_dev), int(initial),
+                self._p(self.outcomes), self._p(self.obstacle_history), self.max_steps, stream),
+                "jmpc_episode_outcomes_scene")
+            return
         _cabi.check(e._lib.jmpc_episode_outcomes(
             e._h, self.B, self._p(self.state), self._p(self.course_id), self._p(obs) if has_obs else None,
             self.n_obs if has_obs else 0, self._p(self.out.record), self._p(self.di),
@@ -373,6 +442,13 @@ class BatchedEpisodes:
                 self._p(self.params), self._p(self.scene_obs), self.n_obs, self._p(self.scene_plans), stream),
                 "jmpc_scene_plans")
 
+    def _presence(self, mask, combine: int):
+        """Clears the bits of absent mates in mask (jmpc_scene_presence); combine = 0 starts from -1."""
+        e = self.e
+        stream = C.c_void_p(self.torch.cuda.current_stream(e.device).cuda_stream)
+        _cabi.check(e._lib.jmpc_scene_presence(e._h, self.B, self.k, int(self._leave), self._p(self.done), self._p(mask),
+                                               int(combine), stream), "jmpc_scene_presence")
+
     def _current_obstacles(self, frame: int):
         """The obstacle rows that loop iteration `frame`'s collision check reads (evaluation `frame`)."""
         if self.scene_obs is not None:
@@ -380,12 +456,19 @@ class BatchedEpisodes:
         return self.obstacles if self.script is None else self.script[min(frame, self.script.shape[0] - 1)]
 
     def _start(self):
-        """Launched once before the first iteration, after __init__ / from_plans wrote the start states: the scene's
-        first exchange, then evaluation 0 of the outcome record."""
+        """Launched once before the first iteration, after __init__ / from_plans wrote the start states and done codes:
+        the waiting codes, the scene's first exchange, then evaluation 0 of the outcome record."""
         if self._started:
             return
+        if self._entering:
+            e = self.e
+            stream = C.c_void_p(self.torch.cuda.current_stream(e.device).cuda_stream)
+            _cabi.check(e._lib.jmpc_scene_depart_init(e._h, self.B, self._p(self.depart), self._p(self.done), stream),
+                        "jmpc_scene_depart_init")
         if self.scene_obs is not None:
             self._scene_exchange()
+        if self.presence is not None and self.outcomes is not None:
+            self._presence(self.presence, 0)
         if self.outcomes is not None:
             self._outcome_eval(self._current_obstacles(0), initial=1)
         self._started = True
@@ -417,12 +500,14 @@ class BatchedEpisodes:
             _cabi.check(lib.jmpc_right_of_way(
                 e._h, self.B, self.k, self.row_rule, self._p(self.agent_idx), self._p(self.done), self._p(self.params),
                 self._p(self.zone), self._p(self.priority), self._p(self.consider), stream), "jmpc_right_of_way")
+        if self.presence is not None:          # the same done codes: who is in the scene
+            self._presence(self._collision_mask, int(self.consider is not None))
         obs = self._current_obstacles(i)
         if obs is not None and obs.shape[1] > 0:
             self.v.copy_(self.state[:, 2])
             e.collision(self.agent_idx, self.v, obs, self.frame_window, self.margin, self.flag, self.course_len,
                         course_id=self.course_id, params=self.params, horizon_s=self.horizon_s, plans=self.scene_plans,
-                        n_planned=self.k - 1, consider=self.consider)
+                        n_planned=self.k - 1, consider=self._collision_mask)
             has_flags = True
         else:
             has_flags = False
@@ -440,12 +525,23 @@ class BatchedEpisodes:
         elif self.obstacles is not None and self.obstacles.shape[1] > 0:
             _cabi.check(lib.jmpc_obstacle_step(e._h, self.B, int(self.obstacles.shape[1]), self._p(self.obstacles),
                                                self._p(self.done), float(e.dt), stream), "jmpc_obstacle_step")
+        if self._entering:                     # the vehicles whose first step is iteration i + 1
+            _cabi.check(lib.jmpc_scene_enter(e._h, self.B, self._p(self.depart), self._p(self.iter_dev),
+                                             self._p(self.done), stream), "jmpc_scene_enter")
         if self.scene_obs is not None:         # all vehicles have moved: the scene's rows of evaluation i + 1
             self._scene_exchange()
+        if self.presence is not None and self.outcomes is not None:
+            self._presence(self.presence, 0)
         if self.outcomes is not None:          # the obstacle poses that iteration i + 1's collision check reads
             self._outcome_eval(self._current_obstacles(i + 1), initial=0)
         _cabi.check(lib.jmpc_counter_add(e._h, self._p(self.iter_dev), 1, stream), "jmpc_counter_add")
         self.iteration += 1
+
+    def _finished(self) -> bool:
+        """No episode is running (done = 0) or waiting to enter (done = WAITING)."""
+        if self._entering:
+            return bool(((self.done != 0) & (self.done != _cabi.WAITING)).all().item())
+        return bool((self.done != 0).all().item())
 
     def run(self, max_steps: Optional[int] = None, check_every: int = 8, use_graph: bool = False):
         """Iterate until every episode reached its goal (or max_steps).  Returns a dict of numpy results; with
@@ -479,11 +575,11 @@ class BatchedEpisodes:
             if graph is not None and max_steps - self.iteration >= check_every:
                 graph.replay()
                 self.iteration += check_every
-                if bool((self.done != 0).all().item()):
+                if self._finished():
                     break
                 continue
             self.iterate()
-            if self.iteration % check_every == 0 and bool((self.done != 0).all().item()):
+            if self.iteration % check_every == 0 and self._finished():
                 break
         # the reference tests the goal at the top of the next iteration
         lib, e = self.e._lib, self.e

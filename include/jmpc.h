@@ -272,7 +272,8 @@ int32_t jmpc_plant_step(jmpc_handle h, int32_t B, double* state, const double* a
  *                      can be captured once as a CUDA graph and replayed.
  *   jmpc_obstacle_step: constant-input motion of obstacles [B][n_obs][6] (moving_obstacles_prediction.py:21-29), with
  *                      one `dt` for the whole batch: a params row's dt reaches the collision prediction and the plant,
- *                      not this step. */
+ *                      not this step.  It advances the obstacles of episodes with done = 0 or done = JMPC_WAITING (a
+ *                      vehicle that has not entered its scene yet, enum jmpc_scene_lifetime) and leaves the others. */
 enum jmpc_done {
   JMPC_DONE_RUNNING = 0,         /* still driving                                                                  */
   JMPC_DONE_GOAL = 1,            /* is_goal fired                                                    mpc.py:314-330 */
@@ -424,6 +425,46 @@ int32_t jmpc_collision_masked(jmpc_handle h, int32_t B, const int32_t* course_id
                               int32_t margin, double horizon_s, const double* params, int32_t* flag,
                               int32_t* course_len_out, void* stream);
 
+/* Lifetimes of scene vehicles (opt-in): an entry iteration per vehicle, and with leave != 0 an end at its goal.
+ * Outside its lifetime a vehicle is absent: it is not stepped, no mate considers it in its collision cut, and no
+ * outcome record measures it.  DEVICE pointers; depart [B] int32 >= 0: the loop iteration of b's first step.
+ *   Waiting code: done = JMPC_WAITING until b enters.  It is nonzero, so the skip mask keeps b out of jmpc_step /
+ *   jmpc_collision*, and jmpc_episode_pre / post / outcomes leave it untouched (no goal test, no History row); its
+ *   extras still advance (jmpc_obstacle_step, jmpc_scripted_obstacle_step).  A vehicle that has not entered when the
+ *   run ends keeps JMPC_WAITING.  jmpc_scene_exchange writes its parked row at the start pose, as for any done != 0.
+ * jmpc_scene_depart_init: done 0 -> JMPC_WAITING where depart > 0.  Enqueue it once, after
+ *   jmpc_episode_init_from_courses / jmpc_scene_init (so a scene that is not driven stays at done 3 / 4).
+ * jmpc_scene_enter: done JMPC_WAITING -> 0 where depart <= *iter_dev + 1.  Enqueue it every iteration after the extras
+ *   advance and before jmpc_scene_exchange: b enters between iteration depart[b] - 1 and evaluation depart[b], with
+ *   its start state (its speed kept).  iter_dev is jmpc_episode_post_dev's counter; no per-iteration host argument.
+ * jmpc_scene_presence: clears bit s of mask [B] for every absent mate in slot s (slots of jmpc_scene_exchange).  Mate m
+ *   is absent iff done[m] = JMPC_WAITING, or leave != 0 and done[m] = JMPC_DONE_GOAL: with leave, a vehicle whose goal
+ *   test fired at the top of iteration g is present in evaluation g and absent from iteration g's collision check on.
+ *   done = 2 (index rule) stays parked and present.  combine = 0 first sets mask[b] = -1; combine = 1 ANDs into it (a
+ *   right-of-way rule's consider mask, which treats every non-running mate as parked and considered).  k in [1, 9].
+ *   Enqueue it after jmpc_episode_pre / jmpc_right_of_way for the mask jmpc_collision_masked reads, and after the
+ *   exchange for the mask jmpc_episode_outcomes_scene reads.
+ * jmpc_episode_outcomes_scene: jmpc_episode_outcomes with present [B] (NULL: every slot present) and depart [B].  Slots
+ *   whose bit is clear add no clearance or contact, and their obstacle_history rows are NaN.  At evaluation
+ *   e = depart[b] > 0 (initial = 0) b's record starts as evaluation 0 starts it: the empty record, then the clearance of
+ *   its start pose, no step columns.  The *_eval columns stay global evaluation indices.  Order of one iteration:
+ *   pre, right_of_way, presence (collision mask), collision_masked, step, post_dev, extras' advance, enter, exchange
+ *   (+ plans), presence (evaluation mask), outcomes_scene, counter_add. */
+enum jmpc_scene_lifetime {
+  JMPC_WAITING = 5               /* has not entered its scene yet: not stepped, absent for its mates              */
+};
+int32_t jmpc_scene_depart_init(jmpc_handle h, int32_t B, const int32_t* depart, int32_t* done, void* stream);
+int32_t jmpc_scene_enter(jmpc_handle h, int32_t B, const int32_t* depart, const int32_t* iter_dev, int32_t* done,
+                         void* stream);
+int32_t jmpc_scene_presence(jmpc_handle h, int32_t B, int32_t k, int32_t leave, const int32_t* done, int32_t* mask,
+                            int32_t combine, void* stream);
+int32_t jmpc_episode_outcomes_scene(jmpc_handle h, int32_t B, const double* state, const int32_t* course_id,
+                                    const double* obstacles, int32_t n_obs, const double* record, const double* di,
+                                    const int32_t* flag, const double* params, const int32_t* done,
+                                    const int32_t* present, const int32_t* depart, const int32_t* iter_dev,
+                                    int32_t initial, double* outcomes, double* obstacle_history, int32_t history_rows,
+                                    void* stream);
+
 /* The reference's scripted obstacles on the device (main/lib/moving_obstacles.py: MovingObstacleTIntersection :166-232,
  * MovingObstacleRoundabout :28-123 including its dt = 0.2 quirk at :45 and the theta overwrite inside its steering
  * property, MovingObstacleArterial :125-164).  DEVICE pointers.
@@ -432,7 +473,8 @@ int32_t jmpc_collision_masked(jmpc_handle h, int32_t B, const int32_t* course_id
  *   obstacles [B][n_obs][6] out: what `get()` returns (x, y, forward_velocity, theta, 0, steering_angle), the tuple
  *             jmpc_collision consumes
  *   advance: 0 = only evaluate get() (before the first loop iteration), 1 = step() first (moving_obstacles.py:113-116)
- * Episodes with done != 0 are left untouched. */
+ * Episodes with done = 0 or done = JMPC_WAITING (enum jmpc_scene_lifetime: the obstacles keep to the loop's clock while
+ * their vehicle waits to enter) are stepped; the others are left untouched. */
 enum jmpc_obs_kind { JMPC_OBS_CONSTANT = 0, JMPC_OBS_TINTERSECTION = 1, JMPC_OBS_ROUNDABOUT = 2, JMPC_OBS_ARTERIAL = 3 };
 enum jmpc_obs_script {
   JMPC_OBS_KIND = 0,     /* jmpc_obs_kind                                                                     */
