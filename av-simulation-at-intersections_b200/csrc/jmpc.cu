@@ -1192,6 +1192,53 @@ int32_t jmpc_scene_presence(jmpc_handle h, int32_t B, int32_t k, int32_t leave, 
   return 0;
 }
 
+// jmpc_scene_trips / jmpc_scene_trips_finish: the checks both share
+static int32_t check_trips(const char* name, jmpc_handle h, const jmpc_trips* t) {
+  char msg[160];
+  auto err = [&](const char* what) { snprintf(msg, sizeof msg, "%s: %s", name, what); return fail(msg); };
+  if (!h) return err("NULL handle");
+  if (!t) return err("NULL trips");
+  if (t->k < 2 || t->k > jmpc::kMaxObstacles + 1) return err("k must be in [2, 9]");
+  if (t->n_scenes < 0 || (long long)t->n_scenes * t->k > h->max_B) return err("n_scenes * k out of range");
+  if (t->n_trips < 0) return err("negative n_trips");
+  if (t->T < 1) return err("T must be >= 1");
+  if (!(t->entry_gap >= 0.0) || !isfinite(t->entry_gap)) return err("entry_gap must be finite and >= 0");
+  if (!t->scene_start || !t->arrival || !t->course_id || !t->course_len || !t->usable || !t->next_unusable || !t->start || !t->params ||
+      !t->cursor || !t->pending || !t->phase || !t->slot_trip || !t->slot || !t->entry || !t->exit || !t->steps ||
+      !t->done || !t->blocked_waits || !t->state || !t->ep_course_id || !t->ep_params ||
+      !t->ep_course_len || !t->target_ind || !t->agent_idx || !t->ep_steps || !t->warm || !t->flag || !t->di ||
+      !t->oa || !t->od || !t->depart || !t->ep_done)
+    return err("NULL array");
+  if (!t->zone != !t->ep_zone) return err("zone and ep_zone go together");
+  if (!t->priority != !t->ep_priority) return err("priority and ep_priority go together");
+  return 0;
+}
+
+int32_t jmpc_scene_trips(jmpc_handle h, const jmpc_trips* trips, const int32_t* iter_dev, int32_t initial,
+                         void* stream) {
+  if (check_trips("jmpc_scene_trips", h, trips)) return -1;
+  if (!initial && !iter_dev) return fail("jmpc_scene_trips: iter_dev is NULL");
+  if (trips->n_scenes == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::scene_trips_kernel<<<(trips->n_scenes + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
+      *trips, iter_dev, initial ? 1 : 0, h->off_front, h->off_rear, h->radius);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
+int32_t jmpc_scene_trips_finish(jmpc_handle h, const jmpc_trips* trips, int32_t n_iterations, void* stream) {
+  if (check_trips("jmpc_scene_trips_finish", h, trips)) return -1;
+  if (n_iterations < 0) return fail("jmpc_scene_trips_finish: negative n_iterations");
+  const int B = trips->n_scenes * trips->k;
+  if (B == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::scene_trips_finish_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(*trips, n_iterations);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
 int32_t jmpc_scene_exchange(jmpc_handle h, int32_t B, int32_t k, int32_t n_extra, const double* state,
                             const double* record, const double* di, const double* params, const int32_t* done,
                             const int32_t* steps, const double* extras, double* obstacles_out, void* stream) {

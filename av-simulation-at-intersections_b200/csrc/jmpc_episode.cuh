@@ -470,6 +470,129 @@ __global__ void scene_presence_kernel(int B, int k, int leave, const int* __rest
   }
   mask[b] = (int)m;
 }
+// ---- trips through scene slots (jmpc_scene_trips, jmpc_scene_trips_finish) -----------------------------------------
+enum { kTripPending = 0, kTripInSlot = 1, kTripClosed = 2 };
+
+// The outcome record's clearance between two poses (x, y, ., yaw) >= gap.  far2: squared distance of the reference
+// points beyond which no circle pair can come within gap (a shortcut that skips the exact test, never a decision).
+__device__ __forceinline__ bool start_clear(const double* p, const double* q, double off_front, double off_rear,
+                                            double reach, double gap, double far2) {
+  const double rx = p[0] - q[0], ry = p[1] - q[1];
+  if (rx * rx + ry * ry > far2) return true;
+  double s, c, px[2], py[2], qx[2], qy[2];
+  sincos(p[3], &s, &c);
+  circle_centre(p[0], p[1], c, s, off_front, px[0], py[0]);
+  circle_centre(p[0], p[1], c, s, off_rear, px[1], py[1]);
+  sincos(q[3], &s, &c);
+  circle_centre(q[0], q[1], c, s, off_front, qx[0], qy[0]);
+  circle_centre(q[0], q[1], c, s, off_rear, qx[1], qy[1]);
+  double clear = INFINITY;
+#pragma unroll
+  for (int n = 0; n < 4; ++n) {
+    const double dx = px[n >> 1] - qx[n & 1], dy = py[n >> 1] - qy[n & 1];
+    clear = fmin(clear, sqrt(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy))) - reach);
+  }
+  return clear >= gap;
+}
+
+// Writes trip t's row from slot b: exit, steps, done and the public outcome columns.
+__device__ __forceinline__ void close_trip(const jmpc_trips& P, int t, int b, int exit, int done) {
+  P.exit[t] = exit;
+  P.steps[t] = P.ep_steps[b];
+  P.done[t] = done;
+  if (P.outcomes && P.ep_outcomes)
+    for (int c = 0; c < JMPC_NOUTCOME; ++c)
+      P.outcomes[(size_t)t * JMPC_NOUTCOME + c] = P.ep_outcomes[(size_t)b * JMPC_OUTCOME_LEN + c];
+}
+
+// Slot b becomes a fresh vehicle on trip t, entering at evaluation `entry`.
+__device__ __forceinline__ void load_trip(const jmpc_trips& P, int t, int b, int entry) {
+  for (int c = 0; c < 4; ++c) P.state[4 * (size_t)b + c] = P.start[4 * (size_t)t + c];
+  for (int c = 0; c < JMPC_NPARAM; ++c)
+    P.ep_params[(size_t)b * JMPC_NPARAM + c] = P.params[(size_t)t * JMPC_NPARAM + c];
+  for (int c = 0; c < P.T; ++c) { P.oa[(size_t)b * P.T + c] = 0.0; P.od[(size_t)b * P.T + c] = 0.0; }
+  P.ep_course_id[b] = P.course_id[t];
+  P.ep_course_len[b] = P.course_len[t];
+  P.target_ind[b] = 0; P.agent_idx[b] = 0; P.ep_steps[b] = 0; P.warm[b] = 0; P.flag[b] = 0;
+  P.di[b] = 0.0;
+  if (P.ep_zone) { P.ep_zone[2 * (size_t)b] = P.zone[2 * (size_t)t]; P.ep_zone[2 * (size_t)b + 1] = P.zone[2 * (size_t)t + 1]; }
+  if (P.ep_priority) P.ep_priority[b] = P.priority[t];
+  P.depart[b] = entry;
+  P.ep_done[b] = JMPC_DONE_RUNNING;
+  P.slot_trip[b] = t;
+  P.phase[t] = kTripInSlot;
+  P.slot[t] = b;
+  P.entry[t] = entry;
+}
+
+// One thread per scene: close, admit, load (jmpc_scene_trips in include/jmpc.h).  A thread per scene suffices: at
+// most 9 slots; the walk starts at the scene's first pending trip, stops at the first trip not yet due, and once no
+// slot is empty jumps from one unusable trip to the next (the waits for a slot are not written: every due pass of a
+// trip either admits it, counts a blocked wait or is a slot wait, so the slot waits follow from entry and arrival).
+__global__ void scene_trips_kernel(const jmpc_trips P, const int* __restrict__ iter_dev, int initial, double off_front,
+                                   double off_rear, double radius) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= P.n_scenes) return;
+  const int k = P.k, b0 = s * k;
+  const int i = initial ? -1 : *iter_dev;
+  const int entry = i + 1;
+  unsigned empty = 0;
+  for (int j = 0; j < k; ++j) {
+    const int b = b0 + j;
+    if (P.ep_done[b] == JMPC_DONE_GOAL) {
+      const int t = P.slot_trip[b];
+      close_trip(P, t, b, i, JMPC_DONE_GOAL);
+      P.phase[t] = kTripClosed;
+      P.slot_trip[b] = -1;
+      P.ep_done[b] = JMPC_WAITING;
+    }
+    if (P.ep_done[b] == JMPC_WAITING) empty |= 1u << j;
+  }
+  const int last = P.scene_start[s + 1];
+  int first = P.cursor[s];
+  while (first < last && P.phase[first] != kTripPending) ++first;
+  P.cursor[s] = first;
+  const double reach = 2.0 * radius;
+  const double far = P.entry_gap + reach + 2.0 * (fabs(off_front) + fabs(off_rear)) + 1.0;
+  const double far2 = far * far;
+  int admitted = 0;
+  for (int t = first; t < last && P.arrival[t] <= entry; ++t) {
+    if (!empty) {                           // the rest wait for a slot (counted by the caller): close unusable ones
+      t = P.next_unusable[t];
+      if (t >= last || P.arrival[t] > entry) break;
+    }
+    if (P.phase[t] != kTripPending) continue;
+    if (!P.usable[t]) {
+      P.done[t] = JMPC_DONE_NO_COURSE;
+      P.phase[t] = kTripClosed;
+      ++admitted;
+      continue;
+    }
+    const double* st = P.start + 4 * (size_t)t;
+    bool clear = true;
+    for (int j = 0; j < k && clear; ++j)
+      if (!((empty >> j) & 1u))
+        clear = start_clear(st, P.state + 4 * (size_t)(b0 + j), off_front, off_rear, reach, P.entry_gap, far2);
+    for (int u = first; u < t && clear; ++u)
+      if (P.phase[u] == kTripPending)
+        clear = start_clear(st, P.start + 4 * (size_t)u, off_front, off_rear, reach, P.entry_gap, far2);
+    if (!clear) { P.blocked_waits[t] += 1; continue; }
+    const int j = __ffs(empty) - 1;
+    empty &= empty - 1;
+    load_trip(P, t, b0 + j, entry);
+    ++admitted;
+  }
+  if (admitted) P.pending[s] -= admitted;
+}
+
+// One thread per slot: the rows of the trips still in a slot when the run ends.
+__global__ void scene_trips_finish_kernel(const jmpc_trips P, int n_iterations) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= P.n_scenes * P.k) return;
+  const int t = P.slot_trip[b];
+  if (t >= 0) close_trip(P, t, b, n_iterations, P.ep_done[b]);
+}
+
 // The extras of a waiting vehicle keep to the loop's clock: they advance as those of a running one.
 __device__ __forceinline__ bool extras_advance(int done) { return done == JMPC_DONE_RUNNING || done == JMPC_WAITING; }
 

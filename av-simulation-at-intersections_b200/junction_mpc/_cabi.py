@@ -27,6 +27,18 @@ class Options(C.Structure):
                 ("warps_per_sm", C.c_int32), ("du_th", C.c_double)]
 
 
+class Trips(C.Structure):
+    """struct jmpc_trips (include/jmpc.h): the trip arrays, trip state, trip table and slot arrays, DEVICE pointers."""
+    _fields_ = ([("n_scenes", C.c_int32), ("k", C.c_int32), ("n_trips", C.c_int32), ("T", C.c_int32),
+                 ("entry_gap", C.c_double)]
+                + [(n, C.c_void_p) for n in (
+                    "scene_start", "arrival", "course_id", "course_len", "usable", "next_unusable", "start", "params",
+                    "zone", "priority", "cursor", "pending", "phase", "slot_trip", "slot", "entry", "exit", "steps",
+                    "done", "blocked_waits", "outcomes", "state", "ep_course_id", "ep_params", "ep_course_len",
+                    "target_ind", "agent_idx", "ep_steps", "warm", "flag", "di", "oa", "od", "ep_zone", "ep_priority",
+                    "depart", "ep_done", "ep_outcomes")])
+
+
 # name -> (restype, argtypes); the exported-symbol test walks this table against include/jmpc.h
 SIGNATURES = {
     "jmpc_abi_version": (C.c_int32, []),
@@ -85,6 +97,8 @@ SIGNATURES = {
                                         C.c_void_p]),
     "jmpc_episode_outcomes_scene": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]
                                     + [C.c_void_p] * 8 + [C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "jmpc_scene_trips": (C.c_int32, [C.c_void_p, C.POINTER(Trips), C.c_void_p, C.c_int32, C.c_void_p]),
+    "jmpc_scene_trips_finish": (C.c_int32, [C.c_void_p, C.POINTER(Trips), C.c_int32, C.c_void_p]),
     "jmpc_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]),
     "jmpc_scripted_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                                 C.c_void_p, C.c_int32, C.c_void_p]),

@@ -11,7 +11,9 @@ With `agents_per_scene=k` every k consecutive episodes form a scene whose MPC-dr
 obstacles (jmpc_scene_exchange); with `share_plans=True` they predict each other along their MPC plans
 (jmpc_scene_plans, jmpc_collision_planned); with `right_of_way` a rule decides which mates each vehicle yields to
 (jmpc_right_of_way, jmpc_collision_masked); with `depart` / `on_goal="leave"` every vehicle has a lifetime in its scene:
-it enters at its departure iteration and may leave at its goal (jmpc_scene_enter, jmpc_scene_presence).
+it enters at its departure iteration and may leave at its goal (jmpc_scene_enter, jmpc_scene_presence); with
+`from_trips` the scenes' slots are fed from a stream of timed trips (jmpc_scene_trips), and `run()` returns one row per
+trip.
 """
 from __future__ import annotations
 
@@ -153,6 +155,154 @@ def lifetime_setup(depart, on_goal: str, k: int, B: int):
     return np.ascontiguousarray(dep, dtype=np.int32), leave
 
 
+def _int_array(a, name: str, n: Optional[int] = None) -> np.ndarray:
+    arr = np.asarray(a)
+    if arr.ndim != 1 or not np.issubdtype(arr.dtype, np.integer):
+        raise ValueError(f"{name} must be a 1-D integer array")
+    if n is not None and len(arr) != n:
+        raise ValueError(f"{name} must be [{n}] (one entry per trip), got shape {arr.shape}")
+    return arr.astype(np.int64)
+
+
+class Trips:
+    """Validated trip arrays for `BatchedEpisodes.from_trips`.  Trip t: scene[t] (its scene), arrival[t] (integer >= 0,
+    the earliest loop iteration of its first step), course_id[t] (a course id, or a plan index with `plans`),
+    state[t] (x, y, v, yaw start state; omitted with plans, whose start states come from the planned courses),
+    params[t] (NPARAM row; default the engine's defaults) and priority[t] (the fixed rule's key; default the trip's
+    rank in its scene's order)."""
+
+    def __init__(self, scene, arrival, course_id, state=None, params=None, priority=None):
+        self.scene = _int_array(scene, "scene")
+        n = self.n = len(self.scene)
+        if n < 1:
+            raise ValueError("Trips needs at least one trip")
+        self.arrival = _int_array(arrival, "arrival", n)
+        if (self.arrival < 0).any():
+            raise ValueError("arrival must be >= 0")
+        if (self.arrival > np.iinfo(np.int32).max).any():
+            raise ValueError("arrival must fit in int32")
+        self.course_id = _int_array(course_id, "course_id", n)
+        self.state = None if state is None else np.asarray(state, np.float64)
+        if self.state is not None and self.state.shape != (n, 4):
+            raise ValueError(f"state must be [{n}, 4], got shape {self.state.shape}")
+        self.params = None if params is None else np.asarray(params, np.float64)
+        if self.params is not None and self.params.shape != (n, NPARAM):
+            raise ValueError(f"params must be [{n}, {NPARAM}], got shape {self.params.shape}")
+        self.priority = None if priority is None else np.asarray(priority, np.float64)
+        if self.priority is not None:
+            if self.priority.shape != (n,):
+                raise ValueError(f"priority must be [{n}] (one key per trip), got shape {self.priority.shape}")
+            if not np.isfinite(self.priority).all():
+                raise ValueError("priority must be finite")
+
+
+def poisson_trips(n_scenes: int, routes, rate_per_hour: float, dt: float, n_iterations: int, entry_speed: float = 0.0,
+                  seed: int = 0) -> Trips:
+    """Seeded Poisson demand: in every scene each approach (route group) of `routes` sends vehicles at rate_per_hour,
+    with exponential gaps in seconds; a vehicle arriving at time a enters no earlier than iteration floor(a / dt), and
+    arrivals from n_iterations on are dropped.  Each vehicle takes a route of its approach uniformly at random.
+    routes[g] is a list of (course_id, (x, y, yaw)) pairs: the trip starts at that pose at entry_speed.  With
+    (course_id, None) pairs (plan indices) the trips carry no state, for `from_trips(plans=...)`."""
+    if rate_per_hour < 0 or dt <= 0 or n_iterations < 0 or n_scenes < 1:
+        raise ValueError("poisson_trips needs rate_per_hour >= 0, dt > 0, n_iterations >= 0 and n_scenes >= 1")
+    rng = np.random.default_rng(seed)
+    rate = rate_per_hour / 3600.0
+    horizon = n_iterations * dt
+    planned = all(pose is None for group in routes for _, pose in group)
+    scene, arrival, cid, state = [], [], [], []
+    for s in range(n_scenes):
+        for group in routes:
+            t = 0.0
+            while rate > 0:
+                t += rng.exponential(1.0 / rate)
+                it = int(math.floor(t / dt))
+                if t >= horizon or it >= n_iterations:
+                    break
+                course, pose = group[int(rng.integers(len(group)))]
+                scene.append(s), arrival.append(it), cid.append(int(course))
+                if not planned:
+                    state.append([pose[0], pose[1], entry_speed, pose[2]])
+    order = np.lexsort((np.arange(len(scene)), arrival, scene))
+    take = lambda a: np.asarray(a)[order] if len(a) else np.zeros(0, np.int64)   # noqa: E731
+    return Trips(take(scene), take(arrival), take(cid),
+                 None if planned else np.asarray(state, np.float64).reshape(-1, 4)[order])
+
+
+def trips_setup(trips: Trips, n_scenes: int, k, n_courses: int, planned: bool, n_extra: int, right_of_way,
+                share_plans: bool, params_default, depart=None, on_goal=None, obstacle_script=None):
+    """Host-side checks of `BatchedEpisodes.from_trips`.  Returns (order, params [N, NPARAM], priority or None): order
+    sorts the trips by (scene, arrival, trip index), the layout the trips pass walks."""
+    if depart is not None or on_goal is not None:
+        raise ValueError("depart / on_goal do not apply to trips: a trip enters at its arrival and leaves at its goal")
+    if obstacle_script is not None:
+        raise ValueError("obstacle_script cannot be combined with trips: give obstacles or obstacle_program")
+    if not isinstance(trips, Trips):
+        raise ValueError("trips must be a Trips object")
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 2 <= k <= MAX_OBSTACLES + 1:
+        raise ValueError(f"trips need agents_per_scene in [2, {MAX_OBSTACLES + 1}], got {k!r}")
+    if (k - 1) + n_extra > MAX_OBSTACLES:
+        raise ValueError(f"{k - 1} scene mates + {n_extra} obstacles exceed the {MAX_OBSTACLES} obstacle slots of an "
+                         "episode")
+    if isinstance(n_scenes, bool) or not isinstance(n_scenes, (int, np.integer)) or n_scenes < 1:
+        raise ValueError(f"n_scenes must be an integer >= 1, got {n_scenes!r}")
+    if trips.scene.min() < 0 or trips.scene.max() >= n_scenes:
+        raise ValueError(f"trip scene out of range [0, {n_scenes})")
+    if trips.course_id.min() < 0 or trips.course_id.max() >= n_courses:
+        raise ValueError(f"trip course_id out of range [0, {n_courses})")
+    if planned and trips.state is not None:
+        raise ValueError("with plans the start states come from the planned courses: give no state")
+    if not planned and trips.state is None:
+        raise ValueError("trips need state [N, 4] unless plans are given")
+    if trips.priority is not None and right_of_way != "fixed":
+        raise ValueError("priority is an argument of the fixed right-of-way rule")
+    order = np.lexsort((np.arange(trips.n), trips.arrival, trips.scene))
+    params = (np.repeat(np.asarray(params_default, np.float64)[None, :], trips.n, axis=0) if trips.params is None
+              else trips.params)[order]
+    if share_plans:
+        dt = params[:, PARAM_INDEX["dt"]]
+        scene = trips.scene[order]
+        first = np.r_[True, scene[1:] != scene[:-1]]
+        ref = dt[np.flatnonzero(first)[np.cumsum(first) - 1]]
+        bad = np.flatnonzero(dt != ref)
+        if len(bad):
+            raise ValueError(f"share_plans=True needs one dt per scene: scene {int(scene[bad[0]])} has trips with dt "
+                             f"{float(ref[bad[0]])} and {float(dt[bad[0]])}")
+    priority = None
+    if right_of_way == "fixed":
+        if trips.priority is not None:
+            priority = trips.priority[order]
+        else:
+            scene = trips.scene[order]
+            start = np.searchsorted(scene, scene, side="left")
+            priority = (np.arange(trips.n) - start).astype(np.float64)
+    return order, np.ascontiguousarray(params), priority
+
+
+TRIP_STATE = ("slot", "entry", "exit", "steps", "done", "blocked_waits")
+
+
+def trip_holding(slot, entry, exit, k: int, obs, evaluation) -> np.ndarray:
+    """The trip that held mate slot `obs` of trip t's slot at evaluation `evaluation` [N] (trip table columns slot,
+    entry, exit [N]; a trip is in its slot at evaluations entry .. exit).  -1 where obs is -1 or an extra (>= k - 1)."""
+    slot, entry, exit, obs, evaluation = (np.asarray(a, np.int64) for a in (slot, entry, exit, obs, evaluation))
+    out = np.full(len(slot), -1, np.int64)
+    held = np.flatnonzero(slot >= 0)
+    q = np.flatnonzero((obs >= 0) & (obs < k - 1) & (slot >= 0))
+    if not len(held) or not len(q):
+        return out
+    span = int(max(entry.max(), exit.max(), evaluation.max())) + 2
+    key = slot[held] * span + entry[held]
+    by = np.argsort(key, kind="stable")
+    key, held = key[by], held[by]
+    j = slot[q] % k
+    mate = slot[q] - j + np.where(obs[q] < j, obs[q], obs[q] + 1)          # jmpc_scene_exchange's mate order
+    pos = np.searchsorted(key, mate * span + evaluation[q], side="right") - 1
+    u = held[np.maximum(pos, 0)]
+    hit = (pos >= 0) & (slot[u] == mate) & (entry[u] <= evaluation[q]) & (evaluation[q] <= exit[u])
+    out[q[hit]] = u[hit]
+    return out
+
+
 def outcome_columns(record) -> dict:
     """[B, >= len(OUTCOME_NAMES)] float64 outcome records -> dict of [B] arrays keyed by OUTCOME_NAMES (the index and
     count columns as int64)."""
@@ -255,6 +405,161 @@ class BatchedEpisodes:
             _cabi.check(engine._lib.jmpc_scene_init(engine._h, B, ep.k, ep._p(ep.done), stream), "jmpc_scene_init")
         ep._plans = (plans, ep.course_id.long())
         return ep
+
+    @classmethod
+    def from_trips(cls, engine: BatchedMPC, trips: Trips, n_scenes: int, agents_per_scene: int = 4, plans=None,
+                   entry_gap: float = 2.0, obstacles=None, obstacle_program=None, frame_window: int = 10,
+                   margin: int = 72, max_steps: int = 256, record_history: bool = True, horizon_s: float = 7.0,
+                   outcomes: bool = False, record_obstacles: bool = False, share_plans: bool = False,
+                   right_of_way=None, junction=None, depart=None, on_goal=None,
+                   obstacle_script=None) -> "BatchedEpisodes":
+        """Scenes fed from a stream of timed trips (jmpc_scene_trips / jmpc_scene_trips_finish in include/jmpc.h).
+        The batch is n_scenes x k slots (episode b = s * k + j is slot j of scene s, k in [2, 9]); a slot holds at most
+        one trip at a time and starts empty.  An empty slot is handled as a vehicle that has not entered under lifetimes:
+        not stepped, absent for its mates, NaN obstacle_history rows, its extras keep the loop's clock.  Once before
+        evaluation 0 and then in every loop iteration i (after the extras advance, before the exchange) the trips pass
+        closes the trips whose goal test fired (they always leave at the goal; a done = 2 vehicle keeps its slot), then
+        admits the scene's due trips (arrival <= i + 1) in (arrival, trip index) order into the lowest empty slot, when
+        their start pose has a clearance >= entry_gap metres to every vehicle in the scene and to every earlier trip
+        still pending (first-in, first-out per approach).  A trip whose planned course is unusable is closed with
+        done = 3.  An admitted slot is a fresh vehicle on the trip's course, params row and start state, entering at
+        evaluation i + 1 (entry).  run() stops when no slot is driving and no trip is pending, and adds `trips`.
+
+        trips: a `Trips` object; with `plans` (a planner result whose courses `engine` holds, as for from_plans) its
+        course_id are plan indices and the start states, dl and usability come from the planned courses.  The other
+        options are those of `__init__`: obstacles / obstacle_program are per-slot extras; share_plans needs one dt per
+        scene across its trips; right_of_way "fixed" takes the trips' priority (default: rank in the scene's order),
+        "first_come" a junction (once or per scene).  depart, on_goal and obstacle_script do not apply to trips."""
+        import torch
+        n_extra = 0
+        if obstacles is not None:
+            n_extra = int(np.shape(obstacles)[1])
+        elif obstacle_program is not None:
+            n_extra = int(np.shape(obstacle_program[0])[1])
+        planned = plans is not None
+        if planned and (engine.course_ok is None or len(engine.course_ok) != len(plans)):
+            raise ValueError("the engine's courses do not come from these plans (BatchedMPC.from_plans)")
+        n_courses = len(plans) if planned else len(engine.course_len)
+        k = agents_per_scene
+        order, params, priority = trips_setup(trips, n_scenes, k, n_courses, planned, n_extra, right_of_way,
+                                              share_plans, engine.default_params, depart, on_goal, obstacle_script)
+        entry_gap = float(entry_gap)
+        if not math.isfinite(entry_gap) or entry_gap < 0:
+            raise ValueError("entry_gap must be finite and >= 0")
+        if planned:
+            _, margin = plan_episode_setup(engine._ok_host, engine._dl_host, trips.course_id, len(plans),
+                                           engine.car_radius)
+        k, B, N = int(k), int(n_scenes) * int(k), trips.n
+        if B > engine.max_batch:
+            raise ValueError(f"n_scenes * k = {B} exceeds the engine's max_batch {engine.max_batch}")
+        row = right_of_way_setup(right_of_way, k, B, None, junction)
+        ep = cls(engine, np.zeros((B, 4)), course_id=np.zeros(B, np.int32), obstacles=obstacles,
+                 obstacle_program=obstacle_program, frame_window=frame_window, margin=margin,
+                 params=np.repeat(engine.default_params[None, :], B, axis=0), max_steps=max_steps,
+                 record_history=record_history, horizon_s=horizon_s, outcomes=outcomes,
+                 record_obstacles=record_obstacles, agents_per_scene=k, share_plans=share_plans, on_goal="leave")
+        dev, i32, f64 = ep.dev, torch.int32, torch.float64
+        t = lambda a, dt: torch.as_tensor(np.ascontiguousarray(a), dtype=dt, device=dev)   # noqa: E731
+        lib, h = engine._lib, engine._h
+        stream = C.c_void_p(torch.cuda.current_stream(engine.device).cuda_stream)
+        scene = trips.scene[order]
+        T = dict(scene_start=t(np.searchsorted(scene, np.arange(n_scenes + 1)), i32), arrival=t(trips.arrival[order], i32),
+                 course_id=t(trips.course_id[order], i32), params=t(params, f64))
+        T["course_len"] = torch.as_tensor(engine.course_len, dtype=i32, device=dev)[T["course_id"].long()].contiguous()
+        usable = torch.zeros(N, dtype=i32, device=dev)          # jmpc_episode_init_from_courses writes 3 where unusable
+        T["start"] = t(np.zeros((N, 4)) if planned else trips.state[order], f64)
+        if planned:
+            for a in range(0, N, engine.max_batch):
+                n = min(engine.max_batch, N - a)
+                _cabi.check(lib.jmpc_episode_init_from_courses(
+                    h, n, ep._p(T["course_id"][a:]), ep._p(engine.course_ok), ep._p(engine.course_dl),
+                    ep._p(T["start"][a:]), ep._p(T["params"][a:]), ep._p(usable[a:]), stream),
+                    "jmpc_episode_init_from_courses")
+        T["usable"] = (usable == 0).to(i32)
+        bad = np.where(T["usable"].cpu().numpy() == 0, np.arange(N), N)     # the first unusable trip at or after t
+        T["next_unusable"] = t(np.minimum.accumulate(bad[::-1])[::-1], i32)
+        T["zone"] = T["priority"] = None
+        if row is not None:
+            ep.row_rule, _, junc = row
+            ep.consider = torch.full((B,), -1, dtype=i32, device=dev)
+            ep._collision_mask = ep.consider
+            if junc is not None:
+                ep.junction = t(junc, f64)
+                ep.zone = torch.full((B, 2), -1, dtype=i32, device=dev)
+                per_trip = t(junc[scene] if len(junc) > 1 else np.repeat(junc, N, axis=0), f64)
+                T["zone"] = torch.empty(N, 2, dtype=i32, device=dev)
+                for a in range(0, N, engine.max_batch):
+                    n = min(engine.max_batch, N - a)
+                    _cabi.check(lib.jmpc_right_of_way_init(
+                        h, n, 1, ep._p(T["course_id"][a:]), ep._p(per_trip[a:]), n, ep._p(T["zone"][a:]), stream),
+                        "jmpc_right_of_way_init")
+            else:
+                ep.priority = torch.zeros(B, dtype=f64, device=dev)
+                T["priority"] = t(priority, f64)
+        z = lambda v: torch.full((N,), v, dtype=i32, device=dev)   # noqa: E731
+        T.update(cursor=T["scene_start"][:-1].clone(), pending=t(np.bincount(scene, minlength=n_scenes), i32),
+                 phase=z(0), slot_trip=torch.full((B,), -1, dtype=i32, device=dev), slot=z(-1), entry=z(-1),
+                 exit=z(-1), steps=z(0), done=z(_cabi.WAITING), blocked_waits=z(0),
+                 outcomes=(torch.full((N, len(OUTCOME_NAMES)), 0.0, dtype=f64, device=dev) if ep.outcomes is not None
+                           else None))
+        if T["outcomes"] is not None:                          # the empty record, for trips that never drive
+            T["outcomes"][:, OUTCOME_NAMES.index("min_clearance")] = math.inf
+            for c in ("min_clearance_eval", "min_clearance_obs", "first_contact_eval", "first_contact_obs"):
+                T["outcomes"][:, OUTCOME_NAMES.index(c)] = -1.0
+        ep.done.fill_(_cabi.WAITING)
+        ep._trips = T
+        ep._trip_order = order
+        ep._trips_struct = _cabi.Trips(
+            n_scenes=int(n_scenes), k=k, n_trips=N, T=ep.T, entry_gap=entry_gap,
+            **{n: T[n].data_ptr() if T[n] is not None else None for n in (
+                "scene_start", "arrival", "course_id", "course_len", "usable", "next_unusable", "start", "params",
+                "zone", "priority", "cursor", "pending", "phase", "slot_trip", "slot", "entry", "exit", "steps", "done",
+                "blocked_waits", "outcomes")},
+            state=ep.state.data_ptr(), ep_course_id=ep.course_id.data_ptr(), ep_params=ep.params.data_ptr(),
+            ep_course_len=ep.course_len.data_ptr(), target_ind=ep.target_ind.data_ptr(),
+            agent_idx=ep.agent_idx.data_ptr(), ep_steps=ep.steps.data_ptr(), warm=ep.warm.data_ptr(),
+            flag=ep.flag.data_ptr(), di=ep.di.data_ptr(), oa=ep.oa.data_ptr(), od=ep.od.data_ptr(),
+            ep_zone=None if ep.zone is None else ep.zone.data_ptr(),
+            ep_priority=None if T["priority"] is None else ep.priority.data_ptr(), depart=ep.depart.data_ptr(),
+            ep_done=ep.done.data_ptr(), ep_outcomes=None if ep.outcomes is None else ep.outcomes.data_ptr())
+        return ep
+
+    def _trips_pass(self, initial: int):
+        e = self.e
+        stream = C.c_void_p(self.torch.cuda.current_stream(e.device).cuda_stream)
+        _cabi.check(e._lib.jmpc_scene_trips(e._h, C.byref(self._trips_struct), self._p(self.iter_dev), int(initial),
+                                            stream), "jmpc_scene_trips")
+
+    def _trip_table(self) -> dict:
+        """The trip table in the caller's trip order (jmpc_scene_trips_finish first)."""
+        e, T = self.e, self._trips
+        stream = C.c_void_p(self.torch.cuda.current_stream(e.device).cuda_stream)
+        _cabi.check(e._lib.jmpc_scene_trips_finish(e._h, C.byref(self._trips_struct), self.iteration, stream),
+                    "jmpc_scene_trips_finish")
+        order = self._trip_order
+        N = len(order)
+
+        def back(a):
+            out = np.empty((N,) + a.shape[1:], a.dtype)
+            out[order] = a
+            return out
+        scene_sorted = np.repeat(np.arange(len(T["scene_start"]) - 1), np.diff(T["scene_start"].cpu().numpy()))
+        res = dict(scene=back(scene_sorted.astype(np.int64)), arrival=back(T["arrival"].cpu().numpy().astype(np.int64)))
+        for n in TRIP_STATE:
+            res[n] = back(T[n].cpu().numpy().astype(np.int64))
+        # every pass in which a trip is due and pending waits for a slot or is blocked: the passes of entries
+        # arrival .. entry - 1, or arrival .. self.iteration for a trip still pending
+        due = np.where(res["entry"] >= 0, res["entry"] - res["arrival"],
+                       np.where(res["done"] == _cabi.WAITING, np.maximum(self.iteration + 1 - res["arrival"], 0), 0))
+        res["slot_waits"] = due - res["blocked_waits"]
+        res["entry_delay"] = np.where(res["entry"] >= 0, res["entry"] - res["arrival"], -1)
+        res["travel"] = np.where((res["entry"] >= 0) & (res["exit"] >= 0), res["exit"] - res["entry"], -1)
+        if T["outcomes"] is not None:
+            res.update(outcome_columns(back(T["outcomes"].cpu().numpy())))
+            for col in ("min_clearance", "first_contact"):
+                res[f"{col}_trip"] = trip_holding(res["slot"], res["entry"], res["exit"], self.k,
+                                                  res[f"{col}_obs"], res[f"{col}_eval"])
+        return res
 
     def __init__(self, engine: BatchedMPC, state0, course_id=None, obstacles=None, obstacle_script=None,
                  frame_window: int = 10, margin: int = 72, params=None, max_steps: int = 256,
@@ -394,6 +699,7 @@ class BatchedEpisodes:
             if record_obstacles:
                 self.obstacle_history = torch.full((self.max_steps + 1, B, n_obs, 6), float("nan"), dtype=f64,
                                                    device=self.dev)
+        self._trips = None                                            # from_trips: the trip arrays and table
         self._started = False
         if self.program is not None:                                 # get() before the first iteration
             self._scripted_step(advance=0)
@@ -460,6 +766,8 @@ class BatchedEpisodes:
         the waiting codes, the scene's first exchange, then evaluation 0 of the outcome record."""
         if self._started:
             return
+        if self._trips is not None:
+            self._trips_pass(initial=1)
         if self._entering:
             e = self.e
             stream = C.c_void_p(self.torch.cuda.current_stream(e.device).cuda_stream)
@@ -525,6 +833,8 @@ class BatchedEpisodes:
         elif self.obstacles is not None and self.obstacles.shape[1] > 0:
             _cabi.check(lib.jmpc_obstacle_step(e._h, self.B, int(self.obstacles.shape[1]), self._p(self.obstacles),
                                                self._p(self.done), float(e.dt), stream), "jmpc_obstacle_step")
+        if self._trips is not None:            # close finished trips, admit the trips whose first step is i + 1
+            self._trips_pass(initial=0)
         if self._entering:                     # the vehicles whose first step is iteration i + 1
             _cabi.check(lib.jmpc_scene_enter(e._h, self.B, self._p(self.depart), self._p(self.iter_dev),
                                              self._p(self.done), stream), "jmpc_scene_enter")
@@ -538,7 +848,9 @@ class BatchedEpisodes:
         self.iteration += 1
 
     def _finished(self) -> bool:
-        """No episode is running (done = 0) or waiting to enter (done = WAITING)."""
+        """No episode is running (done = 0) or waiting to enter (done = WAITING; with trips: no trip is pending)."""
+        if self._trips is not None:
+            return not bool(((self.done == 0).any() | (self._trips["pending"] != 0).any()).item())
         if self._entering:
             return bool(((self.done != 0) & (self.done != _cabi.WAITING)).all().item())
         return bool((self.done != 0).all().item())
@@ -588,6 +900,7 @@ class BatchedEpisodes:
                                          self._p(self.target_ind), self._p(self.steps), self._p(self.agent_idx),
                                          self._p(self.done), float(e.config.goal_dis), float(e.config.stop_speed), stream),
                     "jmpc_episode_pre")
+        trips = self._trip_table() if self._trips is not None else None
         self.torch.cuda.synchronize(e.device)
         res = dict(steps=self.steps.cpu().numpy(), done=self.done.cpu().numpy(), state=self.state.cpu().numpy(),
                    iterations=self.iteration)
@@ -601,6 +914,8 @@ class BatchedEpisodes:
             res["outcomes"] = outcome_columns(self.outcomes.cpu().numpy())
             if self.obstacle_history is not None:
                 res["obstacle_history"] = self.obstacle_history[:min(self.iteration, self.max_steps) + 1].cpu().numpy()
+        if trips is not None:
+            res["trips"] = trips
         if self._plans is not None:
             plans, pid = self._plans
             res.update(plan_status=plans.status[pid].cpu().numpy(), plan_cost=plans.cost[pid].cpu().numpy(),

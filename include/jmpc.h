@@ -465,6 +465,82 @@ int32_t jmpc_episode_outcomes_scene(jmpc_handle h, int32_t B, const double* stat
                                     int32_t initial, double* outcomes, double* obstacle_history, int32_t history_rows,
                                     void* stream);
 
+/* Trips (opt-in): scenes fed from a stream of timed trips instead of a fixed cast of k vehicles.  The batch is
+ * B = n_scenes * k episodes as above, k in [2, 9]; episode b = s * k + j is now SLOT j of scene s, and a slot holds at
+ * most one trip at a time.  An empty slot has done = JMPC_WAITING and no trip, so it is handled exactly as a vehicle
+ * that has not entered under lifetimes: not stepped, absent for its mates (jmpc_scene_presence with leave = 1), NaN
+ * obstacle_history rows, its extras keep the loop's clock.  All slots start empty.  DEVICE pointers throughout.
+ *   Trip t (n_trips of them) has a scene, an arrival iteration arrival[t] >= 0 (the earliest loop iteration of its
+ *   first step), a course, a start state, a params row and the right-of-way inputs of a vehicle (zone, priority).  The
+ *   trips of scene s are t = scene_start[s] .. scene_start[s + 1] - 1, sorted by (arrival, trip index): the scene's
+ *   order.  The constants (start, params, course_len = the course's length, usable, zone, priority) are prepared once
+ *   with the existing kernels: jmpc_episode_init_from_courses on the trip arrays for planned start states, dl and
+ *   usable (= course_ok), jmpc_right_of_way_init with k = 1 and one junction row per trip for the zones.
+ * jmpc_scene_trips: the trips pass, one thread per scene.  initial = 1 runs it once before evaluation 0 and admits
+ *   arrivals <= 0 with entry 0; otherwise it runs in loop iteration i = *iter_dev where jmpc_scene_enter runs under
+ *   lifetimes (after the extras advance, before the exchange) and admits arrivals <= i + 1 with entry i + 1.  Per scene:
+ *   1. close: a slot whose vehicle has done = 1 (goal test at the top of iteration g = i) writes its trip's row,
+ *      exit = g, steps, done = 1 and, with outcomes, the public columns of its outcome record; the slot becomes empty.
+ *      A done = 2 vehicle (index rule) stays parked and keeps its slot.
+ *   2. admit: the scene's pending trips with arrival <= i + 1, in scene order.  A trip whose course is not usable is
+ *      closed with done = 3 (no slot, blocks nothing).  Any other is admitted iff a slot is empty (the lowest is taken)
+ *      and its start pose is clear: clearance >= entry_gap to every vehicle present in the scene at its current state
+ *      (trips admitted earlier in this pass included, at their start poses) and to every earlier pending trip at its
+ *      start pose, so that an approach is first-in, first-out.  Clearance is the outcome record's (two circles of
+ *      jmpc_set_car_geometry per car, min over the 4 pairs of dist - 2r, no fused multiply-add).  A due trip that is
+ *      not admitted waits: for a slot (no empty slot) or else blocked (start pose not clear).  The pass counts the
+ *      blocked waits; the slot waits are not written: they are (passes due before entry) - blocked_waits, the due
+ *      passes being those of entries arrival .. entry - 1 (of a trip never admitted: arrival .. the last entry).
+ *   3. load: the slot becomes a fresh vehicle, as jmpc_episode_init_from_courses leaves one: state, course_id, params
+ *      row and course_len of the trip, target_ind = agent_idx = steps = warm = flag = 0, di = 0, oa = od = 0, zone
+ *      (first_come) and priority (fixed) of the trip, depart[b] = entry (jmpc_episode_outcomes_scene starts its record
+ *      at that evaluation), done = 0; the trip's slot and entry are written.
+ *   pending [n_scenes] counts the trips not yet admitted or closed (arrived or not); a run is over when no slot has
+ *   done = 0 and every pending count is 0.  iter_dev is jmpc_episode_post_dev's counter: no per-iteration host argument.
+ * jmpc_scene_trips_finish: closes every trip still in a slot with its slot's current done (0 still driving, 2 index
+ *   rule, 1 when the goal test fired after the last iteration), exit = n_iterations, steps and outcome columns.  It
+ *   changes no slot.  A trip never admitted keeps entry = exit = slot = -1 and done = JMPC_WAITING.
+ *   Order of one iteration with trips: pre, right_of_way, presence (collision mask, leave = 1), collision_masked, step,
+ *   post_dev, extras' advance, trips, exchange (+ plans), presence (evaluation mask), outcomes_scene, counter_add; before
+ *   iteration 0: trips (initial = 1), exchange (+ plans), presence, outcomes_scene (initial = 1).
+ *   The caller initialises the trip state: cursor = scene_start[s], pending = the scene's trip count, phase = 0,
+ *   slot_trip = -1, slot = entry = exit = -1, steps = 0, done = JMPC_WAITING, blocked_waits = 0, and every slot's done =
+ *   JMPC_WAITING. */
+typedef struct jmpc_trips {
+  int32_t n_scenes, k, n_trips, T;         /* T: the horizon of oa / od                                            */
+  double entry_gap;                        /* metres, finite, >= 0                                                 */
+  /* trips, constant */
+  const int32_t* scene_start;              /* [n_scenes + 1]                                                       */
+  const int32_t* arrival;                  /* [n_trips]                                                            */
+  const int32_t* course_id;                /* [n_trips]                                                            */
+  const int32_t* course_len;               /* [n_trips] the course's length                                        */
+  const int32_t* usable;                   /* [n_trips] 0: closed with done = 3 when due                           */
+  const int32_t* next_unusable;            /* [n_trips] the first u >= t with usable[u] = 0, n_trips if none      */
+  const double* start;                     /* [n_trips][4] x, y, v, yaw                                            */
+  const double* params;                    /* [n_trips][JMPC_NPARAM]                                               */
+  const int32_t* zone;                     /* [n_trips][2] or NULL (first_come)                                    */
+  const double* priority;                  /* [n_trips] or NULL (fixed)                                            */
+  /* trip state and the trip table */
+  int32_t* cursor;                         /* [n_scenes] first trip of the scene that may still be pending         */
+  int32_t* pending;                        /* [n_scenes]                                                           */
+  int32_t* phase;                          /* [n_trips] 0 pending, 1 in a slot, 2 closed                           */
+  int32_t* slot_trip;                      /* [B] trip in the slot, -1 empty                                       */
+  int32_t *slot, *entry, *exit, *steps, *done, *blocked_waits;   /* [n_trips]                                   */
+  double* outcomes;                        /* [n_trips][JMPC_NOUTCOME] or NULL                                     */
+  /* the episodes (slots) */
+  double* state; int32_t* ep_course_id; double* ep_params; int32_t* ep_course_len;
+  int32_t *target_ind, *agent_idx, *ep_steps, *warm, *flag;
+  double *di, *oa, *od;                    /* [B], [B][T], [B][T]                                                  */
+  int32_t* ep_zone;                        /* [B][2] or NULL (first_come)                                          */
+  double* ep_priority;                     /* [B] or NULL (fixed)                                                  */
+  int32_t* depart;                         /* [B]                                                                  */
+  int32_t* ep_done;                        /* [B]                                                                  */
+  const double* ep_outcomes;               /* [B][JMPC_OUTCOME_LEN] or NULL                                        */
+} jmpc_trips;
+int32_t jmpc_scene_trips(jmpc_handle h, const jmpc_trips* trips, const int32_t* iter_dev, int32_t initial,
+                         void* stream);
+int32_t jmpc_scene_trips_finish(jmpc_handle h, const jmpc_trips* trips, int32_t n_iterations, void* stream);
+
 /* The reference's scripted obstacles on the device (main/lib/moving_obstacles.py: MovingObstacleTIntersection :166-232,
  * MovingObstacleRoundabout :28-123 including its dt = 0.2 quirk at :45 and the theta overwrite inside its steering
  * property, MovingObstacleArterial :125-164).  DEVICE pointers.
