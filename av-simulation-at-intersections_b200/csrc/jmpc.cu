@@ -1239,6 +1239,49 @@ int32_t jmpc_scene_trips_finish(jmpc_handle h, const jmpc_trips* trips, int32_t 
   return 0;
 }
 
+int32_t jmpc_signals(jmpc_handle h, int32_t B, int32_t k, const jmpc_signal_plan* plan, const int32_t* offset,
+                     const int32_t* owner, const int32_t* group, const int32_t* zone, const int32_t* course_id,
+                     const int32_t* agent_idx, const double* state, const double* params, const int32_t* done,
+                     int32_t checked, int32_t* course_len, int32_t* latch, int32_t* hold_steps, int32_t* go,
+                     int32_t* slot_hold_steps, int32_t* slot_go, const int32_t* iter_dev, void* stream) {
+  if (!h) return fail("jmpc_signals: NULL handle");
+  if (B < 0 || B > h->max_B) return fail("jmpc_signals: B out of range");
+  if (k < 1 || B % k != 0) return fail("jmpc_signals: B must be a multiple of k >= 1");
+  if (!plan) return fail("jmpc_signals: NULL plan");
+  if (plan->cycle < 1) return fail("jmpc_signals: cycle must be >= 1");
+  if (plan->n_groups < 1 || plan->n_groups > JMPC_SIGNAL_MAX_GROUPS)
+    return fail("jmpc_signals: n_groups must be in [1, 8]");
+  for (int g = 0; g < plan->n_groups; ++g) {
+    if (plan->green_start[g] < 0 || plan->green_start[g] >= plan->cycle)
+      return fail("jmpc_signals: green_start must be in [0, cycle)");
+    if (plan->green_len[g] < 0 || plan->green_len[g] > plan->cycle)
+      return fail("jmpc_signals: green_len must be in [0, cycle]");
+  }
+  if (!(plan->stop_decel > 0.0) || !isfinite(plan->stop_decel))
+    return fail("jmpc_signals: stop_decel must be finite and > 0");
+  if (plan->margin < 0 || plan->margin > h->max_N)
+    return fail("jmpc_signals: margin must be in [0, max_N]");
+  if (!group || !zone || !agent_idx || !state || !done || !course_len || !latch || !hold_steps || !go || !iter_dev)
+    return fail("jmpc_signals: NULL array");
+  if (!slot_hold_steps != !slot_go) return fail("jmpc_signals: slot_hold_steps and slot_go go together");
+  if (!checked && h->n_courses < 1) return fail("jmpc_signals: no courses uploaded (jmpc_set_courses)");
+  if (B == 0) return 0;
+  CK(cudaSetDevice(h->device));
+  jmpc::SignalArgs a;
+  a.plan = *plan;
+  a.B = B; a.k = k; a.n_courses = h->n_courses;
+  a.offset = offset; a.owner = owner; a.group = group; a.zone = zone; a.course_id = course_id;
+  a.course_n = h->d_course_n;
+  a.agent_idx = agent_idx; a.state = state; a.params = params; a.default_dl = h->defaults[JMPC_P_DL];
+  a.done = done; a.checked = checked ? 1 : 0; a.course_len = course_len; a.latch = latch;
+  a.hold_steps = hold_steps; a.go = go; a.slot_hold_steps = slot_hold_steps; a.slot_go = slot_go;
+  a.iter_dev = iter_dev;
+  jmpc::signal_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(a);
+  CK(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
 int32_t jmpc_scene_exchange(jmpc_handle h, int32_t B, int32_t k, int32_t n_extra, const double* state,
                             const double* record, const double* di, const double* params, const int32_t* done,
                             const int32_t* steps, const double* extras, double* obstacles_out, void* stream) {

@@ -593,6 +593,77 @@ __global__ void scene_trips_finish_kernel(const jmpc_trips P, int n_iterations) 
   if (t >= 0) close_trip(P, t, b, n_iterations, P.ep_done[b]);
 }
 
+// ---- fixed-time traffic signals (jmpc_signals) ----------------------------------------------------------------------
+struct SignalArgs {
+  jmpc_signal_plan plan;
+  int B, k, n_courses;
+  const int* offset;        // [B / k] or nullptr
+  const int* owner;         // [B] or nullptr: owner = b
+  const int* group;         // [n_owner]
+  const int* zone;          // [n_owner][2]
+  const int* course_id;     // [B] or nullptr
+  const int* course_n;      // the handle's course lengths
+  const int* agent_idx; const double* state; const double* params; double default_dl;
+  const int* done;
+  int checked;
+  int* course_len;          // [B] in-out
+  int* latch;               // [B][2] (owner, 1 HOLD / 0 GO)
+  int* hold_steps; int* go;                 // [n_owner]
+  int* slot_hold_steps; int* slot_go;       // [B] or nullptr
+  const int* iter_dev;
+};
+
+// One thread per episode: the red-light cut at L = e - margin, decided once per red phase and owner.
+__global__ void signal_kernel(const SignalArgs A) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= A.B || A.done[b] != JMPC_DONE_RUNNING) return;
+  int len;
+  if (A.checked) {
+    len = A.course_len[b];
+  } else {                                  // what a flag-0 collision check writes
+    len = A.course_n[A.course_id ? min(max(A.course_id[b], 0), A.n_courses - 1) : 0];
+    A.course_len[b] = len;
+  }
+  const int o = A.owner ? A.owner[b] : b;
+  const int g = A.group[o], e = A.zone[2 * (size_t)o];
+  bool red = false;
+  if (g >= 0 && g < A.plan.n_groups && e >= 0) {
+    const long long d = (long long)*A.iter_dev + (A.offset ? A.offset[b / A.k] : 0) - A.plan.green_start[g];
+    long long m = d % A.plan.cycle;
+    if (m < 0) m += A.plan.cycle;
+    red = m >= A.plan.green_len[g];
+  }
+  int* latch = A.latch + 2 * (size_t)b;
+  if (!red) {
+    if (latch[0] != -1) {                   // most latches are already empty: store only to clear one
+      latch[0] = -1;
+      latch[1] = 0;
+    }
+    return;
+  }
+  const int a = A.agent_idx[b], L = e - A.plan.margin;
+  int hold;
+  if (latch[0] == o) {
+    hold = latch[1];
+  } else {
+    const double v = A.state[4 * (size_t)b + 2];
+    const double dl = A.params ? A.params[(size_t)b * JMPC_NPARAM + JMPC_P_DL] : A.default_dl;
+    const double reach = __dmul_rn(__dmul_rn(__dmul_rn(2.0, A.plan.stop_decel), (double)(L - 1 - a)), dl);
+    hold = (a < L && __dmul_rn(v, v) <= reach) ? 1 : 0;
+    latch[0] = o;
+    latch[1] = hold;
+    if (!hold && a < L) {                   // could not stop before the line: a dilemma-zone pass
+      A.go[o] += 1;
+      if (A.slot_go) A.slot_go[b] += 1;
+    }
+  }
+  if (hold) {
+    A.course_len[b] = min(len, max(a + 1, L));
+    A.hold_steps[o] += 1;
+    if (A.slot_hold_steps) A.slot_hold_steps[b] += 1;
+  }
+}
+
 // The extras of a waiting vehicle keep to the loop's clock: they advance as those of a running one.
 __device__ __forceinline__ bool extras_advance(int done) { return done == JMPC_DONE_RUNNING || done == JMPC_WAITING; }
 

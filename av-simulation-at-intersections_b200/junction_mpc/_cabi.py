@@ -39,6 +39,15 @@ class Trips(C.Structure):
                     "depart", "ep_done", "ep_outcomes")])
 
 
+SIGNAL_MAX_GROUPS = 8
+
+
+class SignalPlan(C.Structure):
+    """struct jmpc_signal_plan (include/jmpc.h): a fixed-time signal plan, passed by pointer and copied per call."""
+    _fields_ = [("cycle", C.c_int32), ("n_groups", C.c_int32), ("green_start", C.c_int32 * SIGNAL_MAX_GROUPS),
+                ("green_len", C.c_int32 * SIGNAL_MAX_GROUPS), ("margin", C.c_int32), ("stop_decel", C.c_double)]
+
+
 # name -> (restype, argtypes); the exported-symbol test walks this table against include/jmpc.h
 SIGNATURES = {
     "jmpc_abi_version": (C.c_int32, []),
@@ -99,6 +108,8 @@ SIGNATURES = {
                                     + [C.c_void_p] * 8 + [C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "jmpc_scene_trips": (C.c_int32, [C.c_void_p, C.POINTER(Trips), C.c_void_p, C.c_int32, C.c_void_p]),
     "jmpc_scene_trips_finish": (C.c_int32, [C.c_void_p, C.POINTER(Trips), C.c_int32, C.c_void_p]),
+    "jmpc_signals": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(SignalPlan)] + [C.c_void_p] * 9
+                     + [C.c_int32] + [C.c_void_p] * 8),
     "jmpc_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]),
     "jmpc_scripted_obstacle_step": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                                 C.c_void_p, C.c_int32, C.c_void_p]),

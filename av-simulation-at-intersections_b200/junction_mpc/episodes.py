@@ -13,7 +13,7 @@ obstacles (jmpc_scene_exchange); with `share_plans=True` they predict each other
 (jmpc_right_of_way, jmpc_collision_masked); with `depart` / `on_goal="leave"` every vehicle has a lifetime in its scene:
 it enters at its departure iteration and may leave at its goal (jmpc_scene_enter, jmpc_scene_presence); with
 `from_trips` the scenes' slots are fed from a stream of timed trips (jmpc_scene_trips), and `run()` returns one row per
-trip.
+trip; with `signals` a fixed-time signal plan cuts the courses of vehicles facing red at their stop line (jmpc_signals).
 """
 from __future__ import annotations
 
@@ -168,10 +168,10 @@ class Trips:
     """Validated trip arrays for `BatchedEpisodes.from_trips`.  Trip t: scene[t] (its scene), arrival[t] (integer >= 0,
     the earliest loop iteration of its first step), course_id[t] (a course id, or a plan index with `plans`),
     state[t] (x, y, v, yaw start state; omitted with plans, whose start states come from the planned courses),
-    params[t] (NPARAM row; default the engine's defaults) and priority[t] (the fixed rule's key; default the trip's
-    rank in its scene's order)."""
+    params[t] (NPARAM row; default the engine's defaults), priority[t] (the fixed rule's key; default the trip's
+    rank in its scene's order) and group[t] (its signal group with `signals`, -1 = unsignalised)."""
 
-    def __init__(self, scene, arrival, course_id, state=None, params=None, priority=None):
+    def __init__(self, scene, arrival, course_id, state=None, params=None, priority=None, group=None):
         self.scene = _int_array(scene, "scene")
         n = self.n = len(self.scene)
         if n < 1:
@@ -194,24 +194,33 @@ class Trips:
                 raise ValueError(f"priority must be [{n}] (one key per trip), got shape {self.priority.shape}")
             if not np.isfinite(self.priority).all():
                 raise ValueError("priority must be finite")
+        self.group = None if group is None else _int_array(group, "group", n)
+        if self.group is not None and (self.group < -1).any():
+            raise ValueError("group must be >= -1 (-1: unsignalised)")
 
 
 def poisson_trips(n_scenes: int, routes, rate_per_hour: float, dt: float, n_iterations: int, entry_speed: float = 0.0,
-                  seed: int = 0) -> Trips:
+                  seed: int = 0, groups=None) -> Trips:
     """Seeded Poisson demand: in every scene each approach (route group) of `routes` sends vehicles at rate_per_hour,
     with exponential gaps in seconds; a vehicle arriving at time a enters no earlier than iteration floor(a / dt), and
     arrivals from n_iterations on are dropped.  Each vehicle takes a route of its approach uniformly at random.
     routes[g] is a list of (course_id, (x, y, yaw)) pairs: the trip starts at that pose at entry_speed.  With
-    (course_id, None) pairs (plan indices) the trips carry no state, for `from_trips(plans=...)`."""
+    (course_id, None) pairs (plan indices) the trips carry no state, for `from_trips(plans=...)`.  groups (one integer
+    >= -1 per approach, or None) gives each trip the signal group of its approach (Trips.group); the draws do not
+    depend on it."""
     if rate_per_hour < 0 or dt <= 0 or n_iterations < 0 or n_scenes < 1:
         raise ValueError("poisson_trips needs rate_per_hour >= 0, dt > 0, n_iterations >= 0 and n_scenes >= 1")
+    if groups is not None:
+        groups = np.asarray(groups)
+        if groups.shape != (len(routes),) or not np.issubdtype(groups.dtype, np.integer) or (groups < -1).any():
+            raise ValueError(f"groups must be {len(routes)} integers >= -1 (one signal group per approach)")
     rng = np.random.default_rng(seed)
     rate = rate_per_hour / 3600.0
     horizon = n_iterations * dt
     planned = all(pose is None for group in routes for _, pose in group)
-    scene, arrival, cid, state = [], [], [], []
+    scene, arrival, cid, state, approach = [], [], [], [], []
     for s in range(n_scenes):
-        for group in routes:
+        for g, group in enumerate(routes):
             t = 0.0
             while rate > 0:
                 t += rng.exponential(1.0 / rate)
@@ -219,17 +228,18 @@ def poisson_trips(n_scenes: int, routes, rate_per_hour: float, dt: float, n_iter
                 if t >= horizon or it >= n_iterations:
                     break
                 course, pose = group[int(rng.integers(len(group)))]
-                scene.append(s), arrival.append(it), cid.append(int(course))
+                scene.append(s), arrival.append(it), cid.append(int(course)), approach.append(g)
                 if not planned:
                     state.append([pose[0], pose[1], entry_speed, pose[2]])
     order = np.lexsort((np.arange(len(scene)), arrival, scene))
     take = lambda a: np.asarray(a)[order] if len(a) else np.zeros(0, np.int64)   # noqa: E731
     return Trips(take(scene), take(arrival), take(cid),
-                 None if planned else np.asarray(state, np.float64).reshape(-1, 4)[order])
+                 None if planned else np.asarray(state, np.float64).reshape(-1, 4)[order],
+                 group=None if groups is None else groups[take(approach)])
 
 
 def trips_setup(trips: Trips, n_scenes: int, k, n_courses: int, planned: bool, n_extra: int, right_of_way,
-                share_plans: bool, params_default, depart=None, on_goal=None, obstacle_script=None):
+                share_plans: bool, params_default, depart=None, on_goal=None, obstacle_script=None, signals=None):
     """Host-side checks of `BatchedEpisodes.from_trips`.  Returns (order, params [N, NPARAM], priority or None): order
     sorts the trips by (scene, arrival, trip index), the layout the trips pass walks."""
     if depart is not None or on_goal is not None:
@@ -255,6 +265,13 @@ def trips_setup(trips: Trips, n_scenes: int, k, n_courses: int, planned: bool, n
         raise ValueError("trips need state [N, 4] unless plans are given")
     if trips.priority is not None and right_of_way != "fixed":
         raise ValueError("priority is an argument of the fixed right-of-way rule")
+    if signals is None and trips.group is not None:
+        raise ValueError("group is an argument of signals: give signals too")
+    if signals is not None:
+        signal_plan_check(signals, int(n_scenes))
+        if trips.group is None:
+            raise ValueError("signals need Trips.group (one signal group per trip, -1 = unsignalised)")
+        signal_groups(trips.group, signals, "Trips.group")
     order = np.lexsort((np.arange(trips.n), trips.arrival, trips.scene))
     params = (np.repeat(np.asarray(params_default, np.float64)[None, :], trips.n, axis=0) if trips.params is None
               else trips.params)[order]
@@ -276,6 +293,99 @@ def trips_setup(trips: Trips, n_scenes: int, k, n_courses: int, planned: bool, n
             start = np.searchsorted(scene, scene, side="left")
             priority = (np.arange(trips.n) - start).astype(np.float64)
     return order, np.ascontiguousarray(params), priority
+
+
+class SignalPlan:
+    """A fixed-time signal plan for `BatchedEpisodes(signals=...)` (jmpc_signals in include/jmpc.h).
+    cycle: C >= 1 loop iterations.  green: one (start, length) window per signal group, 1 to 8 groups, start in [0, C),
+    length in [0, C]; group g is green in loop iteration i of scene s iff ((i + offset[s] - start) mod C) < length, red
+    otherwise (no amber state: the clearance time is the gap between windows).  junction: (x, y, r), r > 0; a
+    vehicle's stop line is the first point of its course within r of (x, y), its zone entry e.  margin: course points
+    between the cut and the stop line, L = e - margin (None: the run's collision margin).  stop_decel: the deceleration
+    (m/s^2, finite, > 0) of the stopping test that decides, once per red phase, whether a vehicle holds at L or goes.
+    offset: one integer per scene (None: 0), shifting each scene's cycle."""
+
+    def __init__(self, cycle, green, junction, margin=None, stop_decel: float = 3.0, offset=None):
+        i32 = np.iinfo(np.int32).max
+        if isinstance(cycle, bool) or not isinstance(cycle, (int, np.integer)) or not 1 <= cycle <= i32:
+            raise ValueError(f"cycle must be an integer >= 1, got {cycle!r}")
+        self.cycle = int(cycle)
+        win = np.asarray(green)
+        if win.ndim != 2 or win.shape[1] != 2 or not 1 <= len(win) <= _cabi.SIGNAL_MAX_GROUPS:
+            raise ValueError(f"green must be 1 to {_cabi.SIGNAL_MAX_GROUPS} (start, length) pairs, one per signal group")
+        if not np.issubdtype(win.dtype, np.integer):
+            raise ValueError("green windows must be integers (loop iterations)")
+        if ((win[:, 0] < 0) | (win[:, 0] >= cycle)).any():
+            raise ValueError(f"green start must be in [0, {cycle})")
+        if ((win[:, 1] < 0) | (win[:, 1] > cycle)).any():
+            raise ValueError(f"green length must be in [0, {cycle}]")
+        self.green = win.astype(np.int64)
+        junc = np.asarray(junction, np.float64)
+        if junc.shape != (3,) or not np.isfinite(junc).all() or not junc[2] > 0:
+            raise ValueError("junction must be (x, y, r), finite with r > 0")
+        self.junction = junc
+        if margin is not None and (isinstance(margin, bool) or not isinstance(margin, (int, np.integer))
+                                   or not 0 <= margin <= i32):
+            raise ValueError(f"margin must be None or an integer >= 0, got {margin!r}")
+        self.margin = None if margin is None else int(margin)
+        stop_decel = float(stop_decel)
+        if not math.isfinite(stop_decel) or stop_decel <= 0:
+            raise ValueError("stop_decel must be finite and > 0")
+        self.stop_decel = stop_decel
+        self.offset = None
+        if offset is not None:
+            off = np.asarray(offset)
+            if off.ndim != 1 or not np.issubdtype(off.dtype, np.integer):
+                raise ValueError("offset must be a 1-D integer array (one per scene)")
+            if (np.abs(off.astype(np.int64)) > 2 ** 30).any():
+                raise ValueError("offset must be within +-2**30")
+            self.offset = off.astype(np.int32)
+
+    @property
+    def n_groups(self) -> int:
+        return len(self.green)
+
+    def struct(self, margin: int):
+        """struct jmpc_signal_plan, with the run's `margin` where the plan has none."""
+        p = _cabi.SignalPlan(cycle=self.cycle, n_groups=self.n_groups,
+                             margin=int(margin if self.margin is None else self.margin), stop_decel=self.stop_decel)
+        for g, (start, length) in enumerate(self.green):
+            p.green_start[g], p.green_len[g] = int(start), int(length)
+        return p
+
+
+def signal_groups(group, signals: SignalPlan, name: str, n: Optional[int] = None) -> np.ndarray:
+    """Checks per-vehicle (or per-trip) signal groups against the plan: integers in [-1, G).  Returns int32."""
+    grp = np.asarray(group)
+    if grp.ndim != 1 or not np.issubdtype(grp.dtype, np.integer):
+        raise ValueError(f"{name} must be a 1-D integer array")
+    if n is not None and len(grp) != n:
+        raise ValueError(f"{name} must be [{n}] (one signal group per episode), got shape {grp.shape}")
+    if ((grp < -1) | (grp >= signals.n_groups)).any():
+        raise ValueError(f"{name} must be in [-1, {signals.n_groups}) (-1: unsignalised)")
+    return np.ascontiguousarray(grp, dtype=np.int32)
+
+
+def signal_plan_check(signals, n_scenes: int) -> None:
+    """The plan against the run: a SignalPlan whose offset, if any, has one entry per scene.  The pass reads
+    offset[b / k] on the device, where its length cannot be checked."""
+    if not isinstance(signals, SignalPlan):
+        raise ValueError("signals must be a SignalPlan")
+    if signals.offset is not None and signals.offset.shape != (n_scenes,):
+        raise ValueError(f"the plan's offset must be [{n_scenes}] (one per scene), got shape {signals.offset.shape}")
+
+
+def signal_setup(signals, signal_group, B: int, k: int):
+    """Host-side checks of the signals option of `BatchedEpisodes`.  Returns None without signals, else
+    (group int32 [B], offset int32 [B / k] or None)."""
+    if signals is None:
+        if signal_group is not None:
+            raise ValueError("signal_group is an argument of signals: give signals too")
+        return None
+    signal_plan_check(signals, B // k)
+    if signal_group is None:
+        raise ValueError("signals need signal_group [B] (one signal group per episode, -1 = unsignalised)")
+    return signal_groups(signal_group, signals, "signal_group", B), signals.offset
 
 
 TRIP_STATE = ("slot", "entry", "exit", "steps", "done", "blocked_waits")
@@ -370,7 +480,8 @@ class BatchedEpisodes:
                    frame_window: int = 10, max_steps: int = 256, record_history: bool = True, horizon_s: float = 7.0,
                    obstacle_script=None, outcomes: bool = False, record_obstacles: bool = False,
                    agents_per_scene: int = 1, share_plans: bool = False, right_of_way=None, priority=None,
-                   junction=None, depart=None, on_goal: str = "park") -> "BatchedEpisodes":
+                   junction=None, depart=None, on_goal: str = "park", signals=None,
+                   signal_group=None) -> "BatchedEpisodes":
         """Episodes on the planned courses of `engine` (filled by `BatchedMPC.from_plans(plans)` /
         `set_courses_from_plans(plans)`), the second half of main/scenarios/mpc_intersection.py:63-163 for a batch:
         episode b drives plan `plan_id[b]` (default: one episode per plan; zeros = one course, many controllers).
@@ -378,8 +489,9 @@ class BatchedEpisodes:
         course are written on the device (jmpc_episode_init_from_courses); such episodes are never stepped.
         `params` [B, NPARAM] (default: the engine's defaults) supplies every other parameter row.  `run()` adds
         plan_status, plan_cost and expansions per episode.  `outcomes` / `record_obstacles` / `agents_per_scene` /
-        `share_plans` / `right_of_way` / `priority` / `junction` / `depart` / `on_goal` as in `__init__`; evaluation 0 of the outcome record sees
-        the planned start states; the junction zones are found on the planned courses, and first_come distances use
+        `share_plans` / `right_of_way` / `priority` / `junction` / `depart` / `on_goal` / `signals` / `signal_group` as
+        in `__init__`; evaluation 0 of the outcome record sees the planned start states; the junction zones and stop
+        lines are found on the planned courses, and first_come distances and the signals' stopping test use
         each course's dl.  With agents_per_scene > 1 a scene with a done = 3 vehicle is not driven: its other vehicles get
         done = 4 (jmpc_scene_init); such vehicles never wait either: the waiting code is set after this pass."""
         if engine.course_ok is None or len(engine.course_ok) != len(plans):
@@ -396,7 +508,7 @@ class BatchedEpisodes:
                  record_history=record_history, horizon_s=horizon_s, obstacle_program=obstacle_program,
                  outcomes=outcomes, record_obstacles=record_obstacles, agents_per_scene=agents_per_scene,
                  share_plans=share_plans, right_of_way=right_of_way, priority=priority, junction=junction,
-                 depart=depart, on_goal=on_goal)
+                 depart=depart, on_goal=on_goal, signals=signals, signal_group=signal_group)
         stream = C.c_void_p(torch.cuda.current_stream(engine.device).cuda_stream)
         _cabi.check(engine._lib.jmpc_episode_init_from_courses(
             engine._h, B, ep._p(ep.course_id), ep._p(engine.course_ok), ep._p(engine.course_dl), ep._p(ep.state),
@@ -412,7 +524,7 @@ class BatchedEpisodes:
                    margin: int = 72, max_steps: int = 256, record_history: bool = True, horizon_s: float = 7.0,
                    outcomes: bool = False, record_obstacles: bool = False, share_plans: bool = False,
                    right_of_way=None, junction=None, depart=None, on_goal=None,
-                   obstacle_script=None) -> "BatchedEpisodes":
+                   obstacle_script=None, signals=None) -> "BatchedEpisodes":
         """Scenes fed from a stream of timed trips (jmpc_scene_trips / jmpc_scene_trips_finish in include/jmpc.h).
         The batch is n_scenes x k slots (episode b = s * k + j is slot j of scene s, k in [2, 9]); a slot holds at most
         one trip at a time and starts empty.  An empty slot is handled as a vehicle that has not entered under lifetimes:
@@ -429,7 +541,9 @@ class BatchedEpisodes:
         course_id are plan indices and the start states, dl and usability come from the planned courses.  The other
         options are those of `__init__`: obstacles / obstacle_program are per-slot extras; share_plans needs one dt per
         scene across its trips; right_of_way "fixed" takes the trips' priority (default: rank in the scene's order),
-        "first_come" a junction (once or per scene).  depart, on_goal and obstacle_script do not apply to trips."""
+        "first_come" a junction (once or per scene); signals takes each trip's group from Trips.group (the latch,
+        hold_steps and go belong to the trip; run() also gives the per-slot counts).  depart, on_goal and
+        obstacle_script do not apply to trips."""
         import torch
         n_extra = 0
         if obstacles is not None:
@@ -442,7 +556,8 @@ class BatchedEpisodes:
         n_courses = len(plans) if planned else len(engine.course_len)
         k = agents_per_scene
         order, params, priority = trips_setup(trips, n_scenes, k, n_courses, planned, n_extra, right_of_way,
-                                              share_plans, engine.default_params, depart, on_goal, obstacle_script)
+                                              share_plans, engine.default_params, depart, on_goal, obstacle_script,
+                                              signals)
         entry_gap = float(entry_gap)
         if not math.isfinite(entry_gap) or entry_gap < 0:
             raise ValueError("entry_gap must be finite and >= 0")
@@ -507,6 +622,10 @@ class BatchedEpisodes:
             for c in ("min_clearance_eval", "min_clearance_obs", "first_contact_eval", "first_contact_obs"):
                 T["outcomes"][:, OUTCOME_NAMES.index(c)] = -1.0
         ep.done.fill_(_cabi.WAITING)
+        if signals is not None:                                # per trip: its group and stop line; owner = slot_trip
+            same = T["zone"] is not None and bool((junc == signals.junction).all())
+            zone = T["zone"] if same else ep._zones(T["course_id"], signals.junction)   # first_come's zones if equal
+            ep._signals_init(signals, t(trips.group[order], i32), zone, N, owner=T["slot_trip"])
         ep._trips = T
         ep._trip_order = order
         ep._trips_struct = _cabi.Trips(
@@ -554,6 +673,9 @@ class BatchedEpisodes:
         res["slot_waits"] = due - res["blocked_waits"]
         res["entry_delay"] = np.where(res["entry"] >= 0, res["entry"] - res["arrival"], -1)
         res["travel"] = np.where((res["entry"] >= 0) & (res["exit"] >= 0), res["exit"] - res["entry"], -1)
+        if self.signals is not None:
+            res["signal_hold_steps"] = back(self.signal_hold.cpu().numpy().astype(np.int64))
+            res["signal_go"] = back(self.signal_go.cpu().numpy().astype(np.int64))
         if T["outcomes"] is not None:
             res.update(outcome_columns(back(T["outcomes"].cpu().numpy())))
             for col in ("min_clearance", "first_contact"):
@@ -565,7 +687,8 @@ class BatchedEpisodes:
                  frame_window: int = 10, margin: int = 72, params=None, max_steps: int = 256,
                  record_history: bool = True, horizon_s: float = 7.0, obstacle_program=None, outcomes: bool = False,
                  record_obstacles: bool = False, agents_per_scene: int = 1, share_plans: bool = False,
-                 right_of_way=None, priority=None, junction=None, depart=None, on_goal: str = "park"):
+                 right_of_way=None, priority=None, junction=None, depart=None, on_goal: str = "park",
+                 signals=None, signal_group=None):
         """outcomes: keep one outcome record per episode on the device (jmpc_episode_outcomes): contact and clearance
         against the obstacles, cut / limit steps, failed solves, comfort and tracking columns; `run()` returns it as
         `outcomes`.  It observes only: the episodes are exactly those of outcomes=False.  record_obstacles (needs
@@ -612,7 +735,18 @@ class BatchedEpisodes:
         contact to the outcome record, whose obstacle_history rows for them are NaN.  A vehicle's outcome record starts
         at evaluation depart[b]; the *_eval columns stay global evaluation indices, and `steps` counts its own steps.
         A vehicle that has not entered when the run ends keeps done = WAITING.  depart all zero with "park" is the run
-        without lifetimes, with nothing launched or allocated for them."""
+        without lifetimes, with nothing launched or allocated for them.
+
+        signals (a `SignalPlan`) and signal_group (integer [B] in [-1, G), -1 = unsignalised): fixed-time traffic
+        signals (jmpc_signals in include/jmpc.h).  Vehicle b's stop line is e, the first point of its course within the
+        plan's junction (jmpc_right_of_way_init; a course that never enters it is unsignalised), and its cut point is
+        L = e - margin.  Every iteration, after the collision check and before the step, a vehicle whose group is red
+        decides once per red phase: it holds iff a < L and v * v <= 2 stop_decel (L - 1 - a) dl (a its course index,
+        v its speed, dl its params' dl), else it goes.  A held vehicle's course is cut at max(a + 1, L) as a collision
+        cut is, until it sees green; a vehicle that goes is left alone, and one that goes with a < L (it could not
+        stop) counts a GO pass.  run() adds `signal_hold_steps` and `signal_go` per episode.  The collision flag,
+        History, the outcome record and the masks are unchanged: a signal stop is not a cut step.  signals=None
+        launches and allocates nothing for signals."""
         import torch
         self.torch = torch
         self.e = engine
@@ -679,6 +813,11 @@ class BatchedEpisodes:
                 _cabi.check(engine._lib.jmpc_right_of_way_init(
                     engine._h, B, self.k, self._p(self.course_id), self._p(self.junction), int(junc.shape[0]),
                     self._p(self.zone), stream), "jmpc_right_of_way_init")
+        # signals: per-episode group and stop line, the latch and the counters (jmpc_signals, every iteration)
+        self.signals = None
+        sig = signal_setup(signals, signal_group, B, self.k)
+        if sig is not None:
+            self._signals_init(signals, t(sig[0], i32), self._zones(self.course_id, signals.junction), B)
         # lifetimes: depart [B] int32; the collision mask (a rule's `consider` ANDed with presence, or presence alone)
         # and the evaluation mask `presence` [B], both written by jmpc_scene_presence every iteration (k > 1)
         self.depart = self.presence = None
@@ -703,6 +842,53 @@ class BatchedEpisodes:
         self._started = False
         if self.program is not None:                                 # get() before the first iteration
             self._scripted_step(advance=0)
+
+    def _zones(self, course_id, junction):
+        """(entry, exit) [n, 2] int32 of every course in course_id [n] (None: course 0 for all B episodes) in the zone
+        junction = (x, y, r) (jmpc_right_of_way_init, in launches of at most max_batch)."""
+        torch, e = self.torch, self.e
+        stream = C.c_void_p(torch.cuda.current_stream(e.device).cuda_stream)
+        n = self.B if course_id is None else int(course_id.shape[0])
+        junc = torch.as_tensor(np.asarray(junction, np.float64)[None, :], device=self.dev)
+        zone = torch.empty(n, 2, dtype=torch.int32, device=self.dev)
+        for a in range(0, n, e.max_batch):
+            m = min(e.max_batch, n - a)
+            _cabi.check(e._lib.jmpc_right_of_way_init(
+                e._h, m, 1, None if course_id is None else self._p(course_id[a:]), self._p(junc), 1,
+                self._p(zone[a:]), stream), "jmpc_right_of_way_init")
+        return zone
+
+    def _signals_init(self, signals: "SignalPlan", group, zone, n_owner: int, owner=None):
+        """The signal pass's arrays: group and zone [n_owner], the latch [B, 2] = (-1, 0), the counters per owner and,
+        with an owner array (trips), per slot."""
+        torch, i32 = self.torch, self.torch.int32
+        self._signal_plan = signals.struct(self.margin)
+        if not 0 <= self._signal_plan.margin <= self.e.max_N:
+            raise ValueError(f"the signal margin must be in [0, {self.e.max_N}] (the engine's max_N), got "
+                             f"{self._signal_plan.margin}")
+        self.signals = signals
+        self.signal_offset = (None if signals.offset is None
+                              else torch.as_tensor(signals.offset, dtype=i32, device=self.dev))
+        self.signal_group, self.signal_zone, self.signal_owner = group, zone, owner
+        self.signal_latch = torch.zeros(self.B, 2, dtype=i32, device=self.dev)
+        self.signal_latch[:, 0] = -1
+        self.signal_hold = torch.zeros(n_owner, dtype=i32, device=self.dev)
+        self.signal_go = torch.zeros(n_owner, dtype=i32, device=self.dev)
+        self.signal_slot_hold = self.signal_slot_go = None
+        if owner is not None:
+            self.signal_slot_hold = torch.zeros(self.B, dtype=i32, device=self.dev)
+            self.signal_slot_go = torch.zeros(self.B, dtype=i32, device=self.dev)
+
+    def _signal_pass(self, checked: bool):
+        e = self.e
+        stream = C.c_void_p(self.torch.cuda.current_stream(e.device).cuda_stream)
+        _cabi.check(e._lib.jmpc_signals(
+            e._h, self.B, self.k, C.byref(self._signal_plan), self._p(self.signal_offset), self._p(self.signal_owner),
+            self._p(self.signal_group), self._p(self.signal_zone), self._p(self.course_id), self._p(self.agent_idx),
+            self._p(self.state), self._p(self.params), self._p(self.done), int(checked), self._p(self.course_len),
+            self._p(self.signal_latch), self._p(self.signal_hold), self._p(self.signal_go),
+            self._p(self.signal_slot_hold), self._p(self.signal_slot_go), self._p(self.iter_dev), stream),
+            "jmpc_signals")
 
     def _scripted_step(self, advance: int):
         e = self.e
@@ -819,6 +1005,8 @@ class BatchedEpisodes:
             has_flags = True
         else:
             has_flags = False
+        if self.signals is not None:           # the red-light cut: after the collision check, before the step
+            self._signal_pass(has_flags)
         e.step(self.state, self.target_ind, self.oa, self.od, self.out, course_id=self.course_id,
                course_len=self.course_len, warm=self.warm, params=self.params)
         # history row, flag copy and time stamp are indexed by the device-side iteration counter: nothing in the loop
@@ -914,6 +1102,10 @@ class BatchedEpisodes:
             res["outcomes"] = outcome_columns(self.outcomes.cpu().numpy())
             if self.obstacle_history is not None:
                 res["obstacle_history"] = self.obstacle_history[:min(self.iteration, self.max_steps) + 1].cpu().numpy()
+        if self.signals is not None:
+            per_slot = self.signal_owner is not None
+            res["signal_hold_steps"] = (self.signal_slot_hold if per_slot else self.signal_hold).cpu().numpy()
+            res["signal_go"] = (self.signal_slot_go if per_slot else self.signal_go).cpu().numpy()
         if trips is not None:
             res["trips"] = trips
         if self._plans is not None:

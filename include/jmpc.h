@@ -541,6 +541,52 @@ int32_t jmpc_scene_trips(jmpc_handle h, const jmpc_trips* trips, const int32_t* 
                          void* stream);
 int32_t jmpc_scene_trips_finish(jmpc_handle h, const jmpc_trips* trips, int32_t n_iterations, void* stream);
 
+/* Fixed-time traffic signals (opt-in): a red light is one more course cut at the stop line, made the way a collision
+ * cut is (course_len = max(agent_idx + 1, stop)), in the course_len array jmpc_step reads.  DEVICE pointers.
+ *   Plan: a cycle C >= 1 loop iterations, G in [1, 8] signal groups, a green window per group (green_start[g] in
+ *   [0, C), green_len[g] in [0, C]), an offset per scene (offset [B / k] int32, NULL = 0), a stop margin in course
+ *   points and a stopping deceleration stop_decel (finite, > 0).  Group g is green in loop iteration i of scene s iff
+ *   ((i + offset[s] - green_start[g]) mod C) < green_len[g], with the non-negative modulus; the time between windows
+ *   is red (no separate amber state: the clearance time is the gap between windows).
+ *   Per vehicle: a group (-1 = unsignalised, e.g. a free right turn) and a stop line e = the zone entry index that
+ *   jmpc_right_of_way_init computes for the plan's junction (x, y, r); the cut point is L = e - margin; a course with
+ *   e = -1 is unsignalised.
+ *   Owner o of episode b: owner[b] (with trips: the slot's trip, jmpc_trips.slot_trip) or b (owner = NULL).  group
+ *   [n_owner] int32 and zone [n_owner][2] (entry, exit) are indexed by the owner; so are hold_steps and go [n_owner].
+ *   latch [B][2] = (owner, decision: 1 HOLD, 0 GO), owner -1 = empty; a latch stored for another owner counts as
+ *   empty, so a trip loaded into a slot starts undecided.  The caller initialises latch to (-1, 0).
+ * jmpc_signals: the signal pass, one thread per episode, in loop iteration i = *iter_dev after jmpc_collision* and
+ *   before jmpc_step.  For each episode with done = 0:
+ *   1. checked = 0 (no collision check ran this iteration): course_len = the course's full length, as a flag-0 check
+ *      writes it.
+ *   2. g < 0 (or g >= G), e < 0 or g green: the latch is cleared; course_len is left as it is.
+ *   3. otherwise, unless the latch holds a decision for o, decide once, a = agent_idx[b], v = state[b][2],
+ *      dl = params[b][JMPC_P_DL] (params NULL: the handle's default): HOLD iff a < L and
+ *      v * v <= 2.0 * stop_decel * (double)(L - 1 - a) * dl, evaluated left to right with every product rounded (no
+ *      fused multiply-add); else GO, and a GO with a < L (a vehicle that could not stop) counts go[o] += 1.  The
+ *      decision holds until the vehicle sees green: a held vehicle that creeps to a >= L stays held, and one under an
+ *      always-red group is held for good.
+ *   4. HOLD: course_len = min(course_len, max(a + 1, L)) and hold_steps[o] += 1.  GO changes nothing.
+ *   slot_hold_steps / slot_go [B] or NULL: the same counts per episode (with trips: per slot).  The collision flag,
+ *   the outcome record, History, obstacle_history, the masks and the exchange are untouched: a signal stop is not a
+ *   cut step.  iter_dev is jmpc_episode_post_dev's counter; no per-iteration host argument, so the call can be captured
+ *   in a CUDA graph.  Order of one iteration with signals: pre, right_of_way, presence (collision mask),
+ *   collision_masked, signals, step, post_dev, ... as without. */
+#define JMPC_SIGNAL_MAX_GROUPS 8
+typedef struct jmpc_signal_plan {
+  int32_t cycle;                                   /* C >= 1 loop iterations                                        */
+  int32_t n_groups;                                /* G in [1, JMPC_SIGNAL_MAX_GROUPS]                              */
+  int32_t green_start[JMPC_SIGNAL_MAX_GROUPS];     /* [0, C)                                                        */
+  int32_t green_len[JMPC_SIGNAL_MAX_GROUPS];       /* [0, C]                                                        */
+  int32_t margin;                                  /* course points between the cut and the stop line, [0, max_N] */
+  double stop_decel;                               /* m/s^2, finite, > 0                                            */
+} jmpc_signal_plan;
+int32_t jmpc_signals(jmpc_handle h, int32_t B, int32_t k, const jmpc_signal_plan* plan, const int32_t* offset,
+                     const int32_t* owner, const int32_t* group, const int32_t* zone, const int32_t* course_id,
+                     const int32_t* agent_idx, const double* state, const double* params, const int32_t* done,
+                     int32_t checked, int32_t* course_len, int32_t* latch, int32_t* hold_steps, int32_t* go,
+                     int32_t* slot_hold_steps, int32_t* slot_go, const int32_t* iter_dev, void* stream);
+
 /* The reference's scripted obstacles on the device (main/lib/moving_obstacles.py: MovingObstacleTIntersection :166-232,
  * MovingObstacleRoundabout :28-123 including its dt = 0.2 quirk at :45 and the theta overwrite inside its steering
  * property, MovingObstacleArterial :125-164).  DEVICE pointers.
