@@ -121,11 +121,14 @@ def _device_collision(jm, engine, agent_idx, v, obst, fw, margin, plans=None, n_
     return flag.cpu().numpy(), clen.cpu().numpy()
 
 
-def _near_workload(jm, config, B, seed=99):
-    """The synthetic workload with half of every obstacle slot moved next to the path, so that several slots cut."""
+def _near_workload(jm, config, B, seed=99, n_obs=None):
+    """The synthetic workload with half of every obstacle slot moved next to the path, so that several slots cut.
+    n_obs: that many obstacle slots (synth.make_obstacles) instead of the config's."""
     w = jm["synth"].make_workload(config, B=B)
     course = w["courses"][0]
     rng = np.random.default_rng(seed)
+    if n_obs is not None:
+        w["obstacles"] = jm["synth"].make_obstacles(rng, B, n_obs)
     for s in range(w["obstacles"].shape[1]):
         near = rng.random(B) < 0.5
         k = np.minimum(w["agent_idx"] + rng.integers(0, 200, B), len(course) - 1)
@@ -134,10 +137,12 @@ def _near_workload(jm, config, B, seed=99):
     return w
 
 
-@pytest.mark.parametrize("config", [3, 4])
-def test_masked_check_is_the_check_on_the_considered_rows(jm, config):
+@pytest.mark.parametrize("config,n_slots", [(3, None), (4, None), (4, 8)], ids=["3", "4", "4-8slots"])
+def test_masked_check_is_the_check_on_the_considered_rows(jm, config, n_slots):
+    """n_slots = 8: every obstacle slot a scene can have, so that bit 7 and the (1 << n_obs) - 1 limit are used, with
+    n_planned 4 and 8."""
     B = 4096
-    w = _near_workload(jm, config, B)
+    w = _near_workload(jm, config, B, n_obs=n_slots)
     course, obst = w["courses"][0], w["obstacles"]
     n_obs = obst.shape[1]
     margin = C.cutoff_margin(GEO, w["dl"])
@@ -153,55 +158,60 @@ def test_masked_check_is_the_check_on_the_considered_rows(jm, config):
     mask[::7] = 0
     mask[1::7] = -1
     mask = mask.astype(np.int32)
-    n_planned = max(1, n_obs // 2)
-    plans = np.stack([rng.uniform(p[PI["max_decel"]], p[PI["max_accel"]], (B, n_planned, 12)),
-                      rng.uniform(-p[PI["max_steer"]], p[PI["max_steer"]], (B, n_planned, 12))], axis=-1)
+    # n_planned: the lower half of the slots, and with 8 slots also every slot
+    planned = [max(1, n_obs // 2)] + ([n_obs] if n_obs == 8 else [])
+    plans = np.stack([rng.uniform(p[PI["max_decel"]], p[PI["max_accel"]], (B, planned[-1], 12)),
+                      rng.uniform(-p[PI["max_steer"]], p[PI["max_steer"]], (B, planned[-1], 12))], axis=-1)
     full = _device_collision(jm, engine, a_idx, v, obst, fw, margin)
-    full_planned = _device_collision(jm, engine, a_idx, v, obst, fw, margin, plans, n_planned)
     got = _device_collision(jm, engine, a_idx, v, obst, fw, margin, consider=mask)
-    got_planned = _device_collision(jm, engine, a_idx, v, obst, fw, margin, plans, n_planned, consider=mask)
     low = mask.astype(np.int64) & ((1 << n_obs) - 1)
+    assert ((low >> (n_obs - 1)) & 1).any() and ((low >> (n_obs - 1)) & 1 == 0).any()
     changed = 0
-    for m in np.unique(low):
-        idx = np.flatnonzero(low == m)
-        keep = [s for s in range(n_obs) if (m >> s) & 1]
-        if not keep:                                   # no considered slot: the n_obs = 0 result
-            for g in (got, got_planned):
-                assert (g[0][idx] == 0).all() and (g[1][idx] == len(course)).all()
-            continue
-        ref = _device_collision(jm, engine, a_idx[idx], v[idx], obst[idx][:, keep], fw, margin)
-        kp = [s for s in keep if s < n_planned]
-        ref_p = _device_collision(jm, engine, a_idx[idx], v[idx], obst[idx][:, keep], fw, margin,
-                                  plans[idx][:, kp] if kp else None, len(kp))
-        for g, r in ((got, ref), (got_planned, ref_p)):
-            assert np.array_equal(g[0][idx], r[0]) and np.array_equal(g[1][idx], r[1]), (config, m)
-        changed += int(((got[0][idx] != full[0][idx]) | (got[1][idx] != full[1][idx])).sum())
-    # the all-ones mask (and any mask with every slot's bit) is the unmasked call
-    every = low == (1 << n_obs) - 1
-    for g, r in ((got, full), (got_planned, full_planned)):
-        assert np.array_equal(g[0][every], r[0][every]) and np.array_equal(g[1][every], r[1][every])
-    all_ones = _device_collision(jm, engine, a_idx, v, obst, fw, margin, plans, n_planned, consider=np.full(B, -1))
-    assert np.array_equal(all_ones[0], full_planned[0]) and np.array_equal(all_ones[1], full_planned[1])
-    # a spot check against the oracle on the considered rows
-    for i in rng.choice(B, 24, replace=False):
-        keep = [s for s in range(n_obs) if (int(mask[i]) >> s) & 1]
-        f, cl = C.collision_cut(GEO, course, int(a_idx[i]), float(v[i]), RW.considered_rows(obst[i], mask[i]), dt=0.2,
-                                frame_window=fw, max_accel=p[PI["max_accel"]], max_speed=p[PI["sim_max_speed"]],
-                                margin=margin)
-        assert (int(f), cl) == (int(got[0][i]), int(got[1][i])), i
-        pl = [plans[i, s] if s < n_planned else None for s in keep]
-        f, cl = SP.collision_cut(GEO, course, int(a_idx[i]), float(v[i]), RW.considered_rows(obst[i], mask[i]),
-                                 dt=0.2, frame_window=fw, max_accel=p[PI["max_accel"]],
-                                 max_speed=p[PI["sim_max_speed"]], margin=margin, plans=pl)
-        assert (int(f), cl) == (int(got_planned[0][i]), int(got_planned[1][i])), i
-    # the skip mask: skipped instances are left untouched
-    skip = (rng.random(B) < 0.3).astype(np.int32)
-    sk = _device_collision(jm, engine, a_idx, v, obst, fw, margin, plans, n_planned, consider=mask, skip=skip)
-    assert (sk[0][skip != 0] == -7).all() and (sk[1][skip != 0] == -7).all()
-    assert np.array_equal(sk[0][skip == 0], got_planned[0][skip == 0])
-    assert np.array_equal(sk[1][skip == 0], got_planned[1][skip == 0])
-    print(f"\n[masked check] config {config}: {B} instances, {len(np.unique(low))} distinct masks, the mask changed the "
-          f"flag or cut of {changed}; flagged unmasked / masked {int((full[0] == 1).sum())} / {int((got[0] == 1).sum())}")
+    for n_planned in planned:
+        pn = plans[:, :n_planned]
+        full_planned = _device_collision(jm, engine, a_idx, v, obst, fw, margin, pn, n_planned)
+        got_planned = _device_collision(jm, engine, a_idx, v, obst, fw, margin, pn, n_planned, consider=mask)
+        for m in np.unique(low):
+            idx = np.flatnonzero(low == m)
+            keep = [s for s in range(n_obs) if (m >> s) & 1]
+            if not keep:                                   # no considered slot: the n_obs = 0 result
+                for g in (got, got_planned):
+                    assert (g[0][idx] == 0).all() and (g[1][idx] == len(course)).all()
+                continue
+            ref = _device_collision(jm, engine, a_idx[idx], v[idx], obst[idx][:, keep], fw, margin)
+            kp = [s for s in keep if s < n_planned]
+            ref_p = _device_collision(jm, engine, a_idx[idx], v[idx], obst[idx][:, keep], fw, margin,
+                                      plans[idx][:, kp] if kp else None, len(kp))
+            for g, r in ((got, ref), (got_planned, ref_p)):
+                assert np.array_equal(g[0][idx], r[0]) and np.array_equal(g[1][idx], r[1]), (config, m)
+            changed += int(((got[0][idx] != full[0][idx]) | (got[1][idx] != full[1][idx])).sum())
+        # the all-ones mask (and any mask with every slot's bit) is the unmasked call
+        every = low == (1 << n_obs) - 1
+        for g, r in ((got, full), (got_planned, full_planned)):
+            assert np.array_equal(g[0][every], r[0][every]) and np.array_equal(g[1][every], r[1][every])
+        all_ones = _device_collision(jm, engine, a_idx, v, obst, fw, margin, pn, n_planned, consider=np.full(B, -1))
+        assert np.array_equal(all_ones[0], full_planned[0]) and np.array_equal(all_ones[1], full_planned[1])
+        # a spot check against the oracle on the considered rows
+        for i in rng.choice(B, 24, replace=False):
+            keep = [s for s in range(n_obs) if (int(mask[i]) >> s) & 1]
+            f, cl = C.collision_cut(GEO, course, int(a_idx[i]), float(v[i]), RW.considered_rows(obst[i], mask[i]),
+                                    dt=0.2, frame_window=fw, max_accel=p[PI["max_accel"]],
+                                    max_speed=p[PI["sim_max_speed"]], margin=margin)
+            assert (int(f), cl) == (int(got[0][i]), int(got[1][i])), i
+            pl = [plans[i, s] if s < n_planned else None for s in keep]
+            f, cl = SP.collision_cut(GEO, course, int(a_idx[i]), float(v[i]), RW.considered_rows(obst[i], mask[i]),
+                                     dt=0.2, frame_window=fw, max_accel=p[PI["max_accel"]],
+                                     max_speed=p[PI["sim_max_speed"]], margin=margin, plans=pl)
+            assert (int(f), cl) == (int(got_planned[0][i]), int(got_planned[1][i])), i
+        # the skip mask: skipped instances are left untouched
+        skip = (rng.random(B) < 0.3).astype(np.int32)
+        sk = _device_collision(jm, engine, a_idx, v, obst, fw, margin, pn, n_planned, consider=mask, skip=skip)
+        assert (sk[0][skip != 0] == -7).all() and (sk[1][skip != 0] == -7).all()
+        assert np.array_equal(sk[0][skip == 0], got_planned[0][skip == 0])
+        assert np.array_equal(sk[1][skip == 0], got_planned[1][skip == 0])
+    print(f"\n[masked check] config {config}, n_obs {n_obs}, n_planned {planned}: {B} instances, "
+          f"{len(np.unique(low))} distinct masks, the mask changed the flag or cut of {changed}; flagged unmasked / "
+          f"masked {int((full[0] == 1).sum())} / {int((got[0] == 1).sum())}")
     assert changed > 0
     # argument errors of the new entry points
     cabi, lib, h = jm["cabi"], engine._lib, engine._h
